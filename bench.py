@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                      (the reference's CPU forward on the host cores)
+    python bench.py ... --dump-outputs DIR                    (also save the last timed step's logits under DIR)
 
 One "step" = one forward of the hot path over the rank's shard of the global batch (BASELINE.json config 3:
 global batch 4096 sharded 4096/2048/1024/512 per GPU; strong scaling, no collective on the data path).
@@ -86,6 +87,22 @@ def timed_steps(fn, steps, warmup=3):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / steps
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname: str, logits: torch.Tensor, rank: int, world: int) -> str:
+    """Save what the timed path returned in its last step (the [per-GPU batch, 1000] f32 logits) as DIR/logits.npy, or
+    DIR/logits_rank<r>.npy per rank when sharded.  Above 64 MB in all, every k-th row is kept (a fixed stride, so two runs
+    with the same arguments save the same images).  Inputs and weights are seeded: two builds compare output for output."""
+    import numpy as np
+    a = logits.float().cpu().numpy()
+    stride = -(-a.nbytes // (DUMP_LIMIT_BYTES // world))
+    os.makedirs(dirname, exist_ok=True)
+    path = os.path.join(dirname, "logits.npy" if world == 1 else f"logits_rank{rank}.npy")
+    np.save(path, np.ascontiguousarray(a[::stride]))
+    return path
 
 
 def build_hf(workload: str, seed: int = 0):
@@ -176,8 +193,10 @@ def run_reference(args):
             model(pixel_values=x)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            model(pixel_values=x).logits
+            out = model(pixel_values=x).logits
         el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, 0, 1)
     ips = sample * args.steps / el
     line = {
         "impl": "reference", "metric": "images_per_sec", "value": ips, "unit": "img/s", "n_gpus": args.gpus,
@@ -327,7 +346,10 @@ def main():
     ap.add_argument("--preroll-s", type=float, default=2.0, help="seconds of untimed steps before the timed region (sustained clocks)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the other BASELINE configs, the library baseline and config 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="save the logits of the last timed step as DIR/logits.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -398,6 +420,8 @@ def main():
     ms_step = float(t.item()) / args.steps
     value = gbatch / (ms_step / 1e3)
     assert torch.isfinite(out).all()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank, n_gpus)
 
     # ------------------------------------------------------------------ end to end through the public API, host buffers
     # Headline e2e: f32 pinned pixels (what the reference's loader hands over).  The C ABI also takes bf16 and raw u8
