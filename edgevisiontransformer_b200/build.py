@@ -15,17 +15,13 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-# EVT_BUILD_OUT / EVT_NVCC_EXTRA: build a differently configured library next to the shipped one for same-box A/B runs
-# (loaded through EVT_LIB_PATH), e.g. EVT_NVCC_EXTRA="-DEVT_EPI_WARPS_ACT=12" EVT_BUILD_OUT=libevt_w12.so
+# EVT_BUILD_OUT / EVT_NVCC_EXTRA: build a second library (another commit's sources, or extra nvcc flags) under its own name for
+# same-box A/B runs against the shipped one (loaded through EVT_LIB_PATH), e.g. EVT_BUILD_OUT=libevt_prev.so
 OUT = os.path.join(HERE, os.environ.get("EVT_BUILD_OUT", "libevt.so"))
 OBJ_DIR = os.path.join(CSRC, "build" + ("_" + os.path.splitext(os.path.basename(OUT))[0] if "EVT_BUILD_OUT" in os.environ else ""))
 
 SOURCES = ["common.cu", "gemm.cu", "gemm2.cu", "gemm_ln.cu", "gemm_rowln.cu", "attention.cu", "layernorm.cu", "embed.cu", "performer.cu", "swin.cu", "swin_model.cu", "model.cu"]
-# Kernels that lost their A/B (kept as negative results, DESIGN.md): the GEMM + LayerNorm epilogue fusion (gemm3.cu) and the
-# single-group ping-pong attention variants.  EVT_EXPERIMENTAL=1 in the environment builds them into the library.
-EXPERIMENTAL = os.environ.get("EVT_EXPERIMENTAL", "0") not in ("", "0")
-if EXPERIMENTAL:
-    SOURCES.insert(3, "gemm3.cu")
+# Kernels that lost their A/B tests are not kept in the tree: DESIGN.md records each result and the commit its source is at.
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -33,7 +29,7 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC",
     "--expt-relaxed-constexpr",
     "-Xptxas", "-v",
-] + (["-DEVT_EXPERIMENTAL=1"] if EXPERIMENTAL else []) + os.environ.get("EVT_NVCC_EXTRA", "").split()
+] + os.environ.get("EVT_NVCC_EXTRA", "").split()
 
 
 def nvcc() -> str:

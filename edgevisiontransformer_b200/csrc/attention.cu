@@ -1,24 +1,24 @@
 // Fused short-sequence attention for sm_100a: softmax(Q K^T * scale) V with all keys of one head
 // resident on chip (S <= 256 tokens, head size 64).  Persistent, warp-specialised, one CTA per SM:
 //
-//   work item          (image b, head h, query tile mt of 128 rows); a CTA walks (b, h) pairs blockIdx.x, +gridDim.x, ..
-//                      and the query tiles of each pair, so the K/V re-read of the second tile hits L2.
-//   warp 8 (1 thread)  TMA producer: Q [128x64], K [SKx64], V [SKx64] (bf16, 128B swizzle) straight out of the packed
-//                      QKV activation matrix into a ring of 2-4 shared-memory stages -- loads run items ahead.
-//   warp 9 (1 thread)  MMA issuer: S = Q K^T (tcgen05.mma M=128, N=SK, 4 x K=16) into one of two TMEM slots, later
-//                      O = P V (A operand = P read from TMEM, B = V as an MN-major smem operand, SK/16 MMAs) -- no
-//                      transposes anywhere, no score tensor in HBM.  QK of item j is issued before PV of item j-1.
+//   work unit          (image b, head h): a CTA walks the (b, h) pairs blockIdx.x, +gridDim.x, .. and both 128-row
+//                      query tiles of each pair (items); small batches split the tiles of a pair across CTAs instead.
+//   warp 8 (1 thread)  TMA producer: K [SKx64] and V [SKx64] once per pair into a ring of 2-4 stages, each query tile as
+//                      four 32-row boxes into a 2-deep Q ring (bf16, 128B swizzle) straight out of the packed QKV matrix.
+//   warp 9 (1 thread)  S = Q K^T issuer (tcgen05.mma M=128, N=SK, 4 x K=16) into one of two TMEM slots.
+//   warp 10 (1 thread) O = P V issuer (A operand = P read from TMEM, B = V as an MN-major smem operand, SK/16 MMAs) --
+//                      no transposes anywhere, no score tensor in HBM.
 //   warps 0-3 / 4-7    softmax group 0 / 1, one per TMEM slot (items alternate between the slots, so one group's
 //                      exponentials overlap the other's MMAs, O read-out and stores).  One thread per query row:
 //                      row max (FMNMX3), exp2 on packed f32x2 pairs, bf16 P written back over the consumed S columns
-//                      (tcgen05.st), row sum; then O * 1/sum -> bf16 context.
+//                      (tcgen05.st), row sum; then O * 1/sum -> bf16 context through a swizzled staging tile and a
+//                      3-D TMA store.
 //
 // SK = S rounded up to 16; key columns >= S are masked to probability 0, so the extra K/V rows the TMA box
 // picks up (next image's tokens, or zero fill past the end of the matrix) never contribute.
 // TMEM: 2 slots x 256 columns (S at [0,SK), P overlaid at [0,SK/2), O overlaid at [128,192)).
 #include <cuda_bf16.h>
 
-#include <cstdlib>
 #include <math_constants.h>
 
 #include "common.h"
@@ -32,28 +32,11 @@ constexpr int kQRows = 128;
 constexpr int kAttnThreads = 160;   // tf32 kernel below
 constexpr int kSoftmaxWarps = 8;
 constexpr int kProdWarp = 8;
-constexpr int kIssueWarp = 9;
-constexpr int kThreadsP = 32 * (kSoftmaxWarps + 2);
 constexpr int kSlotCols = 256;
 constexpr int kOCol = 128;
-constexpr int kMaxStages = 4;
-#ifndef EVT_ATTN_POLY_PAIRS
-#define EVT_ATTN_POLY_PAIRS 1
-#endif
 // Of every 4 pairs of exponentials, how many run on the FMA pipe (0..4).  Measured at B = 1024, S = 197, 12 heads on one box:
 // 0 -> 0.319 ms, 1 -> 0.309, 2 -> 0.318, 3 -> 0.342 (0.330 before the division-free item bookkeeping).
-constexpr int kPolyPairs = EVT_ATTN_POLY_PAIRS;
-
-struct AttnParams {
-  __nv_bfloat16* ctx;
-  const float* head_mask;
-  long long ldc;
-  int S, SK, heads, B;
-  int n_mt;      // query tiles per work unit: tiles per (image, head), or 1 when the tiles are split across CTAs
-  int q_tiles;   // query tiles per (image, head)
-  int n_stages;  // shared-memory ring depth
-  float scale_log2e;
-};
+constexpr int kPolyPairs = 1;
 
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;
@@ -100,31 +83,6 @@ __device__ __forceinline__ void ex2_poly_pair(float t0, float t1, float& p0, flo
   upk2(r, r0, r1);
   p0 = __int_as_float(__float_as_int(q0) + (__float_as_int(r0) << 23));
   p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(r1) << 23));
-}
-
-// Item j of this CTA -> (image, head, query tile).  Consecutive items share (b, h); the tile order flips on every
-// other pair so that each softmax group (slot = j & 1) sees full and ragged query tiles alternately.
-// Small batches (fewer work units than SMs) split the query tiles of a pair across CTAs instead (n_mt = 1, unit =
-// (pair, tile)): batch 1 with 12 heads then runs on 24 SMs, one tile each, instead of 12 SMs with two tiles in sequence.
-struct Item {
-  int b, h, mt;
-};
-__device__ __forceinline__ Item item_of(const AttnParams& p, int j) {
-  const int ql = j / p.n_mt;
-  const int s = j - ql * p.n_mt;
-  const int unit = blockIdx.x + ql * gridDim.x;
-  Item it;
-  if (p.n_mt != p.q_tiles) {  // split mode: unit = pair * q_tiles + tile
-    const int pair = unit / p.q_tiles;
-    it.mt = unit - pair * p.q_tiles;
-    it.b = pair / p.heads;
-    it.h = pair - it.b * p.heads;
-    return it;
-  }
-  it.b = unit / p.heads;
-  it.h = unit - it.b * p.heads;
-  it.mt = p.n_mt == 2 ? (s ^ (ql & 1)) : s;
-  return it;
 }
 
 // Row max over W score columns held in r (columns >= nvalid ignored when MASKED).
@@ -246,216 +204,12 @@ __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_v
   return sum;
 }
 
-#ifdef EVT_EXPERIMENTAL  // the round-1 kernel, kept for A/B timing (EVT_ATTN_V1=1)
-__global__ void __launch_bounds__(kThreadsP, 1)
-attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV, const AttnParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int kv_bytes = p.SK * 128;
-  const int stage_bytes = kQRows * 128 + 2 * kv_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + p.n_stages * stage_bytes);
-  uint64_t* full = bars;                      // [kMaxStages] producer -> issuer
-  uint64_t* empty = bars + kMaxStages;        // [kMaxStages] issuer (commit) -> producer
-  uint64_t* s_ready = bars + 2 * kMaxStages;  // [2] issuer (commit) -> softmax group
-  uint64_t* p_ready = s_ready + 2;            // [2] softmax group (4 warps) -> issuer
-  uint64_t* o_ready = p_ready + 2;            // [2] issuer (commit) -> softmax group
-  uint64_t* slot_free = o_ready + 2;          // [2] softmax group (4 warps) -> issuer
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(slot_free + 2);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int a = p.heads * kHD;
-  const int total_units = p.B * p.heads * (p.q_tiles / p.n_mt);
-  const int my_units = (total_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
-  const int n_items = my_units * p.n_mt;
-
-  if (warp == kProdWarp && lane == 0) {
-    ptx::prefetch_tmap(&tmQ);
-    ptx::prefetch_tmap(&tmKV);
-    for (int s = 0; s < kMaxStages; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      ptx::mbar_init(&s_ready[s], 1);
-      ptx::mbar_init(&p_ready[s], 4);
-      ptx::mbar_init(&o_ready[s], 1);
-      ptx::mbar_init(&slot_free[s], 4);
-    }
-    ptx::fence_mbar_init();
-  }
-  if (warp == kIssueWarp) ptx::tmem_alloc<512>(tmem_ptr);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  ptx::grid_dep_launch();
-  ptx::grid_dep_wait();  // qkv (previous kernel's output) is complete from here on
-
-  if (warp == kProdWarp) {
-    // ------------------------------------------------------------ TMA producer
-    if (lane == 0) {
-      int st = 0;
-      uint32_t ph = 0;
-      for (int j = 0; j < n_items; ++j) {
-        const Item it = item_of(p, j);
-        ptx::mbar_wait(&empty[st], ph ^ 1);
-        uint8_t* sQ = smem + st * stage_bytes;
-        uint8_t* sK = sQ + kQRows * 128;
-        uint8_t* sV = sK + kv_bytes;
-        const int row0 = it.b * p.S;
-        ptx::mbar_arrive_expect_tx(&full[st], stage_bytes);
-        ptx::tma_load_2d(sQ, &tmQ, &full[st], it.h * kHD, row0 + it.mt * kQRows);
-        ptx::tma_load_2d(sK, &tmKV, &full[st], a + it.h * kHD, row0);
-        ptx::tma_load_2d(sV, &tmKV, &full[st], 2 * a + it.h * kHD, row0);
-        if (++st == p.n_stages) {
-          st = 0;
-          ph ^= 1;
-        }
-      }
-    }
-  } else if (warp == kIssueWarp) {
-    // ------------------------------------------------------------ MMA issuer
-    if (lane == 0) {
-      const uint32_t idesc_qk = ptx::make_idesc(kQRows, p.SK, 1, 0, 0);
-      const uint32_t idesc_pv = ptx::make_idesc(kQRows, kHD, 1, 0, 1);
-      const int nk = p.SK / 16;
-      auto issue_pv = [&](int jj) {  // O = P V of item jj; P from TMEM (8 columns per K=16), V MN-major (2048 B per step)
-        const int sl = jj & 1;
-        const int st = jj % p.n_stages;
-        ptx::mbar_wait(&p_ready[sl], (jj >> 1) & 1);
-        ptx::tc_fence_after();
-        const uint32_t slot = tmem_base + sl * kSlotCols;
-        const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(smem + st * stage_bytes + kQRows * 128 + kv_bytes));
-        for (int k = 0; k < nk; ++k)
-          ptx::mma_f16_ts(slot + kOCol, slot + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, k != 0 ? 1u : 0u);
-        ptx::mma_commit(&o_ready[sl]);
-        ptx::mma_commit(&empty[st]);  // Q, K, V of this stage are no longer needed
-      };
-      int st = 0;
-      uint32_t ph = 0;
-      for (int j = 0; j < n_items; ++j) {
-        const int sl = j & 1;
-        ptx::mbar_wait(&full[st], ph);
-        ptx::mbar_wait(&slot_free[sl], ((j >> 1) & 1) ^ 1);
-        ptx::tc_fence_after();
-        {  // S = Q K^T
-          const uint32_t sq = ptx::smem_u32(smem + st * stage_bytes);
-          const uint64_t qd = ptx::smem_desc_sw128(sq);
-          const uint64_t kd = ptx::smem_desc_sw128(sq + kQRows * 128);
-          const uint32_t slot = tmem_base + sl * kSlotCols;
-#pragma unroll
-          for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
-          ptx::mma_commit(&s_ready[sl]);
-        }
-        if (j > 0) issue_pv(j - 1);
-        if (++st == p.n_stages) {
-          st = 0;
-          ph ^= 1;
-        }
-      }
-      if (n_items > 0) issue_pv(n_items - 1);
-    }
-  } else {
-    // ------------------------------------------------------------ softmax groups
-    const int grp = warp >> 2;
-    const int quad = warp & 3;
-    const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + grp * kSlotCols;
-    const int n16 = p.SK / 16;                    // 16-column score chunks; only the last one can hold masked keys
-    const int last_valid = p.S - (n16 - 1) * 16;  // valid columns in it (1..16)
-    const uint64_t scale2 = pk2(p.scale_log2e, p.scale_log2e);
-    // Item bookkeeping without divisions inside the loop (item_of costs two integer divisions, and the compiler
-    // re-derived it after every barrier wait: 11 % of the softmax warps' instructions): this group's items are
-    // j = grp, grp + 2, ...; the (image, head) pair index advances by dql * gridDim.x per iteration.
-    const int dql = p.n_mt == 2 ? 1 : 2;
-    const int step_pairs = dql * static_cast<int>(gridDim.x);
-    const int db = step_pairs / p.heads, dh = step_pairs - db * p.heads;
-    Item it = item_of(p, grp);
-#pragma unroll 1
-    for (int j = grp; j < n_items; j += 2) {
-      const uint32_t ph = (j >> 1) & 1;
-      const int qrow0 = it.mt * kQRows + quad * 32;
-      const bool warp_live = qrow0 < p.S;  // rows 224..255 of the second tile when S = 197: nothing to do
-      ptx::mbar_wait(&s_ready[grp], ph);
-      ptx::tc_fence_after();
-      float sum = 1.f;
-      if (warp_live) {
-        sum = softmax_row(t_row, n16, last_valid, p.scale_log2e);
-        ptx::tmem_st_wait();
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&p_ready[grp]);
-      // epilogue: O / sum
-      float inv;
-      asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(sum));  // sum >= 1 (the max contributes 2^0)
-      if (p.head_mask != nullptr) inv *= p.head_mask[it.h];
-      ptx::mbar_wait(&o_ready[grp], ph);
-      ptx::tc_fence_after();
-      uint32_t o0[32], o1[32];
-      if (warp_live) {
-        ptx::tmem_ld_x32(t_row + kOCol, o0);
-        ptx::tmem_ld_x32(t_row + kOCol + 32, o1);
-        ptx::tmem_ld_wait();
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&slot_free[grp]);  // the slot can take the next S while we convert and store
-      const int qrow = qrow0 + lane;
-      if (warp_live && qrow < p.S) {
-        __nv_bfloat16* dst = p.ctx + (static_cast<long long>(it.b) * p.S + qrow) * p.ldc + it.h * kHD;
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-#pragma unroll
-          for (int jj = 0; jj < 32; jj += 8) {
-            const uint32_t* r = half == 0 ? &o0[jj] : &o1[jj];
-            uint4 o;
-            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(r[0]) * inv, __uint_as_float(r[1]) * inv);
-            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(r[2]) * inv, __uint_as_float(r[3]) * inv);
-            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(r[4]) * inv, __uint_as_float(r[5]) * inv);
-            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(r[6]) * inv, __uint_as_float(r[7]) * inv);
-            o.x = *reinterpret_cast<uint32_t*>(&t0);
-            o.y = *reinterpret_cast<uint32_t*>(&t1);
-            o.z = *reinterpret_cast<uint32_t*>(&t2);
-            o.w = *reinterpret_cast<uint32_t*>(&t3);
-            *reinterpret_cast<uint4*>(dst + half * 32 + jj) = o;
-          }
-        }
-      }
-      // next item of this group
-      if (p.n_mt != p.q_tiles) {  // split mode (small batches only): units are (pair, tile), no incremental form
-        if (j + 2 < n_items) it = item_of(p, j + 2);
-        continue;
-      }
-      it.h += dh;
-      it.b += db;
-      if (it.h >= p.heads) {
-        it.h -= p.heads;
-        ++it.b;
-      }
-      if (p.n_mt == 2) it.mt ^= 1;  // s = grp is fixed, the tile order flips with every step of ql
-    }
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == kIssueWarp) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(tmem_base);
-  }
-}
-
-
-
-#endif  // EVT_EXPERIMENTAL
-
 // ------------------------------------------------------------------------------------------------------------
-// Round-2 kernel.  Same arithmetic and TMEM slot layout as attention_kernel above (the softmax code is shared); what
-// changed is everything around it, driven by the round-1 warp-sample profile (56 % of the softmax warps' time was spent
-// WAITING, 31 % for O = P V alone, although the tensor pipe was 25 % busy):
-//   * the single issuer thread was the bottleneck: written under `lane == 0`, every tcgen05.mma was wrapped by ptxas in an
+// Why the kernel is organised this way (a warp-sample profile of the first, single-issuer version: 56 % of the softmax
+// warps' time was spent WAITING, 31 % for O = P V alone, although the tensor pipe was 25 % busy):
+//   * a single issuer thread was the bottleneck: written under `lane == 0`, every tcgen05.mma was wrapped by ptxas in an
 //     ELECT / R2UR.BROADCAST / BRA.U.ANY loop and the descriptor arithmetic ran on per-thread registers (~110 cycles per MMA
-//     issued, 3650 per item).  The roles are now chosen with elect.sync (uniform datapath, MMAs issue back to back), and
+//     issued, 3650 per item).  The roles are chosen with elect.sync (uniform datapath, MMAs issue back to back), and
 //     S = Q K^T and O = P V are issued by TWO warps, so a P that is ready never queues behind the other group's slot wait.
 //   * K and V of an (image, head) pair are loaded ONCE for both query tiles (ring of n_kv pair stages, Q tiles in their
 //     own 2-deep ring -- one per softmax group): 138 -> 85 KB of L2 -> SM traffic per pair.
@@ -480,7 +234,6 @@ struct Attn2Params {
   int n_mt;      // query tiles per work unit (q_tiles, or 1 when the tiles of a pair are split across CTAs)
   int q_tiles;   // query tiles per (image, head)
   int n_kv;      // K/V ring depth
-  int rot_mask;  // 3: rotate the block -> quadrant assignment from unit to unit; 0: fixed (EVT_ATTN_NOROT=1, A/B timing)
   float scale_log2e;
 };
 
@@ -583,7 +336,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
           const int mt = tile_of(p, u, ql, s);
 #pragma unroll
           for (int q = 0; q < 4; ++q)  // rows past the end of the image (and whole empty blocks) arrive as zeros
-            ptx::tma_load_3d(q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &q_full[g], u.h * kHD, 32 * block_of(mt, q, ql & p.rot_mask), u.b);
+            ptx::tma_load_3d(q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &q_full[g], u.h * kHD, 32 * block_of(mt, q, ql & 3), u.b);
         }
         if (++kst == p.n_kv) {
           kst = 0;
@@ -659,7 +412,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     uint8_t* stg_row = stg + lane * 128;
     const int sw = lane & 7;
     // This group's items are j = grp, grp + 2, ...: unit ql = j / n_mt advances by dql per iteration.  (b, h) follow
-    // incrementally -- two integer divisions per item were 11 % of the softmax warps' instructions in round 1.
+    // incrementally -- two integer divisions per item were 11 % of the softmax warps' instructions in the first version.
     const int dql = p.n_mt == 2 ? 1 : 2;
     const int step_pairs = dql * static_cast<int>(gridDim.x);
     const int db = step_pairs / p.heads, dh = step_pairs - db * p.heads;
@@ -682,7 +435,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         }
       }
       const int mt = tile_of(p, u, ql, p.n_mt == 2 ? grp : 0);
-      const int qrow0 = 32 * block_of(mt, quad, ql & p.rot_mask);
+      const int qrow0 = 32 * block_of(mt, quad, ql & 3);
       const bool warp_live = qrow0 < p.S;  // block 7 (rows 224..255) when S = 197: nothing to do
       float hm = 1.f;
       if (p.head_mask != nullptr) hm = p.head_mask[u.h];
@@ -749,269 +502,6 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     ptx::tmem_dealloc<512>(tmem_base);
   }
 }
-
-#ifdef EVT_EXPERIMENTAL
-// ------------------------------------------------------------------------------------------------------------
-// EXPERIMENTAL variant (EVT_ATTN_PP=1): ONE softmax group of four warps and TWO score buffers in TMEM
-//   S0 [0, 208)  S1 [208, 416)  O [416, 480)            (2 x 208 + 64 = 480 of 512 columns)
-// so that S = Q K^T of item j+1 runs on the tensor pipe while the group exponentiates item j, and O = P V of item j runs
-// under the row-max / exponential passes of item j+1: the group never waits for an MMA in steady state (in the default
-// kernel each group's chain QK -> softmax -> PV -> read-out is serial: 32 % of its time is spent waiting for the two
-// MMAs).  Price: one softmax warp per SM sub-partition instead of two, so the MUFU pipe has no second warp to fill the
-// gaps of the first.  Issue order per item j:  QK(j+1);  wait P(j) -> PV(j).  The tensor pipe executes in issue order,
-// which is what makes the buffer re-use safe: QK(j+2) overwrites the buffer whose P(j) was read by PV(j), issued before it.
-constexpr int kPPSCols = 208;
-constexpr int kPPOCol = 416;
-constexpr int kPPMaxHalfChunks = 7;  // 13 score chunks of 16 columns split 7 + 6 between the two threads of a row
-
-// HALVES = 1: one thread per query row (four softmax warps).  HALVES = 2: two threads per row (eight softmax warps, the
-// second MUFU client per sub-partition back): thread h of a row owns the score chunks [h * 7, ...) and the context columns
-// [32 h, 32 h + 32).  Row maximum and row sum are exchanged through shared memory with a 64-thread named barrier per
-// lane quadrant; because P overlays S, a thread keeps its bf16 P half in registers until BOTH threads have consumed
-// their score columns (the second barrier) and only then writes it to TMEM.
-template <int HALVES>
-__global__ void __launch_bounds__(32 * (4 * HALVES + 2), 1)
-attention_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV, const AttnParams p) {
-  constexpr int kSoftWarps = 4 * HALVES, kProd = kSoftWarps, kIssue = kSoftWarps + 1;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int kv_bytes = p.SK * 128;
-  const int stage_bytes = kQRows * 128 + 2 * kv_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + p.n_stages * stage_bytes);
-  uint64_t* full = bars;                      // [kMaxStages] producer -> issuer
-  uint64_t* empty = bars + kMaxStages;        // [kMaxStages] issuer (commit) -> producer
-  uint64_t* s_ready = bars + 2 * kMaxStages;  // [2] issuer (commit) -> softmax warps, one per score buffer
-  uint64_t* p_ready = s_ready + 2;            // [1] softmax warps: P(j) written and O(j-1) read out
-  uint64_t* o_ready = p_ready + 1;            // [1] issuer (commit) -> softmax warps
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(o_ready + 1);
-  float* xch = reinterpret_cast<float*>(bars + 2 * kMaxStages + 8);  // [2 (max | sum)][2 halves][128 rows]
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int a = p.heads * kHD;
-  const int total_units = p.B * p.heads * (p.q_tiles / p.n_mt);
-  const int my_units = (total_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
-  const int n_items = my_units * p.n_mt;
-
-  if (warp == kProd && lane == 0) {
-    ptx::prefetch_tmap(&tmQ);
-    ptx::prefetch_tmap(&tmKV);
-    for (int s = 0; s < kMaxStages; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    ptx::mbar_init(&s_ready[0], 1);
-    ptx::mbar_init(&s_ready[1], 1);
-    ptx::mbar_init(p_ready, kSoftWarps);
-    ptx::mbar_init(o_ready, 1);
-    ptx::fence_mbar_init();
-  }
-  if (warp == kIssue) ptx::tmem_alloc<512>(tmem_ptr);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  ptx::grid_dep_launch();
-  ptx::grid_dep_wait();
-
-  if (warp == kProd) {
-    // ------------------------------------------------------------ TMA producer (as in attention_kernel)
-    if (lane == 0) {
-      int st = 0;
-      uint32_t ph = 0;
-      for (int j = 0; j < n_items; ++j) {
-        const Item it = item_of(p, j);
-        ptx::mbar_wait(&empty[st], ph ^ 1);
-        uint8_t* sQ = smem + st * stage_bytes;
-        uint8_t* sK = sQ + kQRows * 128;
-        uint8_t* sV = sK + kv_bytes;
-        const int row0 = it.b * p.S;
-        ptx::mbar_arrive_expect_tx(&full[st], stage_bytes);
-        ptx::tma_load_2d(sQ, &tmQ, &full[st], it.h * kHD, row0 + it.mt * kQRows);
-        ptx::tma_load_2d(sK, &tmKV, &full[st], a + it.h * kHD, row0);
-        ptx::tma_load_2d(sV, &tmKV, &full[st], 2 * a + it.h * kHD, row0);
-        if (++st == p.n_stages) {
-          st = 0;
-          ph ^= 1;
-        }
-      }
-    }
-  } else if (warp == kIssue) {
-    // ------------------------------------------------------------ MMA issuer
-    if (lane == 0 && n_items > 0) {
-      const uint32_t idesc_qk = ptx::make_idesc(kQRows, p.SK, 1, 0, 0);
-      const uint32_t idesc_pv = ptx::make_idesc(kQRows, kHD, 1, 0, 1);
-      const int nk = p.SK / 16;
-      int st = 0;          // stage of the item whose QK is issued next
-      uint32_t ph = 0;
-      auto issue_qk = [&](int jj) {
-        ptx::mbar_wait(&full[st], ph);
-        ptx::tc_fence_after();
-        const uint32_t sq = ptx::smem_u32(smem + st * stage_bytes);
-        const uint64_t qd = ptx::smem_desc_sw128(sq);
-        const uint64_t kd = ptx::smem_desc_sw128(sq + kQRows * 128);
-        const uint32_t sbuf = tmem_base + (jj & 1) * kPPSCols;
-#pragma unroll
-        for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(sbuf, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
-        ptx::mma_commit(&s_ready[jj & 1]);
-        if (++st == p.n_stages) {
-          st = 0;
-          ph ^= 1;
-        }
-      };
-      issue_qk(0);
-      for (int j = 0; j < n_items; ++j) {
-        if (j + 1 < n_items) issue_qk(j + 1);       // runs under the exponentials of item j
-        ptx::mbar_wait(p_ready, j & 1);             // P(j) complete, O(j-1) read out
-        ptx::tc_fence_after();
-        const int stj = j % p.n_stages;
-        const uint32_t sbuf = tmem_base + (j & 1) * kPPSCols;
-        const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(smem + stj * stage_bytes + kQRows * 128 + kv_bytes));
-        for (int k = 0; k < nk; ++k)
-          ptx::mma_f16_ts(tmem_base + kPPOCol, sbuf + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, k != 0 ? 1u : 0u);
-        ptx::mma_commit(o_ready);
-        ptx::mma_commit(&empty[stj]);
-      }
-    }
-  } else {
-    // ------------------------------------------------------------ softmax warps: thread = (query row, half)
-    const int quad = warp & 3;
-    const int half = warp >> 2;
-    const int row_in_tile = quad * 32 + lane;
-    const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
-    const int n16 = p.SK / 16;
-    const int last_valid = p.S - (n16 - 1) * 16;
-    const int c_split = HALVES == 2 ? (n16 + 1) / 2 : n16;
-    const int c0 = half == 0 ? 0 : c_split, c1 = half == 0 ? c_split : n16;
-    constexpr int kOC = 64 / HALVES;               // context columns of this thread
-    float* xmax = xch;
-    float* xsum = xch + 2 * 128;
-    const uint64_t scale2 = pk2(p.scale_log2e, p.scale_log2e);
-    Item prev = {0, 0, 0};
-    float prev_inv = 0.f;
-    bool prev_live = false;
-#pragma unroll 1
-    for (int j = 0; j <= n_items; ++j) {
-      Item it = {0, 0, 0};
-      float sum = 1.f;
-      bool live = false;
-      if (j < n_items) {
-        it = item_of(p, j);
-        live = it.mt * kQRows + quad * 32 < p.S;
-        ptx::mbar_wait(&s_ready[j & 1], (j >> 1) & 1);
-        ptx::tc_fence_after();
-        if (live) {
-          if constexpr (HALVES == 1) {
-            sum = softmax_row(lane_base + (j & 1) * kPPSCols, n16, last_valid, p.scale_log2e);
-            ptx::tmem_st_wait();
-          } else {
-            const uint32_t t_row = lane_base + (j & 1) * kPPSCols;
-            uint32_t buf[2][16];
-            // pass 1: maximum over this thread's chunks
-            float m[4] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
-            if (c0 < c1) ptx::tmem_ld_x16(t_row + c0 * 16, buf[0]);
-#pragma unroll
-            for (int i = 0; i < kPPMaxHalfChunks; ++i) {
-              const int c = c0 + i;
-              if (c < c1) {
-                ptx::tmem_ld_wait();
-                if (c + 1 < c1) ptx::tmem_ld_x16(t_row + (c + 1) * 16, buf[(i + 1) & 1]);
-                if (c == n16 - 1) chunk_max<16, true>(buf[i & 1], last_valid, m);
-                else chunk_max<16, false>(buf[i & 1], 16, m);
-              }
-            }
-            float mx = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3]));
-            xmax[half * 128 + row_in_tile] = mx;
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");
-            mx = fmaxf(mx, xmax[(half ^ 1) * 128 + row_in_tile]);
-            const float nm = -mx * p.scale_log2e;
-            const uint64_t negm2 = pk2(nm, nm);
-            // pass 2: exponentials of this thread's chunks; the bf16 P half stays in registers
-            uint64_t sum2[2] = {0ull, 0ull};
-            uint32_t pk[kPPMaxHalfChunks][8];
-            if (c0 < c1) ptx::tmem_ld_x16(t_row + c0 * 16, buf[0]);
-#pragma unroll
-            for (int i = 0; i < kPPMaxHalfChunks; ++i) {
-              const int c = c0 + i;
-              if (c < c1) {
-                ptx::tmem_ld_wait();
-                if (c + 1 < c1) ptx::tmem_ld_x16(t_row + (c + 1) * 16, buf[(i + 1) & 1]);
-                if (c == n16 - 1) chunk_exp<16, true>(buf[i & 1], last_valid, scale2, negm2, sum2, pk[i]);
-                else chunk_exp<16, false>(buf[i & 1], 16, scale2, negm2, sum2, pk[i]);
-              }
-            }
-            float s0, s1, s2, s3;
-            upk2(sum2[0], s0, s1);
-            upk2(sum2[1], s2, s3);
-            const float part = (s0 + s1) + (s2 + s3);
-            xsum[half * 128 + row_in_tile] = part;
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");   // both threads of the row are done reading S
-            sum = part + xsum[(half ^ 1) * 128 + row_in_tile];
-#pragma unroll
-            for (int i = 0; i < kPPMaxHalfChunks; ++i)
-              if (c0 + i < c1) ptx::tmem_st_x8(t_row + (c0 + i) * 8, pk[i]);
-            ptx::tmem_st_wait();
-          }
-        }
-      }
-      // O of the previous item: complete long ago in steady state (its MMAs ran under the passes above)
-      uint32_t o[kOC];
-      if (j > 0) {
-        ptx::mbar_wait(o_ready, (j - 1) & 1);
-        ptx::tc_fence_after();
-        if (prev_live) {
-          if constexpr (HALVES == 1) {
-            ptx::tmem_ld_x32(lane_base + kPPOCol, reinterpret_cast<uint32_t(&)[32]>(o[0]));
-            ptx::tmem_ld_x32(lane_base + kPPOCol + 32, reinterpret_cast<uint32_t(&)[32]>(o[32]));
-          } else {
-            ptx::tmem_ld_x32(lane_base + kPPOCol + half * 32, reinterpret_cast<uint32_t(&)[32]>(o[0]));
-          }
-          ptx::tmem_ld_wait();
-        }
-      }
-      if (j < n_items) {
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(p_ready);   // P(j) is in TMEM and O(j-1) is in registers: PV(j) may run
-      }
-      if (j > 0) {
-        const int qrow = prev.mt * kQRows + row_in_tile;
-        if (prev_live && qrow < p.S) {
-          __nv_bfloat16* dst = p.ctx + (static_cast<long long>(prev.b) * p.S + qrow) * p.ldc + prev.h * kHD + (HALVES == 2 ? half * 32 : 0);
-#pragma unroll
-          for (int jj = 0; jj < kOC; jj += 8) {
-            uint4 v;
-            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(o[jj]) * prev_inv, __uint_as_float(o[jj + 1]) * prev_inv);
-            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(o[jj + 2]) * prev_inv, __uint_as_float(o[jj + 3]) * prev_inv);
-            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(o[jj + 4]) * prev_inv, __uint_as_float(o[jj + 5]) * prev_inv);
-            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(o[jj + 6]) * prev_inv, __uint_as_float(o[jj + 7]) * prev_inv);
-            v.x = *reinterpret_cast<uint32_t*>(&t0);
-            v.y = *reinterpret_cast<uint32_t*>(&t1);
-            v.z = *reinterpret_cast<uint32_t*>(&t2);
-            v.w = *reinterpret_cast<uint32_t*>(&t3);
-            *reinterpret_cast<uint4*>(dst + jj) = v;
-          }
-        }
-      }
-      float inv;
-      asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(sum));
-      if (p.head_mask != nullptr && j < n_items) inv *= p.head_mask[it.h];
-      prev = it;
-      prev_inv = inv;
-      prev_live = live;
-    }
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == kIssue) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(tmem_base);
-  }
-}
-
-
-#endif  // EVT_EXPERIMENTAL
 
 // ------------------------------------------------------------------------------------------------------------
 // tf32 accuracy mode: Q, K, V and the context are fp32 in HBM; the tensor core reads them as tf32 (kind::tf32,
@@ -1221,52 +711,6 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   CUtensorMap tmKV;
   int rc = make_tmap_2d(&tmKV, qkv, 2, rows, 3ull * heads * kHD, static_cast<uint64_t>(ldq), SK, kHD);
   if (rc != EVT_OK) return rc;
-#ifdef EVT_EXPERIMENTAL
-  // round-1 kernels, selectable for A/B timing: EVT_ATTN_V1=1 (two softmax groups, one issuer), EVT_ATTN_PP=1|2 (ping-pong)
-  static const bool use_v1 = getenv("EVT_ATTN_V1") != nullptr && atoi(getenv("EVT_ATTN_V1")) != 0;
-  static const int pp_mode = getenv("EVT_ATTN_PP") != nullptr ? atoi(getenv("EVT_ATTN_PP")) : 0;
-  if (use_v1 || pp_mode != 0) {
-    CUtensorMap tmQ;
-    rc = make_tmap_2d(&tmQ, qkv, 2, rows, 3ull * heads * kHD, static_cast<uint64_t>(ldq), kQRows, kHD);
-    if (rc != EVT_OK) return rc;
-    AttnParams p;
-    p.ctx = reinterpret_cast<__nv_bfloat16*>(ctx);
-    p.head_mask = head_mask;
-    p.ldc = ldc;
-    p.S = S;
-    p.SK = SK;
-    p.heads = heads;
-    p.B = B;
-    p.q_tiles = q_tiles;
-    p.n_mt = n_mt;
-    p.scale_log2e = scale_log2e;
-    const int stage_bytes = kQRows * 128 + 2 * SK * 128;
-    const int bar_bytes = (2 * kMaxStages + 8) * 8 + 16;
-    int n_stages = (max_smem - 1024 - bar_bytes) / stage_bytes;
-    if (n_stages > kMaxStages) n_stages = kMaxStages;
-    if (n_stages < 2) return fail(EVT_ERR_UNSUPPORTED, "attention: sequence too long for two shared-memory stages");
-    p.n_stages = n_stages;
-    const int smem = 1024 + n_stages * stage_bytes + bar_bytes;
-    static int configured_dev = -1;
-    if (configured_dev != dev) {
-      EVT_CUDA(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-      EVT_CUDA(cudaFuncSetAttribute(attention_pp_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-      EVT_CUDA(cudaFuncSetAttribute(attention_pp_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-      configured_dev = dev;
-    }
-    if (pp_mode != 0 && SK <= kPPSCols && smem + 2048 <= max_smem) {
-      if (pp_mode == 2)
-        EVT_CUDA(launch_pdl(attention_pp_kernel<2>, dim3(grid), dim3(32 * 10), smem + 2048, stream, pdl, tmQ, tmKV, p));
-      else
-        EVT_CUDA(launch_pdl(attention_pp_kernel<1>, dim3(grid), dim3(32 * 6), smem + 2048, stream, pdl, tmQ, tmKV, p));
-      EVT_LAUNCH_CHECK("attention_pp_kernel");
-      return EVT_OK;
-    }
-    EVT_CUDA(launch_pdl(attention_kernel, dim3(grid), dim3(kThreadsP), smem, stream, pdl, tmQ, tmKV, p));
-    EVT_LAUNCH_CHECK("attention_kernel");
-    return EVT_OK;
-  }
-#endif  // EVT_EXPERIMENTAL
   CUtensorMap tmO, tmQ;
   rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
                          static_cast<uint64_t>(ldq), 32, kHD);
@@ -1283,8 +727,6 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   q.n_mt = n_mt;
   q.q_tiles = q_tiles;
   q.scale_log2e = scale_log2e;
-  static const bool no_rot = getenv("EVT_ATTN_NOROT") != nullptr && atoi(getenv("EVT_ATTN_NOROT")) != 0;  // A/B timing
-  q.rot_mask = no_rot ? 0 : 3;
   const int fixed = 1024 + 2 * kQTileBytes + kSoftmaxWarps * kStgWarpBytes + (2 * kMaxKV + 12) * 8 + 16;
   int n_kv = (max_smem - fixed) / (2 * SK * 128);
   if (n_kv > kMaxKV) n_kv = kMaxKV;

@@ -78,13 +78,6 @@ bool pdl_enabled() {
   }();
   return on;
 }
-bool gemm_ln_fusion_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("EVT_FUSE_LN");
-    return e != nullptr && atoi(e) != 0;
-  }();
-  return on;
-}
 static std::atomic<int> g_split_k{[] {
   const char* e = getenv("EVT_GEMM_SPLIT_K");
   return e == nullptr ? 1 : (atoi(e) != 0);

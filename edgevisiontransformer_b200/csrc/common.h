@@ -85,7 +85,6 @@ struct StaticWeightsScope {
   StaticWeightsScope();
   ~StaticWeightsScope();
 };
-bool gemm_ln_fusion_enabled();  // EVT_FUSE_LN=1 routes the model runtime through the experimental GEMM+LayerNorm kernel
 bool gemm_split_k_enabled();  // evt_gemm_set_split_k / EVT_GEMM_SPLIT_K
 int gemm_pair_mode();  // -1 auto, 0 never, 1 whenever applicable (evt_gemm_set_pair_mode / EVT_GEMM_PAIR)
 

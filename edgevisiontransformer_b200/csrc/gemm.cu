@@ -13,8 +13,6 @@
 // once) while the whole weight matrix stays in L2.  M, N and K tails are handled by TMA zero fill on the
 // load side and by clipping / predication on the store side, so no operand is ever padded in HBM (only leading
 // dimensions must be multiples of 16 bytes).
-#include <cstdlib>
-
 #include "gemm_common.cuh"
 #include "ops.h"
 
@@ -201,17 +199,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 // Tile width: the one that pads N least; when that leaves SMs without a tile (small M: the latency path), the
 // narrower width that puts the most CTAs to work.
 int choose_bn(int64_t M, int N) {
-  // tuning override: EVT_GEMM_BN="N:bn[,N:bn...]" forces the tile width for the given output widths
-  static const char* force = getenv("EVT_GEMM_BN");
-  if (force != nullptr) {
-    for (const char* q = force; *q != 0;) {
-      const long n = strtol(q, const_cast<char**>(&q), 10);
-      if (*q != ':') break;
-      const long bn = strtol(q + 1, const_cast<char**>(&q), 10);
-      if (n == N && (bn == 256 || bn == 192 || bn == 128 || bn == 64)) return static_cast<int>(bn);
-      if (*q == ',') ++q;
-    }
-  }
   const int cands[4] = {256, 192, 128, 64};
   const long tiles_m = static_cast<long>((M + BM - 1) / BM);
   int best = 256;
@@ -346,11 +333,10 @@ int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_d
   // off, and a forced kernel choice (evt_gemm_set_pair_mode) never splits.
   p.k_splits = 1;
   p.kb_per_split = p.num_kb;
-  // The tf32 (accuracy) mode does not split unless EVT_TF32_SPLIT_K=1: DeiT-Tiny batch 1 would drop from 0.477 to 0.427 ms, but
-  // the unordered f32 reduce-adds flip tf32 roundings downstream and the logit error of BASELINE config 1 moves from a
-  // reproducible 7.5e-4 to 9.2e-4 in one run -- a random variable that close to the 1e-3 contract is not worth 0.05 ms.
-  static const bool tf32_split = getenv("EVT_TF32_SPLIT_K") != nullptr && atoi(getenv("EVT_TF32_SPLIT_K")) != 0;
-  if ((!tf32 || tf32_split) && tma_out && residual != nullptr && gemm_pair_mode() < 0 && gemm_split_k_enabled()) {
+  // The tf32 (accuracy) mode never splits: DeiT-Tiny batch 1 would drop from 0.477 to 0.427 ms, but the unordered f32
+  // reduce-adds flip tf32 roundings downstream and the logit error of BASELINE config 1 moves from a reproducible 7.5e-4
+  // to 9.2e-4 in one run -- a random variable that close to the 1e-3 contract is not worth 0.05 ms.
+  if (!tf32 && tma_out && residual != nullptr && gemm_pair_mode() < 0 && gemm_split_k_enabled()) {
     const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
     if (tiles * 2 <= num_sms() && p.num_kb >= 4) {
       int splits = static_cast<int>(num_sms() / tiles);

@@ -22,22 +22,13 @@ namespace {
 
 using namespace gemm_detail;
 
-#ifndef EVT_EPI_WARPS_ACT
-#define EVT_EPI_WARPS_ACT 8
-#endif
-constexpr int kEpiWarpsAct = EVT_EPI_WARPS_ACT;  // epilogue warps of the bf16-output kernels with a fused activation
-
-// EW = epilogue warps per CTA (8, or 16 = 4 per TMEM lane quadrant with one 64-column chunk each).  16 was tried for the
-// FC1 + GELU kernel (-DEVT_EPI_WARPS_ACT=16) on the theory that the epilogue's latency per tile holds up the accumulator
-// hand-off: it measured SLOWER (FC1 0.944 vs 0.912 ms in the step, 1101 vs 1248 TFLOP/s alone) -- 576 threads leave 96
-// registers per thread (the unrolled GELU loses its interleaving) and the extra staging costs a pipeline stage; 12 (three
-// groups, rotating) measured equal within noise.  Default 8.
+// EW = epilogue warps per CTA (8, or 16 = 4 per TMEM lane quadrant with one 64-column chunk each); launch_pair chooses.
 template <int BN, int EW>
 struct Cfg2 {
   static constexpr int kABytes = BM * kStageRowBytes;
   static constexpr int kBBytes = (BN / 2) * kStageRowBytes;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStagingBytes = EW * kStgBytes * kStgBufs;
+  static constexpr int kStagingBytes = EW * kStgBytes;
   static constexpr int kMaxStages = (232448 - 1024 - kStagingBytes - 256) / kStageBytes;
   static constexpr int kStages = kMaxStages < (BN == 128 ? 8 : 6) ? kMaxStages : (BN == 128 ? 8 : 6);
   static constexpr int kTmemCols = BN == 128 ? 256 : 512;
@@ -177,12 +168,11 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   } else {
     // ------------------------------------------------------------ epilogue warps 0..7 (both CTAs, own 128 rows)
     const int quad = warp & 3;
-    uint8_t* stg = staging + warp * kStgBytes * kStgBufs;
-    int stg_sel = 0;
+    uint8_t* stg = staging + warp * kStgBytes;
     int as = 0;
     uint32_t aphase = 0;
-    // With a group count that does not divide the chunk count (12 warps = 3 groups, 4 chunks of 64 columns) the group that
-    // takes two chunks rotates from tile to tile, so every warp does 4 chunks per 3 tiles.
+    // With a group count that does not divide the chunk count (BN = 192, bf16 out: 3 chunks of 64 columns for 2 or 4 groups)
+    // the group assignment rotates from tile to tile, so every warp gets the same share of chunks over 2 (or 4) tiles.
     constexpr int kGroups = EW / 4;
     constexpr bool kRotate = ((BN / (OUT_F32 ? 32 : 64)) % kGroups) != 0;
     const int grp0 = warp >> 2;
@@ -200,7 +190,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       ptx::mbar_wait(&tfull[as], aphase);
       ptx::tc_fence_after();
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + as * BN;
-      epilogue_tile<BN, false, OUT_F32, ACT, true, EW / 4, kStgBufs>(p, &tmO, stg, grp, lane, m0, nt0, t_row, &stg_sel);
+      epilogue_tile<BN, false, OUT_F32, ACT, true, EW / 4>(p, &tmO, stg, grp, lane, m0, nt0, t_row);
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_cluster(ptx::mapa(&tempty[as], 0));
@@ -259,14 +249,16 @@ int launch_pair_ew(const void* W, int64_t ldw, const CUtensorMap& tmA, const CUt
 // Epilogue warps per CTA.  With a fused activation and a SHORT K loop (K <= 384: DeiT-Tiny / -Small / T2T FC1, three to six
 // k-blocks per tile) the tile time is the epilogue's, and sixteen warps (four per TMEM lane quadrant, one 64-column chunk each)
 // finish it sooner: FC1 74.6 -> 68.9 us at D = 384 (batch 256), 49.1 -> 45.2 us for the pruned Tiny (batch 1024), same box.  With
-// a long K loop the MMAs bound the tile and sixteen warps LOSE (DeiT-Base FC1 0.944 vs 0.912 ms: 96 registers per thread, one
-// pipeline stage less), so eight stay the default there.  Without an activation sixteen warps lose as well (QKV at D = 384:
-// 55 vs 49 us): the plain bf16 epilogue is bound by its TMA stores, not by instruction latency.
+// a long K loop the MMAs bound the tile and sixteen warps LOSE (DeiT-Base FC1 0.944 vs 0.912 ms in the step, 1101 vs 1248
+// TFLOP/s alone: 576 threads leave 96 registers per thread, the unrolled GELU loses its interleaving, and the extra staging
+// costs a pipeline stage), so eight stay there; twelve (three groups, rotating) measured equal to eight within noise.  Without
+// an activation sixteen warps lose as well (QKV at D = 384: 55 vs 49 us): the plain bf16 epilogue is bound by its TMA stores,
+// not by instruction latency.
 template <int BN, bool OUT_F32, int ACT>
 int launch_pair(const void* W, int64_t ldw, const CUtensorMap& tmA, const CUtensorMap& tmO, const GemmParams& p, cudaStream_t stream) {
   if constexpr (ACT != EVT_ACT_NONE && !OUT_F32) {
-    if (kEpiWarpsAct == 8 && p.K <= 384) return launch_pair_ew<BN, OUT_F32, ACT, 16>(W, ldw, tmA, tmO, p, stream);
-    return launch_pair_ew<BN, OUT_F32, ACT, kEpiWarpsAct>(W, ldw, tmA, tmO, p, stream);
+    if (p.K <= 384) return launch_pair_ew<BN, OUT_F32, ACT, 16>(W, ldw, tmA, tmO, p, stream);
+    return launch_pair_ew<BN, OUT_F32, ACT, 8>(W, ldw, tmA, tmO, p, stream);
   } else {
     return launch_pair_ew<BN, OUT_F32, ACT, 8>(W, ldw, tmA, tmO, p, stream);
   }

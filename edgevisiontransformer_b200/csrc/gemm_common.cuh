@@ -17,13 +17,6 @@ constexpr int kProducerWarp = kEpiWarps;
 constexpr int kMmaWarp = kEpiWarps + 1;
 constexpr int kThreads = 32 * (kEpiWarps + 2);
 constexpr int kStgBytes = 32 * 128;  // per epilogue warp: 32 dense 128-byte rows, 128B-swizzled
-#ifndef EVT_GELU_ESTRIN
-#define EVT_GELU_ESTRIN 0
-#endif
-#ifndef EVT_STG_BUFS
-#define EVT_STG_BUFS 1
-#endif
-constexpr int kStgBufs = EVT_STG_BUFS;  // CTA-pair kernel: staging tiles per epilogue warp (2 = never wait for the previous TMA store)
 
 template <int BN>
 struct Cfg {
@@ -122,21 +115,11 @@ __device__ __forceinline__ void gelu_erf_pair(float& x0, float& x1) {
     q = fma2(q, a, pk2(-4.585517347e-01f, -4.585517347e-01f));
     q = fma2(q, a, pk2(-1.151212096e+00f, -1.151212096e+00f));
   } else {
-#if EVT_GELU_ESTRIN
-    // Estrin form: dependency depth 3 instead of 5 at the price of two extra multiplies
-    const uint64_t a2 = mul2(a, a);
-    const uint64_t p45 = fma2(a, pk2(2.554092680e-05f, 2.554092680e-05f), pk2(-6.528479280e-04f, -6.528479280e-04f));
-    const uint64_t p23 = fma2(a, pk2(7.452332415e-03f, 7.452332415e-03f), pk2(-5.191940814e-02f, -5.191940814e-02f));
-    const uint64_t p01 = fma2(a, pk2(-4.602991641e-01f, -4.602991641e-01f), pk2(-1.150684714e+00f, -1.150684714e+00f));
-    const uint64_t a4 = mul2(a2, a2);
-    q = fma2(p45, a4, fma2(p23, a2, p01));
-#else
     q = fma2(a, pk2(2.554092680e-05f, 2.554092680e-05f), pk2(-6.528479280e-04f, -6.528479280e-04f));
     q = fma2(q, a, pk2(7.452332415e-03f, 7.452332415e-03f));
     q = fma2(q, a, pk2(-5.191940814e-02f, -5.191940814e-02f));
     q = fma2(q, a, pk2(-4.602991641e-01f, -4.602991641e-01f));
     q = fma2(q, a, pk2(-1.150684714e+00f, -1.150684714e+00f));
-#endif
   }
   float t0, t1;
   upk2(fma2(q, a, pk2(-1.0f, -1.0f)), t0, t1);
@@ -220,10 +203,9 @@ __device__ __forceinline__ void prefetch_bias(const GemmParams& p, int grp, int 
 // on packed f32x2 pairs; the converted chunk then goes through a 128B-swizzled 4 KB smem tile (stg) to a TMA store /
 // TMA f32 reduce-add, or to coalesced global stores on the generic path.
 //   m0: first global row of this warp's block; nt0: first column of the tile; t_row: TMEM address (lane | column).
-template <int BN, bool TF32, bool OUT_F32, int ACT, bool TMA_OUT, int NGRP = 2, int STG = 1>
-__device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtensorMap* tmO, uint8_t* stg0, int grp, int lane,
-                                              int m0, int nt0, uint32_t t_row, int* stg_sel = nullptr) {
-  uint8_t* stg = stg0;  // STG == 2: the warp alternates between two staging tiles (stg0, stg0 + kStgBytes); *stg_sel persists
+template <int BN, bool TF32, bool OUT_F32, int ACT, bool TMA_OUT, int NGRP = 2>
+__device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtensorMap* tmO, uint8_t* stg, int grp, int lane,
+                                              int m0, int nt0, uint32_t t_row) {
   constexpr int CH = OUT_F32 ? 32 : 64;
   constexpr int NCH = BN / CH;
   const int sw = lane & 7;
@@ -294,13 +276,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtenso
       // stage: dense 128-byte rows, 16-byte pieces XOR-swizzled by (row & 7) -- the layout a SWIZZLE_128B
       // tensor map expects, and conflict-free for both the row-per-thread writes and the row-segment reads.
       if constexpr (TMA_OUT) {
-        if constexpr (STG == 2) {
-          stg = stg0 + (*stg_sel & 1) * kStgBytes;
-          ++*stg_sel;
-          if (ptx::elect_one()) ptx::bulk_wait_read<1>();  // the store before the previous one has finished reading this tile
-        } else {
-          if (ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous store of this warp has finished reading stg
-        }
+        if (ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous store of this warp has finished reading stg
       }
       __syncwarp();
       // explicit st.shared: through the C++ pointer these were generic ST.E with descriptor set-up (see ptx.cuh)

@@ -21,8 +21,12 @@
 //   warps 10-13  LayerNorm: eight threads per row, 16 rows at a time out of the staged chunk, f32 mean and centred variance
 //                (three shuffle levels), bf16 result written straight into the A tiles; optionally the normalised f32
 //                row is written back to x (TF dialect: the skip carries LN(x))
-#include <cstdlib>
-
+//
+// The model runtime does not use it: measured on B200 (same box, per launch, batch 1024 / 256):
+//   pruned DeiT-Tiny  QKV 83.8 us fused vs 38.3 (LayerNorm) + 33.9 (GEMM);  FC1 94.1 vs 38.3 + 48.1  -> 240 k vs 255 k img/s
+//   DeiT-Small        QKV 138 vs 23.6 + 47.0;  FC1 176 vs 23.6 + 72.9 (96 KB of A tiles leave a 2-deep W ring)
+// One persistent CTA per SM keeps ~50 KB of the residual stream in flight where the stand-alone LayerNorm kernel keeps
+// the whole SM's worth of warps loading.  The op stays available (evt_layernorm_gemm).  See DESIGN.md.
 #include "gemm_common.cuh"
 #include "ops.h"
 
@@ -374,20 +378,6 @@ int dispatch_ln_kb(int kb, const CUtensorMap& w, const CUtensorMap& o, const LnG
 }
 
 }  // namespace
-
-bool gemm_ln_supported(int64_t M, int N, int K) {
-  // Off in the model runtime unless EVT_FUSE_LN_A=1: measured on B200 (round 2, same box, per launch, batch 1024 / 256):
-  //   pruned DeiT-Tiny  QKV 83.8 us fused vs 38.3 (LayerNorm) + 33.9 (GEMM);  FC1 94.1 vs 38.3 + 48.1  -> 240 k vs 255 k img/s
-  //   DeiT-Small        QKV 138 vs 23.6 + 47.0;  FC1 176 vs 23.6 + 72.9 (96 KB of A tiles leave a 2-deep W ring)
-  // One persistent CTA per SM keeps ~50 KB of the residual stream in flight where the stand-alone LayerNorm kernel keeps
-  // the whole SM's worth of warps loading; the op stays available (evt_layernorm_gemm) and tested.  See DESIGN.md.
-  static const bool on = getenv("EVT_FUSE_LN_A") != nullptr && atoi(getenv("EVT_FUSE_LN_A")) != 0;
-  if (!on) return false;
-  const bool k_ok = K == 64 || K == 128 || K == 192 || K == 256 || K == 384;
-  // one CTA per 128-row block: worth it once the row blocks fill the GPU (large batch); the latency path keeps the
-  // narrow-tile / split-K kernels
-  return k_ok && N > 0 && (M + BM - 1) / BM >= num_sms();
-}
 
 int gemm_ln_launch(const float* x, int64_t ldx, const float* gamma, const float* beta, float eps, float* x_copy, const void* W,
                    int64_t ldw, const float* bias, void* out, int64_t ldo, int64_t M, int N, int K, int act, cudaStream_t stream) {

@@ -9,8 +9,8 @@
 // (modeling/models/vit.py: the skip connection carries the normalised rows): the residual stream then receives the
 // unrounded f32 LayerNorm output instead of x.
 //
-// Why a second attempt after gemm3.cu (DESIGN.md, negative results): that kernel walked the N tiles of a row block one after
-// the other and had to re-read the new residual from L2 for the normalisation pass.  Here the full row block (256 rows x D
+// Why a second attempt after the first GEMM + LayerNorm epilogue fusion (removed, DESIGN.md, negative results): that kernel
+// walked the N tiles of a row block one after the other and had to re-read the new residual from L2 for the normalisation pass.  Here the full row block (256 rows x D
 // columns of f32) stays in TMEM (192-column accumulator slots, two of them), the old residual comes in through a TMA ring
 // that a dedicated thread keeps full across row blocks, and the three epilogue passes (x' and row sums; centred squares;
 // normalise) read tensor memory only.  HBM traffic per row: K*2 (A) + 4D (x in) + 4D (x out) + 2D (xn) bytes -- the LayerNorm
@@ -39,16 +39,6 @@ constexpr int kResBytes = BM * 128;        // ring entry: 128 rows x 32 f32
 constexpr int kXnStgBytes = 32 * 64;       // bf16 staging tile of one epilogue warp: 32 rows x 32 bf16, 64B-swizzled
 constexpr int kMaxD = 384;
 constexpr int kSmemLimit = 232448;
-// A/B knobs of the D = 384 configuration (build.py: EVT_NVCC_EXTRA): operand stages of the K loop against residual-ring depth
-#ifndef EVT_ROWLN_STAGES2
-#define EVT_ROWLN_STAGES2 3
-#endif
-#ifndef EVT_ROWLN_DEPTH2
-#define EVT_ROWLN_DEPTH2 6
-#endif
-#ifndef EVT_ROWLN_DEPTHMIN_COPY2
-#define EVT_ROWLN_DEPTHMIN_COPY2 4
-#endif
 
 struct RowLnParams {
   const float* bias;   // [D] or null
@@ -73,8 +63,9 @@ struct CfgR {
   static constexpr int kStageBytes = kABytes + kBBytes;
   // NT == 1: two accumulator slots double-buffer the row blocks, the K loop is short and hidden -> two stages are enough.
   // NT == 2: one K loop per slot (the A tile is re-read from L2), so that pass 1 of slot 0 runs under the MMAs of slot 1.  A
-  // single K loop feeding both slots (A read once, 40 KB stages) measured slower: out-proj 66 vs 56 us at D = 384.
-  static constexpr int kStages = NT == 1 ? 2 : EVT_ROWLN_STAGES2;
+  // single K loop feeding both slots (A read once, 40 KB stages) measured slower: out-proj 66 vs 56 us at D = 384, and so did
+  // four stages with a 4-deep residual ring (57 -> 65 us).
+  static constexpr int kStages = NT == 1 ? 2 : 3;
   static constexpr int kCopyBytes = COPY ? EW * kStgBytes : 0;  // f32 staging of the normalised rows (TF dialect)
   static constexpr int kVecBytes = 3 * kMaxD * 4;               // bias, gamma, beta
   static constexpr int kStatBytes = 2 * G * BM * 4;             // [sum | squares][column group][row]
@@ -83,8 +74,8 @@ struct CfgR {
   // multiple of G -- then an entry is only ever consumed by ONE group, and a consumer has seen round k-1 of an entry before
   // it waits for round k.  (A depth of 5 with two groups deadlocked: a group waiting for round 1 of an entry whose round 0 --
   // the other group's chunk -- had not landed yet passed its parity wait on the untouched barrier.)
-  static constexpr int kDepthWant = G == 4 ? 8 : (NT == 2 ? EVT_ROWLN_DEPTH2 : 6);
-  static constexpr int kDepthMin = G == 3 ? 3 : (NT == 2 && COPY ? EVT_ROWLN_DEPTHMIN_COPY2 : 4);
+  static constexpr int kDepthWant = G == 4 ? 8 : 6;
+  static constexpr int kDepthMin = G == 3 ? 3 : 4;
   static constexpr int kResDepth = (kFixed + EW * kXnStgBytes + kDepthWant * kResBytes <= kSmemLimit) ? kDepthWant : kDepthMin;
   // (the TF-dialect variant stores the f32 rows from a single staging tile in the same bulk group: one tile there too)
   static constexpr int kXnBufs = (!COPY && kFixed + kResDepth * kResBytes + 2 * EW * kXnStgBytes <= kSmemLimit) ? 2 : 1;
@@ -470,11 +461,6 @@ int launch_rowln(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorM
 }  // namespace
 
 bool gemm_rowln_supported(int64_t M, int N, int K, bool copy_ln) {
-  static const bool off = [] {
-    const char* e = getenv("EVT_FUSE_ROWLN");
-    return e != nullptr && atoi(e) == 0;
-  }();
-  if (off) return false;
   // whole rows in two 192-column accumulator slots; enough 256-row blocks to give every CTA pair one
   (void)copy_ln;
   return (N == kSlotCols || N == 2 * kSlotCols) && K >= 1 && M < (1ll << 31) - 256 &&
@@ -486,8 +472,7 @@ bool gemm_rowln_supported(int64_t M, int N, int K, bool copy_ln) {
 // epilogue: with a long K loop (HF DeiT-Small FC2, K = 1536: 104 us against 72 + 25 for the two kernels) the fusion loses; it
 // wins for the out-projection (56 against 41 + 25) and in the TF dialect, whose LayerNorm kernel also writes the f32 rows back.
 bool gemm_rowln_pays(int N, int K, bool copy_ln) {
-  static const bool always = getenv("EVT_ROWLN_ALWAYS") != nullptr && atoi(getenv("EVT_ROWLN_ALWAYS")) != 0;  // A/B timing
-  return always || N == kSlotCols || copy_ln || K <= 2 * kSlotCols;
+  return N == kSlotCols || copy_ln || K <= 2 * kSlotCols;
 }
 
 int gemm_rowln_launch(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias, float* resid, int64_t ldr,

@@ -2,8 +2,6 @@
 // mean then centred variance (exact for eps = 1e-12 as well as 1e-5), fp32 statistics.
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include "common.h"
 #include "ptx.cuh"
 
@@ -299,8 +297,7 @@ template <int OUT>
 int launch_rows(const float* x, long long xs, const float* g, const float* b, void* y, long long ys, float* yc,
                 long long rows, int D, float eps, cudaStream_t st) {
   // warps (= rows, or row groups) per block; 4 measured 2 % faster than 8 at 201 728 x 768 inside the forward
-  static const int wpb_env = getenv("EVT_LN_WPB") ? atoi(getenv("EVT_LN_WPB")) : 4;
-  const int wpb = wpb_env >= 1 && wpb_env <= 8 ? wpb_env : 4;
+  constexpr int wpb = 4;
   const unsigned grid = static_cast<unsigned>((rows + wpb - 1) / wpb);
   const bool fast = (D % 2 == 0) && D <= 64 * kMaxVec && (xs % 2 == 0) && (ys % 2 == 0) &&
                     (reinterpret_cast<uintptr_t>(x) % 8 == 0) && (reinterpret_cast<uintptr_t>(y) % 8 == 0) &&

@@ -509,15 +509,8 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
                                              0, 0, 0, rows, 192, pw.in_dim, EVT_ACT_NONE, st));
       // single_attn + attn_output + LayerNorm + MLP (transformer_encoder.py:67-99): the attention contraction's apply kernel carries
       // each tile through the tail, y = the performer's output rows
-      static const bool two_calls = getenv("EVT_T2T_TWO_CALLS") != nullptr;  // A/B only: performer + tail as separate kernels
-      if (two_calls) {
-        uint8_t* ya = w.t_x[i];  // the unfolded rows are dead once kqv exists: their buffer takes the attention output
-        EVT_TRY(performer_launch(w.t_kqv[i], 192, pw.w, ya, w.t_y[i], w.t_ws[i], batch, T, 64, 32, 1e-8f, st));
-        EVT_TRY(performer_mlp_launch(ya, w.t_y[i], pw.wo, pw.bo, pw.g2, pw.b2, pw.w1, pw.bb1, pw.w2, pw.bb2, rows, tf_eps, st));
-      } else {
-        EVT_TRY(performer_block_launch(w.t_kqv[i], 192, pw.w, w.t_y[i], w.t_ws[i], batch, T, 1e-8f, pw.wo, pw.bo, pw.g2, pw.b2, pw.w1,
-                                       pw.bb1, pw.w2, pw.bb2, tf_eps, st));
-      }
+      EVT_TRY(performer_block_launch(w.t_kqv[i], 192, pw.w, w.t_y[i], w.t_ws[i], batch, T, 1e-8f, pw.wo, pw.bo, pw.g2, pw.b2, pw.w1,
+                                     pw.bb1, pw.w2, pw.bb2, tf_eps, st));
       EVT_TRY(mark(EVT_STAGE_EMBED));
       src = w.t_y[i], src_dt = EVT_F32, side = so, ch = 64;
     }
@@ -546,37 +539,18 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
                                            EVT_ACT_NONE, st));
     EVT_STAGE(EVT_STAGE_EMBED, prefix_tokens_launch(m->prefix, m->pos, w.resid, batch, s.tokens, m->n_prefix, D, st));
   }
-  // encoder.  EXPERIMENTAL (EVT_FUSE_LN=1, off by default): with bf16 operands and the HF dataflow the LayerNorm that
-  // FOLLOWS each residual projection can run inside that GEMM's epilogue (gemm3.cu).  It is bit-identical on the residual
-  // stream but measured SLOWER on B200 (0.42 vs 0.22 ms for out-proj + LN at 100k rows): the second pass over the new
-  // residual does not stay in L2 (DRAM reads 750 MB vs 465 MB expected), so no traffic is saved -- see DESIGN.md.
-#ifdef EVT_EXPERIMENTAL
-  const bool fuse_ln = !tf32 && !tf && gemm_ln_fusion_enabled() && gemm_res_ln_supported(M, D, D) &&
-                       (M + 255) / 256 >= num_sms() / 2;
-#else
-  constexpr bool fuse_ln = false;  // gemm3.cu is only built with EVT_EXPERIMENTAL=1 (edgevisiontransformer_b200/build.py)
-#endif
-  // Narrow residual streams at large batch (D = 192 / 384: DeiT-Tiny / -Small, T2T): whole rows of a 256-row block fit in tensor
-  // memory, so the LayerNorm that FOLLOWS each residual projection runs in that projection's epilogue (gemm_rowln.cu): 5 launches
-  // per layer instead of 7 and the LayerNorm kernel's read of the f32 residual stream never happens.
-  const bool row_ln = !tf32 && !fuse_ln && gemm_rowln_supported(M, D, D, tf);  // per projection: gemm_rowln_pays
+  // encoder.  Narrow residual streams at large batch (D = 192 / 384: DeiT-Tiny / -Small, T2T): whole rows of a 256-row block
+  // fit in tensor memory, so the LayerNorm that FOLLOWS each residual projection runs in that projection's epilogue
+  // (gemm_rowln.cu): 5 launches per layer instead of 7 and the LayerNorm kernel's read of the f32 residual stream never happens.
+  const bool row_ln = !tf32 && gemm_rowln_supported(M, D, D, tf);  // per projection: gemm_rowln_pays
   bool xn_ready = false;  // w.xn already holds LN1 of the current layer (written by the previous layer's FC2 epilogue)
   for (int l = 0; l < s.layers; ++l) {
     const LayerW& lw = m->layers[l];
     const int a = lw.a;
-    // Narrow residual streams at large batch (D <= 384: DeiT-Tiny / -Small, T2T): the LayerNorm runs inside the projection
-    // that consumes it, as the producer of its A operand (gemm_ln.cu) -- 5 launches per layer instead of 7, and the bf16
-    // copy of the normalised rows never goes to HBM.
-    const bool ln_in_gemm = !tf32 && !fuse_ln && !row_ln && gemm_ln_supported(M, 3 * a, D);
-    if (ln_in_gemm) {
-      EVT_STAGE(EVT_STAGE_QKV, gemm_ln_launch(w.resid, D, lw.ln1_g, lw.ln1_b, s.eps, tf ? w.resid : nullptr, lw.wqkv, D, lw.bqkv, w.qkv,
-                                              3 * a, M, 3 * a, D, EVT_ACT_NONE, st));
-    } else {
-      if (!xn_ready)
-        EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln1_g, lw.ln1_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
-      EVT_STAGE(EVT_STAGE_QKV, gemm_launch(w.xn, D, lw.wqkv, D, dt, lw.bqkv, nullptr, 0, 0, 0, w.qkv, adt, 3 * a, 0, 0, 0, M, 3 * a, D,
-                          EVT_ACT_NONE, st));
-    }
+    if (!xn_ready)
+      EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln1_g, lw.ln1_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
+    EVT_STAGE(EVT_STAGE_QKV, gemm_launch(w.xn, D, lw.wqkv, D, dt, lw.bqkv, nullptr, 0, 0, 0, w.qkv, adt, 3 * a, 0, 0, 0, M, 3 * a, D,
+                        EVT_ACT_NONE, st));
     xn_ready = false;
     // head mask row of this layer (are_16_heads mask_heads) and, on request, the context written straight into the caller's
     // buffer (context_layer_val): the output projection then reads its A operand from there
@@ -589,33 +563,15 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
                                     batch, s.tokens, s.heads[l], s.head_size, scale, st));
     else
       EVT_STAGE(EVT_STAGE_ATTN, attention_launch(w.qkv, 3 * a, ctx, a, hmask, batch, s.tokens, s.heads[l], s.head_size, scale, st));
-#ifdef EVT_EXPERIMENTAL
-    if (fuse_ln) {
-      EVT_STAGE(EVT_STAGE_OPROJ, gemm_res_ln_launch(ctx, a, lw.wo, a, lw.bo, w.resid, D, lw.ln2_g, lw.ln2_b, s.eps, w.xn, D, M, D, a, st));
-    } else
-#endif
     if (row_ln && gemm_rowln_pays(D, a, tf)) {
       EVT_STAGE(EVT_STAGE_OPROJ, gemm_rowln_launch(ctx, a, lw.wo, a, lw.bo, w.resid, D, lw.ln2_g, lw.ln2_b, s.eps, tf, w.xn, D, M, D, a, st));
     } else {
       EVT_STAGE(EVT_STAGE_OPROJ, gemm_launch(ctx, a, lw.wo, a, dt, lw.bo, w.resid, D, 0, 0, w.resid, EVT_F32, D, 0, 0, 0, M, D, a,
                           EVT_ACT_NONE, st));
-      if (!ln_in_gemm)
-        EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln2_g, lw.ln2_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
+      EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln2_g, lw.ln2_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
     }
-    if (ln_in_gemm)
-      EVT_STAGE(EVT_STAGE_FC1, gemm_ln_launch(w.resid, D, lw.ln2_g, lw.ln2_b, s.eps, tf ? w.resid : nullptr, lw.w1, D, lw.b1, w.big,
-                                              lw.inter_ld, M, lw.inter, D, s.act, st));
-    else
-      EVT_STAGE(EVT_STAGE_FC1, gemm_launch(w.xn, D, lw.w1, D, dt, lw.b1, nullptr, 0, 0, 0, w.big, adt, lw.inter_ld, 0, 0, 0, M, lw.inter, D, s.act,
-                          st));
-#ifdef EVT_EXPERIMENTAL
-    if (fuse_ln && l + 1 < s.layers) {
-      const LayerW& nx = m->layers[l + 1];
-      EVT_STAGE(EVT_STAGE_FC2, gemm_res_ln_launch(w.big, lw.inter_ld, lw.w2, lw.inter_ld, lw.b2, w.resid, D, nx.ln1_g, nx.ln1_b, s.eps, w.xn, D,
-                                 M, D, lw.inter, st));
-      xn_ready = true;
-    } else
-#endif
+    EVT_STAGE(EVT_STAGE_FC1, gemm_launch(w.xn, D, lw.w1, D, dt, lw.b1, nullptr, 0, 0, 0, w.big, adt, lw.inter_ld, 0, 0, 0, M, lw.inter, D, s.act,
+                        st));
     if (row_ln && l + 1 < s.layers && gemm_rowln_pays(D, lw.inter, tf)) {
       const LayerW& nx = m->layers[l + 1];
       EVT_STAGE(EVT_STAGE_FC2, gemm_rowln_launch(w.big, lw.inter_ld, lw.w2, lw.inter_ld, lw.b2, w.resid, D, nx.ln1_g, nx.ln1_b, s.eps, tf, w.xn,
@@ -724,9 +680,8 @@ extern "C" int evt_gemm_residual_layernorm_ex(const void* A, int64_t lda, const 
   return layernorm_launch(resid, ldr, gamma, beta, xn, EVT_BF16, ldxn, copy_ln ? resid : nullptr, M, N, eps, st);
 }
 
-#ifndef EVT_EXPERIMENTAL
-// The single-kernel version (gemm3.cu) measured slower than the two kernels it replaces (DESIGN.md, negative results) and is
-// only built with EVT_EXPERIMENTAL=1; the entry point keeps its contract by issuing those two kernels.
+// A single-kernel version measured slower than the two kernels it replaces (DESIGN.md, negative results): the entry point
+// issues those two kernels.
 extern "C" int evt_gemm_residual_layernorm(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias, float* resid,
                                            int64_t ldr, const float* gamma, const float* beta, float eps, void* xn, int64_t ldxn,
                                            int64_t M, int N, int K, evt_stream stream) {
@@ -736,4 +691,3 @@ extern "C" int evt_gemm_residual_layernorm(const void* A, int64_t lda, const voi
   if (N % 64 != 0 || N < 64 || N > 1024) return fail(EVT_ERR_UNSUPPORTED, "gemm+ln: N must be a multiple of 64 in [64, 1024]");
   return evt_gemm_residual_layernorm_ex(A, lda, W, ldw, bias, resid, ldr, gamma, beta, eps, 0, xn, ldxn, M, N, K, stream);
 }
-#endif

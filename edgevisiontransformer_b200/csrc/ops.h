@@ -9,24 +9,14 @@ int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_d
                 int64_t ldo, int out_group, int out_group_stride, int out_group_off, int64_t M, int N, int K, int act,
                 cudaStream_t stream);
 
-// x <- x + A W^T + bias (f32 residual stream, in place) and xn <- LayerNorm(x) gamma + beta (bf16), one kernel (gemm3.cu)
-bool gemm_res_ln_supported(int64_t M, int N, int K);
-int gemm_res_ln_launch(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias, float* resid, int64_t ldr,
-                       const float* gamma, const float* beta, float eps, void* xn, int64_t ldxn, int64_t M, int N, int K,
-                       cudaStream_t stream);
-
-// The same for row lengths 192 / 384 with whole rows resident in tensor memory (gemm_rowln.cu); copy_ln: the residual stream
-// receives the normalised rows (TF dialect).  Supported = large M only (every CTA pair gets a 256-row block).
+// x <- x + A W^T + bias (f32 residual stream, in place) and xn <- LayerNorm(x) gamma + beta (bf16) for row lengths 192 / 384,
+// with whole rows resident in tensor memory (gemm_rowln.cu); copy_ln: the residual stream receives the normalised rows (TF
+// dialect).  Supported = large M only (every CTA pair gets a 256-row block).
 bool gemm_rowln_supported(int64_t M, int N, int K, bool copy_ln);
 bool gemm_rowln_pays(int N, int K, bool copy_ln);  // model runtime: the fused kernel beats GEMM + LayerNorm for this projection
 int gemm_rowln_launch(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias, float* resid, int64_t ldr,
                       const float* gamma, const float* beta, float eps, bool copy_ln, void* xn, int64_t ldxn, int64_t M, int N,
                       int K, cudaStream_t stream);
-
-// LayerNorm fused into the A-operand producer of the following projection (gemm_ln.cu); K = D in {64,128,192,256,384}
-bool gemm_ln_supported(int64_t M, int N, int K);
-int gemm_ln_launch(const float* x, int64_t ldx, const float* gamma, const float* beta, float eps, float* x_copy, const void* W,
-                   int64_t ldw, const float* bias, void* out, int64_t ldo, int64_t M, int N, int K, int act, cudaStream_t stream);
 
 int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S,
                      int heads, int head_size, float scale, cudaStream_t stream);

@@ -79,9 +79,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 // handful of instructions per microsecond instead of spinning (the default time limit is ~100 cycles: the round-2
 // attention profile showed 21 retries per wait, 15 % of all issued instructions, competing with the other softmax group
 // for the sub-partition's issue slots).
-#ifndef EVT_MBAR_SUSPEND_NS
-#define EVT_MBAR_SUSPEND_NS 2000
-#endif
+constexpr uint32_t kMbarSuspendNs = 2000;
 __device__ __forceinline__ bool mbar_try_wait_hint(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -89,7 +87,7 @@ __device__ __forceinline__ bool mbar_try_wait_hint(uint64_t* bar, uint32_t parit
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
       "selp.b32 %0, 1, 0, p;\n\t}\n"
       : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"(static_cast<uint32_t>(EVT_MBAR_SUSPEND_NS))
+      : "r"(smem_u32(bar)), "r"(parity), "r"(kMbarSuspendNs)
       : "memory");
   return ok != 0;
 }

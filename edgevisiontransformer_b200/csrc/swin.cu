@@ -14,13 +14,11 @@
 //                             (window, head): q, k, v staged with cp.async into swizzled shared memory, mma.sync
 //                             m16n8k16 bf16 with the probabilities kept in registers (accumulator fragments re-used as A
 //                             fragments).  A 49 x 49 x 32 problem fills 38 % of a 128-row tcgen05 tile and its time is
-//                             exp / load bound, so the warp-level tensor path is used here; packing two windows per
-//                             tcgen05 tile is the follow-up.
+//                             exp / load bound, so the warp-level tensor path is used here (a tcgen05 kernel with two
+//                             windows per tile was measured slower, DESIGN.md).
 //   ln_mean_tokens_kernel     final LayerNorm + average pool over the tokens of an image (SwinModel.layernorm + pooler).
 #include <cuda_bf16.h>
 #include <math_constants.h>
-
-#include <cstdlib>
 
 #include "common.h"
 #include "ptx.cuh"
@@ -352,274 +350,6 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
   }
 }
 
-// ---------------------------------------------------------------------------------------------------- window attention, tcgen05
-// EXPERIMENTAL (built with EVT_EXPERIMENTAL=1, selected with EVT_SWIN_ATTN_TC=1): correct -- the Swin op and model parity
-// tests pass with it -- but SLOWER than the warp-level kernel above on B200: Swin-T batch 256 37.2 k img/s (34.4 k with the
-// table row prefetched ahead of the S wait: more spills) against 40.4 k.  Two CTAs per SM leave 168 registers per thread for a
-// row-per-thread softmax that wants 56 scores + 56 table values + 32 packed probabilities live (100-330 bytes of spills), and
-// each head is a serial QK -> softmax -> PV -> read-out chain with a barrier round trip between the steps; the mma.sync kernel
-// keeps a whole (window, head) in one warp's registers with no hand-offs.  A 49 x 49 x 32 problem is too small for the
-// tcgen05 hand-off latencies to amortise.
-#ifdef EVT_EXPERIMENTAL
-// Two 49-token windows share one 128-row tcgen05 tile (window 0 in TMEM lanes / key columns 0..48, window 1 in
-// 64..112): S = Q K^T is ONE M = 128, N = 128 MMA pair per head whose off-diagonal 64 x 64 blocks are simply never read,
-// P (bf16, written back into TMEM over the consumed scores) is block-diagonal by construction -- zeros outside the row's
-// own window -- so O = P V over all 128 key rows is exact.  Two heads (2 x 32 columns = one 128-byte row) share the Q / K / V
-// tiles; the head is selected by the K offset of the operand descriptors.
-//   work item         (window pair, head pair); persistent CTAs, TWO per SM (256 TMEM columns and ~113 KB of shared memory
-//                     each), so one CTA's serial chain QK -> softmax -> PV -> read-out overlaps the other's
-//   warp 4 (1 thread) TMA producer: Q, K, V as two 64-row boxes each (one per window) into a 2-deep ring
-//   warp 5 (1 thread) MMA issuer
-//   warps 0-3         thread = query row: scores * scale + (relative position bias + shift mask) table, max, exp2, bf16 P,
-//                     sum; then O / sum -> bf16 into a 128B-swizzled staging tile; one 49-row TMA store per window
-constexpr int kTcStages = 2;
-constexpr int kTcTile = 128 * 128;               // one operand tile: 128 rows x 64 bf16
-constexpr int kTcStageBytes = 3 * kTcTile;       // Q | K | V
-constexpr int kTcStgBytes = (56 + kWTok) * 128;  // staging: window 0 at row 0, window 1 at row 56 (1024-byte aligned)
-constexpr int kTcThreads = 192;
-constexpr int kTcSCols = 128, kTcOCol = 128, kTcTmemCols = 256;
-
-struct WinTcParams {
-  const float* tab;
-  long long n_windows, n_items;
-  int n_tab, heads, hp_count;
-  float scale_log2e;
-};
-
-__global__ void __launch_bounds__(kTcThreads, 2)
-window_attention_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ CUtensorMap tmOut, const WinTcParams p) {
-  extern __shared__ uint8_t tc_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tc_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* staging = smem + kTcStages * kTcStageBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kTcStgBytes);
-  uint64_t* full = bars;            // [2] producer -> issuer
-  uint64_t* empty = bars + 2;       // [2] issuer (commit after the item's last PV) -> producer
-  uint64_t* s_ready = bars + 4;     // issuer (commit) -> softmax warps
-  uint64_t* p_ready = bars + 5;     // softmax warps (4 arrivals) -> issuer
-  uint64_t* o_ready = bars + 6;     // issuer (commit) -> softmax warps
-  uint64_t* slot_free = bars + 7;   // softmax warps (4 arrivals): O read out, the slot may take the next S
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 8);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int C = p.heads * kWHd;
-  const long long my_items = (p.n_items - static_cast<long long>(blockIdx.x) + gridDim.x - 1) / gridDim.x;
-
-  if (warp == 4 && ptx::elect_one()) {
-    ptx::prefetch_tmap(&tmIn);
-    ptx::prefetch_tmap(&tmOut);
-    for (int s = 0; s < 2; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    ptx::mbar_init(s_ready, 1);
-    ptx::mbar_init(p_ready, 4);
-    ptx::mbar_init(o_ready, 1);
-    ptx::mbar_init(slot_free, 4);
-    ptx::fence_mbar_init();
-  }
-  if (warp == 5) ptx::tmem_alloc<kTcTmemCols>(tmem_ptr);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  ptx::grid_dep_launch();
-  ptx::grid_dep_wait();
-
-  if (warp == 4) {
-    if (ptx::elect_one()) {
-      int st = 0;
-      uint32_t ph = 0;
-      for (long long it = 0; it < my_items; ++it) {
-        const long long item = blockIdx.x + it * gridDim.x;
-        const long long wp = item / p.hp_count;
-        const int hp = static_cast<int>(item - wp * p.hp_count);
-        ptx::mbar_wait(&empty[st], ph ^ 1);
-        uint8_t* base = smem + st * kTcStageBytes;
-        ptx::mbar_arrive_expect_tx(&full[st], kTcStageBytes);
-        for (int wi = 0; wi < 2; ++wi) {
-          const long long row = (2 * wp + wi) * kWTok;   // a window past the end loads zeros (rows out of range)
-          const int r = row < 0x7fffffffll ? static_cast<int>(row) : 0x7fffffff;
-          for (int m = 0; m < 3; ++m)
-            ptx::tma_load_2d(base + m * kTcTile + wi * (kTcTile / 2), &tmIn, &full[st], m * C + hp * 64, r);
-        }
-        if (++st == kTcStages) {
-          st = 0;
-          ph ^= 1;
-        }
-      }
-    }
-  } else if (warp == 5) {
-    if (ptx::elect_one()) {
-      constexpr uint32_t idesc_qk = ptx::make_idesc(128, 128, 1, 0, 0);
-      constexpr uint32_t idesc_pv = ptx::make_idesc(128, 64, 1, 0, 1);
-      int st = 0;
-      uint32_t ph = 0, hph = 0;  // hph: phase of the per-head barriers (one completion per head processed)
-      for (long long it = 0; it < my_items; ++it) {
-        const long long item = blockIdx.x + it * gridDim.x;
-        const int hp = static_cast<int>(item % p.hp_count);
-        const int nh = p.heads - 2 * hp < 2 ? p.heads - 2 * hp : 2;
-        ptx::mbar_wait(&full[st], ph);
-        const uint32_t sq = ptx::smem_u32(smem + st * kTcStageBytes);
-        const uint64_t qd = ptx::smem_desc_sw128(sq), kd = ptx::smem_desc_sw128(sq + kTcTile), vd = ptx::smem_desc_sw128(sq + 2 * kTcTile);
-        for (int hl = 0; hl < nh; ++hl) {
-          ptx::mbar_wait(slot_free, hph ^ 1);
-          ptx::tc_fence_after();
-#pragma unroll
-          for (int k = 0; k < 2; ++k)  // head hl = K offsets 32 hl .. 32 hl + 31 of the 64-column tiles
-            ptx::mma_f16_ss(tmem_base, qd + 2 * (2 * hl + k), kd + 2 * (2 * hl + k), idesc_qk, k != 0 ? 1u : 0u);
-          ptx::mma_commit(s_ready);
-          ptx::mbar_wait(p_ready, hph);
-          ptx::tc_fence_after();
-#pragma unroll
-          for (int k = 0; k < 8; ++k)  // 16 keys per step: 8 TMEM columns of P, 2048 bytes of V (MN-major)
-            ptx::mma_f16_ts(tmem_base + kTcOCol, tmem_base + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, k != 0 ? 1u : 0u);
-          ptx::mma_commit(o_ready);
-          if (hl == nh - 1) ptx::mma_commit(&empty[st]);
-          hph ^= 1;
-        }
-        if (++st == kTcStages) {
-          st = 0;
-          ph ^= 1;
-        }
-      }
-    }
-  } else {
-    const int r = threadIdx.x;                 // query row of the tile = TMEM lane
-    const int wi = r >> 6, i = r & 63;         // window of the pair, token in the window
-    const uint32_t t_row = tmem_base + (static_cast<uint32_t>(warp * 32) << 16);
-    uint8_t* stg_row = staging + (wi * 56 + i) * 128;
-    const int sw = (wi * 56 + i) & 7;
-    uint32_t hph = 0;
-    for (long long it = 0; it < my_items; ++it) {
-      const long long item = blockIdx.x + it * gridDim.x;
-      const long long wp = item / p.hp_count;
-      const int hp = static_cast<int>(item - wp * p.hp_count);
-      const int nh = p.heads - 2 * hp < 2 ? p.heads - 2 * hp : 2;
-      const long long w = 2 * wp + wi;
-      const bool live = i < kWTok && w < p.n_windows;
-      // tcgen05.ld / .st are warp-collective (.sync.aligned): they are issued under the warp-uniform condition and the rows
-      // past a window's 49 tokens (lanes 17..31 of warps 1 and 3) only discard what they loaded
-      const bool warp_live = w < p.n_windows;
-      for (int hl = 0; hl < nh; ++hl) {
-        const int h = 2 * hp + hl;
-        const float* tb = p.tab + (((w % p.n_tab) * p.heads + h) * static_cast<long long>(kWRows) + i) * kWKeyCols;
-        // the row of the (bias + mask) table is requested BEFORE the wait for S = Q K^T: its L2 latency hides behind the MMA
-        float t[kWKeyCols];
-        if (live) {
-#pragma unroll
-          for (int j = 0; j < kWKeyCols; j += 4) {
-            const float4 bv = __ldg(reinterpret_cast<const float4*>(tb + j));
-            t[j] = bv.x, t[j + 1] = bv.y, t[j + 2] = bv.z, t[j + 3] = bv.w;
-          }
-        }
-        ptx::mbar_wait(s_ready, hph);
-        ptx::tc_fence_after();
-        float sum = 1.f;
-        uint32_t pk[32];   // this row's 64 keys as bf16 pairs (keys >= 56 and masked keys: 0)
-#pragma unroll
-        for (int j = 0; j < 32; ++j) pk[j] = 0u;
-        uint32_t sc[64];
-        if (warp_live) {
-          uint32_t a[32], b[32];
-          ptx::tmem_ld_x32(t_row + wi * 64, a);
-          ptx::tmem_ld_x32(t_row + wi * 64 + 32, b);
-          ptx::tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j) sc[j] = a[j], sc[32 + j] = b[j];
-        }
-        if (live) {
-          float m = -CUDART_INF_F;
-#pragma unroll
-          for (int j = 0; j < kWKeyCols; j += 4) {
-            t[j] = fmaf(__uint_as_float(sc[j]), p.scale_log2e, t[j]);
-            t[j + 1] = fmaf(__uint_as_float(sc[j + 1]), p.scale_log2e, t[j + 1]);
-            t[j + 2] = fmaf(__uint_as_float(sc[j + 2]), p.scale_log2e, t[j + 2]);
-            t[j + 3] = fmaf(__uint_as_float(sc[j + 3]), p.scale_log2e, t[j + 3]);
-            m = fmaxf(fmaxf(m, fmaxf(t[j], t[j + 1])), fmaxf(t[j + 2], t[j + 3]));
-          }
-          float l = 0.f;
-#pragma unroll
-          for (int j = 0; j < kWKeyCols; j += 2) {
-            const float p0 = ex2f(t[j] - m), p1 = ex2f(t[j + 1] - m);   // masked keys: 2^-inf = 0
-            l += p0 + p1;
-            pk[j >> 1] = pack_bf16(p0, p1);
-          }
-          sum = l;
-        }
-        // block-diagonal P: window wi's keys live in columns 32 wi .. 32 wi + 31 of the packed row, zeros elsewhere
-        {
-          uint32_t z[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j) z[j] = 0u;
-          uint32_t lo[16], hi[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j) lo[j] = pk[j], hi[j] = pk[16 + j];
-          if (wi == 0) {
-            ptx::tmem_st_x16(t_row, lo);
-            ptx::tmem_st_x16(t_row + 16, hi);
-            ptx::tmem_st_x16(t_row + 32, z);
-            ptx::tmem_st_x16(t_row + 48, z);
-          } else {
-            ptx::tmem_st_x16(t_row, z);
-            ptx::tmem_st_x16(t_row + 16, z);
-            ptx::tmem_st_x16(t_row + 32, lo);
-            ptx::tmem_st_x16(t_row + 48, hi);
-          }
-        }
-        ptx::tmem_st_wait();
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(p_ready);
-        const float inv = 1.0f / sum;   // sum >= 1: the row maximum contributes 2^0
-        ptx::mbar_wait(o_ready, hph);
-        ptx::tc_fence_after();
-        uint32_t o[32];
-        if (warp_live) {
-          ptx::tmem_ld_x32(t_row + kTcOCol + 32 * hl, o);   // O holds both heads' dims; this head's are columns 32 hl ..
-          ptx::tmem_ld_wait();
-        }
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(slot_free);
-        if (hl == 0 && it > 0) {  // the previous item's TMA stores have read the staging tile (long ago): safe to rewrite it
-          if (warp == 0 && ptx::elect_one()) ptx::bulk_wait_read<0>();
-          asm volatile("bar.sync 1, 128;" ::: "memory");
-        }
-        if (live) {
-#pragma unroll
-          for (int c4 = 0; c4 < 4; ++c4) {
-            uint4 v;
-            v.x = pack_bf16(__uint_as_float(o[8 * c4]) * inv, __uint_as_float(o[8 * c4 + 1]) * inv);
-            v.y = pack_bf16(__uint_as_float(o[8 * c4 + 2]) * inv, __uint_as_float(o[8 * c4 + 3]) * inv);
-            v.z = pack_bf16(__uint_as_float(o[8 * c4 + 4]) * inv, __uint_as_float(o[8 * c4 + 5]) * inv);
-            v.w = pack_bf16(__uint_as_float(o[8 * c4 + 6]) * inv, __uint_as_float(o[8 * c4 + 7]) * inv);
-            *reinterpret_cast<uint4*>(stg_row + (((4 * hl + c4) ^ sw) << 4)) = v;
-          }
-        }
-        hph ^= 1;
-      }
-      // both heads of the pair are staged: one 49-row store per window (columns past C are clipped by the tensor map)
-      ptx::fence_proxy_async_smem();
-      asm volatile("bar.sync 1, 128;" ::: "memory");
-      if (warp == 0 && ptx::elect_one()) {
-        const long long w0 = 2 * wp;
-        ptx::tma_store_2d(&tmOut, staging, hp * 64, static_cast<int>(w0 * kWTok));
-        if (w0 + 1 < p.n_windows) ptx::tma_store_2d(&tmOut, staging + 56 * 128, hp * 64, static_cast<int>((w0 + 1) * kWTok));
-        ptx::bulk_commit();
-      }
-    }
-    if (warp == 0 && ptx::elect_one()) ptx::bulk_wait<0>();
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 5) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc<kTcTmemCols>(tmem_base);
-  }
-}
-
-#endif  // EVT_EXPERIMENTAL
-
 // ---------------------------------------------------------------------------------------------------- final LN + pool
 // One CTA (8 warps) per image: every warp normalises tokens warp, warp + 8, ... and accumulates them; the warps' sums meet
 // in shared memory.  D % 4 == 0, D <= 128 * NV.
@@ -758,39 +488,6 @@ extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx,
   EVT_CHECK_ARG(ldq >= 3ll * heads * kWHd && ldc >= static_cast<int64_t>(heads) * kWHd, "window_attention: leading dimension too small");
   EVT_CHECK_ARG(ldq % 8 == 0 && reinterpret_cast<uintptr_t>(qkv) % 16 == 0, "window_attention: qkv rows must be 16-byte aligned");
   EVT_CHECK_ARG(ldc % 2 == 0 && reinterpret_cast<uintptr_t>(ctx) % 4 == 0, "window_attention: ctx rows must be 4-byte aligned");
-#ifdef EVT_EXPERIMENTAL
-  static const bool tc_on = getenv("EVT_SWIN_ATTN_TC") != nullptr && atoi(getenv("EVT_SWIN_ATTN_TC")) != 0;  // A/B timing
-  if (tc_on && ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0 && n_windows * kWTok < (1ll << 31) - 256) {
-    const int C = heads * kWHd;
-    CUtensorMap tmIn, tmOut;
-    rc = make_tmap_2d(&tmIn, qkv, 2, static_cast<uint64_t>(n_windows) * kWTok, 3ull * C, static_cast<uint64_t>(ldq), 64, 64);
-    if (rc != EVT_OK) return rc;
-    rc = make_tmap_2d(&tmOut, ctx, 2, static_cast<uint64_t>(n_windows) * kWTok, static_cast<uint64_t>(C), static_cast<uint64_t>(ldc), kWTok, 64);
-    if (rc != EVT_OK) return rc;
-    WinTcParams q;
-    q.tab = table;
-    q.n_windows = n_windows;
-    q.n_tab = n_tab;
-    q.heads = heads;
-    q.hp_count = (heads + 1) / 2;
-    q.n_items = ((n_windows + 1) / 2) * q.hp_count;
-    q.scale_log2e = scale * 1.4426950408889634f;
-    const int smem_tc = 1024 + kTcStages * kTcStageBytes + kTcStgBytes + 128;
-    static int tc_dev = -1;
-    int dev_tc = 0;
-    EVT_CUDA(cudaGetDevice(&dev_tc));
-    if (tc_dev != dev_tc) {
-      EVT_CUDA(cudaFuncSetAttribute(window_attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc));
-      tc_dev = dev_tc;
-    }
-    const long long cap_tc = 2ll * num_sms();
-    const unsigned grid_tc = static_cast<unsigned>(q.n_items < cap_tc ? q.n_items : cap_tc);
-    EVT_CUDA(launch_pdl(window_attention_tc_kernel, dim3(grid_tc), dim3(kTcThreads), smem_tc, static_cast<cudaStream_t>(stream),
-                        pdl_for_work(n_windows * kWTok, static_cast<long long>(heads) * kWHd), tmIn, tmOut, q));
-    EVT_LAUNCH_CHECK("window_attention_tc_kernel");
-    return EVT_OK;
-  }
-#endif  // EVT_EXPERIMENTAL
   const long long items = n_windows * heads;
   const int smem = kWWarps * 3 * kWMatBytes;
   static int configured_dev = -1;

@@ -64,8 +64,8 @@ void evt_gemm_set_pair_mode(int mode);
  * reduce-adds whose order is not fixed, so with splitting on (the default) small-batch bf16 results can differ from run
  * to run and from one batch size to another by a last-bit f32 difference in the residual stream (which bf16 roundings
  * downstream turn into logit differences of a few 1e-3, inside the 2e-2 parity budget); 0 turns it off (bit-reproducible,
- * batch-invariant results).  Large batches never split, and the tf32 accuracy mode only with EVT_TF32_SPLIT_K=1 in the
- * environment (DeiT-Tiny batch 1 0.48 -> 0.43 ms, but the logit error stops being reproducible: 7.5e-4 -> 9.2e-4 of the 1e-3 budget).
+ * batch-invariant results).  Large batches never split, and neither does the tf32 accuracy mode (splitting would take
+ * DeiT-Tiny batch 1 from 0.48 to 0.43 ms, but the logit error would stop being reproducible: 7.5e-4 -> 9.2e-4 of the 1e-3 budget).
  * Initial value: environment variable EVT_GEMM_SPLIT_K if set, else 1. */
 void evt_gemm_set_split_k(int enable);
 /* Promise, for the evt_gemm_bias_act* calls the calling thread makes while the count is positive, that W is a weight matrix:

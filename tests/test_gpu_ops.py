@@ -155,7 +155,7 @@ def test_gemm_residual_layernorm_fused(M, N, K):
     unfused = res0.clone()
     try:
         # Deterministic accumulation order on both sides: by default the entry point issues the residual GEMM and the
-        # LayerNorm kernel (the single-kernel version is an EVT_EXPERIMENTAL build option), and a small-M residual GEMM
+        # LayerNorm kernel (a single-kernel version lost its A/B test and was removed), and a small-M residual GEMM
         # splits K over idle SMs, whose reduce-adds land in any order.
         ops.set_gemm_split_k(False)
         xn = ops.linear_residual_layernorm(a, w, bias, res, gamma, beta, eps, k=K)
