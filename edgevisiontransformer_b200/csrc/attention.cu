@@ -706,8 +706,6 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   const long long units = n_pairs * (q_tiles / n_mt);
   const int grid = units < num_sms() ? static_cast<int>(units) : num_sms();
   const bool pdl = pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * kHD);
-  int dev = 0;
-  EVT_CUDA(cudaGetDevice(&dev));
   CUtensorMap tmKV;
   int rc = make_tmap_2d(&tmKV, qkv, 2, rows, 3ull * heads * kHD, static_cast<uint64_t>(ldq), SK, kHD);
   if (rc != EVT_OK) return rc;
@@ -733,11 +731,7 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   if (n_kv < 2) return fail(EVT_ERR_UNSUPPORTED, "attention: sequence too long for two K/V stages");
   q.n_kv = n_kv;
   const int smem2 = fixed + n_kv * 2 * SK * 128;
-  static int dev2 = -1;
-  if (dev2 != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    dev2 = dev;
-  }
+  EVT_TRY(opt_in_smem<attention2_kernel>(max_smem));
   EVT_CUDA(launch_pdl(attention2_kernel, dim3(grid), dim3(kThreads2), smem2, stream, pdl, tmQ, tmKV, tmO, q));
   EVT_LAUNCH_CHECK("attention2_kernel");
   return EVT_OK;
@@ -771,14 +765,7 @@ int attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc
   p.heads = heads;
   p.scale_log2e = scale * 1.4426950408889634f;
   const int smem = 1024 + 2 * kQRows * 128 + 2 * SK * 128 + (SK / 32) * 8192 + 64;
-  static int configured_dev = -1;
-  int dev = 0;
-  EVT_CUDA(cudaGetDevice(&dev));
-  if (configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(attention_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  1024 + 2 * kQRows * 128 + 2 * 256 * 128 + 8 * 8192 + 64));
-    configured_dev = dev;
-  }
+  EVT_TRY(opt_in_smem<attention_tf32_kernel>(1024 + 2 * kQRows * 128 + 2 * 256 * 128 + 8 * 8192 + 64));
   dim3 grid((S + kQRows - 1) / kQRows, heads, B);
   EVT_CUDA(launch_pdl(attention_tf32_kernel, grid, dim3(kAttnThreads), smem, stream, pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * kHD), tmQ, tmKV, p));
   EVT_LAUNCH_CHECK("attention_tf32_kernel");

@@ -85,66 +85,51 @@ static std::atomic<int> g_split_k{[] {
 bool gemm_split_k_enabled() { return g_split_k.load(std::memory_order_relaxed) != 0; }
 int gemm_pair_mode() { return g_pair_mode.load(std::memory_order_relaxed); }
 
-int make_tmap_2d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t rows, uint64_t cols, uint64_t ld,
-                 uint32_t box_rows, uint32_t box_cols) {
+// What the three map shapes share: the entry point, the alignment checks, the shape's own box check (`box_error`: null when the
+// box is valid), then the encode.  A box is box_rows x box_cols of one batch entry (rank 3) or of the whole matrix (rank 2).
+static int encode_tmap(CUtensorMap* out, const void* base, int elem_bytes, int rank, uint64_t cols, uint64_t rows, uint64_t batch,
+                       uint64_t ld, uint32_t box_rows, uint32_t box_cols, int swizzle_bytes, const char* box_error, const char* what) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(EVT_ERR_INVALID, "TMA base pointer not 16-byte aligned");
   if ((ld * elem_bytes) % 16 != 0) return fail(EVT_ERR_INVALID, "TMA leading dimension not a multiple of 16 bytes");
-  if (box_cols * elem_bytes != 128 || box_rows > 256 || box_rows == 0)
-    return fail(EVT_ERR_INVALID, "TMA box must be 128 bytes wide and at most 256 rows");
-  CUtensorMapDataType dt;
-  if (elem_bytes == 2) dt = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-  else if (elem_bytes == 4) dt = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-  else return fail(EVT_ERR_INVALID, "TMA element size must be 2 or 4");
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * static_cast<uint64_t>(elem_bytes)};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(out, dt, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
+  if (box_error) return fail(EVT_ERR_INVALID, box_error);
+  const cuuint64_t dims[3] = {cols, rows, batch};
+  const cuuint64_t strides[2] = {ld * static_cast<uint64_t>(elem_bytes), rows * ld * static_cast<uint64_t>(elem_bytes)};
+  const cuuint32_t box[3] = {box_cols, box_rows, 1};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = enc(out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, const_cast<void*>(base),
+                   dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(EVT_ERR_CUDA, std::string("cuTensorMapEncodeTiled") + what + " failed with CUresult " + std::to_string((int)r));
   return EVT_OK;
+}
+
+static const char* box_128_error(int elem_bytes, uint32_t box_rows, uint32_t box_cols) {
+  return box_cols * elem_bytes != 128 || box_rows > 256 || box_rows == 0 ? "TMA box must be 128 bytes wide and at most 256 rows" : nullptr;
+}
+
+int make_tmap_2d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t rows, uint64_t cols, uint64_t ld,
+                 uint32_t box_rows, uint32_t box_cols) {
+  const char* err = box_128_error(elem_bytes, box_rows, box_cols);
+  if (!err && elem_bytes != 2 && elem_bytes != 4) err = "TMA element size must be 2 or 4";
+  return encode_tmap(out, base, elem_bytes, 2, cols, rows, 1, ld, box_rows, box_cols, 128, err, "");
 }
 
 int make_tmap_2d_sw(CUtensorMap* out, const void* base, int elem_bytes, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows,
                     uint32_t box_cols, int swizzle_bytes) {
   if (swizzle_bytes == 128) return make_tmap_2d(out, base, elem_bytes, rows, cols, ld, box_rows, box_cols);
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(EVT_ERR_INVALID, "TMA base pointer not 16-byte aligned");
-  if ((ld * elem_bytes) % 16 != 0) return fail(EVT_ERR_INVALID, "TMA leading dimension not a multiple of 16 bytes");
-  if (swizzle_bytes != 64 || box_cols * elem_bytes != 64 || box_rows > 256 || box_rows == 0 || (elem_bytes != 2 && elem_bytes != 4))
-    return fail(EVT_ERR_INVALID, "TMA box must be as wide as its swizzle span (64 or 128 bytes) and at most 256 rows");
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * static_cast<uint64_t>(elem_bytes)};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
-                   const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled (64B swizzle) failed with CUresult " + std::to_string((int)r));
-  return EVT_OK;
+  const bool ok = swizzle_bytes == 64 && box_cols * elem_bytes == 64 && box_rows <= 256 && box_rows != 0 && (elem_bytes == 2 || elem_bytes == 4);
+  return encode_tmap(out, base, elem_bytes, 2, cols, rows, 1, ld, box_rows, box_cols, 64,
+                     ok ? nullptr : "TMA box must be as wide as its swizzle span (64 or 128 bytes) and at most 256 rows", " (64B swizzle)");
 }
 
 int make_tmap_3d_rows(CUtensorMap* out, const void* base, int elem_bytes, uint64_t cols, uint64_t rows, uint64_t batch,
                       uint64_t ld, uint32_t box_rows, uint32_t box_cols) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(EVT_ERR_INVALID, "TMA base pointer not 16-byte aligned");
-  if ((ld * elem_bytes) % 16 != 0) return fail(EVT_ERR_INVALID, "TMA leading dimension not a multiple of 16 bytes");
-  if (box_cols * elem_bytes != 128 || box_rows > 256 || box_rows == 0)
-    return fail(EVT_ERR_INVALID, "TMA box must be 128 bytes wide and at most 256 rows");
-  if (elem_bytes != 2) return fail(EVT_ERR_INVALID, "3-D TMA map: bf16 only");
-  cuuint64_t dims[3] = {cols, rows, batch};
-  cuuint64_t strides[2] = {ld * static_cast<uint64_t>(elem_bytes), rows * ld * static_cast<uint64_t>(elem_bytes)};
-  cuuint32_t box[3] = {box_cols, box_rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled (3-D) failed with CUresult " + std::to_string((int)r));
-  return EVT_OK;
+  const char* err = box_128_error(elem_bytes, box_rows, box_cols);
+  if (!err && elem_bytes != 2) err = "3-D TMA map: bf16 only";
+  return encode_tmap(out, base, elem_bytes, 3, cols, rows, batch, ld, box_rows, box_cols, 128, err, " (3-D)");
 }
 
 }  // namespace evt

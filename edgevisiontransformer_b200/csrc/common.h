@@ -36,6 +36,51 @@ void count_launch(int n = 1);
     ::evt::count_launch();                                                                               \
   } while (0)
 
+// Return the status of a call that failed.
+#define EVT_TRY(expr)                     \
+  do {                                    \
+    const int _rc = (expr);               \
+    if (_rc != EVT_OK) return _rc;        \
+  } while (0)
+
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Lays out a workspace: consecutive regions, each starting on a 1 KiB boundary.  A null base only sizes the plan.
+struct WorkspaceCarver {
+  uint8_t* base;
+  size_t bytes = 0;
+  template <typename T = uint8_t>
+  T* take(size_t n) {
+    T* p = reinterpret_cast<T*>(base + bytes);
+    bytes = align_up(bytes + n, 1024);
+    return p;
+  }
+};
+
+// Places a workspace plan (a callable from the 1 KiB-aligned base to a struct with `bytes`) on the caller's buffer, rounded up
+// to 1 KiB: the *_workspace_bytes queries add 1 KiB of slack for that.
+template <typename Plan>
+int place_workspace(void* workspace, size_t workspace_bytes, const Plan& plan, decltype(plan(nullptr))* out, const char* too_small) {
+  uint8_t* base = reinterpret_cast<uint8_t*>(align_up(reinterpret_cast<uintptr_t>(workspace), 1024));
+  *out = plan(base);
+  EVT_CHECK_ARG(out->bytes + (base - static_cast<uint8_t*>(workspace)) <= workspace_bytes, too_small);
+  return EVT_OK;
+}
+
+// Lets `Kernel` use `bytes` of dynamic shared memory, once per device.  The cache is keyed by the kernel pointer, not its type:
+// the instantiations of a kernel template that differ only in non-type template arguments share one function type.
+template <auto Kernel>
+int opt_in_smem(int bytes) {
+  static int done_dev = -1;
+  int dev = 0;
+  EVT_CUDA(cudaGetDevice(&dev));
+  if (done_dev != dev) {
+    EVT_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    done_dev = dev;
+  }
+  return EVT_OK;
+}
+
 int num_sms();
 bool pdl_enabled();  // EVT_PDL=0 launches every kernel with full stream serialization (A/B timing, debugging)
 // Programmatic dependent launch pays on the latency path (batch 1: -12 %, the next kernel's prologue hides behind the

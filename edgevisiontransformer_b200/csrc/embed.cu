@@ -299,7 +299,8 @@ extern "C" int evt_patch_embed_fwd(const void* pixels, int pixel_dtype, const fl
   if (rc != EVT_OK) return rc;
   rc = evt::embed_fill_launch(prefix, pos, bias, out, B, tokens, n_prefix, D, st);
   if (rc != EVT_OK) return rc;
-  return evt::gemm_launch(workspace, K, W, ldw, EVT_BF16, nullptr, out, D, 0, 0, out, EVT_F32, D, 0, 0, 0, M, D, K, EVT_ACT_NONE, st);
+  return evt::gemm_launch(
+      {.A = workspace, .lda = K, .W = W, .ldw = ldw, .residual = out, .ldr = D, .out = out, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D, .K = K}, st);
 }
 extern "C" int evt_prefix_tokens(const float* prefix, const float* pos, float* out, int B, int tokens, int n_prefix,
                                  int D, evt_stream stream) {

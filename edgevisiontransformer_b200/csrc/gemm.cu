@@ -228,16 +228,8 @@ int choose_bn(int64_t M, int N) {
 template <int BN, bool TF32, bool OUT_F32, int ACT, bool TMA_OUT>
 int launch(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmO, const GemmParams& p, cudaStream_t stream) {
   using C = Cfg<BN>;
-  auto kern = gemm_kernel<BN, TF32, OUT_F32, ACT, TMA_OUT>;
-  static bool configured = false;  // per instantiation; attribute is per-device-context but identical everywhere
-  static int configured_dev = -1;
-  int dev = 0;
-  EVT_CUDA(cudaGetDevice(&dev));
-  if (!configured || configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes));
-    configured = true;
-    configured_dev = dev;
-  }
+  constexpr auto kern = gemm_kernel<BN, TF32, OUT_F32, ACT, TMA_OUT>;
+  EVT_TRY(opt_in_smem<kern>(C::kSmemBytes));
   const int num_tiles = p.tiles_m * p.tiles_n * p.k_splits;
   const int grid = num_tiles < num_sms() ? num_tiles : num_sms();
   EVT_CUDA(launch_pdl(kern, dim3(grid), dim3(kThreads), C::kSmemBytes, stream, pdl_for_gemm(p.M, p.N, p.K), tmA, tmW, tmO, p));
@@ -264,66 +256,62 @@ int dispatch_epi(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& 
 
 }  // namespace
 
-// in_dtype: EVT_BF16 (kind::f16) or EVT_F32 (kind::tf32, operands read as fp32 and truncated to tf32 by the MMA)
-int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_dtype, const float* bias,
-                const float* residual, int64_t ldr, int res_row_mod, int res_row_off, void* out, int out_dtype,
-                int64_t ldo, int out_group, int out_group_stride, int out_group_off, int64_t M, int N, int K, int act,
-                cudaStream_t stream) {
-  EVT_CHECK_ARG(A && W && out, "gemm: null pointer");
-  EVT_CHECK_ARG(M > 0 && N > 0 && K > 0, "gemm: M, N, K must be positive");
-  EVT_CHECK_ARG(M < (1ll << 31) - 256, "gemm: M too large");
-  EVT_CHECK_ARG(in_dtype == EVT_BF16 || in_dtype == EVT_F32, "gemm: input dtype must be bf16 or f32(tf32)");
-  EVT_CHECK_ARG(out_dtype == EVT_BF16 || out_dtype == EVT_F32 || out_dtype == EVT_TF32, "gemm: out dtype must be bf16, f32 or tf32");
-  EVT_CHECK_ARG(!(out_dtype == EVT_TF32 && residual != nullptr), "gemm: a tf32-rounded output cannot take a residual");
-  EVT_CHECK_ARG(act >= EVT_ACT_NONE && act <= EVT_ACT_GELU_TANH, "gemm: unknown activation");
-  EVT_CHECK_ARG(lda >= K && ldw >= K && ldo >= N, "gemm: leading dimension smaller than the row length");
-  EVT_CHECK_ARG(out_group >= 0 && res_row_mod >= 0, "gemm: negative row-group parameter");
-  EVT_CHECK_ARG(residual == nullptr || ldr >= N, "gemm: residual leading dimension smaller than N");
-  const bool tf32 = in_dtype == EVT_F32;
+int gemm_launch(const GemmOp& op, cudaStream_t stream) {
+  EVT_CHECK_ARG(op.A && op.W && op.out, "gemm: null pointer");
+  EVT_CHECK_ARG(op.M > 0 && op.N > 0 && op.K > 0, "gemm: M, N, K must be positive");
+  EVT_CHECK_ARG(op.M < (1ll << 31) - 256, "gemm: M too large");
+  EVT_CHECK_ARG(op.in_dtype == EVT_BF16 || op.in_dtype == EVT_F32, "gemm: input dtype must be bf16 or f32(tf32)");
+  EVT_CHECK_ARG(op.out_dtype == EVT_BF16 || op.out_dtype == EVT_F32 || op.out_dtype == EVT_TF32, "gemm: out dtype must be bf16, f32 or tf32");
+  EVT_CHECK_ARG(!(op.out_dtype == EVT_TF32 && op.residual != nullptr), "gemm: a tf32-rounded output cannot take a residual");
+  EVT_CHECK_ARG(op.act >= EVT_ACT_NONE && op.act <= EVT_ACT_GELU_TANH, "gemm: unknown activation");
+  EVT_CHECK_ARG(op.lda >= op.K && op.ldw >= op.K && op.ldo >= op.N, "gemm: leading dimension smaller than the row length");
+  EVT_CHECK_ARG(op.map.out_group >= 0 && op.map.res_row_mod >= 0, "gemm: negative row-group parameter");
+  EVT_CHECK_ARG(op.residual == nullptr || op.ldr >= op.N, "gemm: residual leading dimension smaller than N");
+  const bool tf32 = op.in_dtype == EVT_F32;
   const int eb = tf32 ? 4 : 2;
   const int k_step = kStageRowBytes / eb;
-  const int bn = choose_bn(M, N);
+  const int bn = choose_bn(op.M, op.N);
   CUtensorMap tmA, tmW;
-  int rc = make_tmap_2d(&tmA, A, eb, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), BM, k_step);
+  int rc = make_tmap_2d(&tmA, op.A, eb, static_cast<uint64_t>(op.M), static_cast<uint64_t>(op.K), static_cast<uint64_t>(op.lda), BM, k_step);
   if (rc != EVT_OK) return rc;
-  rc = make_tmap_2d(&tmW, W, eb, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldw), bn, k_step);
+  rc = make_tmap_2d(&tmW, op.W, eb, static_cast<uint64_t>(op.N), static_cast<uint64_t>(op.K), static_cast<uint64_t>(op.ldw), bn, k_step);
   if (rc != EVT_OK) return rc;
   GemmParams p;
-  p.bias = bias;
-  p.residual = residual;
-  p.out = out;
-  p.ldr = ldr;
-  p.ldo = ldo;
-  p.M = static_cast<int>(M);
-  p.N = N;
-  p.K = K;
-  p.res_row_mod = res_row_mod;
-  p.res_row_off = res_row_off;
-  p.out_group = out_group;
-  p.out_group_stride = out_group_stride;
-  p.out_group_off = out_group_off;
-  p.tiles_m = static_cast<int>((M + BM - 1) / BM);
-  p.tiles_n = (N + bn - 1) / bn;
-  p.num_kb = (K + k_step - 1) / k_step;
+  p.bias = op.bias;
+  p.residual = op.residual;
+  p.out = op.out;
+  p.ldr = op.ldr;
+  p.ldo = op.ldo;
+  p.M = static_cast<int>(op.M);
+  p.N = op.N;
+  p.K = op.K;
+  p.res_row_mod = op.map.res_row_mod;
+  p.res_row_off = op.map.res_row_off;
+  p.out_group = op.map.out_group;
+  p.out_group_stride = op.map.out_group_stride;
+  p.out_group_off = op.map.out_group_off;
+  p.tiles_m = static_cast<int>((op.M + BM - 1) / BM);
+  p.tiles_n = (op.N + bn - 1) / bn;
+  p.num_kb = (op.K + k_step - 1) / k_step;
   p.k_step = k_step;
   p.w_static = gemm_weights_static() ? 1 : 0;
   {
-    const int oe = out_dtype != EVT_BF16 ? 4 : 2;
-    bool ok = reinterpret_cast<uintptr_t>(out) % 16 == 0 && (ldo * oe) % 16 == 0;
-    if (bias) ok = ok && reinterpret_cast<uintptr_t>(bias) % 16 == 0;
-    if (residual) ok = ok && reinterpret_cast<uintptr_t>(residual) % 16 == 0 && (ldr * 4) % 16 == 0;
+    const int oe = op.out_dtype != EVT_BF16 ? 4 : 2;
+    bool ok = reinterpret_cast<uintptr_t>(op.out) % 16 == 0 && (op.ldo * oe) % 16 == 0;
+    if (op.bias) ok = ok && reinterpret_cast<uintptr_t>(op.bias) % 16 == 0;
+    if (op.residual) ok = ok && reinterpret_cast<uintptr_t>(op.residual) % 16 == 0 && (op.ldr * 4) % 16 == 0;
     p.vec_ok = ok ? 1 : 0;
   }
-  const bool of32 = out_dtype != EVT_BF16;
-  p.round_tf32 = out_dtype == EVT_TF32 ? 1 : 0;
+  const bool of32 = op.out_dtype != EVT_BF16;
+  p.round_tf32 = op.out_dtype == EVT_TF32 ? 1 : 0;
   // TMA epilogue: contiguous output rows, 16-byte aligned, and the skip connection (if any) updated in place
   const int oeb = of32 ? 4 : 2;
-  const bool tma_out = out_group == 0 && res_row_mod == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0 &&
-                       (ldo * oeb) % 16 == 0 &&
-                       (residual == nullptr || (of32 && residual == reinterpret_cast<const float*>(out) && ldr == ldo));
+  const bool tma_out = op.map.out_group == 0 && op.map.res_row_mod == 0 && reinterpret_cast<uintptr_t>(op.out) % 16 == 0 &&
+                       (op.ldo * oeb) % 16 == 0 &&
+                       (op.residual == nullptr || (of32 && op.residual == reinterpret_cast<const float*>(op.out) && op.ldr == op.ldo));
   CUtensorMap tmO = tmA;
   if (tma_out) {
-    rc = make_tmap_2d(&tmO, out, oeb, static_cast<uint64_t>(M), static_cast<uint64_t>(N), static_cast<uint64_t>(ldo), 32,
+    rc = make_tmap_2d(&tmO, op.out, oeb, static_cast<uint64_t>(op.M), static_cast<uint64_t>(op.N), static_cast<uint64_t>(op.ldo), 32,
                       128 / oeb);
     if (rc != EVT_OK) return rc;
   }
@@ -336,7 +324,7 @@ int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_d
   // The tf32 (accuracy) mode never splits: DeiT-Tiny batch 1 would drop from 0.477 to 0.427 ms, but the unordered f32
   // reduce-adds flip tf32 roundings downstream and the logit error of BASELINE config 1 moves from a reproducible 7.5e-4
   // to 9.2e-4 in one run -- a random variable that close to the 1e-3 contract is not worth 0.05 ms.
-  if (!tf32 && tma_out && residual != nullptr && gemm_pair_mode() < 0 && gemm_split_k_enabled()) {
+  if (!tf32 && tma_out && op.residual != nullptr && gemm_pair_mode() < 0 && gemm_split_k_enabled()) {
     const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
     if (tiles * 2 <= num_sms() && p.num_kb >= 4) {
       int splits = static_cast<int>(num_sms() / tiles);
@@ -351,17 +339,17 @@ int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_d
   // forces the choice (tests exercise both kernels on the same shapes).
   if (!tf32 && tma_out && pair_supported(bn)) {
     const int pair_mode = gemm_pair_mode();
-    const long pair_tiles = static_cast<long>((M + 2 * BM - 1) / (2 * BM)) * p.tiles_n;
+    const long pair_tiles = static_cast<long>((op.M + 2 * BM - 1) / (2 * BM)) * p.tiles_n;
     const bool use_pair = pair_mode < 0 ? pair_tiles >= num_sms() : pair_mode != 0;
-    if (use_pair) return gemm_pair_launch(bn, W, ldw, tmA, tmO, p, of32, act, stream);
+    if (use_pair) return gemm_pair_launch(bn, op.W, op.ldw, tmA, tmO, p, of32, op.act, stream);
   }
-#define EVT_BN_CASE(BNV)                                                                                   \
-  case BNV:                                                                                                \
-    if (tma_out)                                                                                           \
-      return tf32 ? dispatch_epi<BNV, true, true>(tmA, tmW, tmO, p, of32, act, stream)                     \
-                  : dispatch_epi<BNV, false, true>(tmA, tmW, tmO, p, of32, act, stream);                   \
-    return tf32 ? dispatch_epi<BNV, true, false>(tmA, tmW, tmO, p, of32, act, stream)                      \
-                : dispatch_epi<BNV, false, false>(tmA, tmW, tmO, p, of32, act, stream);
+#define EVT_BN_CASE(BNV)                                                                                      \
+  case BNV:                                                                                                   \
+    if (tma_out)                                                                                              \
+      return tf32 ? dispatch_epi<BNV, true, true>(tmA, tmW, tmO, p, of32, op.act, stream)                     \
+                  : dispatch_epi<BNV, false, true>(tmA, tmW, tmO, p, of32, op.act, stream);                   \
+    return tf32 ? dispatch_epi<BNV, true, false>(tmA, tmW, tmO, p, of32, op.act, stream)                      \
+                : dispatch_epi<BNV, false, false>(tmA, tmW, tmO, p, of32, op.act, stream);
   switch (bn) {
     EVT_BN_CASE(256)
     EVT_BN_CASE(192)
@@ -380,8 +368,10 @@ extern "C" int evt_gemm_bias_act(const void* A, int64_t lda, const void* W, int6
                                  int64_t M, int N, int K, int act, evt_stream stream) {
   int rc = evt_device_check();
   if (rc != EVT_OK) return rc;
-  return evt::gemm_launch(A, lda, W, ldw, EVT_BF16, bias, residual, ldr, res_row_mod, res_row_off, out, out_dtype, ldo,
-                          out_group, out_group_stride, out_group_off, M, N, K, act, static_cast<cudaStream_t>(stream));
+  return evt::gemm_launch({.A = A, .lda = lda, .W = W, .ldw = ldw, .in_dtype = EVT_BF16, .bias = bias, .residual = residual, .ldr = ldr,
+                           .out = out, .out_dtype = out_dtype, .ldo = ldo, .M = M, .N = N, .K = K, .act = act,
+                           .map = {.res_row_mod = res_row_mod, .res_row_off = res_row_off, .out_group = out_group, .out_group_stride = out_group_stride,
+                                    .out_group_off = out_group_off}}, static_cast<cudaStream_t>(stream));
 }
 
 // tf32 flavour: A and W are f32 (the MMA reads them as tf32); out is f32.
@@ -391,6 +381,8 @@ extern "C" int evt_gemm_bias_act_tf32(const float* A, int64_t lda, const float* 
                                       int N, int K, int act, evt_stream stream) {
   int rc = evt_device_check();
   if (rc != EVT_OK) return rc;
-  return evt::gemm_launch(A, lda, W, ldw, EVT_F32, bias, residual, ldr, res_row_mod, res_row_off, out, EVT_F32, ldo,
-                          out_group, out_group_stride, out_group_off, M, N, K, act, static_cast<cudaStream_t>(stream));
+  return evt::gemm_launch({.A = A, .lda = lda, .W = W, .ldw = ldw, .in_dtype = EVT_F32, .bias = bias, .residual = residual, .ldr = ldr,
+                           .out = out, .out_dtype = EVT_F32, .ldo = ldo, .M = M, .N = N, .K = K, .act = act,
+                           .map = {.res_row_mod = res_row_mod, .res_row_off = res_row_off, .out_group = out_group, .out_group_stride = out_group_stride,
+                                    .out_group_off = out_group_off}}, static_cast<cudaStream_t>(stream));
 }

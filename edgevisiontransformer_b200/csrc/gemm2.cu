@@ -216,13 +216,13 @@ template <int BN, bool OUT_F32, int ACT, int EW>
 int launch_pair_ew(const void* W, int64_t ldw, const CUtensorMap& tmA, const CUtensorMap& tmO, GemmParams p, cudaStream_t stream) {
   using C = Cfg2<BN, EW>;
   constexpr int kThreads = C::kThreadsCta;
-  auto kern = gemm_pair_kernel<BN, OUT_F32, ACT, EW>;
-  static int configured_dev = -1;
+  constexpr auto kern = gemm_pair_kernel<BN, OUT_F32, ACT, EW>;
+  EVT_TRY(opt_in_smem<kern>(C::kSmemBytes));
+  static int pairs_dev = -1;
   static int max_pairs = 0;
   int dev = 0;
   EVT_CUDA(cudaGetDevice(&dev));
-  if (configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes));
+  if (pairs_dev != dev) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(num_sms() & ~1, 1, 1);
     cfg.blockDim = dim3(kThreads, 1, 1);
@@ -232,7 +232,7 @@ int launch_pair_ew(const void* W, int64_t ldw, const CUtensorMap& tmA, const CUt
     if (n <= 0) return fail(EVT_ERR_CUDA, "gemm: no CTA pair of this configuration fits on the device");
     max_pairs = n;
     if (getenv("EVT_DEBUG")) fprintf(stderr, "evt: gemm_pair_kernel<%d> max active clusters %d, smem %d\n", BN, n, C::kSmemBytes);
-    configured_dev = dev;
+    pairs_dev = dev;
   }
   CUtensorMap tmW;
   int rc = make_tmap_2d(&tmW, W, 2, static_cast<uint64_t>(p.N), static_cast<uint64_t>(p.K), static_cast<uint64_t>(ldw), BN / 2,

@@ -340,14 +340,8 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ 
 template <int BN, int KB, int ACT>
 int launch_ln(const CUtensorMap& tmW, const CUtensorMap& tmO, const LnGemmParams& p, cudaStream_t stream) {
   using C = CfgLn<BN, KB>;
-  auto kern = gemm_ln_kernel<BN, KB, ACT>;
-  static int configured_dev = -1;
-  int dev = 0;
-  EVT_CUDA(cudaGetDevice(&dev));
-  if (configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes));
-    configured_dev = dev;
-  }
+  constexpr auto kern = gemm_ln_kernel<BN, KB, ACT>;
+  EVT_TRY(opt_in_smem<kern>(C::kSmemBytes));
   const int grid = p.g.tiles_m < num_sms() ? p.g.tiles_m : num_sms();
   EVT_CUDA(launch_pdl(kern, dim3(grid), dim3(kLnThreads), C::kSmemBytes, stream, pdl_for_gemm(p.g.M, p.g.N, p.g.K), tmW, tmO, p));
   EVT_LAUNCH_CHECK("gemm_ln_kernel");

@@ -432,13 +432,13 @@ template <int NT, bool COPY, int EW>
 int launch_rowln(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmRin, const CUtensorMap& tmRout,
                  const CUtensorMap& tmXn, const RowLnParams& p, cudaStream_t stream) {
   using C = CfgR<NT, COPY, EW>;
-  auto kern = gemm_rowln_kernel<NT, COPY, EW>;
-  static int configured_dev = -1;
+  constexpr auto kern = gemm_rowln_kernel<NT, COPY, EW>;
+  EVT_TRY(opt_in_smem<kern>(C::kSmemBytes));
+  static int pairs_dev = -1;
   static int max_pairs = 0;
   int dev = 0;
   EVT_CUDA(cudaGetDevice(&dev));
-  if (configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes));
+  if (pairs_dev != dev) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(num_sms() & ~1, 1, 1);
     cfg.blockDim = dim3(C::kThreads, 1, 1);
@@ -449,7 +449,7 @@ int launch_rowln(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorM
     max_pairs = n;
     if (getenv("EVT_DEBUG"))
       fprintf(stderr, "evt: gemm_rowln_kernel<%d,%d,%d> smem %d ring %d xn bufs %d\n", NT, (int)COPY, EW, C::kSmemBytes, C::kResDepth, C::kXnBufs);
-    configured_dev = dev;
+    pairs_dev = dev;
   }
   const int pairs = p.row_blocks < max_pairs ? p.row_blocks : max_pairs;
   EVT_CUDA(launch_pdl(kern, dim3(2 * pairs), dim3(C::kThreads), C::kSmemBytes, stream, pdl_for_gemm(p.M, p.D, p.K), tmA, tmW, tmRin,

@@ -10,11 +10,10 @@
 // residual stream, because there the skip connection carries LN(x).
 #include <cuda_bf16.h>
 
-#include <cstring>
-#include <map>
 #include <string>
 #include <vector>
 
+#include "loader.h"
 #include "ops.h"
 #include "ptx.cuh"
 
@@ -58,7 +57,6 @@ __global__ void __launch_bounds__(256) gather_rows_cast_kernel(const float* __re
 }
 
 inline int padn(int v, int n) { return (v + n - 1) / n * n; }
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct LayerW {
   uint8_t *wqkv = nullptr, *wo = nullptr, *w1 = nullptr, *w2 = nullptr;  // bf16 or f32 (tf32 mode) matrices
@@ -124,7 +122,7 @@ inline int t2t_side(int image, int stage) {
   return s;
 }
 
-Workspace plan_workspace(const evt_model* m, int batch, void* base) {
+Workspace plan_workspace(const evt_model* m, int batch, uint8_t* base) {
   const evt_model_spec& s = m->spec;
   const size_t M = static_cast<size_t>(batch) * s.tokens;
   const size_t Mp = static_cast<size_t>(batch) * m->patches;
@@ -133,42 +131,29 @@ Workspace plan_workspace(const evt_model* m, int batch, void* base) {
     amax = std::max(amax, s.heads[l] * s.head_size);
     imax_ld = std::max(imax_ld, padn(s.inter[l], m->pad));
   }
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    size_t o = off;
-    off = align_up(off + bytes, 1024);
-    return o;
-  };
-  uint8_t* b = reinterpret_cast<uint8_t*>(base);
+  WorkspaceCarver c{base};
   Workspace w;
-  const size_t o_resid = take(M * s.hidden * 4);
   const size_t es = m->es;
-  const size_t o_xn = take(M * s.hidden * es);
-  const size_t o_qkv = take(M * 3 * amax * es);
-  const size_t o_ctx = take(M * amax * es);
+  w.resid = c.take<float>(M * s.hidden * 4);
+  w.xn = c.take(M * s.hidden * es);
+  w.qkv = c.take(M * 3 * amax * es);
+  w.ctx = c.take(M * amax * es);
   // the patch matrix has one row per TOKEN when the library builds it (pixels path), see forward_impl
-  const size_t o_big = take(std::max(M * imax_ld, (s.embed_k > 0 ? Mp : M) * static_cast<size_t>(m->patch_k)) * es);
-  const size_t o_cls = take(static_cast<size_t>(batch) * s.hidden * (s.head_rows > 1 ? s.head_rows : 1) * es);
-  const size_t o_hh = take(static_cast<size_t>(batch) * std::max(padn(s.head_hidden, m->pad), 8) * es);
+  w.big = c.take(std::max(M * imax_ld, (s.embed_k > 0 ? Mp : M) * static_cast<size_t>(m->patch_k)) * es);
+  w.clsn = c.take(static_cast<size_t>(batch) * s.hidden * (s.head_rows > 1 ? s.head_rows : 1) * es);
+  w.hh = c.take(static_cast<size_t>(batch) * std::max(padn(s.head_hidden, m->pad), 8) * es);
   if (s.t2t) {
     for (int i = 0; i < 2; ++i) {
       const size_t T = static_cast<size_t>(t2t_side(s.image, i)) * t2t_side(s.image, i) * batch;
       const size_t in_ld = i == 0 ? 152 : 576;
-      const size_t ox = take(T * in_ld * 2), ok = take(T * 192 * 2), oy = take(T * 64 * 4);
-      const size_t ow = take(performer_workspace_bytes(batch, t2t_side(s.image, i) * t2t_side(s.image, i)));
-      w.t_x[i] = b + ox, w.t_kqv[i] = b + ok, w.t_y[i] = reinterpret_cast<float*>(b + oy);
-      w.t_ws[i] = b + ow;
+      w.t_x[i] = c.take(T * in_ld * 2);
+      w.t_kqv[i] = c.take(T * 192 * 2);
+      w.t_y[i] = c.take<float>(T * 64 * 4);
+      w.t_ws[i] = c.take(performer_workspace_bytes(batch, t2t_side(s.image, i) * t2t_side(s.image, i)));
     }
-    w.t_pm = b + take(Mp * 576 * 2);
+    w.t_pm = c.take(Mp * 576 * 2);
   }
-  w.resid = reinterpret_cast<float*>(b + o_resid);
-  w.xn = b + o_xn;
-  w.qkv = b + o_qkv;
-  w.ctx = b + o_ctx;
-  w.big = b + o_big;
-  w.clsn = b + o_cls;
-  w.hh = b + o_hh;
-  w.bytes = off;
+  w.bytes = c.bytes;
   return w;
 }
 
@@ -204,93 +189,97 @@ int validate_spec(const evt_model_spec* s) {
   return EVT_OK;
 }
 
-struct Loader {
-  evt_model* m;
-  std::map<std::string, const evt_tensor_view*> by_name;
-  cudaStream_t st;
-
-  const evt_tensor_view* find(const std::string& name) const {
-    auto it = by_name.find(name);
-    return it == by_name.end() ? nullptr : it->second;
-  }
-  static int64_t numel(const evt_tensor_view* v) {
-    int64_t n = 1;
-    for (int i = 0; i < v->ndim; ++i) n *= v->shape[i];
-    return n;
-  }
-  int need(const std::string& name, int64_t n, const evt_tensor_view** out) const {
-    const evt_tensor_view* v = find(name);
-    if (!v) return fail(EVT_ERR_INVALID, "missing weight '" + name + "'");
-    if (!v->data) return fail(EVT_ERR_INVALID, "weight '" + name + "' has a null data pointer");
-    if (numel(v) != n)
-      return fail(EVT_ERR_INVALID, "weight '" + name + "' has " + std::to_string(numel(v)) + " elements, expected " + std::to_string(n));
-    *out = v;
-    return EVT_OK;
-  }
-  int alloc(size_t bytes, void** out) {
-    void* p = nullptr;
-    cudaError_t e = cudaMalloc(&p, std::max<size_t>(bytes, 16));
-    if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("cudaMalloc: ") + cudaGetErrorString(e));
-    m->allocs.push_back(p);
-    *out = p;
-    return EVT_OK;
-  }
-  // f32 copy of a vector / table; zero-filled when `optional` and absent
-  int vec(const std::string& name, int64_t n, bool optional, float** out) {
-    void* p;
-    int rc = alloc(n * 4, &p);
-    if (rc) return rc;
-    const evt_tensor_view* v = find(name);
-    if (!v && optional) {
-      EVT_CUDA(cudaMemsetAsync(p, 0, n * 4, st));
-    } else {
-      rc = need(name, n, &v);
-      if (rc) return rc;
-      EVT_CUDA(cudaMemcpyAsync(p, v->data, n * 4, cudaMemcpyDeviceToDevice, st));
-    }
-    *out = reinterpret_cast<float*>(p);
-    return EVT_OK;
-  }
-  // operand-typed [rows, ld] from f32 [rows, cols] into dst (already allocated), zero padded
-  int mat_into(const std::string& name, int64_t rows, int cols, int ld, uint8_t* dst) {
-    const evt_tensor_view* v;
-    int rc = need(name, rows * cols, &v);
-    if (rc) return rc;
-    const long long total = rows * ld;
-    const unsigned grid = static_cast<unsigned>((total + 255) / 256);
-    const float* src = reinterpret_cast<const float*>(v->data);
-    if (m->es == 2) convert_pad_kernel<<<grid, 256, 0, st>>>(src, reinterpret_cast<__nv_bfloat16*>(dst), rows, cols, ld);
-    else convert_pad_kernel<<<grid, 256, 0, st>>>(src, reinterpret_cast<float*>(dst), rows, cols, ld);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("convert_pad: ") + cudaGetErrorString(e));
-    return EVT_OK;
-  }
-  // bf16 [rows_out, ld] from an f32 Keras kernel [cols_out, rows_out]
-  int mat_t(const std::string& name, int rows_out, int cols_out, int ld, __nv_bfloat16** out) {
-    const evt_tensor_view* v;
-    int rc = need(name, static_cast<int64_t>(rows_out) * cols_out, &v);
-    if (rc) return rc;
-    void* p;
-    rc = alloc(static_cast<size_t>(rows_out) * ld * 2, &p);
-    if (rc) return rc;
-    *out = reinterpret_cast<__nv_bfloat16*>(p);
-    const long long total = static_cast<long long>(rows_out) * ld;
-    convert_pad_transposed_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float*>(v->data), *out,
-                                                                                               rows_out, cols_out, ld);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("convert_pad_transposed: ") + cudaGetErrorString(e));
-    return EVT_OK;
-  }
-  int mat(const std::string& name, int64_t rows, int cols, int ld, uint8_t** out) {
-    void* p;
-    int rc = alloc(static_cast<size_t>(rows) * ld * m->es, &p);
-    if (rc) return rc;
-    *out = reinterpret_cast<uint8_t*>(p);
-    return mat_into(name, rows, cols, ld, *out);
-  }
-};
-
 }  // namespace
+
+int Loader::index(const evt_tensor_view* tensors, int n) {
+  for (int i = 0; i < n; ++i) {
+    EVT_CHECK_ARG(tensors[i].name != nullptr, "tensor view without a name");
+    EVT_CHECK_ARG(tensors[i].ndim >= 1 && tensors[i].ndim <= 4, "tensor view rank must be 1..4");
+    by_name[tensors[i].name] = &tensors[i];
+  }
+  return EVT_OK;
+}
+
+const evt_tensor_view* Loader::find(const std::string& name) const {
+  auto it = by_name.find(name);
+  return it == by_name.end() ? nullptr : it->second;
+}
+
+int Loader::need(const std::string& name, int64_t n, const evt_tensor_view** out) const {
+  const evt_tensor_view* v = find(name);
+  if (!v) return fail(EVT_ERR_INVALID, "missing weight '" + name + "'");
+  if (!v->data) return fail(EVT_ERR_INVALID, "weight '" + name + "' has a null data pointer");
+  int64_t numel = 1;
+  for (int i = 0; i < v->ndim; ++i) numel *= v->shape[i];
+  if (numel != n)
+    return fail(EVT_ERR_INVALID, "weight '" + name + "' has " + std::to_string(numel) + " elements, expected " + std::to_string(n));
+  *out = v;
+  return EVT_OK;
+}
+
+int Loader::alloc(size_t bytes, void** out) {
+  void* p = nullptr;
+  cudaError_t e = cudaMalloc(&p, std::max<size_t>(bytes, 16));
+  if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+  allocs->push_back(p);
+  *out = p;
+  return EVT_OK;
+}
+
+int Loader::vec_into(const std::string& name, int64_t n, bool optional, float* dst) {
+  const evt_tensor_view* v = find(name);
+  if (!v && optional) {
+    EVT_CUDA(cudaMemsetAsync(dst, 0, n * 4, st));
+  } else {
+    EVT_TRY(need(name, n, &v));
+    EVT_CUDA(cudaMemcpyAsync(dst, v->data, n * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  return EVT_OK;
+}
+
+int Loader::vec(const std::string& name, int64_t n, bool optional, float** out) {
+  void* p;
+  EVT_TRY(alloc(n * 4, &p));
+  *out = static_cast<float*>(p);
+  return vec_into(name, n, optional, *out);
+}
+
+int Loader::mat_into(const std::string& name, int64_t rows, int cols, int ld, void* dst) {
+  const evt_tensor_view* v;
+  EVT_TRY(need(name, rows * cols, &v));
+  const long long total = rows * ld;
+  const unsigned grid = static_cast<unsigned>((total + 255) / 256);
+  const float* src = static_cast<const float*>(v->data);
+  if (es == 2) convert_pad_kernel<<<grid, 256, 0, st>>>(src, static_cast<__nv_bfloat16*>(dst), rows, cols, ld);
+  else convert_pad_kernel<<<grid, 256, 0, st>>>(src, static_cast<float*>(dst), rows, cols, ld);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("convert_pad: ") + cudaGetErrorString(e));
+  return EVT_OK;
+}
+
+int Loader::mat_t(const std::string& name, int rows_out, int cols_out, int ld, __nv_bfloat16** out) {
+  const evt_tensor_view* v;
+  EVT_TRY(need(name, static_cast<int64_t>(rows_out) * cols_out, &v));
+  void* p;
+  EVT_TRY(alloc(static_cast<size_t>(rows_out) * ld * 2, &p));
+  *out = static_cast<__nv_bfloat16*>(p);
+  const long long total = static_cast<long long>(rows_out) * ld;
+  convert_pad_transposed_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(static_cast<const float*>(v->data), *out,
+                                                                                             rows_out, cols_out, ld);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("convert_pad_transposed: ") + cudaGetErrorString(e));
+  return EVT_OK;
+}
+
+int Loader::host_copy(const std::string& name, int64_t n, std::vector<float>* out) {
+  const evt_tensor_view* v;
+  EVT_TRY(need(name, n, &v));
+  out->resize(n);
+  EVT_CUDA(cudaMemcpyAsync(out->data(), v->data, n * 4, cudaMemcpyDeviceToHost, st));
+  EVT_CUDA(cudaStreamSynchronize(st));
+  return EVT_OK;
+}
+
 }  // namespace evt
 
 using namespace evt;
@@ -326,21 +315,9 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
   EVT_CHECK_ARG(m != nullptr && tensors != nullptr && n > 0, "evt_model_load_weights: bad arguments");
   if (m->loaded) return fail(EVT_ERR_STATE, "weights already loaded; create a new model to reload");
   const evt_model_spec& s = m->spec;
-  Loader L;
-  L.m = m;
-  L.st = static_cast<cudaStream_t>(stream);
-  for (int i = 0; i < n; ++i) {
-    EVT_CHECK_ARG(tensors[i].name != nullptr, "tensor view without a name");
-    EVT_CHECK_ARG(tensors[i].ndim >= 1 && tensors[i].ndim <= 4, "tensor view rank must be 1..4");
-    L.by_name[tensors[i].name] = &tensors[i];
-  }
+  Loader L{&m->allocs, static_cast<cudaStream_t>(stream), m->es};
+  EVT_TRY(L.index(tensors, n));
   const int D = s.hidden;
-  int rc;
-#define EVT_TRY(expr) \
-  do {                \
-    rc = (expr);      \
-    if (rc != EVT_OK) return rc; \
-  } while (0)
   const std::string e = "vit.embeddings.";
   EVT_TRY(L.mat(e + "patch_embeddings.projection.weight", D, m->patch_k, m->patch_k, &m->w_patch));
   EVT_TRY(L.vec(e + "patch_embeddings.projection.bias", D, false, &m->b_patch));
@@ -349,13 +326,8 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
     void* p;
     EVT_TRY(L.alloc(static_cast<size_t>(m->n_prefix) * D * 4, &p));
     m->prefix = reinterpret_cast<float*>(p);
-    const evt_tensor_view* v;
-    EVT_TRY(L.need(e + "cls_token", D, &v));
-    EVT_CUDA(cudaMemcpyAsync(m->prefix, v->data, D * 4, cudaMemcpyDeviceToDevice, L.st));
-    if (m->n_prefix == 2) {
-      EVT_TRY(L.need(e + "distillation_token", D, &v));
-      EVT_CUDA(cudaMemcpyAsync(m->prefix + D, v->data, D * 4, cudaMemcpyDeviceToDevice, L.st));
-    }
+    EVT_TRY(L.vec_into(e + "cls_token", D, false, m->prefix));
+    if (m->n_prefix == 2) EVT_TRY(L.vec_into(e + "distillation_token", D, false, m->prefix + D));
   }
   for (int l = 0; l < s.layers; ++l) {
     LayerW& w = m->layers[l];
@@ -372,13 +344,7 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
     for (int t = 0; t < 3; ++t) {
       const std::string base = p + "attention.attention." + names[t];
       EVT_TRY(L.mat_into(base + ".weight", w.a, D, D, w.wqkv + static_cast<size_t>(t) * w.a * D * m->es));
-      const evt_tensor_view* v = L.find(base + ".bias");
-      if (v) {
-        EVT_TRY(L.need(base + ".bias", w.a, &v));
-        EVT_CUDA(cudaMemcpyAsync(w.bqkv + t * w.a, v->data, w.a * 4, cudaMemcpyDeviceToDevice, L.st));
-      } else {
-        EVT_CUDA(cudaMemsetAsync(w.bqkv + t * w.a, 0, w.a * 4, L.st));
-      }
+      EVT_TRY(L.vec_into(base + ".bias", w.a, true, w.bqkv + t * w.a));
     }
     EVT_TRY(L.mat(p + "attention.output.dense.weight", D, w.a, w.a, &w.wo));
     EVT_TRY(L.vec(p + "attention.output.dense.bias", D, true, &w.bo));
@@ -424,7 +390,6 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
   }
   EVT_TRY(L.mat("classifier.weight", s.num_labels, cls_in, padn(cls_in, m->pad), &m->w_cls));
   EVT_TRY(L.vec("classifier.bias", s.num_labels, true, &m->b_cls));
-#undef EVT_TRY
   EVT_CUDA(cudaStreamSynchronize(L.st));
   m->loaded = true;
   return EVT_OK;
@@ -454,10 +419,9 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   static const evt_forward_opts kNoOpts = {};
   const evt_forward_opts& o = opts != nullptr ? *opts : kNoOpts;
   EVT_CHECK_ARG(o.head_mask == nullptr || o.head_mask_ld > 0, "head_mask_ld must be positive when a head mask is given");
-  void* base = reinterpret_cast<void*>(align_up(reinterpret_cast<uintptr_t>(workspace), 1024));
-  const size_t slack = reinterpret_cast<uintptr_t>(base) - reinterpret_cast<uintptr_t>(workspace);
-  Workspace w = plan_workspace(m, batch, base);
-  EVT_CHECK_ARG(w.bytes + slack <= workspace_bytes, "workspace too small for this batch (see evt_model_workspace_bytes)");
+  Workspace w;
+  EVT_TRY(place_workspace(workspace, workspace_bytes, [&](uint8_t* base) { return plan_workspace(m, batch, base); }, &w,
+                          "workspace too small for this batch (see evt_model_workspace_bytes)"));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   StaticWeightsScope weights_are_static;  // every GEMM below multiplies by a weight matrix this model owns
   const int D = s.hidden;
@@ -465,12 +429,6 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   const int64_t Mp = static_cast<int64_t>(batch) * m->patches;
   const bool tf = s.dialect == EVT_DIALECT_TF;
   const float scale = 1.0f / sqrtf(static_cast<float>(s.head_size));
-  int rc;
-#define EVT_TRY(expr) \
-  do {                \
-    rc = (expr);      \
-    if (rc != EVT_OK) return rc; \
-  } while (0)
   // profiling tap: events on the launching stream between launches (no effect on the launches themselves)
   auto mark = [&](int stage) -> int {
     if (!m->profiling) return EVT_OK;
@@ -505,8 +463,8 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
       const int so = t2t_side(s.image, i), T = so * so;
       const int64_t rows = static_cast<int64_t>(batch) * T;
       EVT_STAGE(EVT_STAGE_EMBED, unfold_ln_launch(src, src_dt, w.t_x[i], pw.in_ld, pw.g1, pw.b1, tf_eps, batch, side, side, ch, k, st_, pad_, st));
-      EVT_STAGE(EVT_STAGE_EMBED, gemm_launch(w.t_x[i], pw.in_ld, pw.wkqv, pw.in_ld, EVT_BF16, pw.bkqv, nullptr, 0, 0, 0, w.t_kqv[i], EVT_BF16, 192,
-                                             0, 0, 0, rows, 192, pw.in_dim, EVT_ACT_NONE, st));
+      EVT_STAGE(EVT_STAGE_EMBED, gemm_launch({.A = w.t_x[i], .lda = pw.in_ld, .W = pw.wkqv, .ldw = pw.in_ld, .bias = pw.bkqv, .out = w.t_kqv[i],
+                                              .out_dtype = EVT_BF16, .ldo = 192, .M = rows, .N = 192, .K = pw.in_dim}, st));
       // single_attn + attn_output + LayerNorm + MLP (transformer_encoder.py:67-99): the attention contraction's apply kernel carries
       // each tile through the tail, y = the performer's output rows
       EVT_TRY(performer_block_launch(w.t_kqv[i], 192, pw.w, w.t_y[i], w.t_ws[i], batch, T, 1e-8f, pw.wo, pw.bo, pw.g2, pw.b2, pw.w1,
@@ -530,13 +488,16 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
     EVT_STAGE(EVT_STAGE_EMBED, im2col_launch(pixels, o.pixel_dtype, o.pixel_scale, o.pixel_bias, w.big, dt, batch, s.image, s.image, s.patch, st,
                                              s.tokens, m->n_prefix));
     EVT_STAGE(EVT_STAGE_EMBED, embed_fill_launch(m->prefix, m->pos, m->b_patch, w.resid, batch, s.tokens, m->n_prefix, D, st));
-    EVT_STAGE(EVT_STAGE_EMBED, gemm_launch(w.big, m->patch_k, m->w_patch, m->patch_k, dt, nullptr, w.resid, D, 0, 0, w.resid, EVT_F32, D,
-                                           0, 0, 0, M, D, m->patch_k, EVT_ACT_NONE, st));
+    EVT_STAGE(EVT_STAGE_EMBED, gemm_launch({.A = w.big, .lda = m->patch_k, .W = m->w_patch, .ldw = m->patch_k, .in_dtype = dt, .residual = w.resid,
+                                            .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D, .K = m->patch_k}, st));
   } else {
     EVT_CHECK_ARG(patch_ld >= m->patch_k, "patch matrix leading dimension smaller than the embedding K");
-    EVT_STAGE(EVT_STAGE_EMBED, gemm_launch(patch_matrix, patch_ld, m->w_patch, m->patch_k, dt, m->b_patch, m->pos, D, m->patches,
-                                           m->n_prefix, w.resid, EVT_F32, D, m->patches, s.tokens, m->n_prefix, Mp, D, m->patch_k,
-                                           EVT_ACT_NONE, st));
+    // patch row p of image b: output row b * tokens + n_prefix + p, position-embedding row n_prefix + p
+    EVT_STAGE(EVT_STAGE_EMBED,
+              gemm_launch({.A = patch_matrix, .lda = patch_ld, .W = m->w_patch, .ldw = m->patch_k, .in_dtype = dt, .bias = m->b_patch,
+                           .residual = m->pos, .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = Mp, .N = D, .K = m->patch_k,
+                           .map = {.res_row_mod = m->patches, .res_row_off = m->n_prefix, .out_group = m->patches,
+                                   .out_group_stride = s.tokens, .out_group_off = m->n_prefix}}, st));
     EVT_STAGE(EVT_STAGE_EMBED, prefix_tokens_launch(m->prefix, m->pos, w.resid, batch, s.tokens, m->n_prefix, D, st));
   }
   // encoder.  Narrow residual streams at large batch (D = 192 / 384: DeiT-Tiny / -Small, T2T): whole rows of a 256-row block
@@ -549,8 +510,8 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
     const int a = lw.a;
     if (!xn_ready)
       EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln1_g, lw.ln1_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
-    EVT_STAGE(EVT_STAGE_QKV, gemm_launch(w.xn, D, lw.wqkv, D, dt, lw.bqkv, nullptr, 0, 0, 0, w.qkv, adt, 3 * a, 0, 0, 0, M, 3 * a, D,
-                        EVT_ACT_NONE, st));
+    EVT_STAGE(EVT_STAGE_QKV, gemm_launch({.A = w.xn, .lda = D, .W = lw.wqkv, .ldw = D, .in_dtype = dt, .bias = lw.bqkv, .out = w.qkv,
+                                          .out_dtype = adt, .ldo = 3 * a, .M = M, .N = 3 * a, .K = D}, st));
     xn_ready = false;
     // head mask row of this layer (are_16_heads mask_heads) and, on request, the context written straight into the caller's
     // buffer (context_layer_val): the output projection then reads its A operand from there
@@ -566,20 +527,21 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
     if (row_ln && gemm_rowln_pays(D, a, tf)) {
       EVT_STAGE(EVT_STAGE_OPROJ, gemm_rowln_launch(ctx, a, lw.wo, a, lw.bo, w.resid, D, lw.ln2_g, lw.ln2_b, s.eps, tf, w.xn, D, M, D, a, st));
     } else {
-      EVT_STAGE(EVT_STAGE_OPROJ, gemm_launch(ctx, a, lw.wo, a, dt, lw.bo, w.resid, D, 0, 0, w.resid, EVT_F32, D, 0, 0, 0, M, D, a,
-                          EVT_ACT_NONE, st));
+      EVT_STAGE(EVT_STAGE_OPROJ, gemm_launch({.A = ctx, .lda = a, .W = lw.wo, .ldw = a, .in_dtype = dt, .bias = lw.bo, .residual = w.resid,
+                                              .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D, .K = a}, st));
       EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln2_g, lw.ln2_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
     }
-    EVT_STAGE(EVT_STAGE_FC1, gemm_launch(w.xn, D, lw.w1, D, dt, lw.b1, nullptr, 0, 0, 0, w.big, adt, lw.inter_ld, 0, 0, 0, M, lw.inter, D, s.act,
-                        st));
+    EVT_STAGE(EVT_STAGE_FC1, gemm_launch({.A = w.xn, .lda = D, .W = lw.w1, .ldw = D, .in_dtype = dt, .bias = lw.b1, .out = w.big,
+                                          .out_dtype = adt, .ldo = lw.inter_ld, .M = M, .N = lw.inter, .K = D, .act = s.act}, st));
     if (row_ln && l + 1 < s.layers && gemm_rowln_pays(D, lw.inter, tf)) {
       const LayerW& nx = m->layers[l + 1];
       EVT_STAGE(EVT_STAGE_FC2, gemm_rowln_launch(w.big, lw.inter_ld, lw.w2, lw.inter_ld, lw.b2, w.resid, D, nx.ln1_g, nx.ln1_b, s.eps, tf, w.xn,
                                                  D, M, D, lw.inter, st));
       xn_ready = true;
     } else {
-      EVT_STAGE(EVT_STAGE_FC2, gemm_launch(w.big, lw.inter_ld, lw.w2, lw.inter_ld, dt, lw.b2, w.resid, D, 0, 0, w.resid, EVT_F32, D, 0, 0, 0, M,
-                          D, lw.inter, EVT_ACT_NONE, st));
+      EVT_STAGE(EVT_STAGE_FC2, gemm_launch({.A = w.big, .lda = lw.inter_ld, .W = lw.w2, .ldw = lw.inter_ld, .in_dtype = dt, .bias = lw.b2,
+                                            .residual = w.resid, .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D,
+                                            .K = lw.inter}, st));
     }
   }
   // head: only the cls row of every image is consumed (SITE/models/vit/modeling_vit.py:641)
@@ -608,17 +570,16 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   }
   if (s.head_hidden > 0) {
     const int hl = padn(s.head_hidden, m->pad);
-    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch(w.clsn, D, m->w_pre, D, dt, m->b_pre, nullptr, 0, 0, 0, w.hh, adt, hl, 0, 0, 0, batch, s.head_hidden, D,
-                        EVT_ACT_GELU_TANH, st));
-    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch(w.hh, hl, m->w_cls, hl, dt, m->b_cls, nullptr, 0, 0, 0, logits, EVT_F32, s.num_labels, 0, 0, 0, batch,
-                        s.num_labels, s.head_hidden, EVT_ACT_NONE, st));
+    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch({.A = w.clsn, .lda = D, .W = m->w_pre, .ldw = D, .in_dtype = dt, .bias = m->b_pre, .out = w.hh,
+                                           .out_dtype = adt, .ldo = hl, .M = batch, .N = s.head_hidden, .K = D, .act = EVT_ACT_GELU_TANH}, st));
+    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch({.A = w.hh, .lda = hl, .W = m->w_cls, .ldw = hl, .in_dtype = dt, .bias = m->b_cls, .out = logits,
+                                           .out_dtype = EVT_F32, .ldo = s.num_labels, .M = batch, .N = s.num_labels, .K = s.head_hidden}, st));
   } else {
     const int kc = head_rows * D;
-    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch(w.clsn, kc, m->w_cls, kc, dt, m->b_cls, nullptr, 0, 0, 0, logits, EVT_F32, s.num_labels, 0, 0, 0, batch,
-                        s.num_labels, kc, EVT_ACT_NONE, st));
+    EVT_STAGE(EVT_STAGE_HEAD, gemm_launch({.A = w.clsn, .lda = kc, .W = m->w_cls, .ldw = kc, .in_dtype = dt, .bias = m->b_cls, .out = logits,
+                                           .out_dtype = EVT_F32, .ldo = s.num_labels, .M = batch, .N = s.num_labels, .K = kc}, st));
   }
 #undef EVT_STAGE
-#undef EVT_TRY
   return EVT_OK;
 }
 
@@ -675,8 +636,8 @@ extern "C" int evt_gemm_residual_layernorm_ex(const void* A, int64_t lda, const 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (gemm_rowln_supported(M, N, K, copy_ln != 0))
     return gemm_rowln_launch(A, lda, W, ldw, bias, resid, ldr, gamma, beta, eps, copy_ln != 0, xn, ldxn, M, N, K, st);
-  rc = gemm_launch(A, lda, W, ldw, EVT_BF16, bias, resid, ldr, 0, 0, resid, EVT_F32, ldr, 0, 0, 0, M, N, K, EVT_ACT_NONE, st);
-  if (rc != EVT_OK) return rc;
+  EVT_TRY(gemm_launch({.A = A, .lda = lda, .W = W, .ldw = ldw, .bias = bias, .residual = resid, .ldr = ldr, .out = resid,
+                       .out_dtype = EVT_F32, .ldo = ldr, .M = M, .N = N, .K = K}, st));
   return layernorm_launch(resid, ldr, gamma, beta, xn, EVT_BF16, ldxn, copy_ln ? resid : nullptr, M, N, eps, st);
 }
 

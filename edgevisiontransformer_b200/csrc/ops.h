@@ -1,13 +1,35 @@
-// Internal launchers shared between the op-level C ABI and the model runtime.
+// Internal launchers shared between the op-level C ABI and the model runtimes.
 #pragma once
 #include "common.h"
 
 namespace evt {
 
-int gemm_launch(const void* A, int64_t lda, const void* W, int64_t ldw, int in_dtype, const float* bias,
-                const float* residual, int64_t ldr, int res_row_mod, int res_row_off, void* out, int out_dtype,
-                int64_t ldo, int out_group, int out_group_stride, int out_group_off, int64_t M, int N, int K, int act,
-                cudaStream_t stream);
+// out[M, N] = act(A[M, K] W[N, K]^T + bias) (+ residual), row-major with leading dimensions in elements.  Call sites name the
+// fields with designated initializers, in declaration order.
+struct GemmOp {
+  // Rows of out and of the residual for outputs that are not one dense block (evt_gemm_bias_act in include/evt.h); the default
+  // is the identity.
+  struct RowMap {
+    int res_row_mod = 0, res_row_off = 0;
+    int out_group = 0, out_group_stride = 0, out_group_off = 0;
+  };
+  const void* A = nullptr;
+  int64_t lda = 0;
+  const void* W = nullptr;
+  int64_t ldw = 0;
+  int in_dtype = EVT_BF16;  // EVT_BF16 (kind::f16) or EVT_F32 (kind::tf32: operands read as fp32, truncated to tf32 by the MMA)
+  const float* bias = nullptr;
+  const float* residual = nullptr;
+  int64_t ldr = 0;
+  void* out = nullptr;
+  int out_dtype = EVT_BF16;
+  int64_t ldo = 0;
+  int64_t M = 0;
+  int N = 0, K = 0;
+  int act = EVT_ACT_NONE;
+  RowMap map = {};
+};
+int gemm_launch(const GemmOp& op, cudaStream_t stream);
 
 // x <- x + A W^T + bias (f32 residual stream, in place) and xn <- LayerNorm(x) gamma + beta (bf16) for row lengths 192 / 384,
 // with whole rows resident in tensor memory (gemm_rowln.cu); copy_ln: the residual stream receives the normalised rows (TF
@@ -34,6 +56,13 @@ int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, cons
 int embed_fill_launch(const float* prefix, const float* pos, const float* bias, float* out, int B, int tokens, int n_prefix, int D,
                       cudaStream_t st);
 int im2col4_launch(const float* pixels, void* cols, int B, int H, int W, int P, cudaStream_t st);  // swin.cu, P % 4 == 0
+// swin.cu: evt_gather_layernorm, evt_window_attention_fwd and evt_layernorm_mean_tokens without the device check
+int gather_layernorm_launch(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype, float* copy_f32,
+                            int64_t images, int T_in, int T_out, int G, int C, float eps, cudaStream_t st);
+int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                            int window_tokens, int heads, int head_size, float scale, cudaStream_t st);
+int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
+                                 cudaStream_t st);
 int prefix_tokens_launch(const float* prefix, const float* pos, float* out, int B, int tokens, int n_prefix, int D,
                          cudaStream_t st);
 int cast_launch(const float* x, void* y, int64_t n, cudaStream_t st);

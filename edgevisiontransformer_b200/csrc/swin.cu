@@ -20,7 +20,7 @@
 #include <cuda_bf16.h>
 #include <math_constants.h>
 
-#include "common.h"
+#include "ops.h"
 #include "ptx.cuh"
 
 namespace evt {
@@ -446,15 +446,8 @@ int im2col4_launch(const float* pixels, void* cols, int B, int H, int W, int P, 
   return EVT_OK;
 }
 
-}  // namespace evt
-
-using namespace evt;
-
-extern "C" int evt_gather_layernorm(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype,
-                                    float* copy_f32, int64_t images, int T_in, int T_out, int G, int C, float eps,
-                                    evt_stream stream) {
-  int rc = evt_device_check();
-  if (rc != EVT_OK) return rc;
+int gather_layernorm_launch(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype, float* copy_f32,
+                            int64_t images, int T_in, int T_out, int G, int C, float eps, cudaStream_t st) {
   EVT_CHECK_ARG(x && idx, "gather_layernorm: null pointer");
   EVT_CHECK_ARG(y != nullptr || copy_f32 != nullptr, "gather_layernorm: nothing to write");
   EVT_CHECK_ARG(y == nullptr || (gamma && beta), "gather_layernorm: LayerNorm output needs gamma and beta");
@@ -464,7 +457,6 @@ extern "C" int evt_gather_layernorm(const float* x, const int* idx, const float*
   EVT_CHECK_ARG(eps >= 0.f, "gather_layernorm: negative eps");
   const long long rows = images * T_out;
   const int D = G * C;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (G == 1 && C == 96) return launch_gather_ln_sub<8, 3>(x, idx, gamma, beta, y, y_dtype, copy_f32, rows, T_in, T_out, eps, st);
   if (G == 1 && C == 192) return launch_gather_ln_sub<16, 3>(x, idx, gamma, beta, y, y_dtype, copy_f32, rows, T_in, T_out, eps, st);
   const int nv = (D + 127) / 128;
@@ -476,11 +468,8 @@ extern "C" int evt_gather_layernorm(const float* x, const int* idx, const float*
   return launch_gather_ln<24>(x, idx, gamma, beta, y, y_dtype, copy_f32, rows, T_in, T_out, G, C, eps, st);
 }
 
-extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab,
-                                        int64_t n_windows, int window_tokens, int heads, int head_size, float scale,
-                                        evt_stream stream) {
-  int rc = evt_device_check();
-  if (rc != EVT_OK) return rc;
+int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                            int window_tokens, int heads, int head_size, float scale, cudaStream_t st) {
   EVT_CHECK_ARG(qkv && ctx && table, "window_attention: null pointer");
   EVT_CHECK_ARG(n_windows > 0 && heads > 0 && n_tab > 0, "window_attention: sizes must be positive");
   if (window_tokens != kWTok || head_size != kWHd)
@@ -490,17 +479,11 @@ extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx,
   EVT_CHECK_ARG(ldc % 2 == 0 && reinterpret_cast<uintptr_t>(ctx) % 4 == 0, "window_attention: ctx rows must be 4-byte aligned");
   const long long items = n_windows * heads;
   const int smem = kWWarps * 3 * kWMatBytes;
-  static int configured_dev = -1;
-  int dev = 0;
-  EVT_CUDA(cudaGetDevice(&dev));
-  if (configured_dev != dev) {
-    EVT_CUDA(cudaFuncSetAttribute(window_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured_dev = dev;
-  }
+  EVT_TRY(opt_in_smem<window_attention_kernel>(smem));
   const long long ctas_needed = (items + kWWarps - 1) / kWWarps;
   const long long cap = static_cast<long long>(num_sms()) * 4;  // 4 CTAs of 48 KB per SM, grid-stride over the rest
   const unsigned grid = static_cast<unsigned>(ctas_needed < cap ? ctas_needed : cap);
-  EVT_CUDA(launch_pdl(window_attention_kernel, dim3(grid), dim3(kWWarps * 32), smem, static_cast<cudaStream_t>(stream),
+  EVT_CUDA(launch_pdl(window_attention_kernel, dim3(grid), dim3(kWWarps * 32), smem, st,
                       pdl_for_work(n_windows * kWTok, static_cast<long long>(heads) * kWHd), reinterpret_cast<const __nv_bfloat16*>(qkv), static_cast<long long>(ldq),
                       reinterpret_cast<__nv_bfloat16*>(ctx), static_cast<long long>(ldc), table, n_tab, heads, items,
                       scale * 1.4426950408889634f));
@@ -508,13 +491,10 @@ extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx,
   return EVT_OK;
 }
 
-extern "C" int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T,
-                                         int D, float eps, evt_stream stream) {
-  int rc = evt_device_check();
-  if (rc != EVT_OK) return rc;
+int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
+                                 cudaStream_t st) {
   EVT_CHECK_ARG(x && gamma && beta && y, "layernorm_mean_tokens: null pointer");
   EVT_CHECK_ARG(images > 0 && T > 0 && D > 0 && D % 4 == 0 && D <= 1536, "layernorm_mean_tokens: D must be a multiple of 4, <= 1536");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const dim3 grid(static_cast<unsigned>(images));
   __nv_bfloat16* yo = reinterpret_cast<__nv_bfloat16*>(y);
   const int nv = (D + 127) / 128;
@@ -523,4 +503,31 @@ extern "C" int evt_layernorm_mean_tokens(const float* x, const float* gamma, con
   else EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<12>, grid, dim3(256), 0, st, false, x, gamma, beta, yo, T, D, eps));
   EVT_LAUNCH_CHECK("ln_mean_tokens_kernel");
   return EVT_OK;
+}
+
+}  // namespace evt
+
+extern "C" int evt_gather_layernorm(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype,
+                                    float* copy_f32, int64_t images, int T_in, int T_out, int G, int C, float eps,
+                                    evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::gather_layernorm_launch(x, idx, gamma, beta, y, y_dtype, copy_f32, images, T_in, T_out, G, C, eps,
+                                      static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab,
+                                        int64_t n_windows, int window_tokens, int heads, int head_size, float scale,
+                                        evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::window_attention_launch(qkv, ldq, ctx, ldc, table, n_tab, n_windows, window_tokens, heads, head_size, scale,
+                                      static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T,
+                                         int D, float eps, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::layernorm_mean_tokens_launch(x, gamma, beta, y, images, T, D, eps, static_cast<cudaStream_t>(stream));
 }

@@ -7,28 +7,20 @@
 //
 // Data layout (see modeling_swin.py): inside a stage the f32 residual stream [B*T, C] is kept in the WINDOW ORDER of the
 // current block.  A block whose cyclic shift differs from the previous one starts with a row gather fused into its
-// layernorm_before (evt_gather_layernorm); patch merging is the same kernel with a 4-row gather.
+// layernorm_before (gather_layernorm_launch); patch merging is the same kernel with a 4-row gather.
 #include <cuda_bf16.h>
 
 #include <cmath>
-#include <cstring>
-#include <map>
 #include <string>
 #include <vector>
 
+#include "loader.h"
 #include "ops.h"
 
 namespace evt {
 namespace {
 
 constexpr float kLog2e = 1.4426950408889634f;
-
-__global__ void __launch_bounds__(256) swin_convert_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, long long n) {
-  const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (t < n) dst[t] = __float2bfloat16_rn(src[t]);
-}
-
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // raster index (y*W + x) of every position of the window order: r = ((wh*nWw + ww)*ws + i)*ws + j holds the token at
 // y = (wh*ws + i + shift) % H, x = (ww*ws + j + shift) % W   (roll by -shift, then window_partition; SwinLayer.forward :606-613)
@@ -123,105 +115,28 @@ using namespace evt;
 
 namespace {
 
-struct SwinLoader {
-  evt_swin* m;
-  std::map<std::string, const evt_tensor_view*> by_name;
-  cudaStream_t st;
-  static int64_t numel(const evt_tensor_view* v) {
-    int64_t n = 1;
-    for (int i = 0; i < v->ndim; ++i) n *= v->shape[i];
-    return n;
-  }
-  int need(const std::string& name, int64_t n, const evt_tensor_view** out) const {
-    auto it = by_name.find(name);
-    if (it == by_name.end()) return fail(EVT_ERR_INVALID, "missing weight '" + name + "'");
-    if (!it->second->data) return fail(EVT_ERR_INVALID, "weight '" + name + "' has a null data pointer");
-    if (numel(it->second) != n)
-      return fail(EVT_ERR_INVALID, "weight '" + name + "' has " + std::to_string(numel(it->second)) + " elements, expected " + std::to_string(n));
-    *out = it->second;
-    return EVT_OK;
-  }
-  int alloc(size_t bytes, void** out) {
-    void* p = nullptr;
-    cudaError_t e = cudaMalloc(&p, std::max<size_t>(bytes, 16));
-    if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("cudaMalloc: ") + cudaGetErrorString(e));
-    m->allocs.push_back(p);
-    *out = p;
-    return EVT_OK;
-  }
-  int vec(const std::string& name, int64_t n, float** out) {
-    const evt_tensor_view* v;
-    int rc = need(name, n, &v);
-    if (rc) return rc;
-    void* p;
-    rc = alloc(n * 4, &p);
-    if (rc) return rc;
-    EVT_CUDA(cudaMemcpyAsync(p, v->data, n * 4, cudaMemcpyDeviceToDevice, st));
-    *out = reinterpret_cast<float*>(p);
-    return EVT_OK;
-  }
-  int bf16_into(const std::string& name, int64_t n, __nv_bfloat16* dst) {
-    const evt_tensor_view* v;
-    int rc = need(name, n, &v);
-    if (rc) return rc;
-    swin_convert_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float*>(v->data), dst, n);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(EVT_ERR_CUDA, std::string("swin_convert: ") + cudaGetErrorString(e));
-    return EVT_OK;
-  }
-  int bf16(const std::string& name, int64_t n, __nv_bfloat16** out) {
-    void* p;
-    int rc = alloc(n * 2, &p);
-    if (rc) return rc;
-    *out = reinterpret_cast<__nv_bfloat16*>(p);
-    return bf16_into(name, n, *out);
-  }
-  template <typename T>
-  int upload(const std::vector<T>& h, T** out) {
-    void* p;
-    int rc = alloc(h.size() * sizeof(T), &p);
-    if (rc) return rc;
-    EVT_CUDA(cudaMemcpyAsync(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, st));
-    EVT_CUDA(cudaStreamSynchronize(st));  // the host vector goes out of scope
-    *out = reinterpret_cast<T*>(p);
-    return EVT_OK;
-  }
-  int host_copy(const std::string& name, int64_t n, std::vector<float>* out) {
-    const evt_tensor_view* v;
-    int rc = need(name, n, &v);
-    if (rc) return rc;
-    out->resize(n);
-    EVT_CUDA(cudaMemcpyAsync(out->data(), v->data, n * 4, cudaMemcpyDeviceToHost, st));
-    EVT_CUDA(cudaStreamSynchronize(st));
-    return EVT_OK;
-  }
-};
-
 struct SwinWs {
   uint8_t *cols, *xn, *qkv, *ctx, *h, *pooled;
   float *ra, *rb;
   size_t bytes;
 };
 
-SwinWs plan(const evt_swin* m, int batch, void* base) {
+SwinWs plan(const evt_swin* m, int batch, uint8_t* base) {
   const evt_swin_spec& s = m->spec;
   const size_t T0 = static_cast<size_t>(m->grid) * m->grid * batch;
   const size_t C0 = s.embed_dim;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    size_t o = off;
-    off = align_up(off + bytes, 1024);
-    return o;
-  };
-  uint8_t* b = reinterpret_cast<uint8_t*>(base);
+  WorkspaceCarver c{base};
   SwinWs w;
   // T * C is largest in stage 1 and halves with every patch merging
-  const size_t o_cols = take(T0 * m->patch_ld * 2), o_ra = take(T0 * C0 * 4), o_rb = take(T0 * C0 * 4), o_xn = take(T0 * C0 * 2);
-  const size_t o_qkv = take(T0 * 3 * C0 * 2), o_ctx = take(T0 * C0 * 2), o_h = take(T0 * 4 * C0 * 2);
-  const size_t o_pool = take(static_cast<size_t>(batch) * C0 * (1u << (s.stages - 1)) * 2);
-  w.cols = b + o_cols, w.ra = reinterpret_cast<float*>(b + o_ra), w.rb = reinterpret_cast<float*>(b + o_rb), w.xn = b + o_xn;
-  w.qkv = b + o_qkv, w.ctx = b + o_ctx, w.h = b + o_h, w.pooled = b + o_pool;
-  w.bytes = off;
+  w.cols = c.take(T0 * m->patch_ld * 2);
+  w.ra = c.take<float>(T0 * C0 * 4);
+  w.rb = c.take<float>(T0 * C0 * 4);
+  w.xn = c.take(T0 * C0 * 2);
+  w.qkv = c.take(T0 * 3 * C0 * 2);
+  w.ctx = c.take(T0 * C0 * 2);
+  w.h = c.take(T0 * 4 * C0 * 2);
+  w.pooled = c.take(static_cast<size_t>(batch) * C0 * (1u << (s.stages - 1)) * 2);
+  w.bytes = c.bytes;
   return w;
 }
 
@@ -262,29 +177,16 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
   EVT_CHECK_ARG(m != nullptr && tensors != nullptr && n > 0, "evt_swin_load_weights: bad arguments");
   if (m->loaded) return fail(EVT_ERR_STATE, "weights already loaded; create a new model to reload");
   const evt_swin_spec& s = m->spec;
-  SwinLoader L;
-  L.m = m;
-  L.st = static_cast<cudaStream_t>(stream);
-  for (int i = 0; i < n; ++i) {
-    EVT_CHECK_ARG(tensors[i].name != nullptr, "tensor view without a name");
-    L.by_name[tensors[i].name] = &tensors[i];
-  }
-  int rc;
-#define EVT_TRY(expr)            \
-  do {                           \
-    rc = (expr);                 \
-    if (rc != EVT_OK) return rc; \
-  } while (0)
-  const int ws = s.window, N = ws * ws;
+  Loader L{&m->allocs, static_cast<cudaStream_t>(stream), 2};
+  EVT_TRY(L.index(tensors, n));
+  const int ws = s.window;
   const std::string e = "swin.embeddings.";
   const int C0 = s.embed_dim;
-  {  // patch-embedding weight [C0, 3, 4, 4] -> bf16 [C0, patch_ld] (K = 48 is already a multiple of 8)
-    EVT_CHECK_ARG(m->patch_ld == m->patch_k, "patch embedding K must be a multiple of 8");
-    EVT_TRY(L.bf16(e + "patch_embeddings.projection.weight", static_cast<int64_t>(C0) * m->patch_k, &m->w_patch));
-  }
-  EVT_TRY(L.vec(e + "patch_embeddings.projection.bias", C0, &m->b_patch));
-  EVT_TRY(L.vec(e + "norm.weight", C0, &m->g_embed));
-  EVT_TRY(L.vec(e + "norm.bias", C0, &m->b_embed));
+  // patch-embedding weight [C0, 3, 4, 4] -> bf16 [C0, patch_ld]
+  EVT_TRY(L.mat(e + "patch_embeddings.projection.weight", C0, m->patch_k, m->patch_ld, &m->w_patch));
+  EVT_TRY(L.vec(e + "patch_embeddings.projection.bias", C0, false, &m->b_patch));
+  EVT_TRY(L.vec(e + "norm.weight", C0, false, &m->g_embed));
+  EVT_TRY(L.vec(e + "norm.bias", C0, false, &m->b_embed));
   int H = m->grid;
   std::vector<int> order(static_cast<size_t>(H) * H);
   for (size_t i = 0; i < order.size(); ++i) order[i] = static_cast<int>(i);  // raster after the patch embedding
@@ -315,8 +217,8 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
         EVT_TRY(L.upload(idx, &blk.idx));
         order = want;
       }
-      EVT_TRY(L.vec(p + "layernorm_before.weight", C, &blk.ln1_g));
-      EVT_TRY(L.vec(p + "layernorm_before.bias", C, &blk.ln1_b));
+      EVT_TRY(L.vec(p + "layernorm_before.weight", C, false, &blk.ln1_g));
+      EVT_TRY(L.vec(p + "layernorm_before.bias", C, false, &blk.ln1_b));
       void* q;
       EVT_TRY(L.alloc(static_cast<size_t>(3) * C * C * 2, &q));
       blk.wqkv = reinterpret_cast<__nv_bfloat16*>(q);
@@ -324,10 +226,8 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
       blk.bqkv = reinterpret_cast<float*>(q);
       const char* names[3] = {"query", "key", "value"};
       for (int t = 0; t < 3; ++t) {
-        EVT_TRY(L.bf16_into(p + "attention.self." + names[t] + ".weight", static_cast<int64_t>(C) * C, blk.wqkv + static_cast<size_t>(t) * C * C));
-        const evt_tensor_view* v;
-        EVT_TRY(L.need(p + "attention.self." + names[t] + ".bias", C, &v));
-        EVT_CUDA(cudaMemcpyAsync(blk.bqkv + t * C, v->data, C * 4, cudaMemcpyDeviceToDevice, L.st));
+        EVT_TRY(L.mat_into(p + "attention.self." + names[t] + ".weight", C, C, C, blk.wqkv + static_cast<size_t>(t) * C * C));
+        EVT_TRY(L.vec_into(p + "attention.self." + names[t] + ".bias", C, false, blk.bqkv + t * C));
       }
       std::vector<float> bias_table;
       EVT_TRY(L.host_copy(p + "attention.self.relative_position_bias_table", static_cast<int64_t>(2 * ws - 1) * (2 * ws - 1) * stg.heads, &bias_table));
@@ -339,14 +239,14 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
         blk.n_tab = 1;
         EVT_TRY(L.upload(attention_table(bias_table, stg.heads, ws, nullptr, 1), &blk.table));
       }
-      EVT_TRY(L.bf16(p + "attention.output.dense.weight", static_cast<int64_t>(C) * C, &blk.wo));
-      EVT_TRY(L.vec(p + "attention.output.dense.bias", C, &blk.bo));
-      EVT_TRY(L.vec(p + "layernorm_after.weight", C, &blk.ln2_g));
-      EVT_TRY(L.vec(p + "layernorm_after.bias", C, &blk.ln2_b));
-      EVT_TRY(L.bf16(p + "intermediate.dense.weight", static_cast<int64_t>(4) * C * C, &blk.w1));
-      EVT_TRY(L.vec(p + "intermediate.dense.bias", 4 * C, &blk.b1));
-      EVT_TRY(L.bf16(p + "output.dense.weight", static_cast<int64_t>(4) * C * C, &blk.w2));
-      EVT_TRY(L.vec(p + "output.dense.bias", C, &blk.b2));
+      EVT_TRY(L.mat(p + "attention.output.dense.weight", C, C, C, &blk.wo));
+      EVT_TRY(L.vec(p + "attention.output.dense.bias", C, false, &blk.bo));
+      EVT_TRY(L.vec(p + "layernorm_after.weight", C, false, &blk.ln2_g));
+      EVT_TRY(L.vec(p + "layernorm_after.bias", C, false, &blk.ln2_b));
+      EVT_TRY(L.mat(p + "intermediate.dense.weight", 4 * C, C, C, &blk.w1));
+      EVT_TRY(L.vec(p + "intermediate.dense.bias", 4 * C, false, &blk.b1));
+      EVT_TRY(L.mat(p + "output.dense.weight", C, 4 * C, 4 * C, &blk.w2));
+      EVT_TRY(L.vec(p + "output.dense.bias", C, false, &blk.b2));
     }
     if (si + 1 < s.stages) {
       // SwinPatchMerging (:326-349): rows (2y, 2x), (2y+1, 2x), (2y, 2x+1), (2y+1, 2x+1) concatenated; the next stage starts in
@@ -364,20 +264,18 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
       }
       stg.merge = true;
       EVT_TRY(L.upload(idx, &stg.m_idx));
-      EVT_TRY(L.vec(p + "norm.weight", 4 * C, &stg.m_g));
-      EVT_TRY(L.vec(p + "norm.bias", 4 * C, &stg.m_b));
-      EVT_TRY(L.bf16(p + "reduction.weight", static_cast<int64_t>(2) * C * 4 * C, &stg.m_w));
+      EVT_TRY(L.vec(p + "norm.weight", 4 * C, false, &stg.m_g));
+      EVT_TRY(L.vec(p + "norm.bias", 4 * C, false, &stg.m_b));
+      EVT_TRY(L.mat(p + "reduction.weight", 2 * C, 4 * C, 4 * C, &stg.m_w));
       order = nxt;
       H = H2;
     }
   }
   const int Cf = C0 << (s.stages - 1);
-  EVT_TRY(L.vec("swin.layernorm.weight", Cf, &m->g_final));
-  EVT_TRY(L.vec("swin.layernorm.bias", Cf, &m->b_final));
-  EVT_TRY(L.bf16("classifier.weight", static_cast<int64_t>(s.num_labels) * Cf, &m->w_cls));
-  EVT_TRY(L.vec("classifier.bias", s.num_labels, &m->b_cls));
-#undef EVT_TRY
-  (void)N;
+  EVT_TRY(L.vec("swin.layernorm.weight", Cf, false, &m->g_final));
+  EVT_TRY(L.vec("swin.layernorm.bias", Cf, false, &m->b_final));
+  EVT_TRY(L.mat("classifier.weight", s.num_labels, Cf, Cf, &m->w_cls));
+  EVT_TRY(L.vec("classifier.bias", s.num_labels, false, &m->b_cls));
   EVT_CUDA(cudaStreamSynchronize(L.st));
   m->loaded = true;
   return EVT_OK;
@@ -402,26 +300,19 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
   if (!m->loaded) return fail(EVT_ERR_STATE, "evt_swin_forward called before evt_swin_load_weights");
   EVT_CHECK_ARG(batch > 0 && batch <= 65535, "batch must be in 1..65535");
   const evt_swin_spec& s = m->spec;
-  void* base = reinterpret_cast<void*>(align_up(reinterpret_cast<uintptr_t>(workspace), 1024));
-  const size_t slack = reinterpret_cast<uintptr_t>(base) - reinterpret_cast<uintptr_t>(workspace);
-  SwinWs w = plan(m, batch, base);
-  EVT_CHECK_ARG(w.bytes + slack <= workspace_bytes, "workspace too small for this batch (see evt_swin_workspace_bytes)");
+  SwinWs w;
+  EVT_TRY(place_workspace(workspace, workspace_bytes, [&](uint8_t* base) { return plan(m, batch, base); }, &w,
+                          "workspace too small for this batch (see evt_swin_workspace_bytes)"));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   StaticWeightsScope weights_are_static;
-  int rc;
-#define EVT_TRY(expr)            \
-  do {                           \
-    rc = (expr);                 \
-    if (rc != EVT_OK) return rc; \
-  } while (0)
   const float eps = s.eps;
   const float scale = 1.0f / sqrtf(32.f);
   int T = m->grid * m->grid;
   // SwinEmbeddings (:262-301): 4 x 4 patch conv as im2col + GEMM, LayerNorm, rows gathered into the first window order
   EVT_TRY(im2col4_launch(pixels, w.cols, batch, s.image, s.image, s.patch, st));
-  EVT_TRY(gemm_launch(w.cols, m->patch_ld, m->w_patch, m->patch_ld, EVT_BF16, m->b_patch, nullptr, 0, 0, 0, w.rb, EVT_F32, s.embed_dim, 0, 0, 0,
-                      static_cast<int64_t>(batch) * T, s.embed_dim, m->patch_k, EVT_ACT_NONE, st));
-  EVT_TRY(evt_gather_layernorm(w.rb, m->idx_embed, m->g_embed, m->b_embed, w.ra, EVT_F32, nullptr, batch, T, T, 1, s.embed_dim, eps, stream));
+  EVT_TRY(gemm_launch({.A = w.cols, .lda = m->patch_ld, .W = m->w_patch, .ldw = m->patch_ld, .bias = m->b_patch, .out = w.rb,
+                       .out_dtype = EVT_F32, .ldo = s.embed_dim, .M = static_cast<int64_t>(batch) * T, .N = s.embed_dim, .K = m->patch_k}, st));
+  EVT_TRY(gather_layernorm_launch(w.rb, m->idx_embed, m->g_embed, m->b_embed, w.ra, EVT_F32, nullptr, batch, T, T, 1, s.embed_dim, eps, st));
   float* resid = w.ra;
   float* other = w.rb;
   for (int si = 0; si < s.stages; ++si) {
@@ -430,31 +321,34 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
     const int64_t M = static_cast<int64_t>(batch) * T;
     for (const SwinBlock& blk : stg.blocks) {
       if (blk.idx != nullptr) {  // cyclic shift / reverse shift folded into layernorm_before; the residual stream is re-ordered too
-        EVT_TRY(evt_gather_layernorm(resid, blk.idx, blk.ln1_g, blk.ln1_b, w.xn, EVT_BF16, other, batch, T, T, 1, C, eps, stream));
+        EVT_TRY(gather_layernorm_launch(resid, blk.idx, blk.ln1_g, blk.ln1_b, w.xn, EVT_BF16, other, batch, T, T, 1, C, eps, st));
         std::swap(resid, other);
       } else {
         EVT_TRY(layernorm_launch(resid, C, blk.ln1_g, blk.ln1_b, w.xn, EVT_BF16, C, nullptr, M, C, eps, st));
       }
-      EVT_TRY(gemm_launch(w.xn, C, blk.wqkv, C, EVT_BF16, blk.bqkv, nullptr, 0, 0, 0, w.qkv, EVT_BF16, 3 * C, 0, 0, 0, M, 3 * C, C, EVT_ACT_NONE, st));
-      EVT_TRY(evt_window_attention_fwd(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / 49, 49, stg.heads, 32, scale, stream));
-      EVT_TRY(gemm_launch(w.ctx, C, blk.wo, C, EVT_BF16, blk.bo, resid, C, 0, 0, resid, EVT_F32, C, 0, 0, 0, M, C, C, EVT_ACT_NONE, st));
+      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.wqkv, .ldw = C, .bias = blk.bqkv, .out = w.qkv, .out_dtype = EVT_BF16, .ldo = 3 * C,
+                           .M = M, .N = 3 * C, .K = C}, st));
+      EVT_TRY(window_attention_launch(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / 49, 49, stg.heads, 32, scale, st));
+      EVT_TRY(gemm_launch({.A = w.ctx, .lda = C, .W = blk.wo, .ldw = C, .bias = blk.bo, .residual = resid, .ldr = C, .out = resid,
+                           .out_dtype = EVT_F32, .ldo = C, .M = M, .N = C, .K = C}, st));
       EVT_TRY(layernorm_launch(resid, C, blk.ln2_g, blk.ln2_b, w.xn, EVT_BF16, C, nullptr, M, C, eps, st));
-      EVT_TRY(gemm_launch(w.xn, C, blk.w1, C, EVT_BF16, blk.b1, nullptr, 0, 0, 0, w.h, EVT_BF16, 4 * C, 0, 0, 0, M, 4 * C, C, EVT_ACT_GELU_ERF, st));
-      EVT_TRY(gemm_launch(w.h, 4 * C, blk.w2, 4 * C, EVT_BF16, blk.b2, resid, C, 0, 0, resid, EVT_F32, C, 0, 0, 0, M, C, 4 * C, EVT_ACT_NONE, st));
+      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.w1, .ldw = C, .bias = blk.b1, .out = w.h, .out_dtype = EVT_BF16, .ldo = 4 * C,
+                           .M = M, .N = 4 * C, .K = C, .act = EVT_ACT_GELU_ERF}, st));
+      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = blk.w2, .ldw = 4 * C, .bias = blk.b2, .residual = resid, .ldr = C, .out = resid,
+                           .out_dtype = EVT_F32, .ldo = C, .M = M, .N = C, .K = 4 * C}, st));
     }
     if (stg.merge) {
       // 2 x 2 neighbourhood concat + LayerNorm(4C) as one gather, then the bias-free reduction to 2C
-      EVT_TRY(evt_gather_layernorm(resid, stg.m_idx, stg.m_g, stg.m_b, w.h, EVT_BF16, nullptr, batch, T, T / 4, 4, C, eps, stream));
+      EVT_TRY(gather_layernorm_launch(resid, stg.m_idx, stg.m_g, stg.m_b, w.h, EVT_BF16, nullptr, batch, T, T / 4, 4, C, eps, st));
       T /= 4;
-      EVT_TRY(gemm_launch(w.h, 4 * C, stg.m_w, 4 * C, EVT_BF16, nullptr, nullptr, 0, 0, 0, other, EVT_F32, 2 * C, 0, 0, 0,
-                          static_cast<int64_t>(batch) * T, 2 * C, 4 * C, EVT_ACT_NONE, st));
+      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = stg.m_w, .ldw = 4 * C, .out = other, .out_dtype = EVT_F32, .ldo = 2 * C,
+                           .M = static_cast<int64_t>(batch) * T, .N = 2 * C, .K = 4 * C}, st));
       std::swap(resid, other);
     }
   }
   const int Cf = s.embed_dim << (s.stages - 1);
-  EVT_TRY(evt_layernorm_mean_tokens(resid, m->g_final, m->b_final, w.pooled, batch, T, Cf, eps, stream));
-  EVT_TRY(gemm_launch(w.pooled, Cf, m->w_cls, Cf, EVT_BF16, m->b_cls, nullptr, 0, 0, 0, logits, EVT_F32, s.num_labels, 0, 0, 0, batch, s.num_labels,
-                      Cf, EVT_ACT_NONE, st));
-#undef EVT_TRY
+  EVT_TRY(layernorm_mean_tokens_launch(resid, m->g_final, m->b_final, w.pooled, batch, T, Cf, eps, st));
+  EVT_TRY(gemm_launch({.A = w.pooled, .lda = Cf, .W = m->w_cls, .ldw = Cf, .bias = m->b_cls, .out = logits, .out_dtype = EVT_F32,
+                       .ldo = s.num_labels, .M = batch, .N = s.num_labels, .K = Cf}, st));
   return EVT_OK;
 }
