@@ -76,6 +76,7 @@ SIGNATURES = {
     "evt_gemm_residual_layernorm_ex": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _p, _p, _f, _i, _p, _i64, _i64, _i, _i, _p]),
     "evt_attention_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _f, _p]),
     "evt_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _f, _p]),
+    "evt_attention_query_rows_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _i, _f, _p]),
     "evt_im2col_patch": (_i, [_p, _p, _i, _i, _i, _i, _p]),
     "evt_patch_embed_workspace_bytes": (_i, [_i, _i, _i, _i, _i, C.POINTER(C.c_size_t)]),
     "evt_patch_embed_fwd": (_i, [_p, _i, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p]),

@@ -14,6 +14,8 @@
 //                      (tcgen05.st), row sum; then O * 1/sum -> bf16 context through a swizzled staging tile and a
 //                      3-D TMA store.
 //
+// Sq <= S: only the first Sq query rows of every image are computed and stored (context [B, Sq, heads*64]); K and V are
+// still all S rows, so those rows come out exactly as in the full run (Sq = 1: the cls row of the last encoder layer).
 // SK = S rounded up to 16; key columns >= S are masked to probability 0, so the extra K/V rows the TMA box
 // picks up (next image's tokens, or zero fill past the end of the matrix) never contribute.
 // TMEM: 2 slots x 256 columns (S at [0,SK), P overlaid at [0,SK/2), O overlaid at [128,192)).
@@ -231,6 +233,7 @@ constexpr int kMaxKV = 4;
 struct Attn2Params {
   const float* head_mask;
   int S, SK, heads, B;
+  int Sq;        // query rows per image (S, or fewer: only rows < Sq are computed and stored)
   int n_mt;      // query tiles per work unit (q_tiles, or 1 when the tiles of a pair are split across CTAs)
   int q_tiles;   // query tiles per (image, head)
   int n_kv;      // K/V ring depth
@@ -436,7 +439,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       }
       const int mt = tile_of(p, u, ql, p.n_mt == 2 ? grp : 0);
       const int qrow0 = 32 * block_of(mt, quad, ql & 3);
-      const bool warp_live = qrow0 < p.S;  // block 7 (rows 224..255) when S = 197: nothing to do
+      const bool warp_live = qrow0 < p.Sq;  // block 7 (rows 224..255) when S = 197, or a block past Sq: nothing to do
       float hm = 1.f;
       if (p.head_mask != nullptr) hm = p.head_mask[u.h];
       ptx::mbar_wait(&s_ready[grp], ph);
@@ -687,10 +690,11 @@ attention_tf32_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 
 }  // namespace
 
-int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S,
+int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                      int heads, int head_size, float scale, cudaStream_t stream) {
   EVT_CHECK_ARG(qkv && ctx, "attention: null pointer");
   EVT_CHECK_ARG(B > 0 && S > 0 && heads > 0, "attention: B, S, heads must be positive");
+  EVT_CHECK_ARG(Sq > 0 && Sq <= S, "attention: query rows must be in 1..S");
   if (head_size != kHD) return fail(EVT_ERR_UNSUPPORTED, "attention: only head size 64 is implemented");
   if (S > 256) return fail(EVT_ERR_UNSUPPORTED, "attention: sequence length above 256 is not implemented");
   EVT_CHECK_ARG(ldq >= 3ll * heads * kHD && ldc >= static_cast<int64_t>(heads) * kHD, "attention: leading dimension too small");
@@ -698,7 +702,7 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");
   const int SK = (S + 15) / 16 * 16;
   const uint64_t rows = static_cast<uint64_t>(B) * S;
-  const int q_tiles = (S + kQRows - 1) / kQRows;
+  const int q_tiles = (Sq + kQRows - 1) / kQRows;
   const long long n_pairs = static_cast<long long>(B) * heads;
   const int n_mt = (q_tiles > 1 && n_pairs * q_tiles <= num_sms()) ? 1 : q_tiles;  // split the tiles across CTAs at small batch
   const float scale_log2e = scale * 1.4426950408889634f;
@@ -710,15 +714,17 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   int rc = make_tmap_2d(&tmKV, qkv, 2, rows, 3ull * heads * kHD, static_cast<uint64_t>(ldq), SK, kHD);
   if (rc != EVT_OK) return rc;
   CUtensorMap tmO, tmQ;
-  rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
-                         static_cast<uint64_t>(ldq), 32, kHD);
+  // Q: the first Sq rows of every image (rows past them arrive as zeros); context: Sq rows per image, packed
+  rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                         static_cast<uint64_t>(ldq), 32, kHD, static_cast<uint64_t>(S));
   if (rc != EVT_OK) return rc;
-  rc = make_tmap_3d_rows(&tmO, ctx, 2, static_cast<uint64_t>(heads) * kHD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
+  rc = make_tmap_3d_rows(&tmO, ctx, 2, static_cast<uint64_t>(heads) * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
                          static_cast<uint64_t>(ldc), 32, kHD);
   if (rc != EVT_OK) return rc;
   Attn2Params q;
   q.head_mask = head_mask;
   q.S = S;
+  q.Sq = Sq;
   q.SK = SK;
   q.heads = heads;
   q.B = B;
@@ -778,7 +784,16 @@ extern "C" int evt_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_
                                  int S, int heads, int head_size, float scale, evt_stream stream) {
   int rc = evt_device_check();
   if (rc != EVT_OK) return rc;
-  return evt::attention_launch(qkv, ldq, ctx, ldc, head_mask, B, S, heads, head_size, scale,
+  return evt::attention_launch(qkv, ldq, ctx, ldc, head_mask, B, S, S, heads, head_size, scale,
+                               static_cast<cudaStream_t>(stream));
+}
+
+// Only the first Sq query rows of every image (all S keys): ctx is [B*Sq, ldc].
+extern "C" int evt_attention_query_rows_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask,
+                                            int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::attention_launch(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, head_size, scale,
                                static_cast<cudaStream_t>(stream));
 }
 

@@ -88,14 +88,15 @@ int gemm_pair_mode() { return g_pair_mode.load(std::memory_order_relaxed); }
 // What the three map shapes share: the entry point, the alignment checks, the shape's own box check (`box_error`: null when the
 // box is valid), then the encode.  A box is box_rows x box_cols of one batch entry (rank 3) or of the whole matrix (rank 2).
 static int encode_tmap(CUtensorMap* out, const void* base, int elem_bytes, int rank, uint64_t cols, uint64_t rows, uint64_t batch,
-                       uint64_t ld, uint32_t box_rows, uint32_t box_cols, int swizzle_bytes, const char* box_error, const char* what) {
+                       uint64_t ld, uint32_t box_rows, uint32_t box_cols, int swizzle_bytes, const char* box_error, const char* what,
+                       uint64_t batch_rows = 0) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) return fail(EVT_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(EVT_ERR_INVALID, "TMA base pointer not 16-byte aligned");
   if ((ld * elem_bytes) % 16 != 0) return fail(EVT_ERR_INVALID, "TMA leading dimension not a multiple of 16 bytes");
   if (box_error) return fail(EVT_ERR_INVALID, box_error);
   const cuuint64_t dims[3] = {cols, rows, batch};
-  const cuuint64_t strides[2] = {ld * static_cast<uint64_t>(elem_bytes), rows * ld * static_cast<uint64_t>(elem_bytes)};
+  const cuuint64_t strides[2] = {ld * static_cast<uint64_t>(elem_bytes), (batch_rows ? batch_rows : rows) * ld * static_cast<uint64_t>(elem_bytes)};
   const cuuint32_t box[3] = {box_cols, box_rows, 1};
   const cuuint32_t estr[3] = {1, 1, 1};
   CUresult r = enc(out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, const_cast<void*>(base),
@@ -126,10 +127,11 @@ int make_tmap_2d_sw(CUtensorMap* out, const void* base, int elem_bytes, uint64_t
 }
 
 int make_tmap_3d_rows(CUtensorMap* out, const void* base, int elem_bytes, uint64_t cols, uint64_t rows, uint64_t batch,
-                      uint64_t ld, uint32_t box_rows, uint32_t box_cols) {
+                      uint64_t ld, uint32_t box_rows, uint32_t box_cols, uint64_t batch_rows) {
   const char* err = box_128_error(elem_bytes, box_rows, box_cols);
   if (!err && elem_bytes != 2) err = "3-D TMA map: bf16 only";
-  return encode_tmap(out, base, elem_bytes, 3, cols, rows, batch, ld, box_rows, box_cols, 128, err, " (3-D)");
+  if (!err && batch_rows != 0 && batch_rows < rows) err = "3-D TMA map: batch entries closer than their row count";
+  return encode_tmap(out, base, elem_bytes, 3, cols, rows, batch, ld, box_rows, box_cols, 128, err, " (3-D)", batch_rows);
 }
 
 }  // namespace evt

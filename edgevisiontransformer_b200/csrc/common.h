@@ -143,7 +143,8 @@ int make_tmap_2d_sw(CUtensorMap* out, const void* base, int elem_bytes, uint64_t
 // 3-D view [batch][rows][cols] of a row-major matrix of batch * rows rows (leading dimension ld): a box is box_rows x
 // box_cols of ONE batch entry, so rows past the end of an image are zero-filled on loads and clipped on stores instead of
 // running into the next image.  128-byte swizzle.
+// batch_rows: matrix rows from one batch entry to the next (0 = rows; more: only the first `rows` of each entry are in view).
 int make_tmap_3d_rows(CUtensorMap* out, const void* base, int elem_bytes, uint64_t cols, uint64_t rows, uint64_t batch,
-                      uint64_t ld, uint32_t box_rows, uint32_t box_cols);
+                      uint64_t ld, uint32_t box_rows, uint32_t box_cols, uint64_t batch_rows = 0);
 
 }  // namespace evt

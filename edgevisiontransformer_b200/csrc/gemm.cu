@@ -254,7 +254,41 @@ int dispatch_epi(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& 
   }
 }
 
+// TMA epilogue: contiguous output rows, 16-byte aligned, and the skip connection (if any) updated in place
+bool tma_out_ok(const GemmOp& op) {
+  const int oeb = op.out_dtype != EVT_BF16 ? 4 : 2;
+  return op.map.out_group == 0 && op.map.res_row_mod == 0 && reinterpret_cast<uintptr_t>(op.out) % 16 == 0 && (op.ldo * oeb) % 16 == 0 &&
+         (op.residual == nullptr || (oeb == 4 && op.residual == reinterpret_cast<const float*>(op.out) && op.ldr == op.ldo));
+}
+
+// Split K when a reduce-add epilogue leaves most SMs idle (out-proj / FC2 at batch 1: 6 tiles for 148 SMs).  The
+// partial products meet in the f32 residual stream through the same TMA reduce-add; their order is not fixed, so
+// results can differ in the last bit from run to run -- only in this small-M regime; evt_gemm_set_split_k(0) turns it
+// off, a forced kernel choice (evt_gemm_set_pair_mode) never splits, and op.max_k_splits bounds the count.
+// The tf32 (accuracy) mode never splits: DeiT-Tiny batch 1 would drop from 0.477 to 0.427 ms, but the unordered f32
+// reduce-adds flip tf32 roundings downstream and the logit error of BASELINE config 1 moves from a reproducible 7.5e-4
+// to 9.2e-4 in one run -- a random variable that close to the 1e-3 contract is not worth 0.05 ms.
+int k_splits(const GemmOp& op, bool tma_out, long tiles, int num_kb) {
+  if (op.in_dtype == EVT_F32 || !tma_out || op.residual == nullptr || gemm_pair_mode() >= 0 || !gemm_split_k_enabled()) return 1;
+  if (tiles * 2 > num_sms() || num_kb < 4) return 1;
+  int splits = static_cast<int>(num_sms() / tiles);
+  if (splits > num_kb / 2) splits = num_kb / 2;  // at least two K blocks per split
+  if (op.max_k_splits > 0 && splits > op.max_k_splits) splits = op.max_k_splits;
+  return splits > 1 ? splits : 1;
+}
+
 }  // namespace
+
+int gemm_k_splits(const GemmOp& op) {
+  const int k_step = kStageRowBytes / (op.in_dtype == EVT_F32 ? 4 : 2);
+  const int bn = choose_bn(op.M, op.N);
+  const long tiles = static_cast<long>((op.M + BM - 1) / BM) * ((op.N + bn - 1) / bn);
+  const int num_kb = (op.K + k_step - 1) / k_step;
+  const int splits = k_splits(op, tma_out_ok(op), tiles, num_kb);
+  if (splits == 1) return 1;
+  const int kb_per_split = (num_kb + splits - 1) / splits;
+  return (num_kb + kb_per_split - 1) / kb_per_split;
+}
 
 int gemm_launch(const GemmOp& op, cudaStream_t stream) {
   EVT_CHECK_ARG(op.A && op.W && op.out, "gemm: null pointer");
@@ -304,36 +338,20 @@ int gemm_launch(const GemmOp& op, cudaStream_t stream) {
   }
   const bool of32 = op.out_dtype != EVT_BF16;
   p.round_tf32 = op.out_dtype == EVT_TF32 ? 1 : 0;
-  // TMA epilogue: contiguous output rows, 16-byte aligned, and the skip connection (if any) updated in place
   const int oeb = of32 ? 4 : 2;
-  const bool tma_out = op.map.out_group == 0 && op.map.res_row_mod == 0 && reinterpret_cast<uintptr_t>(op.out) % 16 == 0 &&
-                       (op.ldo * oeb) % 16 == 0 &&
-                       (op.residual == nullptr || (of32 && op.residual == reinterpret_cast<const float*>(op.out) && op.ldr == op.ldo));
+  const bool tma_out = tma_out_ok(op);
   CUtensorMap tmO = tmA;
   if (tma_out) {
     rc = make_tmap_2d(&tmO, op.out, oeb, static_cast<uint64_t>(op.M), static_cast<uint64_t>(op.N), static_cast<uint64_t>(op.ldo), 32,
                       128 / oeb);
     if (rc != EVT_OK) return rc;
   }
-  // Split K when a reduce-add epilogue leaves most SMs idle (out-proj / FC2 at batch 1: 6 tiles for 148 SMs).  The
-  // partial products meet in the f32 residual stream through the same TMA reduce-add; their order is not fixed, so
-  // results can differ in the last bit from run to run -- only in this small-M regime; evt_gemm_set_split_k(0) turns it
-  // off, and a forced kernel choice (evt_gemm_set_pair_mode) never splits.
   p.k_splits = 1;
   p.kb_per_split = p.num_kb;
-  // The tf32 (accuracy) mode never splits: DeiT-Tiny batch 1 would drop from 0.477 to 0.427 ms, but the unordered f32
-  // reduce-adds flip tf32 roundings downstream and the logit error of BASELINE config 1 moves from a reproducible 7.5e-4
-  // to 9.2e-4 in one run -- a random variable that close to the 1e-3 contract is not worth 0.05 ms.
-  if (!tf32 && tma_out && op.residual != nullptr && gemm_pair_mode() < 0 && gemm_split_k_enabled()) {
-    const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
-    if (tiles * 2 <= num_sms() && p.num_kb >= 4) {
-      int splits = static_cast<int>(num_sms() / tiles);
-      if (splits > p.num_kb / 2) splits = p.num_kb / 2;  // at least two K blocks per split
-      if (splits > 1) {
-        p.kb_per_split = (p.num_kb + splits - 1) / splits;
-        p.k_splits = (p.num_kb + p.kb_per_split - 1) / p.kb_per_split;
-      }
-    }
+  const int splits = k_splits(op, tma_out, static_cast<long>(p.tiles_m) * p.tiles_n, p.num_kb);
+  if (splits > 1) {
+    p.kb_per_split = (p.num_kb + splits - 1) / splits;
+    p.k_splits = (p.num_kb + p.kb_per_split - 1) / p.kb_per_split;
   }
   // Large problems run on CTA pairs (cta_group::2, 256-row tiles): half the W traffic per SM.  evt_gemm_set_pair_mode
   // forces the choice (tests exercise both kernels on the same shapes).

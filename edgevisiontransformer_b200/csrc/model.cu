@@ -504,10 +504,31 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   // fit in tensor memory, so the LayerNorm that FOLLOWS each residual projection runs in that projection's epilogue
   // (gemm_rowln.cu): 5 launches per layer instead of 7 and the LayerNorm kernel's read of the f32 residual stream never happens.
   const bool row_ln = !tf32 && gemm_rowln_supported(M, D, D, tf);  // per projection: gemm_rowln_pays
+  // Classification-row tail: the head reads only row 0 of every image, and after the K / V of the last layer everything
+  // in that layer is row-wise, so its attention runs for the cls query alone (all keys), and the out-projection, LN2,
+  // FC1 and FC2 run on `batch` rows: row i is image i's cls row (residual stream stride tokens * D, context and FC1
+  // output packed).  Same launches, same kernels, so the cls row gets the same bits as in a full layer.  Full layer
+  // instead when a caller asks for the last layer's context of every row (ctx_out), in the tf32 mode (its attention
+  // kernel has no query-row count) and for the two-head distilled DeiT (rows 0 and 1 of every image are not one strided
+  // row set).
+  const int64_t tok_stride = static_cast<int64_t>(s.tokens) * D;
+  const bool cls_tail = !tf32 && s.head_rows <= 1 && !(o.ctx_out != nullptr && o.ctx_out[s.layers - 1] != nullptr);
   bool xn_ready = false;  // w.xn already holds LN1 of the current layer (written by the previous layer's FC2 epilogue)
   for (int l = 0; l < s.layers; ++l) {
     const LayerW& lw = m->layers[l];
     const int a = lw.a;
+    const bool tail = cls_tail && l == s.layers - 1;
+    const int64_t rows = tail ? batch : M;        // rows after attention
+    const int64_t rs = tail ? tok_stride : D;     // their stride in the residual stream
+    // A residual GEMM of the tail splits K only where the full-size one would: no unordered reduce-adds are added to a
+    // forward whose full-size launches have a fixed summation order.
+    auto on_rows = [&](GemmOp op) {
+      if (!tail) return op;
+      op.max_k_splits = gemm_k_splits(op) > 1 ? 0 : 1;
+      op.M = rows;
+      op.ldr = op.ldo = rs;
+      return op;
+    };
     if (!xn_ready)
       EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln1_g, lw.ln1_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
     EVT_STAGE(EVT_STAGE_QKV, gemm_launch({.A = w.xn, .lda = D, .W = lw.wqkv, .ldw = D, .in_dtype = dt, .bias = lw.bqkv, .out = w.qkv,
@@ -523,29 +544,29 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
       EVT_STAGE(EVT_STAGE_ATTN, attention_tf32_launch(reinterpret_cast<const float*>(w.qkv), 3 * a, reinterpret_cast<float*>(ctx), a, hmask,
                                     batch, s.tokens, s.heads[l], s.head_size, scale, st));
     else
-      EVT_STAGE(EVT_STAGE_ATTN, attention_launch(w.qkv, 3 * a, ctx, a, hmask, batch, s.tokens, s.heads[l], s.head_size, scale, st));
-    if (row_ln && gemm_rowln_pays(D, a, tf)) {
+      EVT_STAGE(EVT_STAGE_ATTN, attention_launch(w.qkv, 3 * a, ctx, a, hmask, batch, s.tokens, tail ? 1 : s.tokens, s.heads[l], s.head_size,
+                                                 scale, st));
+    if (!tail && row_ln && gemm_rowln_pays(D, a, tf)) {
       EVT_STAGE(EVT_STAGE_OPROJ, gemm_rowln_launch(ctx, a, lw.wo, a, lw.bo, w.resid, D, lw.ln2_g, lw.ln2_b, s.eps, tf, w.xn, D, M, D, a, st));
     } else {
-      EVT_STAGE(EVT_STAGE_OPROJ, gemm_launch({.A = ctx, .lda = a, .W = lw.wo, .ldw = a, .in_dtype = dt, .bias = lw.bo, .residual = w.resid,
-                                              .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D, .K = a}, st));
-      EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, D, lw.ln2_g, lw.ln2_b, w.xn, adt, D, tf ? w.resid : nullptr, M, D, s.eps, st));
+      EVT_STAGE(EVT_STAGE_OPROJ, gemm_launch(on_rows({.A = ctx, .lda = a, .W = lw.wo, .ldw = a, .in_dtype = dt, .bias = lw.bo, .residual = w.resid,
+                                                      .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D, .K = a}), st));
+      EVT_STAGE(EVT_STAGE_LN, layernorm_launch(w.resid, rs, lw.ln2_g, lw.ln2_b, w.xn, adt, D, tf ? w.resid : nullptr, rows, D, s.eps, st));
     }
     EVT_STAGE(EVT_STAGE_FC1, gemm_launch({.A = w.xn, .lda = D, .W = lw.w1, .ldw = D, .in_dtype = dt, .bias = lw.b1, .out = w.big,
-                                          .out_dtype = adt, .ldo = lw.inter_ld, .M = M, .N = lw.inter, .K = D, .act = s.act}, st));
+                                          .out_dtype = adt, .ldo = lw.inter_ld, .M = rows, .N = lw.inter, .K = D, .act = s.act}, st));
     if (row_ln && l + 1 < s.layers && gemm_rowln_pays(D, lw.inter, tf)) {
       const LayerW& nx = m->layers[l + 1];
       EVT_STAGE(EVT_STAGE_FC2, gemm_rowln_launch(w.big, lw.inter_ld, lw.w2, lw.inter_ld, lw.b2, w.resid, D, nx.ln1_g, nx.ln1_b, s.eps, tf, w.xn,
                                                  D, M, D, lw.inter, st));
       xn_ready = true;
     } else {
-      EVT_STAGE(EVT_STAGE_FC2, gemm_launch({.A = w.big, .lda = lw.inter_ld, .W = lw.w2, .ldw = lw.inter_ld, .in_dtype = dt, .bias = lw.b2,
-                                            .residual = w.resid, .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D,
-                                            .K = lw.inter}, st));
+      EVT_STAGE(EVT_STAGE_FC2, gemm_launch(on_rows({.A = w.big, .lda = lw.inter_ld, .W = lw.w2, .ldw = lw.inter_ld, .in_dtype = dt, .bias = lw.b2,
+                                                    .residual = w.resid, .ldr = D, .out = w.resid, .out_dtype = EVT_F32, .ldo = D, .M = M, .N = D,
+                                                    .K = lw.inter}), st));
     }
   }
   // head: only the cls row of every image is consumed (SITE/models/vit/modeling_vit.py:641)
-  const int64_t tok_stride = static_cast<int64_t>(s.tokens) * D;
   const int head_rows = s.head_rows > 1 ? s.head_rows : 1;
   if (s.final_ln) {
     // head_rows = 2 (DeiTForImageClassificationWithTeacher, SITE/models/deit/modeling_deit.py: logits = (cls_classifier(x[:, 0]) +

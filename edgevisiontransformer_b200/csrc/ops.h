@@ -28,8 +28,10 @@ struct GemmOp {
   int N = 0, K = 0;
   int act = EVT_ACT_NONE;
   RowMap map = {};
+  int max_k_splits = 0;  // upper bound on the K splits of a small-M reduce-add (0 = no bound; 1 = fixed summation order)
 };
 int gemm_launch(const GemmOp& op, cudaStream_t stream);
+int gemm_k_splits(const GemmOp& op);  // the K splits gemm_launch would use for `op` (1 = none)
 
 // x <- x + A W^T + bias (f32 residual stream, in place) and xn <- LayerNorm(x) gamma + beta (bf16) for row lengths 192 / 384,
 // with whole rows resident in tensor memory (gemm_rowln.cu); copy_ln: the residual stream receives the normalised rows (TF
@@ -40,7 +42,8 @@ int gemm_rowln_launch(const void* A, int64_t lda, const void* W, int64_t ldw, co
                       const float* gamma, const float* beta, float eps, bool copy_ln, void* xn, int64_t ldxn, int64_t M, int N,
                       int K, cudaStream_t stream);
 
-int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S,
+// Sq: query rows per image (1..S; S = all), K and V span all S rows; ctx receives Sq rows per image, packed
+int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                      int heads, int head_size, float scale, cudaStream_t stream);
 
 int attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask, int B, int S,

@@ -172,19 +172,28 @@ def linear_residual_layernorm(a: torch.Tensor, w: torch.Tensor, bias: Optional[t
 
 
 def attention(qkv: torch.Tensor, B: int, S: int, heads: int, head_size: int = 64, scale: Optional[float] = None,
-              head_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """qkv bf16 [B*S, 3*heads*head_size] (q | k | v blocks) -> ctx bf16 [B*S, heads*head_size]."""
+              head_mask: Optional[torch.Tensor] = None, q_rows: Optional[int] = None) -> torch.Tensor:
+    """qkv bf16 [B*S, 3*heads*head_size] (q | k | v blocks) -> ctx bf16 [B*S, heads*head_size].
+    q_rows (bf16 only): just the first q_rows queries of every image, against all S keys -> ctx [B*q_rows, heads*head_size]."""
     _need_cuda(qkv, head_mask)
     if qkv.dtype not in (torch.bfloat16, torch.float32) or qkv.dim() != 2 or qkv.stride(1) != 1:
         raise ValueError("attention wants a 2-D bf16 (or f32 for the tf32 mode) qkv matrix")
     if qkv.shape[0] != B * S or qkv.shape[1] < 3 * heads * head_size:
         raise ValueError("attention: qkv shape does not match B, S, heads")
-    ctx = torch.empty((B * S, heads * head_size), dtype=qkv.dtype, device=qkv.device)
+    if q_rows is not None and qkv.dtype != torch.bfloat16:
+        raise ValueError("attention: q_rows is implemented for bf16 only")
+    Sq = S if q_rows is None else int(q_rows)
+    ctx = torch.empty((B * Sq, heads * head_size), dtype=qkv.dtype, device=qkv.device)
     scale = float(head_size ** -0.5 if scale is None else scale)
     lib = _lib.load()
-    fn = lib.evt_attention_fwd if qkv.dtype == torch.bfloat16 else lib.evt_attention_fwd_tf32
-    _lib.check(fn(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), _ptr(head_mask), B, S, heads, head_size,
-                  scale, _stream()), "attention")
+    if q_rows is not None:
+        rc = lib.evt_attention_query_rows_fwd(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), _ptr(head_mask), B, S,
+                                              Sq, heads, head_size, scale, _stream())
+    else:
+        fn = lib.evt_attention_fwd if qkv.dtype == torch.bfloat16 else lib.evt_attention_fwd_tf32
+        rc = fn(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), _ptr(head_mask), B, S, heads, head_size, scale,
+                _stream())
+    _lib.check(rc, "attention")
     return ctx
 
 

@@ -159,6 +159,11 @@ int evt_gemm_residual_layernorm_ex(const void* A, int64_t lda, const void* W, in
 int evt_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask,
                       int B, int S, int heads, int head_size, float scale, evt_stream stream);
 
+/* evt_attention_fwd for the first Sq (1..S) query rows of every image against all S keys: ctx is bf16 [B*Sq, ldc].
+ * Those rows are bit-identical to the same rows of evt_attention_fwd. */
+int evt_attention_query_rows_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask,
+                                 int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream);
+
 /* tf32 flavour of evt_attention_fwd: qkv and ctx are f32 (leading dims multiples of 4). */
 int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask,
                            int B, int S, int heads, int head_size, float scale, evt_stream stream);
