@@ -6,6 +6,7 @@ each bracketed by a stream synchronise and ``timeit.default_timer``; optional ``
 (benchmark/tensorrt/onnx_trt_test.py:103-105); prints ``Avg latency: X ms, Std: Y ms`` and one JSON line.
 
     python -m edgevisiontransformer_b200.benchmark --model deit_tiny --batch 1 --precision tf32 --graph
+    python -m edgevisiontransformer_b200.benchmark --model deit_base --image-size 384 --batch 256
     python -m edgevisiontransformer_b200.benchmark --model /path/to/pruned_checkpoint --batch 1024
     python -m edgevisiontransformer_b200.benchmark --model attention --h 768 --a 12 --n 197      (op-level, tools.py:735-758)
 """
@@ -27,12 +28,12 @@ T2T = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_
        "t2t_vit_14": (384, 14, 6, 3.0)}
 
 
-def _random_hf(name: str, seed: int = 0):
+def _random_hf(name: str, seed: int = 0, image_size: int = 224):
     from transformers import ViTConfig, ViTForImageClassification
     d, h, i = DEIT[name]
     torch.manual_seed(seed)
-    return ViTForImageClassification(ViTConfig(hidden_size=d, num_hidden_layers=12, num_attention_heads=h,
-                                               intermediate_size=i, num_labels=1000, attn_implementation="eager")).eval()
+    return ViTForImageClassification(ViTConfig(hidden_size=d, num_hidden_layers=12, num_attention_heads=h, intermediate_size=i,
+                                               image_size=image_size, num_labels=1000, attn_implementation="eager")).eval()
 
 
 def _random_t2t_weights(hidden, depth, heads, mlp_ratio, seed=0):
@@ -73,13 +74,14 @@ def _random_t2t_weights(hidden, depth, heads, mlp_ratio, seed=0):
     return sd
 
 
-def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", **op_kw):
-    """-> (callable taking one CUDA tensor, input shape without batch, description)."""
+def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", image_size: int = 224, **op_kw):
+    """-> (callable taking one CUDA tensor, input shape without batch, description).  image_size: deit_* only
+    (224 or 384, the two resolutions of deit_*_patch16_*)."""
     from .. import B200ViTForImageClassification
     if name in DEIT:
-        m = B200ViTForImageClassification.from_hf(_random_hf(name), device=device, max_batch=max_batch, precision=precision,
-                                                  keep_params=False)
-        return m, (3, 224, 224), f"{name} random-init ({precision})"
+        m = B200ViTForImageClassification.from_hf(_random_hf(name, image_size=image_size), device=device, max_batch=max_batch,
+                                                  precision=precision, keep_params=False)
+        return m, (3, image_size, image_size), f"{name} random-init ({precision}, {image_size} px)"
     if name in T2T:
         from ..modeling_t2t import B200T2TViT
         hidden, depth, heads, ratio = T2T[name]
@@ -143,6 +145,7 @@ def main(argv=None) -> int:
     ap.add_argument("--warmup_runs", type=int, default=20)
     ap.add_argument("--topk", type=int, default=None)
     ap.add_argument("--graph", action="store_true", help="CUDA-graph replay (small-batch latency path)")
+    ap.add_argument("--image-size", type=int, default=224, help="deit_* input resolution (384: deit_*_patch16_384, 577 tokens)")
     for k, d in (("h", 768), ("a", 12), ("i", 3072), ("n", 128)):
         ap.add_argument(f"--{k}", type=int, default=d)
     ap.add_argument("--h_k", type=int, default=None)
@@ -150,12 +153,15 @@ def main(argv=None) -> int:
     if not torch.cuda.is_available():
         print("b200_benchmark needs a B200 (sm_100a): the backend has no CPU path")
         return 2
-    model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), h=a.h, a=a.a, i=a.i, n=a.n, h_k=a.h_k)
+    if a.image_size != 224 and a.model not in DEIT:
+        ap.error("--image-size applies to the deit_* models only")
+    model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), image_size=a.image_size, h=a.h, a=a.a, i=a.i,
+                                     n=a.n, h_k=a.h_k)
     avg, std, times = b200_benchmark(model, (a.batch, *shape), a.num_runs, a.warmup_runs, a.topk, graph=a.graph)
     print(f"{desc}: batch {a.batch}")
     print(f"Avg latency: {avg: .3f} ms, Std: {std: .3f} ms")          # tools.py:1009 format
     p50 = float(np.percentile(times, 50))
-    print(json.dumps({"model": a.model, "batch": a.batch, "precision": a.precision, "graph": bool(a.graph),
+    print(json.dumps({"model": a.model, "batch": a.batch, "precision": a.precision, "image_size": a.image_size, "graph": bool(a.graph),
                       "avg_ms": avg, "std_ms": std, "p50_ms": p50, "images_per_sec": a.batch / (avg / 1e3),
                       "num_runs": a.num_runs, "warmup_runs": a.warmup_runs}))
     return 0

@@ -19,6 +19,7 @@
 // SK = S rounded up to 16; key columns >= S are masked to probability 0, so the extra K/V rows the TMA box
 // picks up (next image's tokens, or zero fill past the end of the matrix) never contribute.
 // TMEM: 2 slots x 256 columns (S at [0,SK), P overlaid at [0,SK/2), O overlaid at [128,192)).
+// Longer sequences (257 .. EVT_ATTN_MAX_TOKENS) run attention_long_kernel below; attention_launch picks by S.
 #include <cuda_bf16.h>
 
 #include <math_constants.h>
@@ -507,6 +508,352 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// Long sequences (256 < S <= EVT_ATTN_MAX_TOKENS).  A score row of a head no longer fits in TMEM and one head's K + V no
+// longer fits twice in shared memory, so every 128-row query tile runs against 128-key blocks with an online softmax.
+// Same warp roles, TMEM slots and context store as attention2_kernel:
+//
+//   work item          (image b, head h, 128-row query tile mt), flattened with mt fastest: the tiles of one (image, head)
+//                      run on neighbouring CTAs at the same time, so the K / V blocks they all re-read come from L2.  A CTA
+//                      takes units of two consecutive items, one per softmax group.
+//   warp 8 (1 thread)  TMA producer: each item's Q tile (four 32-row boxes, one Q buffer per group), then K and V of every
+//                      128-key block of both items, interleaved group 0 / group 1, into a ring of kLongStages stages.  The
+//                      3-D map clips at the image end: keys past it arrive as zeros and are masked to probability 0 (a
+//                      zero key scores 0, not -inf).
+//   warp 9 (1 thread)  S = Q K_blk^T (M = 128, N = 128) into columns [0, 128) of the group's slot, once O = P V of the
+//                      previous block has read its P.
+//   warp 10 (1 thread) O += P V_blk: P bf16 from TMEM [0, 64), O at [128, 192).
+//   warps 0-3 / 4-7    softmax groups, one thread per query row.  The running maximum is lazy: a row's P, O and sum stay
+//                      relative to the maximum it last used (mu) until a block's maximum exceeds mu by more than
+//                      kRescaleLog2 (log2 units); only then are O and the sum multiplied by 2^(mu - mu_new).  In between
+//                      P <= 2^kRescaleLog2, and O and the sum share the same stale maximum, so the quotient is exact.
+//                      Every decision is per row: a row comes out the same whatever Sq is and whatever its neighbours hold.
+constexpr int kKeyBlock = 128;
+constexpr int kKeyBlockBytes = kKeyBlock * 128;  // one K or V block, 128 keys x 64 bf16
+constexpr int kLongStages = 4;
+constexpr float kRescaleLog2 = 8.f;
+
+struct AttnLongParams {
+  const float* head_mask;
+  int S, Sq, heads;
+  int n_kb;      // 128-key blocks per item
+  int q_tiles;   // query tiles per (image, head)
+  int n_items;   // B * heads * q_tiles
+  float scale_log2e;
+};
+
+struct LongItem {
+  int b, h, mt;
+};
+__device__ __forceinline__ LongItem long_item(const AttnLongParams& p, int it) {
+  LongItem r;
+  const int bh = it / p.q_tiles;
+  r.mt = it - bh * p.q_tiles;
+  r.b = bh / p.heads;
+  r.h = bh - r.b * p.heads;
+  return r;
+}
+
+// Item of softmax group g in unit ql of this CTA; the group-1 item of the very last unit may not exist.
+__device__ __forceinline__ int item_index(int ql, int g) {
+  return 2 * (static_cast<int>(blockIdx.x) + ql * static_cast<int>(gridDim.x)) + g;
+}
+__device__ __forceinline__ int groups_of(const AttnLongParams& p, int ql) { return item_index(ql, 1) < p.n_items ? 2 : 1; }
+
+// One 128-key block of the online softmax for the query row at t_row (nvalid: valid keys in the block, 1..128).  mu is
+// the row's current maximum times scale * log2(e), sum its running sum; both are updated, and O (TMEM columns
+// [kOCol, kOCol + 64)) is rescaled with them when the maximum moves (has_o: O already holds earlier blocks).
+// bf16 P is written over the consumed S columns; the caller issues tcgen05.wait::st.
+template <bool MASKED>
+__device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool has_o, float scale_log2e, float& mu, float& sum) {
+  const uint64_t scale2 = pk2(scale_log2e, scale_log2e);
+  uint32_t ra[16], rb[16];
+  float m[4] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
+  ptx::tmem_ld_x16(t_row, ra);
+#pragma unroll 1
+  for (int c = 0; c < kKeyBlock / 16; c += 2) {
+    ptx::tmem_ld_wait();
+    ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
+    chunk_max<16, MASKED>(ra, nvalid - c * 16, m);
+    ptx::tmem_ld_wait();
+    if (c + 2 < kKeyBlock / 16) ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
+    chunk_max<16, MASKED>(rb, nvalid - (c + 1) * 16, m);
+  }
+  const float bm = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3])) * scale_log2e;
+  const bool grow = bm > mu + kRescaleLog2;  // always on the first block (mu = -inf)
+  float alpha = 1.f;
+  if (grow) {
+    alpha = ex2_approx(mu - bm);  // 0 on the first block
+    mu = bm;
+    sum *= alpha;
+  }
+  if (has_o && __any_sync(0xffffffffu, grow)) {
+#pragma unroll
+    for (int c = 0; c < kHD / 16; c += 2) {
+      ptx::tmem_ld_x16(t_row + kOCol + c * 16, ra);
+      ptx::tmem_ld_x16(t_row + kOCol + (c + 1) * 16, rb);
+      ptx::tmem_ld_wait();
+#pragma unroll
+      for (int j = 0; j < 16; ++j) {
+        ra[j] = __float_as_uint(__uint_as_float(ra[j]) * alpha);
+        rb[j] = __float_as_uint(__uint_as_float(rb[j]) * alpha);
+      }
+      ptx::tmem_st_x16(t_row + kOCol + c * 16, ra);
+      ptx::tmem_st_x16(t_row + kOCol + (c + 1) * 16, rb);
+    }
+  }
+  const uint64_t negm2 = pk2(-mu, -mu);
+  uint64_t sum2[2] = {0ull, 0ull};
+  uint32_t pk[8];
+  ptx::tmem_ld_x16(t_row, ra);
+#pragma unroll 1
+  for (int c = 0; c < kKeyBlock / 16; c += 2) {
+    ptx::tmem_ld_wait();
+    ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
+    chunk_exp<16, MASKED>(ra, nvalid - c * 16, scale2, negm2, sum2, pk);
+    ptx::tmem_st_x8(t_row + c * 8, pk);
+    ptx::tmem_ld_wait();
+    if (c + 2 < kKeyBlock / 16) ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
+    chunk_exp<16, MASKED>(rb, nvalid - (c + 1) * 16, scale2, negm2, sum2, pk);
+    ptx::tmem_st_x8(t_row + (c + 1) * 8, pk);
+  }
+  float s0, s1, s2, s3;
+  upk2(sum2[0], s0, s1);
+  upk2(sum2[1], s2, s3);
+  sum += (s0 + s1) + (s2 + s3);
+}
+
+__global__ void __launch_bounds__(kThreads2, 1)
+attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
+                      const __grid_constant__ CUtensorMap tmO, const AttnLongParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint8_t* kv_ring = smem;                                    // kLongStages x (K | V) blocks
+  uint8_t* q_ring = smem + kLongStages * 2 * kKeyBlockBytes;  // 2 x Q tile, one per softmax group
+  uint8_t* staging = q_ring + 2 * kQTileBytes;                // 8 x 4 KB context staging
+  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kSoftmaxWarps * kStgWarpBytes);
+  uint64_t* kv_full = bars;                    // [kLongStages] producer -> issuers
+  uint64_t* kv_empty = bars + kLongStages;     // [kLongStages] PV issuer (commit) -> producer
+  uint64_t* q_full = bars + 2 * kLongStages;   // [2] producer -> QK issuer
+  uint64_t* q_empty = q_full + 2;              // [2] QK issuer (commit after an item's last block) -> producer
+  uint64_t* s_ready = q_empty + 2;             // [2] QK issuer (commit) -> softmax group
+  uint64_t* p_ready = s_ready + 2;             // [2] softmax group (4 warps) -> PV issuer
+  uint64_t* pv_done = p_ready + 2;             // [2] PV issuer (commit) -> QK issuer (P read) and softmax group (O final)
+  uint64_t* slot_free = pv_done + 2;           // [2] softmax group (4 warps, O read out) -> QK issuer
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(slot_free + 2);
+
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const int a = p.heads * kHD;
+  const int n_units = (p.n_items + 1) / 2;
+  const int my_units = (n_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
+
+  if (warp == kProdWarp && ptx::elect_one()) {
+    ptx::prefetch_tmap(&tmQ);
+    ptx::prefetch_tmap(&tmKV);
+    ptx::prefetch_tmap(&tmO);
+    for (int s = 0; s < kLongStages; ++s) {
+      ptx::mbar_init(&kv_full[s], 1);
+      ptx::mbar_init(&kv_empty[s], 1);
+    }
+    for (int s = 0; s < 2; ++s) {
+      ptx::mbar_init(&q_full[s], 1);
+      ptx::mbar_init(&q_empty[s], 1);
+      ptx::mbar_init(&s_ready[s], 1);
+      ptx::mbar_init(&p_ready[s], 4);
+      ptx::mbar_init(&pv_done[s], 1);
+      ptx::mbar_init(&slot_free[s], 4);
+    }
+    ptx::fence_mbar_init();
+  }
+  if (warp == kQKWarp) ptx::tmem_alloc<512>(tmem_ptr);
+  ptx::tc_fence_before();
+  __syncthreads();
+  ptx::tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr;
+  ptx::grid_dep_launch();
+  ptx::grid_dep_wait();  // qkv (previous kernel's output) is complete from here on
+
+  // The three single-thread roles walk the same sequence of (unit, key block, group) stages.
+  if (warp == kProdWarp) {
+    // ------------------------------------------------------------ TMA producer
+    if (ptx::elect_one()) {
+      int t = 0;
+      uint32_t kph = 0;
+      for (int ql = 0; ql < my_units; ++ql) {
+        const int n_g = groups_of(p, ql);
+        for (int g = 0; g < n_g; ++g) {
+          const LongItem it = long_item(p, item_index(ql, g));
+          ptx::mbar_wait(&q_empty[g], (ql & 1) ^ 1);
+          ptx::mbar_arrive_expect_tx(&q_full[g], kQTileBytes);
+#pragma unroll
+          for (int q = 0; q < 4; ++q)  // rows past Sq arrive as zeros
+            ptx::tma_load_3d(q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &q_full[g], it.h * kHD, it.mt * kQRows + 32 * q, it.b);
+        }
+        for (int kb = 0; kb < p.n_kb; ++kb) {
+          for (int g = 0; g < n_g; ++g) {
+            const LongItem it = long_item(p, item_index(ql, g));
+            ptx::mbar_wait(&kv_empty[t], kph ^ 1);
+            uint8_t* sK = kv_ring + t * 2 * kKeyBlockBytes;
+            ptx::mbar_arrive_expect_tx(&kv_full[t], 2 * kKeyBlockBytes);
+            ptx::tma_load_3d(sK, &tmKV, &kv_full[t], a + it.h * kHD, kb * kKeyBlock, it.b);
+            ptx::tma_load_3d(sK + kKeyBlockBytes, &tmKV, &kv_full[t], 2 * a + it.h * kHD, kb * kKeyBlock, it.b);
+            if (++t == kLongStages) {
+              t = 0;
+              kph ^= 1;
+            }
+          }
+        }
+      }
+    }
+  } else if (warp == kQKWarp) {
+    // ------------------------------------------------------------ S = Q K^T issuer
+    if (ptx::elect_one()) {
+      const uint32_t idesc_qk = ptx::make_idesc(kQRows, kKeyBlock, 1, 0, 0);
+      int t = 0;
+      uint32_t kph = 0;
+      for (int ql = 0; ql < my_units; ++ql) {
+        const int n_g = groups_of(p, ql);
+        for (int kb = 0; kb < p.n_kb; ++kb) {
+          for (int g = 0; g < n_g; ++g) {
+            ptx::mbar_wait(&kv_full[t], kph);
+            if (kb == 0) {
+              ptx::mbar_wait(&q_full[g], ql & 1);
+              ptx::mbar_wait(&slot_free[g], (ql & 1) ^ 1);  // the previous item's O has been read out
+            } else {
+              ptx::mbar_wait(&pv_done[g], (ql * p.n_kb + kb - 1) & 1);  // the previous block's P has been read
+            }
+            ptx::tc_fence_after();
+            const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(q_ring + g * kQTileBytes));
+            const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + t * 2 * kKeyBlockBytes));
+            const uint32_t slot = tmem_base + g * kSlotCols;
+#pragma unroll
+            for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
+            ptx::mma_commit(&s_ready[g]);
+            if (kb == p.n_kb - 1) ptx::mma_commit(&q_empty[g]);
+            if (++t == kLongStages) {
+              t = 0;
+              kph ^= 1;
+            }
+          }
+        }
+      }
+    }
+  } else if (warp == kPVWarp) {
+    // ------------------------------------------------------------ O += P V issuer
+    if (ptx::elect_one()) {
+      const uint32_t idesc_pv = ptx::make_idesc(kQRows, kHD, 1, 0, 1);
+      int t = 0;
+      uint32_t kph = 0;
+      for (int ql = 0; ql < my_units; ++ql) {
+        const int n_g = groups_of(p, ql);
+        for (int kb = 0; kb < p.n_kb; ++kb) {
+          for (int g = 0; g < n_g; ++g) {
+            ptx::mbar_wait(&kv_full[t], kph);  // complete long ago (S of this block exists); taken for the memory ordering
+            ptx::mbar_wait(&p_ready[g], (ql * p.n_kb + kb) & 1);
+            ptx::tc_fence_after();
+            const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + t * 2 * kKeyBlockBytes + kKeyBlockBytes));
+            const uint32_t slot = tmem_base + g * kSlotCols;
+#pragma unroll
+            for (int k = 0; k < kKeyBlock / 16; ++k)
+              ptx::mma_f16_ts(slot + kOCol, slot + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, (kb | k) != 0 ? 1u : 0u);
+            ptx::mma_commit(&pv_done[g]);
+            ptx::mma_commit(&kv_empty[t]);
+            if (++t == kLongStages) {
+              t = 0;
+              kph ^= 1;
+            }
+          }
+        }
+      }
+    }
+  } else {
+    // ------------------------------------------------------------ softmax groups
+    const int grp = warp >> 2;
+    const int quad = warp & 3;
+    const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + grp * kSlotCols;
+    const int last_valid = p.S - (p.n_kb - 1) * kKeyBlock;  // valid keys in the last block (1..128)
+    uint8_t* stg = staging + warp * kStgWarpBytes;
+    uint8_t* stg_row = stg + lane * 128;
+    const int sw = lane & 7;
+#pragma unroll 1
+    for (int ql = 0; ql < my_units; ++ql) {
+      const int idx = item_index(ql, grp);
+      if (idx >= p.n_items) break;
+      const LongItem u = long_item(p, idx);
+      const int qrow0 = u.mt * kQRows + quad * 32;
+      const bool warp_live = qrow0 < p.Sq;  // rows past Sq (or past S in the last tile): nothing to compute
+      float hm = 1.f;
+      if (p.head_mask != nullptr) hm = p.head_mask[u.h];
+      const int c0 = ql * p.n_kb;  // this group's block count before the item: the barrier phases below
+      float mu = -CUDART_INF_F, sum = 0.f;
+#pragma unroll 1
+      for (int kb = 0; kb < p.n_kb; ++kb) {
+        ptx::mbar_wait(&s_ready[grp], (c0 + kb) & 1);
+        if (kb != 0) ptx::mbar_wait(&pv_done[grp], (c0 + kb - 1) & 1);  // O may be rescaled below
+        ptx::tc_fence_after();
+        if (warp_live) {
+          if (kb != p.n_kb - 1) softmax_block<false>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum);
+          else softmax_block<true>(t_row, last_valid, kb != 0, p.scale_log2e, mu, sum);
+          ptx::tmem_st_wait();
+        }
+        ptx::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) ptx::mbar_arrive(&p_ready[grp]);
+      }
+      float inv = 1.f;
+      if (warp_live) asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(sum));  // sum >= 1 (the maximum contributes 2^0)
+      inv *= hm;
+      if (warp_live && ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous context tile has left the staging buffer
+      ptx::mbar_wait(&pv_done[grp], (c0 + p.n_kb - 1) & 1);
+      ptx::tc_fence_after();
+      uint32_t o0[32], o1[32];
+      if (warp_live) {
+        ptx::tmem_ld_x32(t_row + kOCol, o0);
+        ptx::tmem_ld_x32(t_row + kOCol + 32, o1);
+        ptx::tmem_ld_wait();
+      }
+      ptx::tc_fence_before();
+      __syncwarp();
+      if (lane == 0) ptx::mbar_arrive(&slot_free[grp]);
+      if (warp_live) {
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+#pragma unroll
+          for (int jj = 0; jj < 32; jj += 8) {
+            const uint32_t* r = half == 0 ? &o0[jj] : &o1[jj];
+            uint4 o;
+            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(r[0]) * inv, __uint_as_float(r[1]) * inv);
+            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(r[2]) * inv, __uint_as_float(r[3]) * inv);
+            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(r[4]) * inv, __uint_as_float(r[5]) * inv);
+            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(r[6]) * inv, __uint_as_float(r[7]) * inv);
+            o.x = *reinterpret_cast<uint32_t*>(&t0);
+            o.y = *reinterpret_cast<uint32_t*>(&t1);
+            o.z = *reinterpret_cast<uint32_t*>(&t2);
+            o.w = *reinterpret_cast<uint32_t*>(&t3);
+            const int piece = half * 4 + (jj >> 3);
+            ptx::sts_u4(ptx::smem_u32(stg_row) + ((piece ^ sw) << 4), o.x, o.y, o.z, o.w);
+          }
+        }
+        ptx::fence_proxy_async_smem();
+        __syncwarp();
+        if (ptx::elect_one()) {
+          ptx::tma_store_3d(&tmO, stg, u.h * kHD, qrow0, u.b);  // rows >= Sq of the image are clipped by the tensor map
+          ptx::bulk_commit();
+        }
+      }
+    }
+    if (ptx::elect_one()) ptx::bulk_wait<0>();
+  }
+
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (warp == kQKWarp) {
+    ptx::tc_fence_after();
+    ptx::tmem_dealloc<512>(tmem_base);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // tf32 accuracy mode: Q, K, V and the context are fp32 in HBM; the tensor core reads them as tf32 (kind::tf32,
 // K = 8 per MMA) and accumulates in fp32.  A 64-float head row is two 128-byte swizzle atoms, so Q and K are
 // loaded as two TMA boxes of 32 columns each.  V is needed as the B operand of O = P V with the KEY index
@@ -688,6 +1035,42 @@ attention_tf32_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   }
 }
 
+// S > 256: attention_long_kernel.  Argument checks are the caller's (attention_launch).
+int attention_long_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
+                          int heads, float scale, cudaStream_t stream) {
+  AttnLongParams q;
+  q.head_mask = head_mask;
+  q.S = S;
+  q.Sq = Sq;
+  q.heads = heads;
+  q.n_kb = (S + kKeyBlock - 1) / kKeyBlock;
+  q.q_tiles = (Sq + kQRows - 1) / kQRows;
+  const long long n_items = static_cast<long long>(B) * heads * q.q_tiles;
+  EVT_CHECK_ARG(n_items < (1ll << 30), "attention: B * heads * query tiles too large");
+  q.n_items = static_cast<int>(n_items);
+  q.scale_log2e = scale * 1.4426950408889634f;
+  CUtensorMap tmQ, tmKV, tmO;
+  // K / V: 128-key blocks of one image (keys past S arrive as zeros); Q: the first Sq rows of every image; context packed
+  int rc = make_tmap_3d_rows(&tmKV, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
+                             static_cast<uint64_t>(ldq), kKeyBlock, kHD, static_cast<uint64_t>(S));
+  if (rc != EVT_OK) return rc;
+  rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                         static_cast<uint64_t>(ldq), 32, kHD, static_cast<uint64_t>(S));
+  if (rc != EVT_OK) return rc;
+  rc = make_tmap_3d_rows(&tmO, ctx, 2, static_cast<uint64_t>(heads) * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                         static_cast<uint64_t>(ldc), 32, kHD);
+  if (rc != EVT_OK) return rc;
+  const long long units = (n_items + 1) / 2;
+  const int grid = units < num_sms() ? static_cast<int>(units) : num_sms();
+  const int smem = 1024 + kLongStages * 2 * kKeyBlockBytes + 2 * kQTileBytes + kSoftmaxWarps * kStgWarpBytes +
+                   (2 * kLongStages + 12) * 8 + 16;
+  EVT_TRY(opt_in_smem<attention_long_kernel>(smem));
+  const bool pdl = pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * kHD);
+  EVT_CUDA(launch_pdl(attention_long_kernel, dim3(grid), dim3(kThreads2), smem, stream, pdl, tmQ, tmKV, tmO, q));
+  EVT_LAUNCH_CHECK("attention_long_kernel");
+  return EVT_OK;
+}
+
 }  // namespace
 
 int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
@@ -696,10 +1079,12 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   EVT_CHECK_ARG(B > 0 && S > 0 && heads > 0, "attention: B, S, heads must be positive");
   EVT_CHECK_ARG(Sq > 0 && Sq <= S, "attention: query rows must be in 1..S");
   if (head_size != kHD) return fail(EVT_ERR_UNSUPPORTED, "attention: only head size 64 is implemented");
-  if (S > 256) return fail(EVT_ERR_UNSUPPORTED, "attention: sequence length above 256 is not implemented");
+  if (S > EVT_ATTN_MAX_TOKENS)
+    return fail(EVT_ERR_UNSUPPORTED, "attention: sequence length above " + std::to_string(EVT_ATTN_MAX_TOKENS) + " is not implemented");
   EVT_CHECK_ARG(ldq >= 3ll * heads * kHD && ldc >= static_cast<int64_t>(heads) * kHD, "attention: leading dimension too small");
   EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention: ctx must be 16-byte aligned rows");
   EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");
+  if (S > 256) return attention_long_launch(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
   const int SK = (S + 15) / 16 * 16;
   const uint64_t rows = static_cast<uint64_t>(B) * S;
   const int q_tiles = (Sq + kQRows - 1) / kQRows;

@@ -166,7 +166,10 @@ int validate_spec(const evt_model_spec* s) {
   EVT_CHECK_ARG(s->patch % 8 == 0, "patch size must be a multiple of 8");
   const int patches = (s->image / s->patch) * (s->image / s->patch);
   EVT_CHECK_ARG(s->tokens == patches + 1 || s->tokens == patches + 2, "tokens must be patches + 1 (cls) or + 2 (cls, distillation)");
-  if (s->tokens > 256) return fail(EVT_ERR_UNSUPPORTED, "more than 256 tokens per image is not implemented");
+  if (s->tokens > EVT_ATTN_MAX_TOKENS)
+    return fail(EVT_ERR_UNSUPPORTED, "more than " + std::to_string(EVT_ATTN_MAX_TOKENS) + " tokens per image is not implemented");
+  if (s->tokens > 256 && s->precision == EVT_PREC_TF32)  // its attention keeps every key of a head on chip
+    return fail(EVT_ERR_UNSUPPORTED, "the tf32 mode supports at most 256 tokens per image; use the bf16 mode");
   if (s->head_size != 64) return fail(EVT_ERR_UNSUPPORTED, "only head size 64 is implemented");
   EVT_CHECK_ARG(s->num_labels > 0, "num_labels must be positive");
   EVT_CHECK_ARG(s->act == EVT_ACT_GELU_ERF || s->act == EVT_ACT_GELU_TANH, "FFN activation must be erf- or tanh-GELU");

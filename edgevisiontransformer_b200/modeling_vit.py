@@ -209,7 +209,7 @@ class B200ViTForImageClassification(nn.Module):
         sd = model_or_state_dict.state_dict() if hasattr(model_or_state_dict, "state_dict") else model_or_state_dict
         image = kw.pop("image_size", None)
         csd, cfg_kw = timm_vit_to_canonical({k: v for k, v in sd.items()}, patch=kw.pop("patch_size", 16))
-        if image is None:                       # 224 -> 197 tokens, 384 -> 577 (rejected by the library: > 256 tokens)
+        if image is None:                       # from the position rows: 197 / 198 -> 224, 577 / 578 -> 384
             n_prefix = 2 if "vit.embeddings.distillation_token" in csd else 1
             image = int(round((csd["vit.embeddings.position_embeddings"].shape[1] - n_prefix) ** 0.5)) * cfg_kw["patch_size"]
         return cls.from_state_dict(csd, image_size=image, **cfg_kw, **kw)

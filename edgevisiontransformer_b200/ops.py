@@ -173,7 +173,8 @@ def linear_residual_layernorm(a: torch.Tensor, w: torch.Tensor, bias: Optional[t
 
 def attention(qkv: torch.Tensor, B: int, S: int, heads: int, head_size: int = 64, scale: Optional[float] = None,
               head_mask: Optional[torch.Tensor] = None, q_rows: Optional[int] = None) -> torch.Tensor:
-    """qkv bf16 [B*S, 3*heads*head_size] (q | k | v blocks) -> ctx bf16 [B*S, heads*head_size].
+    """qkv bf16 [B*S, 3*heads*head_size] (q | k | v blocks) -> ctx bf16 [B*S, heads*head_size].  S up to 1026
+    (EVT_ATTN_MAX_TOKENS) in bf16, up to 256 for f32 qkv (the tf32 mode).
     q_rows (bf16 only): just the first q_rows queries of every image, against all S keys -> ctx [B*q_rows, heads*head_size]."""
     _need_cuda(qkv, head_mask)
     if qkv.dtype not in (torch.bfloat16, torch.float32) or qkv.dim() != 2 or qkv.stride(1) != 1:

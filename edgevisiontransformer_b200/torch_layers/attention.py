@@ -9,7 +9,7 @@ class Attention(nn.Module):
     """modeling/torch_layers/attention.py:4-48: q/k/v Linear(+bias) -> softmax(q k^T * head_size^-0.5) v -> to_out.
 
     B200 path: x -> bf16, ONE GEMM on the concatenated [3*h*d, hidden] weight (bias in the epilogue), the fused
-    short-sequence attention kernel, then the to_out GEMM (f32 out; an optional residual is added in its epilogue).
+    attention kernel (n up to EVT_ATTN_MAX_TOKENS = 1026), then the to_out GEMM (f32 out; an optional residual is added in its epilogue).
     """
 
     def __init__(self, hidden_size, num_heads, head_size=None):

@@ -148,7 +148,12 @@ int evt_gemm_residual_layernorm_ex(const void* A, int64_t lda, const void* W, in
                                    float* resid, int64_t ldr, const float* gamma, const float* beta, float eps, int copy_ln,
                                    void* xn, int64_t ldxn, int64_t M, int N, int K, evt_stream stream);
 
-/* Fused softmax(Q K^T * scale) V for short sequences (S <= 256, head size 64):
+/* Longest sequence the bf16 attention accepts: ViT / DeiT-B/16 at 512 px with a cls and a distillation token
+ * (32 * 32 + 2 tokens). */
+#define EVT_ATTN_MAX_TOKENS 1026
+
+/* Fused softmax(Q K^T * scale) V, head size 64, any S from 1 to EVT_ATTN_MAX_TOKENS.  S <= 256 keeps every key of a head
+ * on chip; longer sequences run query tiles against 128-key blocks with an online softmax (no score tensor in HBM either way):
  * eager_attention_forward SITE/models/vit/modeling_vit.py:171-196 ==
  * modeling/torch_layers/attention.py:36-45 == modeling/layers/attention.py:30-33.
  *   qkv : bf16 [B*S, ldq]; q of head h at columns [h*64, h*64+64), k at [heads*64 + h*64, ...),
@@ -164,7 +169,7 @@ int evt_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, cons
 int evt_attention_query_rows_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask,
                                  int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream);
 
-/* tf32 flavour of evt_attention_fwd: qkv and ctx are f32 (leading dims multiples of 4). */
+/* tf32 flavour of evt_attention_fwd: qkv and ctx are f32 (leading dims multiples of 4); S <= 256 only. */
 int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask,
                            int B, int S, int heads, int head_size, float scale, evt_stream stream);
 
@@ -282,7 +287,8 @@ typedef struct evt_model_spec {
   int dialect;                 /* evt_dialect */
   int hidden;                  /* D */
   int layers;                  /* L <= EVT_MAX_LAYERS */
-  int tokens;                  /* 197 (cls + 196) or 198 (DeiT distillation token) */
+  int tokens;                  /* patches + 1 (cls) or + 2 (DeiT distillation token): 197 / 198 at 224 px, 577 / 578 at
+                                  384 px; up to EVT_ATTN_MAX_TOKENS in bf16, up to 256 in the tf32 mode */
   int image, patch;            /* 224, 16 */
   int head_size;               /* 64 */
   int num_labels;              /* 1000 */
