@@ -41,32 +41,9 @@ constexpr int kOCol = 128;
 // 0 -> 0.319 ms, 1 -> 0.309, 2 -> 0.318, 3 -> 0.342 (0.330 before the division-free item bookkeeping).
 constexpr int kPolyPairs = 1;
 
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 __device__ __forceinline__ float max3(float a, float b, float c) {
   float d;
   asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-  return d;
-}
-__device__ __forceinline__ uint64_t pk2(float lo, float hi) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
-}
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
 
@@ -75,15 +52,15 @@ __device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
 // rounding of P) and n added into the exponent field.  Used for one element pair in four: the exponential phase of the
 // two softmax groups is MUFU-bound whenever they overlap (ncu: mio-throttle stalls on MUFU.EX2), the FMA pipe is idle.
 __device__ __forceinline__ void ex2_poly_pair(float t0, float t1, float& p0, float& p1) {
-  const uint64_t tt = pk2(fmaxf(t0, -126.f), fmaxf(t1, -126.f));
-  const uint64_t r = add2(tt, pk2(12582912.f, 12582912.f));
-  const uint64_t f = add2(tt, fma2(r, pk2(-1.f, -1.f), pk2(12582912.f, 12582912.f)));  // t - n
-  uint64_t q = fma2(f, pk2(0.0551716685f, 0.0551716685f), pk2(0.2426111251f, 0.2426111251f));
-  q = fma2(q, f, pk2(0.6932609677f, 0.6932609677f));
-  q = fma2(q, f, pk2(0.9999280572f, 0.9999280572f));
+  const uint64_t tt = ptx::pk2(fmaxf(t0, -126.f), fmaxf(t1, -126.f));
+  const uint64_t r = ptx::add2(tt, ptx::pk2(12582912.f, 12582912.f));
+  const uint64_t f = ptx::add2(tt, ptx::fma2(r, ptx::pk2(-1.f, -1.f), ptx::pk2(12582912.f, 12582912.f)));  // t - n
+  uint64_t q = ptx::fma2(f, ptx::pk2(0.0551716685f, 0.0551716685f), ptx::pk2(0.2426111251f, 0.2426111251f));
+  q = ptx::fma2(q, f, ptx::pk2(0.6932609677f, 0.6932609677f));
+  q = ptx::fma2(q, f, ptx::pk2(0.9999280572f, 0.9999280572f));
   float q0, q1, r0, r1;
-  upk2(q, q0, q1);
-  upk2(r, r0, r1);
+  ptx::upk2(q, q0, q1);
+  ptx::upk2(r, r0, r1);
   p0 = __int_as_float(__float_as_int(q0) + (__float_as_int(r0) << 23));
   p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(r1) << 23));
 }
@@ -112,21 +89,20 @@ __device__ __forceinline__ void chunk_exp(const uint32_t (&r)[W], int nvalid, ui
 #pragma unroll
   for (int j = 0; j < W; j += 2) {
     float t0, t1;
-    upk2(fma2(pk2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), scale2, negm2), t0, t1);
+    ptx::upk2(ptx::fma2(ptx::pk2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), scale2, negm2), t0, t1);
     float p0, p1;
     if (((j >> 1) & 3) >= 4 - kPolyPairs) {
       ex2_poly_pair(t0, t1, p0, p1);
     } else {
-      p0 = ex2_approx(t0);
-      p1 = ex2_approx(t1);
+      p0 = ptx::ex2_approx(t0);
+      p1 = ptx::ex2_approx(t1);
     }
     if (MASKED) {
       if (j >= nvalid) p0 = 0.f;
       if (j + 1 >= nvalid) p1 = 0.f;
     }
-    sum2[(j >> 1) & 1] = add2(sum2[(j >> 1) & 1], pk2(p0, p1));
-    __nv_bfloat162 hb = __floats2bfloat162_rn(p0, p1);
-    pk[j >> 1] = *reinterpret_cast<uint32_t*>(&hb);
+    sum2[(j >> 1) & 1] = ptx::add2(sum2[(j >> 1) & 1], ptx::pk2(p0, p1));
+    pk[j >> 1] = ptx::pack_bf16x2(p0, p1);
   }
 }
 
@@ -134,7 +110,7 @@ __device__ __forceinline__ void chunk_exp(const uint32_t (&r)[W], int nvalid, ui
 // f32 row sum returned (the caller issues tcgen05.wait::st).  n16 = score chunks of 16 columns, last_valid = valid columns
 // in the last one.
 __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_valid, float scale_log2e) {
-  const uint64_t scale2 = pk2(scale_log2e, scale_log2e);
+  const uint64_t scale2 = ptx::pk2(scale_log2e, scale_log2e);
   float sum;
   {
     // Both passes walk the row in 16-column chunks, double-buffered: the next tcgen05.ld is in flight while the
@@ -167,7 +143,7 @@ __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_v
     }
     const float mx = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3]));
     const float nm = -mx * scale_log2e;
-    const uint64_t negm2 = pk2(nm, nm);
+    const uint64_t negm2 = ptx::pk2(nm, nm);
     // pass 2: probabilities (bf16) written over the S columns already consumed; fp32 row sum
     uint64_t sum2[2] = {0ull, 0ull};
     {
@@ -200,8 +176,8 @@ __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_v
       }
     }
     float s0, s1, s2, s3;
-    upk2(sum2[0], s0, s1);
-    upk2(sum2[1], s2, s3);
+    ptx::upk2(sum2[0], s0, s1);
+    ptx::upk2(sum2[1], s2, s3);
     sum = (s0 + s1) + (s2 + s3);
   }
   return sum;
@@ -266,58 +242,143 @@ __device__ __forceinline__ int tile_of(const Attn2Params& p, const Unit& u, int 
   return p.n_mt == 2 ? (s ^ (ql & 1)) : s;
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// The skeleton attention2_kernel and attention_long_kernel share: shared memory, prologue, context epilogue, teardown.
+
+// Shared memory: the K/V ring, 2 Q tiles (one per softmax group), 8 context staging tiles, 2 x kMaxKV + 12 mbarriers and the
+// TMEM address.
+struct AttnSmem {
+  uint8_t* kv_ring;
+  uint8_t* q_ring;
+  uint8_t* staging;
+  uint64_t* kv_full;    // [kMaxKV] producer -> issuers
+  uint64_t* kv_empty;   // [kMaxKV] PV issuer (commit) -> producer
+  uint64_t* q_full;     // [2] producer -> QK issuer
+  uint64_t* q_empty;    // [2] QK issuer (commit) -> producer
+  uint64_t* s_ready;    // [2] QK issuer (commit) -> softmax group
+  uint64_t* p_ready;    // [2] softmax group (4 warps) -> PV issuer
+  uint64_t* pv_done;    // [2] PV issuer (commit) -> softmax group (O complete; long kernel: also QK issuer, P read)
+  uint64_t* slot_free;  // [2] softmax group (4 warps, O read out) -> QK issuer
+  uint32_t* tmem_ptr;
+};
+__device__ __forceinline__ AttnSmem attn_smem(uint8_t* smem_raw, int kv_ring_bytes) {
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  AttnSmem m;
+  m.kv_ring = smem;
+  m.q_ring = smem + kv_ring_bytes;
+  m.staging = m.q_ring + 2 * kQTileBytes;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(m.staging + kSoftmaxWarps * kStgWarpBytes);
+  m.kv_full = bars;
+  m.kv_empty = bars + kMaxKV;
+  m.q_full = bars + 2 * kMaxKV;
+  m.q_empty = m.q_full + 2;
+  m.s_ready = m.q_empty + 2;
+  m.p_ready = m.s_ready + 2;
+  m.pv_done = m.p_ready + 2;
+  m.slot_free = m.pv_done + 2;
+  m.tmem_ptr = reinterpret_cast<uint32_t*>(m.slot_free + 2);
+  return m;
+}
+
+// Tensor-map prefetch, barrier init (kv_empty completes after kv_empty_count commits), TMEM allocation (2 slots), PDL.
+// Returns the TMEM base; the previous kernel's output (qkv) is complete from here on.
+__device__ __forceinline__ uint32_t attn_prologue(int warp, const AttnSmem& sm, const CUtensorMap* tmQ, const CUtensorMap* tmKV,
+                                                  const CUtensorMap* tmO, uint32_t kv_empty_count) {
+  if (warp == kProdWarp && ptx::elect_one()) {
+    ptx::prefetch_tmap(tmQ);
+    ptx::prefetch_tmap(tmKV);
+    ptx::prefetch_tmap(tmO);
+    for (int s = 0; s < kMaxKV; ++s) {
+      ptx::mbar_init(&sm.kv_full[s], 1);
+      ptx::mbar_init(&sm.kv_empty[s], kv_empty_count);
+    }
+    for (int s = 0; s < 2; ++s) {
+      ptx::mbar_init(&sm.q_full[s], 1);
+      ptx::mbar_init(&sm.q_empty[s], 1);
+      ptx::mbar_init(&sm.s_ready[s], 1);
+      ptx::mbar_init(&sm.p_ready[s], 4);
+      ptx::mbar_init(&sm.pv_done[s], 1);
+      ptx::mbar_init(&sm.slot_free[s], 4);
+    }
+    ptx::fence_mbar_init();
+  }
+  if (warp == kQKWarp) ptx::tmem_alloc<2 * kSlotCols>(sm.tmem_ptr);
+  ptx::tc_fence_before();
+  __syncthreads();
+  ptx::tc_fence_after();
+  const uint32_t tmem_base = *sm.tmem_ptr;
+  ptx::grid_dep_launch();
+  ptx::grid_dep_wait();
+  return tmem_base;
+}
+
+// Context of one query tile, run by each softmax warp once its P is handed over: wait for O = P V (pv_done, phase), read the
+// warp's 32 rows of O (TMEM lane row t_row), release the slot (slot_free), then O * hm / sum -> bf16, row per thread, into
+// the warp's 128B-swizzled staging tile (16-byte piece i of row r at piece i ^ (r & 7)) and a 3-D TMA store of the tile at
+// (col, row, img); rows past the end of the tensor map are clipped.  A warp with no live row only takes part in the barriers.
+__device__ __forceinline__ void store_context(float sum, float hm, bool warp_live, uint64_t* pv_done, uint32_t phase,
+                                              uint64_t* slot_free, uint32_t t_row, uint8_t* stg, const CUtensorMap* tmO, int col,
+                                              int row, int img) {
+  const int lane = threadIdx.x & 31;
+  const float inv = ptx::rcp_approx(sum) * hm;  // sum >= 1 (the maximum contributes 2^0)
+  if (warp_live && ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous context tile has left the staging buffer
+  ptx::mbar_wait(pv_done, phase);
+  ptx::tc_fence_after();
+  uint32_t o0[32], o1[32];
+  if (warp_live) {
+    ptx::tmem_ld_x32(t_row + kOCol, o0);
+    ptx::tmem_ld_x32(t_row + kOCol + 32, o1);
+    ptx::tmem_ld_wait();
+  }
+  ptx::tc_fence_before();
+  __syncwarp();
+  if (lane == 0) ptx::mbar_arrive(slot_free);  // the slot can take the next S while we convert and store
+  if (!warp_live) return;
+  uint8_t* stg_row = stg + lane * 128;
+  const int sw = lane & 7;
+#pragma unroll
+  for (int half = 0; half < 2; ++half) {
+#pragma unroll
+    for (int jj = 0; jj < 32; jj += 8) {
+      const uint32_t* r = half == 0 ? &o0[jj] : &o1[jj];
+      const uint32_t x = ptx::pack_bf16x2(__uint_as_float(r[0]) * inv, __uint_as_float(r[1]) * inv);
+      const uint32_t y = ptx::pack_bf16x2(__uint_as_float(r[2]) * inv, __uint_as_float(r[3]) * inv);
+      const uint32_t z = ptx::pack_bf16x2(__uint_as_float(r[4]) * inv, __uint_as_float(r[5]) * inv);
+      const uint32_t w = ptx::pack_bf16x2(__uint_as_float(r[6]) * inv, __uint_as_float(r[7]) * inv);
+      const int piece = half * 4 + (jj >> 3);
+      ptx::sts_u4(ptx::smem_u32(stg_row) + ((piece ^ sw) << 4), x, y, z, w);  // explicit STS (a C++ store here is generic)
+    }
+  }
+  ptx::fence_proxy_async_smem();
+  __syncwarp();
+  if (ptx::elect_one()) {
+    ptx::tma_store_3d(tmO, stg, col, row, img);
+    ptx::bulk_commit();
+  }
+}
+
+__device__ __forceinline__ void attn_teardown(int warp, uint32_t tmem_base) {
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (warp == kQKWarp) {
+    ptx::tc_fence_after();
+    ptx::tmem_dealloc<2 * kSlotCols>(tmem_base);
+  }
+}
+
 __global__ void __launch_bounds__(kThreads2, 1)
 attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                   const __grid_constant__ CUtensorMap tmO, const Attn2Params p) {
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int kv_bytes = p.SK * 128;
-  uint8_t* kv_ring = smem;                                   // n_kv x (K | V)
-  uint8_t* q_ring = smem + p.n_kv * 2 * kv_bytes;            // 2 x Q tile, one per softmax group
-  uint8_t* staging = q_ring + 2 * kQTileBytes;               // 8 x 4 KB context staging
-  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kSoftmaxWarps * kStgWarpBytes);
-  uint64_t* kv_full = bars;                   // [kMaxKV] producer -> issuers
-  uint64_t* kv_empty = bars + kMaxKV;         // [kMaxKV] PV issuer (n_mt commits) -> producer
-  uint64_t* q_full = bars + 2 * kMaxKV;       // [2] producer -> QK issuer
-  uint64_t* q_empty = q_full + 2;             // [2] QK issuer (commit) -> producer
-  uint64_t* s_ready = q_empty + 2;            // [2] QK issuer (commit) -> softmax group
-  uint64_t* p_ready = s_ready + 2;            // [2] softmax group (4 warps) -> PV issuer
-  uint64_t* o_ready = p_ready + 2;            // [2] PV issuer (commit) -> softmax group
-  uint64_t* slot_free = o_ready + 2;          // [2] softmax group (4 warps) -> QK issuer
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(slot_free + 2);
-
+  const AttnSmem sm = attn_smem(smem_raw, p.n_kv * 2 * kv_bytes);  // ring: n_kv x (K | V)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int a = p.heads * kHD;
   const int total_units = p.B * p.heads * (p.q_tiles / p.n_mt);
   const int my_units = (total_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
   const int n_items = my_units * p.n_mt;
-
-  if (warp == kProdWarp && ptx::elect_one()) {
-    ptx::prefetch_tmap(&tmQ);
-    ptx::prefetch_tmap(&tmKV);
-    ptx::prefetch_tmap(&tmO);
-    for (int s = 0; s < kMaxKV; ++s) {
-      ptx::mbar_init(&kv_full[s], 1);
-      ptx::mbar_init(&kv_empty[s], p.n_mt);
-    }
-    for (int s = 0; s < 2; ++s) {
-      ptx::mbar_init(&q_full[s], 1);
-      ptx::mbar_init(&q_empty[s], 1);
-      ptx::mbar_init(&s_ready[s], 1);
-      ptx::mbar_init(&p_ready[s], 4);
-      ptx::mbar_init(&o_ready[s], 1);
-      ptx::mbar_init(&slot_free[s], 4);
-    }
-    ptx::fence_mbar_init();
-  }
-  if (warp == kQKWarp) ptx::tmem_alloc<512>(tmem_ptr);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  ptx::grid_dep_launch();
-  ptx::grid_dep_wait();  // qkv (previous kernel's output) is complete from here on
+  const uint32_t tmem_base = attn_prologue(warp, sm, &tmQ, &tmKV, &tmO, p.n_mt);  // n_mt commits release K and V of a unit
 
   if (warp == kProdWarp) {
     // ------------------------------------------------------------ TMA producer
@@ -328,19 +389,19 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       for (int ql = 0; ql < my_units; ++ql) {
         const Unit u = unit_of(p, ql);
         const int row0 = u.b * p.S;
-        ptx::mbar_wait(&kv_empty[kst], kph ^ 1);
-        uint8_t* sK = kv_ring + kst * 2 * kv_bytes;
-        ptx::mbar_arrive_expect_tx(&kv_full[kst], 2 * kv_bytes);
-        ptx::tma_load_2d(sK, &tmKV, &kv_full[kst], a + u.h * kHD, row0);
-        ptx::tma_load_2d(sK + kv_bytes, &tmKV, &kv_full[kst], 2 * a + u.h * kHD, row0);
+        ptx::mbar_wait(&sm.kv_empty[kst], kph ^ 1);
+        uint8_t* sK = sm.kv_ring + kst * 2 * kv_bytes;
+        ptx::mbar_arrive_expect_tx(&sm.kv_full[kst], 2 * kv_bytes);
+        ptx::tma_load_2d(sK, &tmKV, &sm.kv_full[kst], a + u.h * kHD, row0);
+        ptx::tma_load_2d(sK + kv_bytes, &tmKV, &sm.kv_full[kst], 2 * a + u.h * kHD, row0);
         for (int s = 0; s < p.n_mt; ++s, ++j) {
           const int g = j & 1;
-          ptx::mbar_wait(&q_empty[g], ((j >> 1) & 1) ^ 1);
-          ptx::mbar_arrive_expect_tx(&q_full[g], kQTileBytes);
+          ptx::mbar_wait(&sm.q_empty[g], ((j >> 1) & 1) ^ 1);
+          ptx::mbar_arrive_expect_tx(&sm.q_full[g], kQTileBytes);
           const int mt = tile_of(p, u, ql, s);
 #pragma unroll
           for (int q = 0; q < 4; ++q)  // rows past the end of the image (and whole empty blocks) arrive as zeros
-            ptx::tma_load_3d(q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &q_full[g], u.h * kHD, 32 * block_of(mt, q, ql & 3), u.b);
+            ptx::tma_load_3d(sm.q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &sm.q_full[g], u.h * kHD, 32 * block_of(mt, q, ql & 3), u.b);
         }
         if (++kst == p.n_kv) {
           kst = 0;
@@ -356,20 +417,20 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       uint32_t kph = 0;
       int j = 0;
       for (int ql = 0; ql < my_units; ++ql) {
-        ptx::mbar_wait(&kv_full[kst], kph);
-        const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + kst * 2 * kv_bytes));
+        ptx::mbar_wait(&sm.kv_full[kst], kph);
+        const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + kst * 2 * kv_bytes));
         for (int s = 0; s < p.n_mt; ++s, ++j) {
           const int g = j & 1;
           const uint32_t ph = (j >> 1) & 1;
-          ptx::mbar_wait(&q_full[g], ph);
-          ptx::mbar_wait(&slot_free[g], ph ^ 1);
+          ptx::mbar_wait(&sm.q_full[g], ph);
+          ptx::mbar_wait(&sm.slot_free[g], ph ^ 1);
           ptx::tc_fence_after();
-          const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(q_ring + g * kQTileBytes));
+          const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(sm.q_ring + g * kQTileBytes));
           const uint32_t slot = tmem_base + g * kSlotCols;
 #pragma unroll
           for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
-          ptx::mma_commit(&s_ready[g]);
-          ptx::mma_commit(&q_empty[g]);  // the Q tile can be replaced as soon as these MMAs have read it
+          ptx::mma_commit(&sm.s_ready[g]);
+          ptx::mma_commit(&sm.q_empty[g]);  // the Q tile can be replaced as soon as these MMAs have read it
         }
         if (++kst == p.n_kv) {
           kst = 0;
@@ -386,18 +447,18 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       uint32_t kph = 0;
       int j = 0;
       for (int ql = 0; ql < my_units; ++ql) {
-        ptx::mbar_wait(&kv_full[kst], kph);  // complete long ago (S of this unit exists); taken for the memory ordering
-        const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + kst * 2 * kv_bytes + kv_bytes));
+        ptx::mbar_wait(&sm.kv_full[kst], kph);  // complete long ago (S of this unit exists); taken for the memory ordering
+        const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + kst * 2 * kv_bytes + kv_bytes));
         for (int s = 0; s < p.n_mt; ++s, ++j) {
           const int g = j & 1;
-          ptx::mbar_wait(&p_ready[g], (j >> 1) & 1);
+          ptx::mbar_wait(&sm.p_ready[g], (j >> 1) & 1);
           ptx::tc_fence_after();
           const uint32_t slot = tmem_base + g * kSlotCols;
           // P from TMEM (8 columns per K = 16), V MN-major (2048 B per step)
           for (int k = 0; k < nk; ++k)
             ptx::mma_f16_ts(slot + kOCol, slot + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, k != 0 ? 1u : 0u);
-          ptx::mma_commit(&o_ready[g]);
-          ptx::mma_commit(&kv_empty[kst]);  // n_mt arrivals release K and V of the unit
+          ptx::mma_commit(&sm.pv_done[g]);
+          ptx::mma_commit(&sm.kv_empty[kst]);  // n_mt arrivals release K and V of the unit
         }
         if (++kst == p.n_kv) {
           kst = 0;
@@ -412,9 +473,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + grp * kSlotCols;
     const int n16 = p.SK / 16;                    // 16-column score chunks; only the last one can hold masked keys
     const int last_valid = p.S - (n16 - 1) * 16;  // valid columns in it (1..16)
-    uint8_t* stg = staging + warp * kStgWarpBytes;
-    uint8_t* stg_row = stg + lane * 128;
-    const int sw = lane & 7;
+    uint8_t* stg = sm.staging + warp * kStgWarpBytes;
     // This group's items are j = grp, grp + 2, ...: unit ql = j / n_mt advances by dql per iteration.  (b, h) follow
     // incrementally -- two integer divisions per item were 11 % of the softmax warps' instructions in the first version.
     const int dql = p.n_mt == 2 ? 1 : 2;
@@ -443,7 +502,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       const bool warp_live = qrow0 < p.Sq;  // block 7 (rows 224..255) when S = 197, or a block past Sq: nothing to do
       float hm = 1.f;
       if (p.head_mask != nullptr) hm = p.head_mask[u.h];
-      ptx::mbar_wait(&s_ready[grp], ph);
+      ptx::mbar_wait(&sm.s_ready[grp], ph);
       ptx::tc_fence_after();
       float sum = 1.f;
       if (warp_live) {
@@ -452,59 +511,12 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       }
       ptx::tc_fence_before();
       __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&p_ready[grp]);
-      float inv;
-      asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(sum));  // sum >= 1 (the max contributes 2^0)
-      inv *= hm;
-      if (warp_live && ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous context tile has left the staging buffer
-      ptx::mbar_wait(&o_ready[grp], ph);
-      ptx::tc_fence_after();
-      uint32_t o0[32], o1[32];
-      if (warp_live) {
-        ptx::tmem_ld_x32(t_row + kOCol, o0);
-        ptx::tmem_ld_x32(t_row + kOCol + 32, o1);
-        ptx::tmem_ld_wait();
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&slot_free[grp]);  // the slot can take the next S while we convert and store
-      if (warp_live) {
-        // O / sum -> bf16, row per thread into the 128B-swizzled staging tile (16-byte piece i of row r at piece i ^ (r & 7))
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-#pragma unroll
-          for (int jj = 0; jj < 32; jj += 8) {
-            const uint32_t* r = half == 0 ? &o0[jj] : &o1[jj];
-            uint4 o;
-            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(r[0]) * inv, __uint_as_float(r[1]) * inv);
-            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(r[2]) * inv, __uint_as_float(r[3]) * inv);
-            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(r[4]) * inv, __uint_as_float(r[5]) * inv);
-            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(r[6]) * inv, __uint_as_float(r[7]) * inv);
-            o.x = *reinterpret_cast<uint32_t*>(&t0);
-            o.y = *reinterpret_cast<uint32_t*>(&t1);
-            o.z = *reinterpret_cast<uint32_t*>(&t2);
-            o.w = *reinterpret_cast<uint32_t*>(&t3);
-            const int piece = half * 4 + (jj >> 3);
-            ptx::sts_u4(ptx::smem_u32(stg_row) + ((piece ^ sw) << 4), o.x, o.y, o.z, o.w);  // explicit STS (a C++ store here is generic)
-          }
-        }
-        ptx::fence_proxy_async_smem();
-        __syncwarp();
-        if (ptx::elect_one()) {
-          ptx::tma_store_3d(&tmO, stg, u.h * kHD, qrow0, u.b);  // rows >= S of the image are clipped by the tensor map
-          ptx::bulk_commit();
-        }
-      }
+      if (lane == 0) ptx::mbar_arrive(&sm.p_ready[grp]);
+      store_context(sum, hm, warp_live, &sm.pv_done[grp], ph, &sm.slot_free[grp], t_row, stg, &tmO, u.h * kHD, qrow0, u.b);
     }
     if (ptx::elect_one()) ptx::bulk_wait<0>();
   }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == kQKWarp) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(tmem_base);
-  }
+  attn_teardown(warp, tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -530,6 +542,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
 constexpr int kKeyBlock = 128;
 constexpr int kKeyBlockBytes = kKeyBlock * 128;  // one K or V block, 128 keys x 64 bf16
 constexpr int kLongStages = 4;
+static_assert(kLongStages == kMaxKV, "attn_prologue initialises kMaxKV K/V stages");
 constexpr float kRescaleLog2 = 8.f;
 
 struct AttnLongParams {
@@ -565,7 +578,7 @@ __device__ __forceinline__ int groups_of(const AttnLongParams& p, int ql) { retu
 // bf16 P is written over the consumed S columns; the caller issues tcgen05.wait::st.
 template <bool MASKED>
 __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool has_o, float scale_log2e, float& mu, float& sum) {
-  const uint64_t scale2 = pk2(scale_log2e, scale_log2e);
+  const uint64_t scale2 = ptx::pk2(scale_log2e, scale_log2e);
   uint32_t ra[16], rb[16];
   float m[4] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
   ptx::tmem_ld_x16(t_row, ra);
@@ -582,7 +595,7 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
   const bool grow = bm > mu + kRescaleLog2;  // always on the first block (mu = -inf)
   float alpha = 1.f;
   if (grow) {
-    alpha = ex2_approx(mu - bm);  // 0 on the first block
+    alpha = ptx::ex2_approx(mu - bm);  // 0 on the first block
     mu = bm;
     sum *= alpha;
   }
@@ -601,7 +614,7 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
       ptx::tmem_st_x16(t_row + kOCol + (c + 1) * 16, rb);
     }
   }
-  const uint64_t negm2 = pk2(-mu, -mu);
+  const uint64_t negm2 = ptx::pk2(-mu, -mu);
   uint64_t sum2[2] = {0ull, 0ull};
   uint32_t pk[8];
   ptx::tmem_ld_x16(t_row, ra);
@@ -617,8 +630,8 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
     ptx::tmem_st_x8(t_row + (c + 1) * 8, pk);
   }
   float s0, s1, s2, s3;
-  upk2(sum2[0], s0, s1);
-  upk2(sum2[1], s2, s3);
+  ptx::upk2(sum2[0], s0, s1);
+  ptx::upk2(sum2[1], s2, s3);
   sum += (s0 + s1) + (s2 + s3);
 }
 
@@ -626,52 +639,13 @@ __global__ void __launch_bounds__(kThreads2, 1)
 attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                       const __grid_constant__ CUtensorMap tmO, const AttnLongParams p) {
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* kv_ring = smem;                                    // kLongStages x (K | V) blocks
-  uint8_t* q_ring = smem + kLongStages * 2 * kKeyBlockBytes;  // 2 x Q tile, one per softmax group
-  uint8_t* staging = q_ring + 2 * kQTileBytes;                // 8 x 4 KB context staging
-  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kSoftmaxWarps * kStgWarpBytes);
-  uint64_t* kv_full = bars;                    // [kLongStages] producer -> issuers
-  uint64_t* kv_empty = bars + kLongStages;     // [kLongStages] PV issuer (commit) -> producer
-  uint64_t* q_full = bars + 2 * kLongStages;   // [2] producer -> QK issuer
-  uint64_t* q_empty = q_full + 2;              // [2] QK issuer (commit after an item's last block) -> producer
-  uint64_t* s_ready = q_empty + 2;             // [2] QK issuer (commit) -> softmax group
-  uint64_t* p_ready = s_ready + 2;             // [2] softmax group (4 warps) -> PV issuer
-  uint64_t* pv_done = p_ready + 2;             // [2] PV issuer (commit) -> QK issuer (P read) and softmax group (O final)
-  uint64_t* slot_free = pv_done + 2;           // [2] softmax group (4 warps, O read out) -> QK issuer
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(slot_free + 2);
-
+  const AttnSmem sm = attn_smem(smem_raw, kLongStages * 2 * kKeyBlockBytes);  // ring: kLongStages x (K | V) blocks
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int a = p.heads * kHD;
   const int n_units = (p.n_items + 1) / 2;
   const int my_units = (n_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
-
-  if (warp == kProdWarp && ptx::elect_one()) {
-    ptx::prefetch_tmap(&tmQ);
-    ptx::prefetch_tmap(&tmKV);
-    ptx::prefetch_tmap(&tmO);
-    for (int s = 0; s < kLongStages; ++s) {
-      ptx::mbar_init(&kv_full[s], 1);
-      ptx::mbar_init(&kv_empty[s], 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      ptx::mbar_init(&q_full[s], 1);
-      ptx::mbar_init(&q_empty[s], 1);
-      ptx::mbar_init(&s_ready[s], 1);
-      ptx::mbar_init(&p_ready[s], 4);
-      ptx::mbar_init(&pv_done[s], 1);
-      ptx::mbar_init(&slot_free[s], 4);
-    }
-    ptx::fence_mbar_init();
-  }
-  if (warp == kQKWarp) ptx::tmem_alloc<512>(tmem_ptr);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  ptx::grid_dep_launch();
-  ptx::grid_dep_wait();  // qkv (previous kernel's output) is complete from here on
+  const uint32_t tmem_base = attn_prologue(warp, sm, &tmQ, &tmKV, &tmO, 1);
 
   // The three single-thread roles walk the same sequence of (unit, key block, group) stages.
   if (warp == kProdWarp) {
@@ -683,20 +657,20 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         const int n_g = groups_of(p, ql);
         for (int g = 0; g < n_g; ++g) {
           const LongItem it = long_item(p, item_index(ql, g));
-          ptx::mbar_wait(&q_empty[g], (ql & 1) ^ 1);
-          ptx::mbar_arrive_expect_tx(&q_full[g], kQTileBytes);
+          ptx::mbar_wait(&sm.q_empty[g], (ql & 1) ^ 1);
+          ptx::mbar_arrive_expect_tx(&sm.q_full[g], kQTileBytes);
 #pragma unroll
           for (int q = 0; q < 4; ++q)  // rows past Sq arrive as zeros
-            ptx::tma_load_3d(q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &q_full[g], it.h * kHD, it.mt * kQRows + 32 * q, it.b);
+            ptx::tma_load_3d(sm.q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &sm.q_full[g], it.h * kHD, it.mt * kQRows + 32 * q, it.b);
         }
         for (int kb = 0; kb < p.n_kb; ++kb) {
           for (int g = 0; g < n_g; ++g) {
             const LongItem it = long_item(p, item_index(ql, g));
-            ptx::mbar_wait(&kv_empty[t], kph ^ 1);
-            uint8_t* sK = kv_ring + t * 2 * kKeyBlockBytes;
-            ptx::mbar_arrive_expect_tx(&kv_full[t], 2 * kKeyBlockBytes);
-            ptx::tma_load_3d(sK, &tmKV, &kv_full[t], a + it.h * kHD, kb * kKeyBlock, it.b);
-            ptx::tma_load_3d(sK + kKeyBlockBytes, &tmKV, &kv_full[t], 2 * a + it.h * kHD, kb * kKeyBlock, it.b);
+            ptx::mbar_wait(&sm.kv_empty[t], kph ^ 1);
+            uint8_t* sK = sm.kv_ring + t * 2 * kKeyBlockBytes;
+            ptx::mbar_arrive_expect_tx(&sm.kv_full[t], 2 * kKeyBlockBytes);
+            ptx::tma_load_3d(sK, &tmKV, &sm.kv_full[t], a + it.h * kHD, kb * kKeyBlock, it.b);
+            ptx::tma_load_3d(sK + kKeyBlockBytes, &tmKV, &sm.kv_full[t], 2 * a + it.h * kHD, kb * kKeyBlock, it.b);
             if (++t == kLongStages) {
               t = 0;
               kph ^= 1;
@@ -715,21 +689,21 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         const int n_g = groups_of(p, ql);
         for (int kb = 0; kb < p.n_kb; ++kb) {
           for (int g = 0; g < n_g; ++g) {
-            ptx::mbar_wait(&kv_full[t], kph);
+            ptx::mbar_wait(&sm.kv_full[t], kph);
             if (kb == 0) {
-              ptx::mbar_wait(&q_full[g], ql & 1);
-              ptx::mbar_wait(&slot_free[g], (ql & 1) ^ 1);  // the previous item's O has been read out
+              ptx::mbar_wait(&sm.q_full[g], ql & 1);
+              ptx::mbar_wait(&sm.slot_free[g], (ql & 1) ^ 1);  // the previous item's O has been read out
             } else {
-              ptx::mbar_wait(&pv_done[g], (ql * p.n_kb + kb - 1) & 1);  // the previous block's P has been read
+              ptx::mbar_wait(&sm.pv_done[g], (ql * p.n_kb + kb - 1) & 1);  // the previous block's P has been read
             }
             ptx::tc_fence_after();
-            const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(q_ring + g * kQTileBytes));
-            const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + t * 2 * kKeyBlockBytes));
+            const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(sm.q_ring + g * kQTileBytes));
+            const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + t * 2 * kKeyBlockBytes));
             const uint32_t slot = tmem_base + g * kSlotCols;
 #pragma unroll
             for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
-            ptx::mma_commit(&s_ready[g]);
-            if (kb == p.n_kb - 1) ptx::mma_commit(&q_empty[g]);
+            ptx::mma_commit(&sm.s_ready[g]);
+            if (kb == p.n_kb - 1) ptx::mma_commit(&sm.q_empty[g]);
             if (++t == kLongStages) {
               t = 0;
               kph ^= 1;
@@ -748,16 +722,16 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         const int n_g = groups_of(p, ql);
         for (int kb = 0; kb < p.n_kb; ++kb) {
           for (int g = 0; g < n_g; ++g) {
-            ptx::mbar_wait(&kv_full[t], kph);  // complete long ago (S of this block exists); taken for the memory ordering
-            ptx::mbar_wait(&p_ready[g], (ql * p.n_kb + kb) & 1);
+            ptx::mbar_wait(&sm.kv_full[t], kph);  // complete long ago (S of this block exists); taken for the memory ordering
+            ptx::mbar_wait(&sm.p_ready[g], (ql * p.n_kb + kb) & 1);
             ptx::tc_fence_after();
-            const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(kv_ring + t * 2 * kKeyBlockBytes + kKeyBlockBytes));
+            const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + t * 2 * kKeyBlockBytes + kKeyBlockBytes));
             const uint32_t slot = tmem_base + g * kSlotCols;
 #pragma unroll
             for (int k = 0; k < kKeyBlock / 16; ++k)
               ptx::mma_f16_ts(slot + kOCol, slot + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, (kb | k) != 0 ? 1u : 0u);
-            ptx::mma_commit(&pv_done[g]);
-            ptx::mma_commit(&kv_empty[t]);
+            ptx::mma_commit(&sm.pv_done[g]);
+            ptx::mma_commit(&sm.kv_empty[t]);
             if (++t == kLongStages) {
               t = 0;
               kph ^= 1;
@@ -772,9 +746,7 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     const int quad = warp & 3;
     const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + grp * kSlotCols;
     const int last_valid = p.S - (p.n_kb - 1) * kKeyBlock;  // valid keys in the last block (1..128)
-    uint8_t* stg = staging + warp * kStgWarpBytes;
-    uint8_t* stg_row = stg + lane * 128;
-    const int sw = lane & 7;
+    uint8_t* stg = sm.staging + warp * kStgWarpBytes;
 #pragma unroll 1
     for (int ql = 0; ql < my_units; ++ql) {
       const int idx = item_index(ql, grp);
@@ -788,8 +760,8 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       float mu = -CUDART_INF_F, sum = 0.f;
 #pragma unroll 1
       for (int kb = 0; kb < p.n_kb; ++kb) {
-        ptx::mbar_wait(&s_ready[grp], (c0 + kb) & 1);
-        if (kb != 0) ptx::mbar_wait(&pv_done[grp], (c0 + kb - 1) & 1);  // O may be rescaled below
+        ptx::mbar_wait(&sm.s_ready[grp], (c0 + kb) & 1);
+        if (kb != 0) ptx::mbar_wait(&sm.pv_done[grp], (c0 + kb - 1) & 1);  // O may be rescaled below
         ptx::tc_fence_after();
         if (warp_live) {
           if (kb != p.n_kb - 1) softmax_block<false>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum);
@@ -798,59 +770,14 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         }
         ptx::tc_fence_before();
         __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&p_ready[grp]);
+        if (lane == 0) ptx::mbar_arrive(&sm.p_ready[grp]);
       }
-      float inv = 1.f;
-      if (warp_live) asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(sum));  // sum >= 1 (the maximum contributes 2^0)
-      inv *= hm;
-      if (warp_live && ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous context tile has left the staging buffer
-      ptx::mbar_wait(&pv_done[grp], (c0 + p.n_kb - 1) & 1);
-      ptx::tc_fence_after();
-      uint32_t o0[32], o1[32];
-      if (warp_live) {
-        ptx::tmem_ld_x32(t_row + kOCol, o0);
-        ptx::tmem_ld_x32(t_row + kOCol + 32, o1);
-        ptx::tmem_ld_wait();
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&slot_free[grp]);
-      if (warp_live) {
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-#pragma unroll
-          for (int jj = 0; jj < 32; jj += 8) {
-            const uint32_t* r = half == 0 ? &o0[jj] : &o1[jj];
-            uint4 o;
-            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(r[0]) * inv, __uint_as_float(r[1]) * inv);
-            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(r[2]) * inv, __uint_as_float(r[3]) * inv);
-            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(r[4]) * inv, __uint_as_float(r[5]) * inv);
-            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(r[6]) * inv, __uint_as_float(r[7]) * inv);
-            o.x = *reinterpret_cast<uint32_t*>(&t0);
-            o.y = *reinterpret_cast<uint32_t*>(&t1);
-            o.z = *reinterpret_cast<uint32_t*>(&t2);
-            o.w = *reinterpret_cast<uint32_t*>(&t3);
-            const int piece = half * 4 + (jj >> 3);
-            ptx::sts_u4(ptx::smem_u32(stg_row) + ((piece ^ sw) << 4), o.x, o.y, o.z, o.w);
-          }
-        }
-        ptx::fence_proxy_async_smem();
-        __syncwarp();
-        if (ptx::elect_one()) {
-          ptx::tma_store_3d(&tmO, stg, u.h * kHD, qrow0, u.b);  // rows >= Sq of the image are clipped by the tensor map
-          ptx::bulk_commit();
-        }
-      }
+      store_context(sum, hm, warp_live, &sm.pv_done[grp], (c0 + p.n_kb - 1) & 1, &sm.slot_free[grp], t_row, stg, &tmO, u.h * kHD,
+                    qrow0, u.b);
     }
     if (ptx::elect_one()) ptx::bulk_wait<0>();
   }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == kQKWarp) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(tmem_base);
-  }
+  attn_teardown(warp, tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------------------

@@ -9,11 +9,6 @@
 namespace evt {
 namespace {
 
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-
 // One thread = 8 consecutive pixels of one image row (32 / 16 / 8 B in for f32 / bf16 / u8 pixels, 16 B of bf16 or 32 B of
 // tf32-rounded f32 out).  Thread order follows the input (b, c, y, x8) so reads are perfectly coalesced; writes are full
 // 16-byte pieces of patch rows.  Patch p of image b lands in row  b * row_stride + row_off + p  (row_stride = patches,
@@ -75,10 +70,10 @@ __global__ void __launch_bounds__(256) im2col_kernel(const TIN* __restrict__ px,
   const int k = (c * P + i) * P + j;
   if (OUT_BF16) {
     uint4 o;
-    o.x = pack_bf16(v[0], v[1]);
-    o.y = pack_bf16(v[2], v[3]);
-    o.z = pack_bf16(v[4], v[5]);
-    o.w = pack_bf16(v[6], v[7]);
+    o.x = ptx::pack_bf16x2(v[0], v[1]);
+    o.y = ptx::pack_bf16x2(v[2], v[3]);
+    o.z = ptx::pack_bf16x2(v[4], v[5]);
+    o.w = ptx::pack_bf16x2(v[6], v[7]);
     *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(cols_) + row * (3ll * P * P) + k) = o;
   } else {  // tf32 mode keeps the patch matrix in fp32, rounded to nearest tf32 (the tensor core would truncate)
     float* dst = reinterpret_cast<float*>(cols_) + row * (3ll * P * P) + k;
@@ -125,10 +120,10 @@ __global__ void __launch_bounds__(256) cast_kernel(const float* __restrict__ x, 
     const float4 a = *reinterpret_cast<const float4*>(x + t * 8);
     const float4 b = *reinterpret_cast<const float4*>(x + t * 8 + 4);
     uint4 o;
-    o.x = pack_bf16(a.x, a.y);
-    o.y = pack_bf16(a.z, a.w);
-    o.z = pack_bf16(b.x, b.y);
-    o.w = pack_bf16(b.z, b.w);
+    o.x = ptx::pack_bf16x2(a.x, a.y);
+    o.y = ptx::pack_bf16x2(a.z, a.w);
+    o.z = ptx::pack_bf16x2(b.x, b.y);
+    o.w = ptx::pack_bf16x2(b.z, b.w);
     *reinterpret_cast<uint4*>(y + t * 8) = o;
   } else if (t == n8) {
     for (long long i = n8 * 8; i < n; ++i) y[i] = __float2bfloat16_rn(x[i]);

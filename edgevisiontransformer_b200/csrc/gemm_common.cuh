@@ -1,5 +1,5 @@
-// Device code shared by the 1-CTA (gemm.cu) and 2-CTA (gemm2.cu) tcgen05 GEMM kernels: parameters, packed f32x2
-// epilogue math, and the per-warp epilogue of one accumulator tile.
+// Device code shared by the 1-CTA (gemm.cu) and 2-CTA (gemm2.cu) tcgen05 GEMM kernels: parameters, the GELU epilogue
+// math, and the per-warp epilogue of one accumulator tile.
 #pragma once
 #include <cuda_bf16.h>
 
@@ -53,46 +53,15 @@ __device__ __forceinline__ long long map_out_row(const GemmParams& p, long long 
   const long long g = row / p.out_group;
   return g * p.out_group_stride + p.out_group_off + (row - g * p.out_group);
 }
-__device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ float rcp_approx(float x) {
-  float y;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
-// ---- packed f32x2 arithmetic (sm_100: FFMA2 / FMUL2 / FADD2 work on an aligned register pair) ----
-__device__ __forceinline__ uint64_t pk2(float lo, float hi) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
-}
-__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
+// the epilogue math is written with the packed f32x2 and approximate-math primitives of ptx.cuh
+using ptx::add2;
+using ptx::ex2_approx;
+using ptx::fma2;
+using ptx::mul2;
+using ptx::pack_bf16x2;
+using ptx::pk2;
+using ptx::rcp_approx;
+using ptx::upk2;
 
 // erf-GELU of a pair, in place.  erfc(z) = exp2(z Q(z)) on z = |x|/sqrt(2) in [0, 4] with Q a minimax fit of
 // log2(erfc(z))/z (tools/fit_erfc.py; erfc(4) = 1.5e-8 is below f32 resolution of 1, so z is clamped there).  The

@@ -10,12 +10,6 @@ namespace {
 
 constexpr int kMaxVec = 16;  // float2 per lane -> D <= 1024 on the fast path
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
 // D even, D <= 1024, strides even.  NV = ceil(D / 64).
 template <int NV, int OUT>
 __global__ void __launch_bounds__(256) ln_rows_kernel(const float* x, long long x_stride,
@@ -40,7 +34,7 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const float* x, long long 
       v[i] = make_float2(0.f, 0.f);
     }
   }
-  const float mean = warp_sum(s) / static_cast<float>(D);
+  const float mean = ptx::warp_sum(s) / static_cast<float>(D);
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
@@ -50,7 +44,7 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const float* x, long long 
       q += a * a + b * b;
     }
   }
-  const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+  const float rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(D) + eps);
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = i * 64 + lane * 2;
@@ -116,7 +110,7 @@ __global__ void __launch_bounds__(256) ln_rows4_kernel(const float* x, long long
       s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
     }
   }
-  const float mean = warp_sum(s) / static_cast<float>(D);
+  const float mean = ptx::warp_sum(s) / static_cast<float>(D);
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
@@ -126,33 +120,14 @@ __global__ void __launch_bounds__(256) ln_rows4_kernel(const float* x, long long
       q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
     }
   }
-  const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+  const float rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(D) + eps);
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = i * 128 + lane * 4;
     if (c < D) {
       const float4 g = PRE ? gpre[i] : __ldg(reinterpret_cast<const float4*>(gamma + c));
       const float4 b = PRE ? bpre[i] : __ldg(reinterpret_cast<const float4*>(beta + c));
-      float o0 = (v[i].x - mean) * rstd * g.x + b.x;
-      float o1 = (v[i].y - mean) * rstd * g.y + b.y;
-      float o2 = (v[i].z - mean) * rstd * g.z + b.z;
-      float o3 = (v[i].w - mean) * rstd * g.w + b.w;
-      if (y_copy != nullptr) *reinterpret_cast<float4*>(y_copy + row * x_stride + c) = make_float4(o0, o1, o2, o3);  // unrounded
-      if (OUT == EVT_TF32) {
-        o0 = ptx::round_tf32(o0);
-        o1 = ptx::round_tf32(o1);
-        o2 = ptx::round_tf32(o2);
-        o3 = ptx::round_tf32(o3);
-      }
-      if (OUT == EVT_BF16) {
-        __nv_bfloat162 h0 = __floats2bfloat162_rn(o0, o1), h1 = __floats2bfloat162_rn(o2, o3);
-        uint2 w;
-        w.x = *reinterpret_cast<uint32_t*>(&h0);
-        w.y = *reinterpret_cast<uint32_t*>(&h1);
-        *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(y) + row * y_stride + c) = w;
-      } else {
-        *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + row * y_stride + c) = make_float4(o0, o1, o2, o3);
-      }
+      ptx::store_ln4<OUT>(v[i], mean, rstd, g, b, y, y_stride, y_copy, x_stride, row, c);
     }
   }
 }
@@ -184,44 +159,21 @@ __global__ void __launch_bounds__(256) ln_rows4_sub_kernel(const float* x, long 
                  : "l"(xr + c));
     s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
   }
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  const float mean = s / static_cast<float>(D);
+  const float mean = ptx::group_sum<LPR>(s) / static_cast<float>(D);
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const float a0 = v[i].x - mean, a1 = v[i].y - mean, a2 = v[i].z - mean, a3 = v[i].w - mean;
     q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
   }
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
-  const float rstd = rsqrtf(q / static_cast<float>(D) + eps);
+  const float rstd = rsqrtf(ptx::group_sum<LPR>(q) / static_cast<float>(D) + eps);
   if (!live) return;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = (i * LPR + l) * 4;
     const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
     const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-    float o0 = (v[i].x - mean) * rstd * g.x + b.x;
-    float o1 = (v[i].y - mean) * rstd * g.y + b.y;
-    float o2 = (v[i].z - mean) * rstd * g.z + b.z;
-    float o3 = (v[i].w - mean) * rstd * g.w + b.w;
-    if (y_copy != nullptr) *reinterpret_cast<float4*>(y_copy + row * x_stride + c) = make_float4(o0, o1, o2, o3);  // unrounded
-    if (OUT == EVT_TF32) {
-      o0 = ptx::round_tf32(o0);
-      o1 = ptx::round_tf32(o1);
-      o2 = ptx::round_tf32(o2);
-      o3 = ptx::round_tf32(o3);
-    }
-    if (OUT == EVT_BF16) {
-      __nv_bfloat162 h0 = __floats2bfloat162_rn(o0, o1), h1 = __floats2bfloat162_rn(o2, o3);
-      uint2 w;
-      w.x = *reinterpret_cast<uint32_t*>(&h0);
-      w.y = *reinterpret_cast<uint32_t*>(&h1);
-      *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(y) + row * y_stride + c) = w;
-    } else {
-      *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + row * y_stride + c) = make_float4(o0, o1, o2, o3);
-    }
+    ptx::store_ln4<OUT>(v[i], mean, rstd, g, b, y, y_stride, y_copy, x_stride, row, c);
   }
 }
 
@@ -240,13 +192,13 @@ __global__ void __launch_bounds__(256) ln_rows_generic_kernel(const float* x, lo
   const float* xr = x + row * x_stride;
   float s = 0.f;
   for (int c = lane; c < D; c += 32) s += xr[c];
-  const float mean = warp_sum(s) / static_cast<float>(D);
+  const float mean = ptx::warp_sum(s) / static_cast<float>(D);
   float q = 0.f;
   for (int c = lane; c < D; c += 32) {
     const float a = xr[c] - mean;
     q += a * a;
   }
-  const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+  const float rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(D) + eps);
   for (int c = lane; c < D; c += 32) {
     float o = (xr[c] - mean) * rstd * gamma[c] + beta[c];
     if (y_copy != nullptr) y_copy[row * x_stride + c] = o;  // unrounded
@@ -265,12 +217,12 @@ __global__ void __launch_bounds__(1024) ln2d_kernel(const float* __restrict__ x,
   const long long base = static_cast<long long>(blockIdx.x) * nh;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = blockDim.x >> 5;
   auto block_sum = [&](float v) -> float {
-    v = warp_sum(v);
+    v = ptx::warp_sum(v);
     if (lane == 0) red[warp] = v;
     __syncthreads();
     if (warp == 0) {
       float t = lane < nwarp ? red[lane] : 0.f;
-      t = warp_sum(t);
+      t = ptx::warp_sum(t);
       if (lane == 0) stat = t;
     }
     __syncthreads();

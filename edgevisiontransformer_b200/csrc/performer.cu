@@ -21,12 +21,6 @@ namespace {
 constexpr int kEmb = 64;
 constexpr int kM = 32;
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
 // ---------------------------------------------------------------------------------------------- unfold (+ LN)
 // One warp per output row; lane l owns the column pairs (64 i + 2 l, + 1), so stores are packed bf16x2 (128 B per warp
 // instruction).  KK / CC > 0 fix the window and channel count at compile time (T2T: 7 x 7 x 3 and 3 x 3 x 64) -- the
@@ -88,7 +82,7 @@ __global__ void __launch_bounds__(256) unfold_ln_kernel(const TIN* __restrict__ 
   }
   float mean = 0.f, rstd = 1.f;
   if (LN) {
-    mean = warp_sum(sum) / static_cast<float>(L);
+    mean = ptx::warp_sum(sum) / static_cast<float>(L);
     float q = 0.f;
 #pragma unroll
     for (int i = 0; i < NP; ++i) {
@@ -97,7 +91,7 @@ __global__ void __launch_bounds__(256) unfold_ln_kernel(const TIN* __restrict__ 
       if (col < L) q += d0 * d0;
       if (col + 1 < L) q += d1 * d1;
     }
-    rstd = rsqrtf(warp_sum(q) / static_cast<float>(L) + eps);
+    rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(L) + eps);
   }
   __nv_bfloat16* orow = out + row * ldo;  // ldo is even and the base 4-byte aligned (checked by the launcher)
 #pragma unroll
@@ -108,93 +102,6 @@ __global__ void __launch_bounds__(256) unfold_ln_kernel(const TIN* __restrict__ 
       if (col < L) o0 = LN ? (v0[i] - mean) * rstd * gamma[col] + beta[col] : v0[i];
       if (col + 1 < L) o1 = LN ? (v1[i] - mean) * rstd * gamma[col + 1] + beta[col + 1] : v1[i];
       *reinterpret_cast<__nv_bfloat162*>(orow + col) = __floats2bfloat162_rn(o0, o1);
-    }
-  }
-}
-
-// Compile-time window shapes, several output rows per warp: the column -> (ky, kx, c) decomposition, the LayerNorm affine
-// parameters of the lane's columns and the validity of every column are row-invariant and live in registers across the
-// rows of the warp; interior windows (93 % of a 56 x 56 output grid) skip the per-element bounds tests.  Bit-identical to
-// unfold_ln_kernel (same loads, same reduction order).
-template <typename TIN, bool LN, int KK, int CC, int ROWS>
-__global__ void __launch_bounds__(256) unfold_ln_rows_kernel(const TIN* __restrict__ x, __nv_bfloat16* __restrict__ out,
-                                                             long long ldo, const float* __restrict__ gamma,
-                                                             const float* __restrict__ beta, float eps, int H, int W, int s, int p,
-                                                             int oh, int ow, long long rows) {
-  constexpr int L = KK * KK * CC, kC = KK * CC, NP = (L + 63) / 64;
-  const int lane = threadIdx.x & 31;
-  const long long row0 = (static_cast<long long>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * ROWS;
-  if (row0 >= rows) return;
-  int koff[NP][2], kyx[NP][2];
-  float g[NP][2], be[NP][2];
-#pragma unroll
-  for (int i = 0; i < NP; ++i)
-#pragma unroll
-    for (int e = 0; e < 2; ++e) {
-      const int col = i * 64 + 2 * lane + e;
-      const int ky = col / kC, rem = col - ky * kC, kx = rem / CC;
-      koff[i][e] = col < L ? ky * W * CC + rem : -1;
-      kyx[i][e] = (ky << 8) | kx;
-      g[i][e] = (LN && col < L) ? gamma[col] : 0.f;
-      be[i][e] = (LN && col < L) ? beta[col] : 0.f;
-    }
-  int ox = static_cast<int>(row0 % ow);
-  long long t = row0 / ow;
-  int oy = static_cast<int>(t % oh);
-  long long b = t / oh;
-  // (unrolling this loop by 2 or 4 so that several rows' loads are in flight per warp measured no gain: T2T-ViT-14 batch 256
-  //  47.5-47.8 k against 48.1-48.4 k img/s, same box -- occupancy already hides the load latency)
-#pragma unroll 1
-  for (int r = 0; r < ROWS; ++r) {
-    const long long row = row0 + r;
-    if (row >= rows) break;
-    const int iy0 = oy * s - p, ix0 = ox * s - p;
-    const bool interior = iy0 >= 0 && iy0 + KK <= H && ix0 >= 0 && ix0 + KK <= W;
-    const TIN* base = x + ((b * H + iy0) * static_cast<long long>(W) + ix0) * CC;
-    float v[NP][2];
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < NP; ++i) {
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        bool ok = koff[i][e] >= 0;
-        if (!interior) {
-          const int iy = iy0 + (kyx[i][e] >> 8), ix = ix0 + (kyx[i][e] & 255);
-          ok = ok && iy >= 0 && iy < H && ix >= 0 && ix < W;
-        }
-        v[i][e] = ok ? static_cast<float>(base[koff[i][e]]) : 0.f;
-      }
-      sum += v[i][0] + v[i][1];
-    }
-    float mean = 0.f, rstd = 1.f;
-    if (LN) {
-      mean = warp_sum(sum) / static_cast<float>(L);
-      float q = 0.f;
-#pragma unroll
-      for (int i = 0; i < NP; ++i) {
-        const float d0 = v[i][0] - mean, d1 = v[i][1] - mean;
-        if (koff[i][0] >= 0) q += d0 * d0;
-        if (koff[i][1] >= 0) q += d1 * d1;
-      }
-      rstd = rsqrtf(warp_sum(q) / static_cast<float>(L) + eps);
-    }
-    __nv_bfloat16* orow = out + row * ldo;
-#pragma unroll
-    for (int i = 0; i < NP; ++i) {
-      const int col = i * 64 + 2 * lane;
-      if (col < ldo) {
-        float o0 = 0.f, o1 = 0.f;
-        if (koff[i][0] >= 0) o0 = LN ? (v[i][0] - mean) * rstd * g[i][0] + be[i][0] : v[i][0];
-        if (koff[i][1] >= 0) o1 = LN ? (v[i][1] - mean) * rstd * g[i][1] + be[i][1] : v[i][1];
-        *reinterpret_cast<__nv_bfloat162*>(orow + col) = __floats2bfloat162_rn(o0, o1);
-      }
-    }
-    if (++ox == ow) {
-      ox = 0;
-      if (++oy == oh) {
-        oy = 0;
-        ++b;
-      }
     }
   }
 }
@@ -306,20 +213,11 @@ constexpr int kTileTok = 16;
 constexpr int kChunk = 256;  // tokens per block: 4 warps x 4 tiles
 constexpr float kInvSqrtM = 0.17677669529663687f;  // 1/sqrt(32)
 
-__device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
 // (hi, lo) bf16 pairs of two consecutive f32 values: x ~= hi + lo with 16 mantissa bits
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
   const __nv_bfloat16 ha = __float2bfloat16_rn(a), hb = __float2bfloat16_rn(b);
-  hi = pack2(__bfloat162float(ha), __bfloat162float(hb));
-  lo = pack2(a - __bfloat162float(ha), b - __bfloat162float(hb));
+  hi = ptx::pack_bf16x2(__bfloat162float(ha), __bfloat162float(hb));
+  lo = ptx::pack_bf16x2(a - __bfloat162float(ha), b - __bfloat162float(hb));
 }
 __device__ __forceinline__ float sumsq_bf16x2(uint32_t v) {
   const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v));
@@ -396,8 +294,8 @@ __global__ void __launch_bounds__(128) performer_reduce_kernel(const __nv_bfloat
         float acc[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
         for (int ks = 0; ks < 4; ++ks) {
-          mma_bf16(acc, whi[mi][ks], kb[nj][ks][0], kb[nj][ks][1]);
-          mma_bf16(acc, wlo[mi][ks], kb[nj][ks][0], kb[nj][ks][1]);
+          ptx::mma_bf16_16816(acc, whi[mi][ks], kb[nj][ks][0], kb[nj][ks][1]);
+          ptx::mma_bf16_16816(acc, wlo[mi][ks], kb[nj][ks][0], kb[nj][ks][1]);
         }
         // columns of this lane: tokens 8 nj + 2t, + 1
         const float x0 = __shfl_sync(0xffffffffu, xd[nj], (2 * t) * 4);
@@ -409,8 +307,8 @@ __global__ void __launch_bounds__(128) performer_reduce_kernel(const __nv_bfloat
         const float p3 = ok1 ? __expf(acc[3] - x1) * kInvSqrtM : 0.f;
         ksum[mi][0] += p0 + p1;
         ksum[mi][1] += p2 + p3;
-        pa[mi][nj * 2] = pack2(p0, p1);
-        pa[mi][nj * 2 + 1] = pack2(p2, p3);
+        pa[mi][nj * 2] = ptx::pack_bf16x2(p0, p1);
+        pa[mi][nj * 2 + 1] = ptx::pack_bf16x2(p2, p3);
       }
     }
     // kptv^T += kp^T V
@@ -418,13 +316,11 @@ __global__ void __launch_bounds__(128) performer_reduce_kernel(const __nv_bfloat
     for (int np = 0; np < 4; ++np) {
       uint32_t vb[4];  // {b0, b1} of emb n-tile 2 np, {b0, b1} of 2 np + 1
       const int row = (lane & 7) + ((lane >> 3) & 1) * 8, ch = np * 2 + (lane >> 4);
-      asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-                   : "=r"(vb[0]), "=r"(vb[1]), "=r"(vb[2]), "=r"(vb[3])
-                   : "r"(vt + row * 128 + ((ch ^ (row & 7)) << 4)));
+      ptx::ldmatrix_x4_trans(vt + row * 128 + ((ch ^ (row & 7)) << 4), vb);
 #pragma unroll
       for (int mi = 0; mi < 2; ++mi) {
-        mma_bf16(kacc[mi][2 * np], pa[mi], vb[0], vb[1]);
-        mma_bf16(kacc[mi][2 * np + 1], pa[mi], vb[2], vb[3]);
+        ptx::mma_bf16_16816(kacc[mi][2 * np], pa[mi], vb[0], vb[1]);
+        ptx::mma_bf16_16816(kacc[mi][2 * np + 1], pa[mi], vb[2], vb[3]);
       }
     }
   }
@@ -516,7 +412,7 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
     for (int ks = 0; ks < 4; ++ks) {
       uint32_t b0, b1v;
       bfrag(0, nj, ks, b0, b1v);
-      mma_bf16(acc[nj], a[ks], b0, b1v);
+      ptx::mma_bf16_16816(acc[nj], a[ks], b0, b1v);
     }
     const float2 bb = *reinterpret_cast<const float2*>(&sm.vec[0][nj * 8 + 2 * t]);
     y1[nj][0] += acc[nj][0] + bb.x;
@@ -543,8 +439,8 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
       const int nj = 2 * ks + h, col = nj * 8 + 2 * t;
       const float2 gg = *reinterpret_cast<const float2*>(&sm.vec[1][col]);
       const float2 be = *reinterpret_cast<const float2*>(&sm.vec[2][col]);
-      a[ks][2 * h] = pack2((y1[nj][0] - mA) * rA * gg.x + be.x, (y1[nj][1] - mA) * rA * gg.y + be.y);
-      a[ks][2 * h + 1] = pack2((y1[nj][2] - mB) * rB * gg.x + be.x, (y1[nj][3] - mB) * rB * gg.y + be.y);
+      a[ks][2 * h] = ptx::pack_bf16x2((y1[nj][0] - mA) * rA * gg.x + be.x, (y1[nj][1] - mA) * rA * gg.y + be.y);
+      a[ks][2 * h + 1] = ptx::pack_bf16x2((y1[nj][2] - mB) * rB * gg.x + be.x, (y1[nj][3] - mB) * rB * gg.y + be.y);
     }
   }
   // h = gelu_tanh(z w1^T + b1)
@@ -555,7 +451,7 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
     for (int ks = 0; ks < 4; ++ks) {
       uint32_t b0, b1v;
       bfrag(1, nj, ks, b0, b1v);
-      mma_bf16(acc[nj], a[ks], b0, b1v);
+      ptx::mma_bf16_16816(acc[nj], a[ks], b0, b1v);
     }
   }
 #pragma unroll
@@ -567,8 +463,8 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
       float h0 = acc[nj][0] + bb.x, h1 = acc[nj][1] + bb.y, h2 = acc[nj][2] + bb.x, h3 = acc[nj][3] + bb.y;
       gemm_detail::gelu_tanh_pair(h0, h1);
       gemm_detail::gelu_tanh_pair(h2, h3);
-      a[ks][2 * h] = pack2(h0, h1);
-      a[ks][2 * h + 1] = pack2(h2, h3);
+      a[ks][2 * h] = ptx::pack_bf16x2(h0, h1);
+      a[ks][2 * h + 1] = ptx::pack_bf16x2(h2, h3);
     }
   }
   // y = y1 + h w2^T + b2
@@ -579,7 +475,7 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
     for (int ks = 0; ks < 4; ++ks) {
       uint32_t b0, b1v;
       bfrag(2, nj, ks, b0, b1v);
-      mma_bf16(acc[nj], a[ks], b0, b1v);
+      ptx::mma_bf16_16816(acc[nj], a[ks], b0, b1v);
     }
     const float2 bb = *reinterpret_cast<const float2*>(&sm.vec[4][nj * 8 + 2 * t]);
     y1[nj][0] += acc[nj][0] + bb.x;
@@ -628,7 +524,7 @@ __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat1
 #pragma unroll
       for (int r = 0; r < 2; ++r) {
         const float2 x = *reinterpret_cast<const float2*>(st + kM + (ne * 8 + g) * kM + ks * 16 + r * 8 + 2 * t);
-        kvb[ne][ks][r] = pack2(x.x, x.y);
+        kvb[ne][ks][r] = ptx::pack_bf16x2(x.x, x.y);
       }
   float ksm[4][2];  // ksum of this lane's feature columns 8 nf + 2t, + 1
 #pragma unroll
@@ -663,30 +559,30 @@ __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat1
       float acc[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
       for (int ks = 0; ks < 4; ++ks) {
-        mma_bf16(acc, qa[ks], whi[nf][ks][0], whi[nf][ks][1]);
-        mma_bf16(acc, qa[ks], wlo[nf][ks][0], wlo[nf][ks][1]);
+        ptx::mma_bf16_16816(acc, qa[ks], whi[nf][ks][0], whi[nf][ks][1]);
+        ptx::mma_bf16_16816(acc, qa[ks], wlo[nf][ks][0], wlo[nf][ks][1]);
       }
       const float p0 = __expf(acc[0] - xA) * kInvSqrtM, p1 = __expf(acc[1] - xA) * kInvSqrtM;
       const float p2 = __expf(acc[2] - xB) * kInvSqrtM, p3 = __expf(acc[3] - xB) * kInvSqrtM;
       dA = fmaf(p0, ksm[nf][0], fmaf(p1, ksm[nf][1], dA));
       dB = fmaf(p2, ksm[nf][0], fmaf(p3, ksm[nf][1], dB));
-      pa[nf >> 1][(nf & 1) * 2] = pack2(p0, p1);
-      pa[nf >> 1][(nf & 1) * 2 + 1] = pack2(p2, p3);
+      pa[nf >> 1][(nf & 1) * 2] = ptx::pack_bf16x2(p0, p1);
+      pa[nf >> 1][(nf & 1) * 2 + 1] = ptx::pack_bf16x2(p2, p3);
     }
     const float invA = 1.0f / (quad_sum(dA) + eps), invB = 1.0f / (quad_sum(dB) + eps);
     uint32_t ya_frag[4][4];  // TAIL: yattn as the A fragments of the attn_output product (n-tiles 2 ks, 2 ks + 1 = k-step ks)
 #pragma unroll
     for (int ne = 0; ne < 8; ++ne) {
       float y[4] = {0.f, 0.f, 0.f, 0.f};
-      mma_bf16(y, pa[0], kvb[ne][0][0], kvb[ne][0][1]);
-      mma_bf16(y, pa[1], kvb[ne][1][0], kvb[ne][1][1]);
+      ptx::mma_bf16_16816(y, pa[0], kvb[ne][0][0], kvb[ne][0][1]);
+      ptx::mma_bf16_16816(y, pa[1], kvb[ne][1][0], kvb[ne][1][1]);
       const int col = ne * 8 + 2 * t;
       if (TAIL) {
-        ya_frag[ne >> 1][(ne & 1) * 2] = pack2(y[0] * invA, y[1] * invA);
-        ya_frag[ne >> 1][(ne & 1) * 2 + 1] = pack2(y[2] * invB, y[3] * invB);
+        ya_frag[ne >> 1][(ne & 1) * 2] = ptx::pack_bf16x2(y[0] * invA, y[1] * invA);
+        ya_frag[ne >> 1][(ne & 1) * 2 + 1] = ptx::pack_bf16x2(y[2] * invB, y[3] * invB);
       } else {
-        if (okA) *reinterpret_cast<uint32_t*>(yattn + (r0 + g) * kEmb + col) = pack2(y[0] * invA, y[1] * invA);
-        if (okB) *reinterpret_cast<uint32_t*>(yattn + (r0 + g + 8) * kEmb + col) = pack2(y[2] * invB, y[3] * invB);
+        if (okA) *reinterpret_cast<uint32_t*>(yattn + (r0 + g) * kEmb + col) = ptx::pack_bf16x2(y[0] * invA, y[1] * invA);
+        if (okB) *reinterpret_cast<uint32_t*>(yattn + (r0 + g + 8) * kEmb + col) = ptx::pack_bf16x2(y[2] * invB, y[3] * invB);
       }
     }
     if (TAIL) {
@@ -766,14 +662,12 @@ template <typename TIN, bool LN>
 void unfold_ln_dispatch(const TIN* xi, __nv_bfloat16* o, int64_t ldo, const float* gamma, const float* beta, float eps, int B, int H,
                         int W, int C, int k, int s, int p, int oh, int ow, long long rows, cudaStream_t st) {
   const unsigned grid = static_cast<unsigned>((rows + 7) / 8);
-  constexpr int kRowsPerWarp = 4;
-  const unsigned grid_rows = static_cast<unsigned>((rows + 8 * kRowsPerWarp - 1) / (8 * kRowsPerWarp));
   if (k == 7 && C == 3 && ldo == 152) {
     constexpr int kIter = 2;  // 8 warps x 4 rows x 2 iterations = 64 rows per block
     const unsigned g773 = static_cast<unsigned>((rows + 64 - 1) / 64);
     unfold773_kernel<TIN, LN, kIter><<<g773, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, H, W, s, p, oh, ow, rows);
   }
-  else if (k == 7 && C == 3) unfold_ln_rows_kernel<TIN, LN, 7, 3, kRowsPerWarp><<<grid_rows, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, H, W, s, p, oh, ow, rows);
+  else if (k == 7 && C == 3) unfold_ln_kernel<TIN, LN, 7, 3><<<grid, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, B, H, W, C, k, s, p, oh, ow, rows);
   else if (k == 3 && C == 64) unfold_ln_kernel<TIN, LN, 3, 64><<<grid, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, B, H, W, C, k, s, p, oh, ow, rows);
   else unfold_ln_kernel<TIN, LN, 0, 0><<<grid, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, B, H, W, C, k, s, p, oh, ow, rows);
 }

@@ -1,11 +1,15 @@
 // Thin inline-PTX wrappers for the sm_100a features the kernels use:
-// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld / st), fences.
+// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld / st), fences; and the device helpers shared by
+// several kernel files: approximate ex2 / rcp, packed f32x2 arithmetic, bf16x2 packing, lane-group sums, the LayerNorm store
+// of four row elements, mma.sync m16n8k16 and ldmatrix.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+
+#include "../../include/evt.h"
 
 namespace evt {
 namespace ptx {
@@ -341,6 +345,104 @@ __device__ __forceinline__ float round_tf32(float x) {
   uint32_t y;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(y) : "f"(x));
   return __uint_as_float(y);
+}
+
+// ---------------------------------------------------------------- math
+__device__ __forceinline__ float ex2_approx(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+__device__ __forceinline__ float rcp_approx(float x) {
+  float y;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+
+// packed f32x2 arithmetic (sm_100: FFMA2 / FMUL2 / FADD2 work on an aligned register pair)
+__device__ __forceinline__ uint64_t pk2(float lo, float hi) {
+  uint64_t r;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+  return r;
+}
+__device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) {
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+}
+__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
+  uint64_t d;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
+  return d;
+}
+__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
+__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
+
+// two floats -> bf16x2 (round to nearest), a in the low half
+__device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
+  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
+
+// Sum over aligned groups of LANES lanes (xor butterfly, offsets LANES/2 .. 1): every lane of a group gets its group's sum.
+template <int LANES>
+__device__ __forceinline__ float group_sum(float v) {
+#pragma unroll
+  for (int o = LANES / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+__device__ __forceinline__ float warp_sum(float v) { return group_sum<32>(v); }
+
+// LayerNorm output of four consecutive row elements: (v - mean) * rstd * g + b, stored at column c of row `row` of y (row
+// stride y_stride) as bf16 (OUT = EVT_BF16), f32 (EVT_F32) or f32 rounded to tf32 (EVT_TF32).  A non-null `copy` (row stride
+// copy_stride) first receives the unrounded f32 values.
+template <int OUT>
+__device__ __forceinline__ void store_ln4(float4 v, float mean, float rstd, float4 g, float4 b, void* y, long long y_stride,
+                                          float* copy, long long copy_stride, long long row, int c) {
+  float o0 = (v.x - mean) * rstd * g.x + b.x;
+  float o1 = (v.y - mean) * rstd * g.y + b.y;
+  float o2 = (v.z - mean) * rstd * g.z + b.z;
+  float o3 = (v.w - mean) * rstd * g.w + b.w;
+  if (copy != nullptr) *reinterpret_cast<float4*>(copy + row * copy_stride + c) = make_float4(o0, o1, o2, o3);
+  if (OUT == EVT_TF32) {
+    o0 = round_tf32(o0);
+    o1 = round_tf32(o1);
+    o2 = round_tf32(o2);
+    o3 = round_tf32(o3);
+  }
+  if (OUT == EVT_BF16) {
+    uint2 w;
+    w.x = pack_bf16x2(o0, o1);
+    w.y = pack_bf16x2(o2, o3);
+    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(y) + row * y_stride + c) = w;
+  } else {
+    *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + row * y_stride + c) = make_float4(o0, o1, o2, o3);
+  }
+}
+
+// ---------------------------------------------------------------- warp-level tensor core (mma.sync)
+// d += a b, m16n8k16, bf16 operands, f32 accumulate
+__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+// four 8x8 b16 matrices from shared memory (lanes 8i .. 8i+7 give the row addresses of matrix i)
+__device__ __forceinline__ void ldmatrix_x4(uint32_t addr, uint32_t (&r)[4]) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(addr));
+}
+__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t addr, uint32_t (&r)[4]) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(addr));
 }
 
 // ---------------------------------------------------------------- descriptors

@@ -26,19 +26,9 @@
 namespace evt {
 namespace {
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-
 // ---------------------------------------------------------------------------------------------------- gather + LN
 // One warp per output row of D = G * C floats (C % 4 == 0, D <= 128 * NV).
-template <int NV, bool OUT_BF16>
+template <int NV, int OUT>
 __global__ void __launch_bounds__(256) gather_ln_kernel(const float* __restrict__ x, const int* __restrict__ idx,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
                                                         void* __restrict__ y, float* __restrict__ copy, long long rows_out,
@@ -74,7 +64,7 @@ __global__ void __launch_bounds__(256) gather_ln_kernel(const float* __restrict_
     }
   }
   if (y == nullptr) return;
-  const float mean = warp_sum(s) / static_cast<float>(D);
+  const float mean = ptx::warp_sum(s) / static_cast<float>(D);
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
@@ -84,32 +74,21 @@ __global__ void __launch_bounds__(256) gather_ln_kernel(const float* __restrict_
       q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
     }
   }
-  const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+  const float rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(D) + eps);
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = i * 128 + lane * 4;
     if (c < D) {
       const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
       const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-      const float o0 = (v[i].x - mean) * rstd * g.x + b.x;
-      const float o1 = (v[i].y - mean) * rstd * g.y + b.y;
-      const float o2 = (v[i].z - mean) * rstd * g.z + b.z;
-      const float o3 = (v[i].w - mean) * rstd * g.w + b.w;
-      if (OUT_BF16) {
-        uint2 o;
-        o.x = pack_bf16(o0, o1);
-        o.y = pack_bf16(o2, o3);
-        *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(y) + row * D + c) = o;
-      } else {
-        *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + row * D + c) = make_float4(o0, o1, o2, o3);
-      }
+      ptx::store_ln4<OUT>(v[i], mean, rstd, g, b, y, D, nullptr, 0, row, c);
     }
   }
 }
 
 // G = 1 with narrow rows (C = 96 / 192: Swin stages 1 and 2): 32 / LPR rows per warp, every lane carries NV float4
 // (a whole warp per 96-float row leaves a quarter of the lanes idle; these launches cover 802 816 rows at batch 256).
-template <int LPR, int NV, bool OUT_BF16>
+template <int LPR, int NV, int OUT>
 __global__ void __launch_bounds__(256) gather_ln_sub_kernel(const float* __restrict__ x, const int* __restrict__ idx,
                                                             const float* __restrict__ gamma, const float* __restrict__ beta,
                                                             void* __restrict__ y, float* __restrict__ copy, long long rows_out,
@@ -138,36 +117,21 @@ __global__ void __launch_bounds__(256) gather_ln_sub_kernel(const float* __restr
     for (int i = 0; i < NV; ++i) *reinterpret_cast<float4*>(copy + row * C + (i * LPR + l) * 4) = v[i];
   }
   if (y == nullptr) return;
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  const float mean = s / static_cast<float>(C);
+  const float mean = ptx::group_sum<LPR>(s) / static_cast<float>(C);
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const float a0 = v[i].x - mean, a1 = v[i].y - mean, a2 = v[i].z - mean, a3 = v[i].w - mean;
     q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
   }
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
-  const float rstd = rsqrtf(q / static_cast<float>(C) + eps);
+  const float rstd = rsqrtf(ptx::group_sum<LPR>(q) / static_cast<float>(C) + eps);
   if (!live) return;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = (i * LPR + l) * 4;
     const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
     const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-    const float o0 = (v[i].x - mean) * rstd * g.x + b.x;
-    const float o1 = (v[i].y - mean) * rstd * g.y + b.y;
-    const float o2 = (v[i].z - mean) * rstd * g.z + b.z;
-    const float o3 = (v[i].w - mean) * rstd * g.w + b.w;
-    if (OUT_BF16) {
-      uint2 o;
-      o.x = pack_bf16(o0, o1);
-      o.y = pack_bf16(o2, o3);
-      *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(y) + row * C + c) = o;
-    } else {
-      *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + row * C + c) = make_float4(o0, o1, o2, o3);
-    }
+    ptx::store_ln4<OUT>(v[i], mean, rstd, g, b, y, C, nullptr, 0, row, c);
   }
 }
 
@@ -178,10 +142,10 @@ int launch_gather_ln_sub(const float* x, const int* idx, const float* gamma, con
   const unsigned grid = static_cast<unsigned>((rows_out + 8 * RPW - 1) / (8 * RPW));
   const bool pdl = pdl_for_work(rows_out, 4 * LPR * NV);
   if (y_dtype == EVT_BF16)
-    EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, true>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
+    EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, EVT_BF16>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
                         T_in, T_out, eps));
   else
-    EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, false>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
+    EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, EVT_F32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
                         T_in, T_out, eps));
   EVT_LAUNCH_CHECK("gather_ln_sub_kernel");
   return EVT_OK;
@@ -193,10 +157,10 @@ int launch_gather_ln(const float* x, const int* idx, const float* gamma, const f
   const unsigned grid = static_cast<unsigned>((rows_out + 7) / 8);
   const bool pdl = pdl_for_work(rows_out, static_cast<long long>(G) * C);
   if (y_dtype == EVT_BF16)
-    EVT_CUDA(launch_pdl(gather_ln_kernel<NV, true>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
+    EVT_CUDA(launch_pdl(gather_ln_kernel<NV, EVT_BF16>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
                         T_out, G, C, eps));
   else
-    EVT_CUDA(launch_pdl(gather_ln_kernel<NV, false>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
+    EVT_CUDA(launch_pdl(gather_ln_kernel<NV, EVT_F32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
                         T_out, G, C, eps));
   EVT_LAUNCH_CHECK("gather_ln_kernel");
   return EVT_OK;
@@ -210,26 +174,6 @@ constexpr int kWKeyCols = 56; // key columns of the score tile (7 n-tiles of 8);
 constexpr int kWWarps = 4;
 constexpr int kWMatBytes = kWRows * kWHd * 2;  // 4 KB
 
-__device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ float ex2f(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 // byte offset of (row, 16-byte chunk) in a [64 rows][64 bytes] matrix: chunks XOR-swizzled by (row / 2) % 4, so the
 // eight 16-byte rows an ldmatrix phase reads fall into eight different bank groups
 __device__ __forceinline__ uint32_t wofs(int row, int chunk) { return row * 64 + ((chunk ^ ((row >> 1) & 3)) << 4); }
@@ -275,26 +219,26 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
     // K fragments (B operand of S = Q K^T): n-tile nt = keys 8 nt .. 8 nt + 7; registers {ks0.b0, ks0.b1, ks1.b0, ks1.b1}
     uint32_t kb[7][4];
 #pragma unroll
-    for (int nt = 0; nt < 7; ++nt) ldsm_x4(aK + wofs(nt * 8 + (lane & 7), lane >> 3), kb[nt]);
+    for (int nt = 0; nt < 7; ++nt) ptx::ldmatrix_x4(aK + wofs(nt * 8 + (lane & 7), lane >> 3), kb[nt]);
     // V fragments (B operand of O = P V): k-step kk = keys 16 kk .. +15, dims chunk pair cp: {n 2cp: b0, b1, n 2cp+1: b0, b1}
     uint32_t vb[4][2][4];
 #pragma unroll
     for (int kk = 0; kk < 4; ++kk)
 #pragma unroll
       for (int cp = 0; cp < 2; ++cp)
-        ldsm_x4_t(aV + wofs(kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, cp * 2 + (lane >> 4)), vb[kk][cp]);
+        ptx::ldmatrix_x4_trans(aV + wofs(kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, cp * 2 + (lane >> 4)), vb[kk][cp]);
     const float* tb = tab + ((w % n_tab) * heads + h) * static_cast<long long>(kWRows * kWKeyCols);
 #pragma unroll 1
     for (int mt = 0; mt < 4; ++mt) {
       uint32_t qa[2][4];
 #pragma unroll
-      for (int ks = 0; ks < 2; ++ks) ldsm_x4(aQ + wofs(mt * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, ks * 2 + (lane >> 4)), qa[ks]);
+      for (int ks = 0; ks < 2; ++ks) ptx::ldmatrix_x4(aQ + wofs(mt * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, ks * 2 + (lane >> 4)), qa[ks]);
       float s[7][4];
 #pragma unroll
       for (int nt = 0; nt < 7; ++nt) {
         s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
-        mma_bf16(s[nt], qa[0], kb[nt][0], kb[nt][1]);
-        mma_bf16(s[nt], qa[1], kb[nt][2], kb[nt][3]);
+        ptx::mma_bf16_16816(s[nt], qa[0], kb[nt][0], kb[nt][1]);
+        ptx::mma_bf16_16816(s[nt], qa[1], kb[nt][2], kb[nt][3]);
       }
       // scores -> log2 domain with bias / mask; rows g and g + 8 of this m-tile, columns 8 nt + 2 t, + 1
       const float* t0 = tb + (mt * 16 + g) * kWKeyCols + 2 * t;
@@ -319,12 +263,12 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
       uint32_t pa[4][4];  // probabilities as A fragments of the four k-steps (keys 56..63 do not exist -> 0)
 #pragma unroll
       for (int nt = 0; nt < 7; ++nt) {
-        const float p0 = ex2f(s[nt][0] - m0), p1 = ex2f(s[nt][1] - m0);
-        const float p2 = ex2f(s[nt][2] - m1), p3 = ex2f(s[nt][3] - m1);
+        const float p0 = ptx::ex2_approx(s[nt][0] - m0), p1 = ptx::ex2_approx(s[nt][1] - m0);
+        const float p2 = ptx::ex2_approx(s[nt][2] - m1), p3 = ptx::ex2_approx(s[nt][3] - m1);
         l0 += p0 + p1;
         l1 += p2 + p3;
-        pa[nt >> 1][(nt & 1) * 2] = pack_bf16(p0, p1);
-        pa[nt >> 1][(nt & 1) * 2 + 1] = pack_bf16(p2, p3);
+        pa[nt >> 1][(nt & 1) * 2] = ptx::pack_bf16x2(p0, p1);
+        pa[nt >> 1][(nt & 1) * 2 + 1] = ptx::pack_bf16x2(p2, p3);
       }
       pa[3][2] = pa[3][3] = 0u;
       l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
@@ -337,14 +281,14 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
 #pragma unroll
       for (int kk = 0; kk < 4; ++kk)
 #pragma unroll
-        for (int n = 0; n < 4; ++n) mma_bf16(o[n], pa[kk], vb[kk][n >> 1][(n & 1) * 2], vb[kk][n >> 1][(n & 1) * 2 + 1]);
+        for (int n = 0; n < 4; ++n) ptx::mma_bf16_16816(o[n], pa[kk], vb[kk][n >> 1][(n & 1) * 2], vb[kk][n >> 1][(n & 1) * 2 + 1]);
       const float i0 = 1.0f / l0, i1 = 1.0f / l1;  // l >= 1: the row maximum contributes 2^0
       const int r0 = mt * 16 + g, r1 = r0 + 8;
 #pragma unroll
       for (int n = 0; n < 4; ++n) {
         const int col = h * kWHd + n * 8 + 2 * t;
-        if (r0 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r0) * ldc + col) = pack_bf16(o[n][0] * i0, o[n][1] * i0);
-        if (r1 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r1) * ldc + col) = pack_bf16(o[n][2] * i1, o[n][3] * i1);
+        if (r0 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r0) * ldc + col) = ptx::pack_bf16x2(o[n][0] * i0, o[n][1] * i0);
+        if (r1 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r1) * ldc + col) = ptx::pack_bf16x2(o[n][2] * i1, o[n][3] * i1);
       }
     }
   }
@@ -378,7 +322,7 @@ __global__ void __launch_bounds__(256) ln_mean_tokens_kernel(const float* __rest
         s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
       }
     }
-    const float mean = warp_sum(s) / static_cast<float>(D);
+    const float mean = ptx::warp_sum(s) / static_cast<float>(D);
     float q = 0.f;
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
@@ -388,7 +332,7 @@ __global__ void __launch_bounds__(256) ln_mean_tokens_kernel(const float* __rest
         q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
       }
     }
-    const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+    const float rstd = rsqrtf(ptx::warp_sum(q) / static_cast<float>(D) + eps);
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
       acc[i].x += (v[i].x - mean) * rstd;
@@ -431,8 +375,8 @@ __global__ void __launch_bounds__(256) im2col4_kernel(const float* __restrict__ 
   const long long row = (b * (H / P) + py) * (W / P) + pxi;
   const int k = (c * P + i) * P + j;
   uint2 o;
-  o.x = pack_bf16(v.x, v.y);
-  o.y = pack_bf16(v.z, v.w);
+  o.x = ptx::pack_bf16x2(v.x, v.y);
+  o.y = ptx::pack_bf16x2(v.z, v.w);
   *reinterpret_cast<uint2*>(cols + row * (3ll * P * P) + k) = o;
 }
 
