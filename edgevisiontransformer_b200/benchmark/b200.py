@@ -7,6 +7,7 @@ each bracketed by a stream synchronise and ``timeit.default_timer``; optional ``
 
     python -m edgevisiontransformer_b200.benchmark --model deit_tiny --batch 1 --precision tf32 --graph
     python -m edgevisiontransformer_b200.benchmark --model deit_base --image-size 384 --batch 256
+    python -m edgevisiontransformer_b200.benchmark --model swin_large --image-size 384 --batch 256
     python -m edgevisiontransformer_b200.benchmark --model /path/to/pruned_checkpoint --batch 1024
     python -m edgevisiontransformer_b200.benchmark --model attention --h 768 --a 12 --n 197      (op-level, tools.py:735-758)
 """
@@ -23,7 +24,10 @@ import torch
 
 DEIT = {"deit_tiny": (192, 3, 768), "deit_small": (384, 6, 1536), "deit_base": (768, 12, 3072)}
 SWIN = {"swin_tiny": (96, [2, 2, 6, 2], [3, 6, 12, 24]), "swin_small": (96, [2, 2, 18, 2], [3, 6, 12, 24]),
-        "swin_base": (128, [2, 2, 18, 2], [4, 8, 16, 32])}         # swin_*_patch4_window7_224 (tools.py:280)
+        "swin_base": (128, [2, 2, 18, 2], [4, 8, 16, 32]), "swin_large": (192, [2, 2, 18, 2], [6, 12, 24, 48])}
+# swin_*_patch4_window7_224 (tools.py:280); --image-size 384 takes the window12_384 geometry (published for base / large;
+# tiny / small run the same geometry)
+SWIN_WINDOW = {224: 7, 384: 12}
 T2T = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_12": (256, 12, 4, 2.0),
        "t2t_vit_14": (384, 14, 6, 3.0)}
 
@@ -75,8 +79,8 @@ def _random_t2t_weights(hidden, depth, heads, mlp_ratio, seed=0):
 
 
 def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", image_size: int = 224, **op_kw):
-    """-> (callable taking one CUDA tensor, input shape without batch, description).  image_size: deit_* only
-    (224 or 384, the two resolutions of deit_*_patch16_*)."""
+    """-> (callable taking one CUDA tensor, input shape without batch, description).  image_size: deit_* and swin_* (224 or
+    384: deit_*_patch16_{224,384}, swin_*_patch4_window7_224 / swin_*_patch4_window12_384)."""
     from .. import B200ViTForImageClassification
     if name in DEIT:
         m = B200ViTForImageClassification.from_hf(_random_hf(name, image_size=image_size), device=device, max_batch=max_batch,
@@ -92,11 +96,12 @@ def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device
         from transformers import SwinConfig, SwinForImageClassification
         from ..modeling_swin import B200SwinForImageClassification
         dim, depths, heads = SWIN[name]
+        window = SWIN_WINDOW[image_size]
         torch.manual_seed(0)
-        hf = SwinForImageClassification(SwinConfig(image_size=224, patch_size=4, window_size=7, embed_dim=dim, depths=depths,
-                                                   num_heads=heads, num_labels=1000)).eval()
+        hf = SwinForImageClassification(SwinConfig(image_size=image_size, patch_size=4, window_size=window, embed_dim=dim,
+                                                   depths=depths, num_heads=heads, num_labels=1000)).eval()
         m = B200SwinForImageClassification.from_hf(hf, device=device, max_batch=min(max_batch, 1024))
-        return m, (3, 224, 224), f"{name} random-init (bf16)"
+        return m, (3, image_size, image_size), f"{name} random-init (bf16, {image_size} px, window {window})"
     if name in ("attention", "ffn"):
         from .. import torch_layers as tl
         h, n = op_kw.get("h", 768), op_kw.get("n", 128)
@@ -138,14 +143,15 @@ def b200_benchmark(model, input_shape: Sequence[int], num_runs: int = 50, warmup
 
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="b200_benchmark", description=__doc__.split("\n")[0])
-    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | swin_{tiny,small,base} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir")
+    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir")
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--precision", default="bf16", choices=["bf16", "tf32"])
     ap.add_argument("--num_runs", type=int, default=50)
     ap.add_argument("--warmup_runs", type=int, default=20)
     ap.add_argument("--topk", type=int, default=None)
     ap.add_argument("--graph", action="store_true", help="CUDA-graph replay (small-batch latency path)")
-    ap.add_argument("--image-size", type=int, default=224, help="deit_* input resolution (384: deit_*_patch16_384, 577 tokens)")
+    ap.add_argument("--image-size", type=int, default=224,
+                    help="deit_* / swin_* input resolution (384: deit_*_patch16_384, 577 tokens; swin_*_patch4_window12_384)")
     for k, d in (("h", 768), ("a", 12), ("i", 3072), ("n", 128)):
         ap.add_argument(f"--{k}", type=int, default=d)
     ap.add_argument("--h_k", type=int, default=None)
@@ -153,8 +159,10 @@ def main(argv=None) -> int:
     if not torch.cuda.is_available():
         print("b200_benchmark needs a B200 (sm_100a): the backend has no CPU path")
         return 2
-    if a.image_size != 224 and a.model not in DEIT:
-        ap.error("--image-size applies to the deit_* models only")
+    if a.image_size != 224 and a.model not in DEIT and a.model not in SWIN:
+        ap.error("--image-size applies to the deit_* and swin_* models only")
+    if a.model in SWIN and a.image_size not in SWIN_WINDOW:
+        ap.error("swin_* runs at --image-size 224 (window 7) or 384 (window 12)")
     model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), image_size=a.image_size, h=a.h, a=a.a, i=a.i,
                                      n=a.n, h_k=a.h_k)
     avg, std, times = b200_benchmark(model, (a.batch, *shape), a.num_runs, a.warmup_runs, a.topk, graph=a.graph)

@@ -16,6 +16,8 @@
 //                             fragments).  A 49 x 49 x 32 problem fills 38 % of a 128-row tcgen05 tile and its time is
 //                             exp / load bound, so the warp-level tensor path is used here (a tcgen05 kernel with two
 //                             windows per tile was measured slower, DESIGN.md).
+//   window_attention144_kernel the same for 12 x 12 windows (144 tokens, swin_*_window12_384); K and V fragments are
+//                             re-read from shared memory per query m-tile instead of held in registers.
 //   ln_mean_tokens_kernel     final LayerNorm + average pool over the tokens of an image (SwinModel.layernorm + pooler).
 #include <cuda_bf16.h>
 #include <math_constants.h>
@@ -174,9 +176,74 @@ constexpr int kWKeyCols = 56; // key columns of the score tile (7 n-tiles of 8);
 constexpr int kWWarps = 4;
 constexpr int kWMatBytes = kWRows * kWHd * 2;  // 4 KB
 
-// byte offset of (row, 16-byte chunk) in a [64 rows][64 bytes] matrix: chunks XOR-swizzled by (row / 2) % 4, so the
+// 12 x 12 windows (swin_*_window12_384): 144 = 9 m16 query tiles x 18 n8 key tiles, no padding
+constexpr int kW12Tok = 144;
+constexpr int kW12Warps = 4;                    // 4 x 27 KB per CTA: 2 CTAs = 8 warps per SM
+constexpr int kW12MatBytes = kW12Tok * kWHd * 2;  // 9 KB
+
+// byte offset of (row, 16-byte chunk) in a [rows][64 bytes] matrix: chunks XOR-swizzled by (row / 2) % 4, so the
 // eight 16-byte rows an ldmatrix phase reads fall into eight different bank groups
 __device__ __forceinline__ uint32_t wofs(int row, int chunk) { return row * 64 + ((chunk ^ ((row >> 1) & 3)) << 4); }
+
+// cp.async the q, k and v slices of head h of the window whose first row is row0 (TOK rows each) into the warp's three
+// swizzled matrices at aQ, aQ + MAT, aQ + 2 MAT, and wait for them
+template <int TOK, int MAT>
+__device__ __forceinline__ void stage_window(const __nv_bfloat16* __restrict__ qkv, long long ldq, long long row0, int C, int h,
+                                             uint32_t aQ, int lane) {
+  for (int c = lane; c < 3 * TOK * 4; c += 32) {
+    const int mat = c / (TOK * 4), rc = c - mat * (TOK * 4);
+    const int row = rc >> 2, ch = rc & 3;
+    const __nv_bfloat16* src = qkv + (row0 + row) * ldq + mat * C + h * kWHd + ch * 8;
+    const uint32_t dst = aQ + mat * MAT + wofs(row, ch);
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+  }
+  asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
+}
+
+// Scores of the rows g and g + 8 of one m-tile (NT n-tiles) -> log2 domain plus the table rows t0 / t1 (columns
+// 8 nt + 2 t, + 1); m0 / m1 = the row maxima over the quad
+template <int NT>
+__device__ __forceinline__ void scores_rowmax(float (&s)[NT][4], const float* __restrict__ t0, const float* __restrict__ t1,
+                                              float scale_log2e, float& m0, float& m1) {
+  m0 = -CUDART_INF_F, m1 = -CUDART_INF_F;
+#pragma unroll
+  for (int nt = 0; nt < NT; ++nt) {
+    const float2 b0 = __ldg(reinterpret_cast<const float2*>(t0 + nt * 8));
+    const float2 b1 = __ldg(reinterpret_cast<const float2*>(t1 + nt * 8));
+    s[nt][0] = fmaf(s[nt][0], scale_log2e, b0.x);
+    s[nt][1] = fmaf(s[nt][1], scale_log2e, b0.y);
+    s[nt][2] = fmaf(s[nt][2], scale_log2e, b1.x);
+    s[nt][3] = fmaf(s[nt][3], scale_log2e, b1.y);
+    m0 = fmaxf(m0, fmaxf(s[nt][0], s[nt][1]));
+    m1 = fmaxf(m1, fmaxf(s[nt][2], s[nt][3]));
+  }
+  m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1));
+  m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
+  m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1));
+  m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
+}
+
+// Probabilities 2^(s - m) as the A fragments of the (NT + 1) / 2 k-steps of P V (an odd NT leaves the last k-step's upper
+// half zero: those keys do not exist); l0 / l1 = the row sums over the quad
+template <int NT>
+__device__ __forceinline__ void exp_rowsum(const float (&s)[NT][4], float m0, float m1, uint32_t (&pa)[(NT + 1) / 2][4], float& l0,
+                                           float& l1) {
+  l0 = 0.f, l1 = 0.f;
+#pragma unroll
+  for (int nt = 0; nt < NT; ++nt) {
+    const float p0 = ptx::ex2_approx(s[nt][0] - m0), p1 = ptx::ex2_approx(s[nt][1] - m0);
+    const float p2 = ptx::ex2_approx(s[nt][2] - m1), p3 = ptx::ex2_approx(s[nt][3] - m1);
+    l0 += p0 + p1;
+    l1 += p2 + p3;
+    pa[nt >> 1][(nt & 1) * 2] = ptx::pack_bf16x2(p0, p1);
+    pa[nt >> 1][(nt & 1) * 2 + 1] = ptx::pack_bf16x2(p2, p3);
+  }
+  if (NT & 1) pa[NT >> 1][2] = pa[NT >> 1][3] = 0u;
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+}
 
 // qkv  bf16 [n_windows * 49, ldq], columns q | k | v (each heads * 32), head h at h * 32 inside each
 // tab  f32 [n_tab, heads, 64, 56] = (relative position bias + shift mask) * log2(e); key columns >= 49 hold -inf
@@ -207,14 +274,7 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
     const int h = static_cast<int>(item - w * heads);
     const long long row0 = w * kWTok;
     __syncwarp();  // every lane is done with the previous item's shared memory
-    for (int c = lane; c < 3 * kWTok * 4; c += 32) {
-      const int mat = c / (kWTok * 4), rc = c - mat * (kWTok * 4);
-      const int row = rc >> 2, ch = rc & 3;
-      const __nv_bfloat16* src = qkv + (row0 + row) * ldq + mat * C + h * kWHd + ch * 8;
-      const uint32_t dst = aQ + mat * kWMatBytes + wofs(row, ch);
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-    }
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
+    stage_window<kWTok, kWMatBytes>(qkv, ldq, row0, C, h, aQ, lane);
     __syncwarp();
     // K fragments (B operand of S = Q K^T): n-tile nt = keys 8 nt .. 8 nt + 7; registers {ks0.b0, ks0.b1, ks1.b0, ks1.b1}
     uint32_t kb[7][4];
@@ -243,38 +303,10 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
       // scores -> log2 domain with bias / mask; rows g and g + 8 of this m-tile, columns 8 nt + 2 t, + 1
       const float* t0 = tb + (mt * 16 + g) * kWKeyCols + 2 * t;
       const float* t1 = t0 + 8 * kWKeyCols;
-      float m0 = -CUDART_INF_F, m1 = -CUDART_INF_F;
-#pragma unroll
-      for (int nt = 0; nt < 7; ++nt) {
-        const float2 b0 = __ldg(reinterpret_cast<const float2*>(t0 + nt * 8));
-        const float2 b1 = __ldg(reinterpret_cast<const float2*>(t1 + nt * 8));
-        s[nt][0] = fmaf(s[nt][0], scale_log2e, b0.x);
-        s[nt][1] = fmaf(s[nt][1], scale_log2e, b0.y);
-        s[nt][2] = fmaf(s[nt][2], scale_log2e, b1.x);
-        s[nt][3] = fmaf(s[nt][3], scale_log2e, b1.y);
-        m0 = fmaxf(m0, fmaxf(s[nt][0], s[nt][1]));
-        m1 = fmaxf(m1, fmaxf(s[nt][2], s[nt][3]));
-      }
-      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1));
-      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1));
-      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-      float l0 = 0.f, l1 = 0.f;
+      float m0, m1, l0, l1;
+      scores_rowmax<7>(s, t0, t1, scale_log2e, m0, m1);
       uint32_t pa[4][4];  // probabilities as A fragments of the four k-steps (keys 56..63 do not exist -> 0)
-#pragma unroll
-      for (int nt = 0; nt < 7; ++nt) {
-        const float p0 = ptx::ex2_approx(s[nt][0] - m0), p1 = ptx::ex2_approx(s[nt][1] - m0);
-        const float p2 = ptx::ex2_approx(s[nt][2] - m1), p3 = ptx::ex2_approx(s[nt][3] - m1);
-        l0 += p0 + p1;
-        l1 += p2 + p3;
-        pa[nt >> 1][(nt & 1) * 2] = ptx::pack_bf16x2(p0, p1);
-        pa[nt >> 1][(nt & 1) * 2 + 1] = ptx::pack_bf16x2(p2, p3);
-      }
-      pa[3][2] = pa[3][3] = 0u;
-      l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-      l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-      l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-      l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+      exp_rowsum<7>(s, m0, m1, pa, l0, l1);
       float o[4][4];
 #pragma unroll
       for (int n = 0; n < 4; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
@@ -289,6 +321,77 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
         const int col = h * kWHd + n * 8 + 2 * t;
         if (r0 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r0) * ldc + col) = ptx::pack_bf16x2(o[n][0] * i0, o[n][1] * i0);
         if (r1 < kWTok) *reinterpret_cast<uint32_t*>(ctx + (row0 + r1) * ldc + col) = ptx::pack_bf16x2(o[n][2] * i1, o[n][3] * i1);
+      }
+    }
+  }
+}
+
+// The same for 144-token windows.  All K fragments (18 n-tiles x 4) and V fragments (9 k-steps x 8) would take 144
+// registers beside the 72 of the score tile, so both are re-read from shared memory with ldmatrix for every query m-tile
+// (18 + 18 ldmatrix.x4 against 72 mma per m-tile); the score tile of one m-tile holds every key, so the softmax needs no
+// rescale.
+// qkv  bf16 [n_windows * 144, ldq], columns q | k | v (each heads * 32), head h at h * 32 inside each
+// tab  f32 [n_tab, heads, 144, 144] = (relative position bias + shift mask) * log2(e)
+// ctx  bf16 [n_windows * 144, ldc]
+__global__ void __launch_bounds__(kW12Warps * 32) window_attention144_kernel(const __nv_bfloat16* __restrict__ qkv, long long ldq,
+                                                                            __nv_bfloat16* __restrict__ ctx, long long ldc,
+                                                                            const float* __restrict__ tab, int n_tab, int heads,
+                                                                            long long n_items, float scale_log2e) {
+  constexpr int NT = kW12Tok / 8, KS = kW12Tok / 16;
+  extern __shared__ __align__(128) uint8_t wsm[];
+  ptx::grid_dep_launch();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t aQ = ptx::smem_u32(wsm + warp * 3 * kW12MatBytes), aK = aQ + kW12MatBytes, aV = aK + kW12MatBytes;
+  ptx::grid_dep_wait();
+  const int C = heads * kWHd;
+  const int g = lane >> 2, t = lane & 3;
+  for (long long item = static_cast<long long>(blockIdx.x) * kW12Warps + warp; item < n_items;
+       item += static_cast<long long>(gridDim.x) * kW12Warps) {
+    const long long w = item / heads;
+    const int h = static_cast<int>(item - w * heads);
+    const long long row0 = w * kW12Tok;
+    __syncwarp();  // every lane is done with the previous item's shared memory
+    stage_window<kW12Tok, kW12MatBytes>(qkv, ldq, row0, C, h, aQ, lane);
+    __syncwarp();
+    const float* tb = tab + ((w % n_tab) * heads + h) * static_cast<long long>(kW12Tok * kW12Tok);
+#pragma unroll 1
+    for (int mt = 0; mt < KS; ++mt) {
+      uint32_t qa[2][4];
+#pragma unroll
+      for (int ks = 0; ks < 2; ++ks) ptx::ldmatrix_x4(aQ + wofs(mt * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, ks * 2 + (lane >> 4)), qa[ks]);
+      float s[NT][4];
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) {
+        uint32_t kb[4];  // keys 8 nt .. 8 nt + 7: {ks0.b0, ks0.b1, ks1.b0, ks1.b1}
+        ptx::ldmatrix_x4(aK + wofs(nt * 8 + (lane & 7), lane >> 3), kb);
+        s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
+        ptx::mma_bf16_16816(s[nt], qa[0], kb[0], kb[1]);
+        ptx::mma_bf16_16816(s[nt], qa[1], kb[2], kb[3]);
+      }
+      const float* t0 = tb + (mt * 16 + g) * kW12Tok + 2 * t;
+      float m0, m1, l0, l1;
+      scores_rowmax<NT>(s, t0, t0 + 8 * kW12Tok, scale_log2e, m0, m1);
+      uint32_t pa[KS][4];
+      exp_rowsum<NT>(s, m0, m1, pa, l0, l1);
+      float o[4][4];
+#pragma unroll
+      for (int n = 0; n < 4; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
+#pragma unroll
+      for (int kk = 0; kk < KS; ++kk) {
+        uint32_t vb[2][4];  // keys 16 kk .. +15, dims chunk pair cp: {n 2cp: b0, b1, n 2cp+1: b0, b1}
+#pragma unroll
+        for (int cp = 0; cp < 2; ++cp)
+          ptx::ldmatrix_x4_trans(aV + wofs(kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, cp * 2 + (lane >> 4)), vb[cp]);
+#pragma unroll
+        for (int n = 0; n < 4; ++n) ptx::mma_bf16_16816(o[n], pa[kk], vb[n >> 1][(n & 1) * 2], vb[n >> 1][(n & 1) * 2 + 1]);
+      }
+      const float i0 = 1.0f / l0, i1 = 1.0f / l1;  // l >= 1: the row maximum contributes 2^0
+      const long long r0 = row0 + mt * 16 + g, r1 = r0 + 8;
+#pragma unroll
+      for (int n = 0; n < 4; ++n) {
+        const int col = h * kWHd + n * 8 + 2 * t;
+        *reinterpret_cast<uint32_t*>(ctx + r0 * ldc + col) = ptx::pack_bf16x2(o[n][0] * i0, o[n][1] * i0);
+        *reinterpret_cast<uint32_t*>(ctx + r1 * ldc + col) = ptx::pack_bf16x2(o[n][2] * i1, o[n][3] * i1);
       }
     }
   }
@@ -416,12 +519,26 @@ int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc
                             int window_tokens, int heads, int head_size, float scale, cudaStream_t st) {
   EVT_CHECK_ARG(qkv && ctx && table, "window_attention: null pointer");
   EVT_CHECK_ARG(n_windows > 0 && heads > 0 && n_tab > 0, "window_attention: sizes must be positive");
-  if (window_tokens != kWTok || head_size != kWHd)
-    return fail(EVT_ERR_UNSUPPORTED, "window_attention: only 7x7 windows (49 tokens) with head size 32 are implemented");
+  if ((window_tokens != kWTok && window_tokens != kW12Tok) || head_size != kWHd)
+    return fail(EVT_ERR_UNSUPPORTED,
+                "window_attention: only 7x7 (49-token) and 12x12 (144-token) windows with head size 32 are implemented");
   EVT_CHECK_ARG(ldq >= 3ll * heads * kWHd && ldc >= static_cast<int64_t>(heads) * kWHd, "window_attention: leading dimension too small");
   EVT_CHECK_ARG(ldq % 8 == 0 && reinterpret_cast<uintptr_t>(qkv) % 16 == 0, "window_attention: qkv rows must be 16-byte aligned");
   EVT_CHECK_ARG(ldc % 2 == 0 && reinterpret_cast<uintptr_t>(ctx) % 4 == 0, "window_attention: ctx rows must be 4-byte aligned");
   const long long items = n_windows * heads;
+  if (window_tokens == kW12Tok) {
+    const int smem = kW12Warps * 3 * kW12MatBytes;
+    EVT_TRY(opt_in_smem<window_attention144_kernel>(smem));
+    const long long ctas_needed = (items + kW12Warps - 1) / kW12Warps;
+    const long long cap = static_cast<long long>(num_sms()) * 2;  // 2 CTAs of 108 KB per SM, grid-stride over the rest
+    const unsigned grid = static_cast<unsigned>(ctas_needed < cap ? ctas_needed : cap);
+    EVT_CUDA(launch_pdl(window_attention144_kernel, dim3(grid), dim3(kW12Warps * 32), smem, st,
+                        pdl_for_work(n_windows * kW12Tok, static_cast<long long>(heads) * kWHd), reinterpret_cast<const __nv_bfloat16*>(qkv),
+                        static_cast<long long>(ldq), reinterpret_cast<__nv_bfloat16*>(ctx), static_cast<long long>(ldc), table, n_tab, heads,
+                        items, scale * 1.4426950408889634f));
+    EVT_LAUNCH_CHECK("window_attention144_kernel");
+    return EVT_OK;
+  }
   const int smem = kWWarps * 3 * kWMatBytes;
   EVT_TRY(opt_in_smem<window_attention_kernel>(smem));
   const long long ctas_needed = (items + kWWarps - 1) / kWWarps;

@@ -58,22 +58,24 @@ std::vector<float> shift_mask(int H, int ws, int shift) {
     }
   return m;
 }
-// (relative position bias [+ shift mask]) * log2(e) in the window-attention kernel's [n_tab, heads, 64, 56] layout;
+// (relative position bias [+ shift mask]) * log2(e) in the window-attention kernel's layout: [n_tab, heads, 64, 56] for
+// 7 x 7 windows (key columns 49..55 -inf, rows 49..63 finite), [n_tab, heads, 144, 144] for 12 x 12;
 // bias_table [(2ws-1)^2, heads] (SwinSelfAttention :420-438)
 std::vector<float> attention_table(const std::vector<float>& bias_table, int heads, int ws, const std::vector<float>* mask, int n_tab) {
   const int N = ws * ws;
-  std::vector<float> out(static_cast<size_t>(n_tab) * heads * 64 * 56, 0.f);
+  const int rows = N == 49 ? 64 : N, cols = N == 49 ? 56 : N;
+  std::vector<float> out(static_cast<size_t>(n_tab) * heads * rows * cols, 0.f);
   for (int t = 0; t < n_tab; ++t)
     for (int h = 0; h < heads; ++h) {
-      float* o = out.data() + (static_cast<size_t>(t) * heads + h) * 64 * 56;
-      for (int r = 0; r < 64; ++r)
-        for (int c = N; c < 56; ++c) o[r * 56 + c] = -INFINITY;
+      float* o = out.data() + (static_cast<size_t>(t) * heads + h) * rows * cols;
+      for (int r = 0; r < rows; ++r)
+        for (int c = N; c < cols; ++c) o[r * cols + c] = -INFINITY;
       for (int a = 0; a < N; ++a)
         for (int b = 0; b < N; ++b) {
           const int dy = a / ws - b / ws + ws - 1, dx = a % ws - b % ws + ws - 1;
           float v = bias_table[static_cast<size_t>(dy * (2 * ws - 1) + dx) * heads + h];
           if (mask) v += (*mask)[(static_cast<size_t>(t) * N + a) * N + b];
-          o[a * 56 + b] = v * kLog2e;
+          o[a * cols + b] = v * kLog2e;
         }
     }
   return out;
@@ -147,8 +149,8 @@ extern "C" int evt_swin_create(const evt_swin_spec* s, evt_swin** out) {
   if (rc != EVT_OK) return rc;
   EVT_CHECK_ARG(s != nullptr && out != nullptr, "evt_swin_create: null argument");
   EVT_CHECK_ARG(s->stages >= 1 && s->stages <= EVT_SWIN_MAX_STAGES, "stage count out of range");
-  if (s->window != 7) return fail(EVT_ERR_UNSUPPORTED, "only 7 x 7 windows are implemented");
-  EVT_CHECK_ARG(s->patch == 4, "only patch size 4 is implemented (swin_*_patch4_window7)");
+  if (s->window != 7 && s->window != 12) return fail(EVT_ERR_UNSUPPORTED, "only 7 x 7 and 12 x 12 windows are implemented");
+  EVT_CHECK_ARG(s->patch == 4, "only patch size 4 is implemented (swin_*_patch4_window{7,12})");
   EVT_CHECK_ARG(s->image > 0 && s->image % s->patch == 0, "image size must be a multiple of the patch size");
   const int grid = s->image / s->patch;
   EVT_CHECK_ARG(grid % (s->window << (s->stages - 1)) == 0, "image / patch must be a multiple of window * 2^(stages-1)");
@@ -307,6 +309,7 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
   StaticWeightsScope weights_are_static;
   const float eps = s.eps;
   const float scale = 1.0f / sqrtf(32.f);
+  const int ws2 = s.window * s.window;
   int T = m->grid * m->grid;
   // SwinEmbeddings (:262-301): 4 x 4 patch conv as im2col + GEMM, LayerNorm, rows gathered into the first window order
   EVT_TRY(im2col4_launch(pixels, w.cols, batch, s.image, s.image, s.patch, st));
@@ -328,7 +331,7 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
       }
       EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.wqkv, .ldw = C, .bias = blk.bqkv, .out = w.qkv, .out_dtype = EVT_BF16, .ldo = 3 * C,
                            .M = M, .N = 3 * C, .K = C}, st));
-      EVT_TRY(window_attention_launch(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / 49, 49, stg.heads, 32, scale, st));
+      EVT_TRY(window_attention_launch(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / ws2, ws2, stg.heads, 32, scale, st));
       EVT_TRY(gemm_launch({.A = w.ctx, .lda = C, .W = blk.wo, .ldw = C, .bias = blk.bo, .residual = resid, .ldr = C, .out = resid,
                            .out_dtype = EVT_F32, .ldo = C, .M = M, .N = C, .K = C}, st));
       EVT_TRY(layernorm_launch(resid, C, blk.ln2_g, blk.ln2_b, w.xn, EVT_BF16, C, nullptr, M, C, eps, st));

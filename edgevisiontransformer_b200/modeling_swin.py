@@ -4,6 +4,7 @@ The reference builds ``swin_{tiny,small,base}_patch4_window7_224`` from an exter
 (utils.py:14-47 ``get_swin``) and exports / benchmarks it (tools.py:265-292 ``export_onnx_swin``); the same network with HF
 key names is ``transformers.SwinForImageClassification`` (SITE/models/swin/modeling_swin.py), which is what
 :meth:`B200SwinForImageClassification.from_hf` takes.  ``from_microsoft`` renames a state dict of the original repository.
+The 384-pixel checkpoints ``swin_{base,large}_patch4_window12_384`` (12 x 12 windows of 144 tokens) run as well.
 
 Data layout: inside a stage the f32 residual stream ``[B*T, C]`` is kept in the WINDOW ORDER of the current block (image,
 window, token in window).  A block whose cyclic shift differs from the previous one starts with a row gather fused into its
@@ -66,11 +67,13 @@ def shift_mask(H: int, W: int, ws: int, shift: int) -> torch.Tensor:
 
 
 def attention_table(bias_table: torch.Tensor, heads: int, ws: int, mask: torch.Tensor = None) -> torch.Tensor:
-    """(relative position bias [+ shift mask]) * log2(e), padded to the kernel's [n_tab, heads, 64, 56] layout."""
+    """(relative position bias [+ shift mask]) * log2(e) in the kernel's layout: padded to [n_tab, heads, 64, 56] for 7 x 7
+    windows, [n_tab, heads, 144, 144] for 12 x 12."""
     N = ws * ws
     bias = bias_table[relative_position_index(ws).view(-1)].view(N, N, heads).permute(2, 0, 1).float()      # [heads, N, N]
     full = bias.unsqueeze(0) if mask is None else bias.unsqueeze(0) + mask.unsqueeze(1)
-    out = torch.zeros(full.shape[0], heads, 64, 56)
+    rows, cols = ops.window_table_shape(N)
+    out = torch.zeros(full.shape[0], heads, rows, cols)
     out[:, :, :, N:] = -float("inf")
     out[:, :, :N, :N] = full * LOG2E
     return out.contiguous()
@@ -87,7 +90,8 @@ class B200SwinConfig:
 
 
 class B200SwinForImageClassification(nn.Module):
-    """Inference-only.  ``state_dict`` uses HF key names (``swin.embeddings...``, ``swin.encoder.layers.{s}.blocks.{b}...``)."""
+    """Inference-only.  ``state_dict`` uses HF key names (``swin.embeddings...``, ``swin.encoder.layers.{s}.blocks.{b}...``).
+    ``window`` 7 (224 pixels) or 12 (384 pixels)."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], depths: Sequence[int], num_heads: Sequence[int], embed_dim: int,
                  window: int = 7, patch: int = 4, image_size: int = 224, eps: float = 1e-5, device="cuda", max_batch: int = 1024):
@@ -95,8 +99,9 @@ class B200SwinForImageClassification(nn.Module):
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("B200SwinForImageClassification runs only on a CUDA (sm_100a) device; no CPU fallback")
-        if window != 7 or any(embed_dim * 2 ** s != 32 * h for s, h in enumerate(num_heads)):
-            raise ValueError("only 7x7 windows with head size 32 are implemented (swin_{tiny,small,base,large}_patch4_window7)")
+        if window not in (7, 12) or any(embed_dim * 2 ** s != 32 * h for s, h in enumerate(num_heads)):
+            raise ValueError("only 7x7 and 12x12 windows with head size 32 are implemented "
+                             "(swin_{tiny,small,base,large}_patch4_window7_224, swin_{base,large}_patch4_window12_384)")
         grid = image_size // patch
         if image_size % patch or grid % (window * 2 ** (len(depths) - 1)):
             raise ValueError("image_size / patch must be a multiple of window * 2^(stages-1)")
@@ -196,8 +201,18 @@ class B200SwinForImageClassification(nn.Module):
     @classmethod
     def from_microsoft(cls, state_dict: Dict[str, torch.Tensor], depths, num_heads, embed_dim, **kw):
         """State dict of microsoft/Swin-Transformer's ``SwinTransformer`` (what ``get_swin`` + ``load_state_dict(sd['model'])``
-        holds, tools.py:284-288): fused ``attn.qkv``, ``patch_embed`` / ``layers.{s}.blocks.{b}`` / ``norm`` / ``head`` names."""
-        return cls(microsoft_to_hf(state_dict), depths=depths, num_heads=num_heads, embed_dim=embed_dim, **kw)
+        holds, tools.py:284-288): fused ``attn.qkv``, ``patch_embed`` / ``layers.{s}.blocks.{b}`` / ``norm`` / ``head`` names.
+        Unless given, the window is read off the (2w-1)^2 rows of the first relative position bias table and the image size
+        is that of the published checkpoints with that window (7: 224, 12: 384)."""
+        sd = microsoft_to_hf(state_dict)
+        if "window" not in kw:
+            n = sd["swin.encoder.layers.0.blocks.0.attention.self.relative_position_bias_table"].shape[0]
+            side = math.isqrt(n)
+            if side * side != n or side % 2 == 0:
+                raise ValueError(f"relative_position_bias_table has {n} rows, not (2 * window - 1)^2")
+            kw["window"] = (side + 1) // 2
+        kw.setdefault("image_size", {7: 224, 12: 384}.get(kw["window"], 224))
+        return cls(sd, depths=depths, num_heads=num_heads, embed_dim=embed_dim, **kw)
 
     def num_parameters(self) -> int:
         n = sum(t.numel() for t in (self.w_patch, self.b_patch, self.g_embed, self.be_embed, self.g_final, self.b_final,

@@ -218,15 +218,22 @@ def gather_layernorm(x: torch.Tensor, idx: torch.Tensor, gamma: Optional[torch.T
     return y, cp
 
 
+def window_table_shape(window_tokens: int):
+    """(rows, key columns) of one head's bias + mask table in evt_window_attention_fwd: 7 x 7 windows pad 49 to 64 x 56
+    (columns 49..55 -inf), 12 x 12 windows use 144 x 144 as is."""
+    return (64, 56) if window_tokens == 49 else (window_tokens, window_tokens)
+
+
 def window_attention(qkv: torch.Tensor, table: torch.Tensor, n_windows: int, heads: int, window_tokens: int = 49,
                      head_size: int = 32, scale: Optional[float] = None) -> torch.Tensor:
-    """qkv bf16 [n_windows*49, 3*heads*32] in window order, table f32 [n_tab, heads, 64, 56] (log2 domain, include/evt.h)
-    -> ctx bf16 [n_windows*49, heads*32]."""
+    """qkv bf16 [n_windows*N, 3*heads*32] in window order (N = window_tokens, 49 or 144), table f32
+    [n_tab, heads, *window_table_shape(N)] (log2 domain, include/evt.h) -> ctx bf16 [n_windows*N, heads*32]."""
     _need_cuda(qkv, table)
     if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.stride(1) != 1 or qkv.shape[0] != n_windows * window_tokens:
         raise ValueError("window_attention wants a bf16 [n_windows*tokens, 3*heads*head_size] matrix")
-    if table.dtype != torch.float32 or table.dim() != 4 or tuple(table.shape[1:]) != (heads, 64, 56) or not table.is_contiguous():
-        raise ValueError("window_attention: table must be a contiguous f32 [n_tab, heads, 64, 56] tensor")
+    want = (heads, *window_table_shape(window_tokens))
+    if table.dtype != torch.float32 or table.dim() != 4 or tuple(table.shape[1:]) != want or not table.is_contiguous():
+        raise ValueError(f"window_attention: table must be a contiguous f32 [n_tab, {want[0]}, {want[1]}, {want[2]}] tensor")
     ctx = torch.empty((qkv.shape[0], heads * head_size), dtype=torch.bfloat16, device=qkv.device)
     scale = float(head_size ** -0.5 if scale is None else scale)
     lib = _lib.load()

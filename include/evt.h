@@ -252,12 +252,15 @@ int evt_performer_block_fwd(const void* kqv, int64_t ld, const float* w, float* 
 int evt_gather_layernorm(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype,
                          float* copy_f32, int64_t images, int T_in, int T_out, int G, int C, float eps, evt_stream stream);
 
-/* Window attention (SwinSelfAttention.forward :410-459) for 7x7 windows, head size 32:
+/* Window attention (SwinSelfAttention.forward :410-459) for 7x7 (window_tokens = 49) or 12x12 (window_tokens = 144)
+ * windows, head size 32; anything else is EVT_ERR_UNSUPPORTED:
  *   ctx = softmax(q k^T * scale + relative_position_bias + shift_mask) v   per (window, head)
- *   qkv   : bf16 [n_windows * 49, ldq], columns q | k | v (heads*32 each), rows in window order
- *   table : f32 [n_tab, heads, 64, 56] = (bias[h] + mask[w % n_tab]) * log2(e), key columns 49..55 = -inf, rows 49..63
- *           finite; n_tab = windows per image for shifted blocks, 1 otherwise
- *   ctx   : bf16 [n_windows * 49, ldc]. */
+ *   qkv   : bf16 [n_windows * N, ldq] (N = window_tokens), columns q | k | v (heads*32 each), rows in window order
+ *   table : (bias[h] + mask[w % n_tab]) * log2(e), the shift mask being HF's 0 / -100; n_tab = windows per image for
+ *           shifted blocks, 1 otherwise
+ *           N = 49 : f32 [n_tab, heads, 64, 56], key columns 49..55 = -inf, rows 49..63 finite
+ *           N = 144: f32 [n_tab, heads, 144, 144]
+ *   ctx   : bf16 [n_windows * N, ldc]. */
 int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab,
                              int64_t n_windows, int window_tokens, int heads, int head_size, float scale, evt_stream stream);
 
@@ -379,7 +382,8 @@ int evt_model_destroy(evt_model* m);
 /* ------------------------------------------------------------------ Swin model level ----- */
 
 /* The shifted-window classifier the reference builds with utils.get_swin (utils.py:14-47) and exports / benchmarks in
- * tools.py:265-292 (swin_{tiny,small,base}_patch4_window7_224), arithmetic as in SITE/models/swin/modeling_swin.py.
+ * tools.py:265-292 (swin_{tiny,small,base}_patch4_window7_224), arithmetic as in SITE/models/swin/modeling_swin.py;
+ * also the 384-pixel swin_{base,large}_patch4_window12_384 (12 x 12 windows).
  * One call = the whole forward as a fixed launch sequence on `stream` (CUDA-graph capturable).  bf16 operands, f32
  * accumulate / residual stream / LayerNorm / softmax. */
 typedef struct evt_swin evt_swin;
@@ -387,8 +391,8 @@ typedef struct evt_swin evt_swin;
 #define EVT_SWIN_MAX_STAGES 8
 
 typedef struct evt_swin_spec {
-  int image, patch, window;          /* 224, 4, 7 */
-  int embed_dim;                     /* 96 (tiny / small), 128 (base); head size is 32 in every stage */
+  int image, patch, window;          /* 224, 4, 7 (swin_*_window7_224) or 384, 4, 12 (swin_*_window12_384); window 7 or 12 */
+  int embed_dim;                     /* 96 (tiny / small), 128 (base), 192 (large); head size is 32 in every stage */
   int stages;                        /* 4 */
   int depths[EVT_SWIN_MAX_STAGES];   /* blocks per stage, e.g. 2, 2, 6, 2 */
   int heads[EVT_SWIN_MAX_STAGES];    /* heads per stage, e.g. 3, 6, 12, 24 */
