@@ -9,6 +9,7 @@ each bracketed by a stream synchronise and ``timeit.default_timer``; optional ``
     python -m edgevisiontransformer_b200.benchmark --model deit_base --image-size 384 --batch 256
     python -m edgevisiontransformer_b200.benchmark --model swin_large --image-size 384 --batch 256
     python -m edgevisiontransformer_b200.benchmark --model /path/to/pruned_checkpoint --batch 1024
+    python -m edgevisiontransformer_b200.benchmark --model 81.5_T2T_ViT_14.pth.tar --batch 1024    (PyTorch T2T-ViT, tools.py:347-365)
     python -m edgevisiontransformer_b200.benchmark --model attention --h 768 --a 12 --n 197      (op-level, tools.py:735-758)
 """
 from __future__ import annotations
@@ -114,6 +115,10 @@ def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device
         m = B200ViTForImageClassification.from_pretrained(name, device=device, max_batch=max_batch, precision=precision,
                                                           keep_params=False)
         return m, (3, m.config.image_size, m.config.image_size), f"checkpoint {name} heads={m.config.heads} ffn={m.config.intermediate}"
+    if os.path.isfile(name):                 # a PyTorch T2T-ViT checkpoint file (.pth / .pth.tar)
+        from ..modeling_t2t import B200T2TViTTorch
+        m = B200T2TViTTorch.from_checkpoint(name, device=device, max_batch=min(max_batch, 1024), precision=precision, keep_params=False)
+        return m, (3, 224, 224), f"T2T-ViT checkpoint {name} (embed_dim {m.hidden}, depth {m.depth}, {precision}), NCHW input"
     raise ValueError(f"unknown model {name!r}")
 
 
@@ -143,7 +148,7 @@ def b200_benchmark(model, input_shape: Sequence[int], num_runs: int = 50, warmup
 
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="b200_benchmark", description=__doc__.split("\n")[0])
-    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir")
+    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir | T2T-ViT .pth[.tar]")
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--precision", default="bf16", choices=["bf16", "tf32"])
     ap.add_argument("--num_runs", type=int, default=50)

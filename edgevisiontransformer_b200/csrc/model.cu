@@ -181,6 +181,7 @@ int validate_spec(const evt_model_spec* s) {
                   "head_rows = 2 (two-head distilled DeiT) needs 198 tokens, the final LayerNorm and a single Linear head");
   EVT_CHECK_ARG(s->precision == EVT_PREC_BF16 || s->precision == EVT_PREC_TF32, "precision must be bf16 (0) or tf32 (1)");
   EVT_CHECK_ARG(s->embed_k >= 0 && s->embed_k % 8 == 0, "embed_k must be a non-negative multiple of 8");
+  EVT_CHECK_ARG(s->t2t >= 0 && s->t2t <= 2, "t2t must be 0 (patch embedding), 1 (T2T front-end, NHWC f32 pixels) or 2 (T2T front-end, NCHW pixels)");
   if (s->t2t) {
     EVT_CHECK_ARG(s->embed_k == 576 && s->precision == EVT_PREC_BF16, "the T2T front-end needs embed_k = 576 (3 x 3 x 64) and the bf16 mode");
     EVT_CHECK_ARG(t2t_side(s->image, 2) * t2t_side(s->image, 2) == patches, "image size does not give image/16 squared T2T tokens");
@@ -454,24 +455,32 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   const bool tf32 = s.precision == EVT_PREC_TF32;
   const int dt = tf32 ? EVT_F32 : EVT_BF16;   // GEMM operand type
   const int adt = tf32 ? EVT_TF32 : EVT_BF16;  // type activations are WRITTEN in (tf32: f32 storage, rounded to nearest)
-  // tokens-to-token front-end (T2T_module.call, modeling/models/t2t_vit.py:63-88): pixels are NHWC f32 here
+  // tokens-to-token front-end (T2T_module.call, modeling/models/t2t_vit.py:63-88).  spec.t2t = 1: NHWC f32 pixels (the TF T2T);
+  // 2: NCHW pixels of any evt_pixel_dtype (the PyTorch T2T: nn.Unfold over the image, whose stage-1 columns the first kernel writes
+  // in the same (kh, kw, c) order -- the loader permuted the weights).  Stages 2 and 3 read the token-major [B, T, 64] performer
+  // output either way.  The performer MLP's GELU is spec.act (tanh for the TF T2T, erf for the PyTorch one).
   if (s.t2t && patch_matrix == nullptr) {
-    const float tf_eps = 1e-5f;   // tf.keras.layers.LayerNormalization(epsilon=1e-5), transformer_encoder.py:49-50
+    const float tf_eps = 1e-5f;   // tf.keras.layers.LayerNormalization(epsilon=1e-5), transformer_encoder.py:49-50; nn.LayerNorm's default
     const void* src = pixels;
     int src_dt = EVT_F32, side = s.image, ch = 3;
-    EVT_CHECK_ARG(o.pixel_dtype == EVT_PIX_F32, "the T2T front-end takes f32 NHWC pixels");
+    const bool nchw = s.t2t == 2;
+    EVT_CHECK_ARG(nchw || o.pixel_dtype == EVT_PIX_F32, "the T2T front-end with spec.t2t = 1 takes f32 NHWC pixels");
     for (int i = 0; i < 2; ++i) {
       const PerformerW& pw = m->perf[i];
       const int k = i == 0 ? 7 : 3, st_ = i == 0 ? 4 : 2, pad_ = i == 0 ? 2 : 1;
       const int so = t2t_side(s.image, i), T = so * so;
       const int64_t rows = static_cast<int64_t>(batch) * T;
-      EVT_STAGE(EVT_STAGE_EMBED, unfold_ln_launch(src, src_dt, w.t_x[i], pw.in_ld, pw.g1, pw.b1, tf_eps, batch, side, side, ch, k, st_, pad_, st));
+      if (i == 0 && nchw)
+        EVT_STAGE(EVT_STAGE_EMBED, unfold773_nchw_launch(pixels, o.pixel_dtype, o.pixel_scale, o.pixel_bias, w.t_x[0], pw.g1, pw.b1, tf_eps,
+                                                         batch, s.image, s.image, st));
+      else
+        EVT_STAGE(EVT_STAGE_EMBED, unfold_ln_launch(src, src_dt, w.t_x[i], pw.in_ld, pw.g1, pw.b1, tf_eps, batch, side, side, ch, k, st_, pad_, st));
       EVT_STAGE(EVT_STAGE_EMBED, gemm_launch({.A = w.t_x[i], .lda = pw.in_ld, .W = pw.wkqv, .ldw = pw.in_ld, .bias = pw.bkqv, .out = w.t_kqv[i],
                                               .out_dtype = EVT_BF16, .ldo = 192, .M = rows, .N = 192, .K = pw.in_dim}, st));
       // single_attn + attn_output + LayerNorm + MLP (transformer_encoder.py:67-99): the attention contraction's apply kernel carries
       // each tile through the tail, y = the performer's output rows
       EVT_TRY(performer_block_launch(w.t_kqv[i], 192, pw.w, w.t_y[i], w.t_ws[i], batch, T, 1e-8f, pw.wo, pw.bo, pw.g2, pw.b2, pw.w1,
-                                     pw.bb1, pw.w2, pw.bb2, tf_eps, st));
+                                     pw.bb1, pw.w2, pw.bb2, tf_eps, st, s.act));
       EVT_TRY(mark(EVT_STAGE_EMBED));
       src = w.t_y[i], src_dt = EVT_F32, side = so, ch = 64;
     }

@@ -82,7 +82,11 @@ int performer_mlp_launch(const void* ya, float* y, const void* wo, const float* 
 // the whole Token_performer after the kqv projection in three launches: y f32 [B*T, 64] = the performer's output rows
 int performer_block_launch(const void* kqv, int64_t ld, const float* w, float* y, void* workspace, int B, int T, float eps, const void* wo,
                            const float* bo, const float* gamma, const float* beta, const void* w1, const float* b1, const void* w2,
-                           const float* b2, float ln_eps, cudaStream_t st);
+                           const float* b2, float ln_eps, cudaStream_t st, int act = EVT_ACT_GELU_TANH);  // act: the MLP's GELU (evt_act)
+// the first soft split of the PyTorch T2T-ViT (nn.Unfold(7, stride 4, padding 2) over NCHW pixels [B,3,H,W] of an evt_pixel_dtype;
+// u8 takes scale3 / bias3) + the performer's norm1 -> bf16 [B*oh*ow, 152], columns in (kh, kw, c) order, 147.. zero
+int unfold773_nchw_launch(const void* pixels, int pixel_dtype, const float* scale3, const float* bias3, void* out, const float* gamma,
+                          const float* beta, float eps, int B, int H, int W, cudaStream_t st);
 int unfold_launch(const void* x, int x_dtype, void* out, int64_t ldo, int B, int H, int W, int C, int k, int s, int p,
                   cudaStream_t st);
 

@@ -115,25 +115,47 @@ __global__ void __launch_bounds__(256) unfold_ln_kernel(const TIN* __restrict__ 
 // per-row bookkeeping is shared by four rows, and 19 independent loads per lane are in flight.  Offsets and affine parameters
 // of the lane's elements are row-invariant registers; a group of four windows that are all interior (83 % of a 56 x 56 grid)
 // takes a path without any bounds test.
-template <typename TIN, bool LN, int ITER>
-__global__ void __launch_bounds__(256) unfold773_kernel(const TIN* __restrict__ x, __nv_bfloat16* __restrict__ out, long long ldo,
+// NCHW: the same windows read from planar pixels (nn.Unfold over [B,3,H,W], the PyTorch T2T-ViT's first soft split).  Only the
+// row-invariant offsets change, to c H W + ky W + kx; the output columns keep the (kh, kw, c) order, so one device layout of the
+// performer weights serves both.  AFFINE (u8 pixels): value = pixel * scale[c] + bias[c]; a padded element stays 0, i.e. the zero
+// padding is applied to the normalised image, as nn.Unfold pads the normalised tensor.  The u8 instantiation asks for two
+// blocks per SM (128 registers, no spills): left alone ptxas gives it 143, one 8-warp block per SM, too few loads in flight
+// for this latency-bound gather.  0 = no occupancy hint, which leaves every other instantiation's code as it was.
+struct PixAffine {
+  float scale[3], bias[3];
+};
+template <typename TIN, bool LN, int ITER, bool NCHW = false, bool AFFINE = false>
+__global__ void __launch_bounds__(256, AFFINE ? 2 : 0) unfold773_kernel(const TIN* __restrict__ x, __nv_bfloat16* __restrict__ out, long long ldo,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                                                        int H, int W, int s, int p, int oh, int ow, long long rows) {
+                                                        int H, int W, int s, int p, int oh, int ow, long long rows, const PixAffine af) {
   constexpr int KK = 7, CC = 3, L = KK * KK * CC, kRun = KK * CC, NE = 19;  // 147, 21; 8 lanes x 19 elements = 152
   const int lane = threadIdx.x & 31;
   const int j = lane & 7, slot = lane >> 3;
   const long long warp_id = static_cast<long long>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   int off[NE];
   float g[NE], be[NE];
+  // element j + 8 i has channel (j + 8 i) % 3 = (j + 2 i) % 3: three per-lane affine pairs, picked by i % 3 at compile time
+  float sc[3], bi[3];
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+    const int c = (j + 2 * r) % 3;
+    sc[r] = c == 0 ? af.scale[0] : c == 1 ? af.scale[1] : af.scale[2];
+    bi[r] = c == 0 ? af.bias[0] : c == 1 ? af.bias[1] : af.bias[2];
+  }
 #pragma unroll
   for (int i = 0; i < NE; ++i) {
     const int e = j + 8 * i;
     const bool in = e < L;
     const int ky = in ? e / kRun : 0;
-    off[i] = in ? ky * W * CC + (e - ky * kRun) : -1;
+    const int kx = in ? (e - ky * kRun) / CC : 0, c = in ? e - ky * kRun - kx * CC : 0;
+    off[i] = !in ? -1 : NCHW ? c * H * W + ky * W + kx : ky * W * CC + (e - ky * kRun);
     g[i] = (LN && in) ? gamma[e] : 0.f;
     be[i] = (LN && in) ? beta[e] : 0.f;
   }
+  auto val = [&](TIN raw, int i) -> float {
+    if constexpr (AFFINE) return fmaf(static_cast<float>(raw), sc[i % 3], bi[i % 3]);
+    else return static_cast<float>(raw);
+  };
 #pragma unroll 1
   for (int it = 0; it < ITER; ++it) {
     const long long row = (warp_id * ITER + it) * 4 + slot;
@@ -144,13 +166,14 @@ __global__ void __launch_bounds__(256) unfold773_kernel(const TIN* __restrict__ 
     const int oy = static_cast<int>(t % oh);
     const long long b = t / oh;
     const int iy0 = oy * s - p, ix0 = ox * s - p;
-    const TIN* base = x + ((b * H + iy0) * static_cast<long long>(W) + ix0) * CC;
+    const TIN* base = NCHW ? x + (b * CC * H + iy0) * static_cast<long long>(W) + ix0
+                           : x + ((b * H + iy0) * static_cast<long long>(W) + ix0) * CC;
     const bool interior = iy0 >= 0 && iy0 + KK <= H && ix0 >= 0 && ix0 + KK <= W;
     float v[NE];
     if (__all_sync(0xffffffffu, interior)) {
 #pragma unroll
-      for (int i = 0; i < NE - 1; ++i) v[i] = static_cast<float>(base[off[i]]);
-      v[NE - 1] = off[NE - 1] >= 0 ? static_cast<float>(base[off[NE - 1]]) : 0.f;
+      for (int i = 0; i < NE - 1; ++i) v[i] = val(base[off[i]], i);
+      v[NE - 1] = off[NE - 1] >= 0 ? val(base[off[NE - 1]], NE - 1) : 0.f;
     } else {
 #pragma unroll
       for (int i = 0; i < NE; ++i) {
@@ -158,7 +181,7 @@ __global__ void __launch_bounds__(256) unfold773_kernel(const TIN* __restrict__ 
         const int ky = e / kRun, kx = (e - ky * kRun) / CC;
         const int iy = iy0 + ky, ix = ix0 + kx;
         const bool ok = off[i] >= 0 && iy >= 0 && iy < H && ix >= 0 && ix < W;
-        v[i] = ok ? static_cast<float>(base[off[i]]) : 0.f;
+        v[i] = ok ? val(base[off[i]], i) : 0.f;
       }
     }
     float mean = 0.f, rstd = 1.f;
@@ -361,7 +384,8 @@ __global__ void __launch_bounds__(256) performer_reduce_final_kernel(const float
 // Everything the Token_performer does after the attention contraction (modeling/layers/transformer_encoder.py:93-99), for 64-wide
 // tokens, in ONE pass over the rows:
 //     y  = v + attn_output(ya)            (Dense 64 -> 64; v = the f32 copy of the value rows the apply kernel wrote)
-//     y += mlp(LayerNorm(y))              (Dense 64 -> 64, tanh-GELU, Dense 64 -> 64)
+//     y += mlp(LayerNorm(y))              (Dense 64 -> 64, GELU, Dense 64 -> 64)
+// ACT is the GELU of the MLP: tanh for the TensorFlow T2T (its Dense layers), erf for the PyTorch one (nn.GELU).
 // Before: GEMM (f32 reduce-add), LayerNorm kernel, GEMM + GELU, GEMM (reduce-add) -- four launches moving 1920 bytes per token;
 // here 640 (ya in, y in, y out).  Per 16-token tile a warp chains three m16n8k16 products whose accumulator fragments are the
 // next product's A fragments (two adjacent n-tiles = one k-step), the LayerNorm statistics are quad reductions over the
@@ -396,6 +420,7 @@ __device__ __forceinline__ void tail_load(TailSmem& sm, const TailWeights& w) {
 
 // One 16-token tile.  a: A fragments of ya (bf16, 4 k-steps); y1: on entry v in accumulator-fragment layout (rows g / g + 8,
 // columns 8 nj + 2t, + 1), on exit the performer's output rows.
+template <int ACT>
 __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4], float (&y1)[8][4], int g, int t, float eps) {
   auto bfrag = [&](int m, int nj, int ks, uint32_t& b0, uint32_t& b1v) {
     const __nv_bfloat16* rp = &sm.ws[m][(nj * 8 + g) * kWRow + ks * 16 + 2 * t];
@@ -443,7 +468,7 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
       a[ks][2 * h + 1] = ptx::pack_bf16x2((y1[nj][2] - mB) * rB * gg.x + be.x, (y1[nj][3] - mB) * rB * gg.y + be.y);
     }
   }
-  // h = gelu_tanh(z w1^T + b1)
+  // h = gelu(z w1^T + b1); h is a bf16 operand, so the erf form takes the bf16-accuracy polynomial of the FC1 epilogue
 #pragma unroll
   for (int nj = 0; nj < 8; ++nj) {
     acc[nj][0] = acc[nj][1] = acc[nj][2] = acc[nj][3] = 0.f;
@@ -461,8 +486,8 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
       const int nj = 2 * ks + h;
       const float2 bb = *reinterpret_cast<const float2*>(&sm.vec[3][nj * 8 + 2 * t]);
       float h0 = acc[nj][0] + bb.x, h1 = acc[nj][1] + bb.y, h2 = acc[nj][2] + bb.x, h3 = acc[nj][3] + bb.y;
-      gemm_detail::gelu_tanh_pair(h0, h1);
-      gemm_detail::gelu_tanh_pair(h2, h3);
+      gemm_detail::apply_act_pair<ACT, false, false>(h0, h1);
+      gemm_detail::apply_act_pair<ACT, false, false>(h2, h3);
       a[ks][2 * h] = ptx::pack_bf16x2(h0, h1);
       a[ks][2 * h + 1] = ptx::pack_bf16x2(h2, h3);
     }
@@ -490,7 +515,7 @@ __device__ __forceinline__ void tail_tile(const TailSmem& sm, uint32_t (&a)[4][4
 // TAIL: the tile goes straight on through attn_output + LayerNorm + MLP (tail_tile above) -- ya and v never leave the registers,
 // vout receives the performer's finished output rows and yattn is not written: 512 bytes of HBM traffic per token (q, v in; y out)
 // instead of 640 here + 640 in the tail kernel.  Bit-identical to the two kernels (same roundings, same order).
-template <bool TAIL>
+template <bool TAIL, int ACT = EVT_ACT_GELU_TANH>
 __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat16* __restrict__ kqv, long long ld,
                                                               const float* __restrict__ w, const float* __restrict__ stats,
                                                               __nv_bfloat16* __restrict__ yattn, float* __restrict__ vout,
@@ -595,7 +620,7 @@ __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat1
         if (okB) vB = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(base + (g + 8) * ld + col));
         y1[nj][0] = vA.x, y1[nj][1] = vA.y, y1[nj][2] = vB.x, y1[nj][3] = vB.y;
       }
-      tail_tile(sm_tail[0], ya_frag, y1, g, t, tw.eps);
+      tail_tile<ACT>(sm_tail[0], ya_frag, y1, g, t, tw.eps);
 #pragma unroll
       for (int nj = 0; nj < 8; ++nj) {
         const int col = nj * 8 + 2 * t;
@@ -617,6 +642,7 @@ __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat1
 
 
 
+template <int ACT>
 __global__ void __launch_bounds__(128) performer_mlp_kernel(const __nv_bfloat16* __restrict__ ya, float* __restrict__ y, const TailWeights tw,
                                                             long long rows) {
   __shared__ TailSmem sm;
@@ -646,7 +672,7 @@ __global__ void __launch_bounds__(128) performer_mlp_kernel(const __nv_bfloat16*
       if (okB) vB = *reinterpret_cast<const float2*>(y + (r0 + g + 8) * kEmb + col);
       y1[nj][0] = vA.x, y1[nj][1] = vA.y, y1[nj][2] = vB.x, y1[nj][3] = vB.y;
     }
-    tail_tile(sm, a, y1, g, t, tw.eps);
+    tail_tile<ACT>(sm, a, y1, g, t, tw.eps);
 #pragma unroll
     for (int nj = 0; nj < 8; ++nj) {
       const int col = nj * 8 + 2 * t;
@@ -665,7 +691,7 @@ void unfold_ln_dispatch(const TIN* xi, __nv_bfloat16* o, int64_t ldo, const floa
   if (k == 7 && C == 3 && ldo == 152) {
     constexpr int kIter = 2;  // 8 warps x 4 rows x 2 iterations = 64 rows per block
     const unsigned g773 = static_cast<unsigned>((rows + 64 - 1) / 64);
-    unfold773_kernel<TIN, LN, kIter><<<g773, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, H, W, s, p, oh, ow, rows);
+    unfold773_kernel<TIN, LN, kIter><<<g773, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, H, W, s, p, oh, ow, rows, PixAffine{});
   }
   else if (k == 7 && C == 3) unfold_ln_kernel<TIN, LN, 7, 3><<<grid, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, B, H, W, C, k, s, p, oh, ow, rows);
   else if (k == 3 && C == 64) unfold_ln_kernel<TIN, LN, 3, 64><<<grid, 256, 0, st>>>(xi, o, ldo, gamma, beta, eps, B, H, W, C, k, s, p, oh, ow, rows);
@@ -699,6 +725,39 @@ int unfold_ln_launch(const void* x, int x_dtype, void* out, int64_t ldo, const f
     return fail(EVT_ERR_INVALID, "unfold_ln: x dtype must be f32 or bf16");
   }
   EVT_LAUNCH_CHECK("unfold_ln");
+  return EVT_OK;
+}
+
+template <typename TIN, bool AFFINE>
+void unfold773_nchw_typed(const void* px, __nv_bfloat16* o, const float* gamma, const float* beta, float eps, int H, int W, int oh, int ow,
+                          long long rows, const PixAffine& af, cudaStream_t st) {
+  constexpr int kIter = 2;
+  const unsigned grid = static_cast<unsigned>((rows + 64 - 1) / 64);
+  unfold773_kernel<TIN, true, kIter, true, AFFINE><<<grid, 256, 0, st>>>(reinterpret_cast<const TIN*>(px), o, 152, gamma, beta, eps, H, W,
+                                                                          4, 2, oh, ow, rows, af);
+}
+
+int unfold773_nchw_launch(const void* pixels, int pixel_dtype, const float* scale3, const float* bias3, void* out, const float* gamma,
+                          const float* beta, float eps, int B, int H, int W, cudaStream_t st) {
+  EVT_CHECK_ARG(pixels && out && gamma && beta, "unfold773_nchw: null pointer");
+  EVT_CHECK_ARG(B > 0 && H >= 7 && W >= 7, "unfold773_nchw: bad sizes");
+  EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(out) % 4 == 0, "unfold773_nchw: out must be 4-byte aligned");
+  const int oh = (H + 2 * 2 - 7) / 4 + 1, ow = (W + 2 * 2 - 7) / 4 + 1;
+  const long long rows = static_cast<long long>(B) * oh * ow;
+  __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
+  PixAffine af = {{1.f, 1.f, 1.f}, {0.f, 0.f, 0.f}};
+  if (pixel_dtype == EVT_PIX_U8) {
+    EVT_CHECK_ARG(scale3 && bias3, "unfold773_nchw: u8 pixels need a per-channel scale and bias");
+    for (int c = 0; c < 3; ++c) af.scale[c] = scale3[c], af.bias[c] = bias3[c];
+    unfold773_nchw_typed<uint8_t, true>(pixels, o, gamma, beta, eps, H, W, oh, ow, rows, af, st);
+  } else if (pixel_dtype == EVT_PIX_BF16) {
+    unfold773_nchw_typed<__nv_bfloat16, false>(pixels, o, gamma, beta, eps, H, W, oh, ow, rows, af, st);
+  } else if (pixel_dtype == EVT_PIX_F32) {
+    unfold773_nchw_typed<float, false>(pixels, o, gamma, beta, eps, H, W, oh, ow, rows, af, st);
+  } else {
+    return fail(EVT_ERR_INVALID, "unfold773_nchw: unknown pixel dtype");
+  }
+  EVT_LAUNCH_CHECK("unfold773_nchw");
   return EVT_OK;
 }
 
@@ -764,7 +823,7 @@ int performer_mlp_launch(const void* ya, float* y, const void* wo, const float* 
   TailWeights tw;
   tw.wo = reinterpret_cast<const __nv_bfloat16*>(wo), tw.w1 = reinterpret_cast<const __nv_bfloat16*>(w1), tw.w2 = reinterpret_cast<const __nv_bfloat16*>(w2);
   tw.bo = bo, tw.gamma = gamma, tw.beta = beta, tw.b1 = b1, tw.b2 = b2, tw.eps = eps;
-  performer_mlp_kernel<<<grid, 128, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(ya), y, tw, rows);
+  performer_mlp_kernel<EVT_ACT_GELU_TANH><<<grid, 128, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(ya), y, tw, rows);
   EVT_LAUNCH_CHECK("performer_mlp");
   return EVT_OK;
 }
@@ -796,8 +855,9 @@ int performer_launch(const void* kqv, int64_t ld, const float* w, void* yattn, f
 // The whole Token_performer after the kqv projection: attention contraction + attn_output + LayerNorm + MLP; y f32 [B*T, 64]
 int performer_block_launch(const void* kqv, int64_t ld, const float* w, float* y, void* workspace, int B, int T, float eps, const void* wo,
                            const float* bo, const float* gamma, const float* beta, const void* w1, const float* b1, const void* w2,
-                           const float* b2, float ln_eps, cudaStream_t st) {
+                           const float* b2, float ln_eps, cudaStream_t st, int act) {
   EVT_CHECK_ARG(kqv && w && y && workspace && wo && gamma && beta && w1 && w2, "performer_block: null pointer");
+  EVT_CHECK_ARG(act == EVT_ACT_GELU_TANH || act == EVT_ACT_GELU_ERF, "performer_block: the MLP activation must be tanh- or erf-GELU");
   EVT_CHECK_ARG(B > 0 && T > 0 && B <= 65535, "performer_block: B in 1..65535 and T > 0");
   EVT_CHECK_ARG(ld >= 3 * kEmb && ld % 8 == 0 && reinterpret_cast<uintptr_t>(kqv) % 16 == 0,
                 "performer_block: kqv rows must be 16-byte aligned with a leading dimension >= 192");
@@ -814,7 +874,11 @@ int performer_block_launch(const void* kqv, int64_t ld, const float* w, float* y
   TailWeights tw;
   tw.wo = reinterpret_cast<const __nv_bfloat16*>(wo), tw.w1 = reinterpret_cast<const __nv_bfloat16*>(w1), tw.w2 = reinterpret_cast<const __nv_bfloat16*>(w2);
   tw.bo = bo, tw.gamma = gamma, tw.beta = beta, tw.b1 = b1, tw.b2 = b2, tw.eps = ln_eps;
-  performer_apply_kernel<true><<<grid, 128, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(kqv), ld, w, stats, nullptr, y, T, eps, tw);
+  const __nv_bfloat16* kqv16 = reinterpret_cast<const __nv_bfloat16*>(kqv);
+  if (act == EVT_ACT_GELU_ERF)
+    performer_apply_kernel<true, EVT_ACT_GELU_ERF><<<grid, 128, 0, st>>>(kqv16, ld, w, stats, nullptr, y, T, eps, tw);
+  else
+    performer_apply_kernel<true, EVT_ACT_GELU_TANH><<<grid, 128, 0, st>>>(kqv16, ld, w, stats, nullptr, y, T, eps, tw);
   EVT_LAUNCH_CHECK("performer_apply_tail");
   return EVT_OK;
 }

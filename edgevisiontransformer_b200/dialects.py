@@ -11,10 +11,15 @@ The different skip-connection semantics (skip carries LN(x)) is a runtime flag (
 timm / facebookresearch-deit dialect (``torch.hub.load('facebookresearch/deit:main', 'deit_*_patch16_224')``,
 utils.py:52-62, tools.py:244-263): same function as HF ViT with a fused ``attn.qkv`` Linear (rows q | k | v, head-major
 inside each), LayerNorm eps 1e-6 and flat key names -> pure renaming + split, see ``timm_vit_to_canonical``.
+
+PyTorch T2T-ViT (yitu-opensource/T2T-ViT, ``tokens_type='performer'``; the reference's tools.py:347-365 loads these files):
+timm-layout encoder blocks without qkv bias, plus the tokens-to-token module, whose ``nn.Unfold`` soft splits order their
+columns ``(c, kh, kw)`` -> permuted to the ``(kh, kw, c)`` order of the library's soft splits, see ``t2t_torch_to_canonical``.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Tuple
+import math
+from typing import Dict, List, Optional, Tuple
 
 import torch
 
@@ -85,6 +90,14 @@ def timm_vit_to_canonical(sd: Dict[str, torch.Tensor], patch: int = 16) -> Tuple
         out["distillation_classifier.weight"], out["distillation_classifier.bias"] = sd["head_dist.weight"], sd["head_dist.bias"]
     else:
         out["classifier.weight"], out["classifier.bias"] = sd["head.weight"], sd["head.bias"]
+    if _timm_blocks_to_canonical(sd, out, D) == 0:
+        raise ValueError("not a timm VisionTransformer state dict (no blocks.0.attn.qkv.weight)")
+    return out, dict(layer_norm_eps=1e-6, hidden_act="gelu", patch_size=patch)
+
+
+def _timm_blocks_to_canonical(sd: Dict[str, torch.Tensor], out: Dict[str, torch.Tensor], D: int, q_scale: float = 1.0) -> int:
+    """timm ``Block`` s ``blocks.{l}.*`` (fused ``attn.qkv``, rows q | k | v) -> ``vit.encoder.layer.{l}.*``; returns the depth.
+    ``q_scale`` multiplies the query rows (weight and bias): how a softmax scale other than head_size ** -0.5 is folded in."""
     l = 0
     while f"blocks.{l}.attn.qkv.weight" in sd:
         p, q = f"blocks.{l}.", f"vit.encoder.layer.{l}."
@@ -93,14 +106,79 @@ def timm_vit_to_canonical(sd: Dict[str, torch.Tensor], patch: int = 16) -> Tuple
             raise ValueError(f"blocks.{l}.attn.qkv.weight has {w.shape[0]} rows, expected 3 x {D}")
         b = sd.get(p + "attn.qkv.bias")
         for i, n in enumerate(("query", "key", "value")):
-            out[q + f"attention.attention.{n}.weight"] = w[i * D:(i + 1) * D].contiguous()
-            if b is not None:
-                out[q + f"attention.attention.{n}.bias"] = b[i * D:(i + 1) * D].contiguous()
+            for t, suffix in ((w, "weight"), (b, "bias")):
+                if t is not None:
+                    rows = t[i * D:(i + 1) * D]
+                    out[q + f"attention.attention.{n}.{suffix}"] = (rows * q_scale if i == 0 and q_scale != 1.0 else rows).contiguous()
         for src, dst in (("attn.proj", "attention.output.dense"), ("mlp.fc1", "intermediate.dense"), ("mlp.fc2", "output.dense"),
                          ("norm1", "layernorm_before"), ("norm2", "layernorm_after")):
             out[q + dst + ".weight"] = sd[p + src + ".weight"]
             out[q + dst + ".bias"] = sd[p + src + ".bias"]
         l += 1
-    if l == 0:
-        raise ValueError("not a timm VisionTransformer state dict (no blocks.0.attn.qkv.weight)")
-    return out, dict(layer_norm_eps=1e-6, hidden_act="gelu", patch_size=patch)
+    return l
+
+
+def unwrap_checkpoint(ck: dict, use_ema: bool = True) -> Dict[str, torch.Tensor]:
+    """The state dict inside a training checkpoint: ``state_dict_ema`` (when ``use_ema``), ``state_dict`` or ``model``, else
+    ``ck`` itself; ``module.`` (DataParallel / DDP) prefixes stripped.  timm's checkpoint saver writes the first two."""
+    for k in (("state_dict_ema",) if use_ema else ()) + ("state_dict", "model"):
+        if isinstance(ck.get(k), dict):
+            ck = ck[k]
+            break
+    return {(k[len("module."):] if k.startswith("module.") else k): v for k, v in ck.items() if torch.is_tensor(v)}
+
+
+def _ckk_to_kkc(t: torch.Tensor, C: int, k: int) -> torch.Tensor:
+    """Last dimension ordered (c, kh, kw) -- nn.Unfold's columns -- reordered to (kh, kw, c)."""
+    lead = t.shape[:-1]
+    return t.reshape(*lead, C, k, k).movedim(-3, -1).reshape(*lead, C * k * k).contiguous()
+
+
+T2T_TORCH_HEAD_SIZE = 64
+
+
+def t2t_torch_to_canonical(sd: Dict[str, torch.Tensor], qk_scale: Optional[float] = None, use_ema: bool = True
+                           ) -> Tuple[Dict[str, torch.Tensor], dict]:
+    """PyTorch T2T-ViT (``T2T_ViT`` with ``tokens_type='performer'``) state dict or training checkpoint -> (canonical state
+    dict, from_state_dict kwargs).
+
+    * ``tokens_to_token.attention{1,2}.*`` -> ``t2t.performer{1,2}.*`` in the Keras naming the runtime loads (INTEGRATION.md
+      §3): kernels ``[in, out]``; the rows of ``kqv.kernel`` and of ``norm1.{gamma,beta}`` permuted from ``(c, kh, kw)`` to
+      ``(kh, kw, c)`` (stage 1: C = 3, k = 7; stage 2: C = 64, k = 3); ``w`` as stored (already times sqrt(m)).
+    * ``tokens_to_token.project`` -> the token-embedding projection, its 576 input columns permuted the same way (C = 64, k = 3).
+    * ``cls_token``, ``pos_embed`` (the sinusoid table stored in the checkpoint) -> the embeddings.
+    * ``blocks.*``, ``norm.*``, ``head.*`` as in ``timm_vit_to_canonical``.  ``qk_scale`` (default head_size ** -0.5, the
+      scale the runtime applies) is folded into the query rows.
+    Refuses ``tokens_type='transformer'`` checkpoints and any image size other than 224."""
+    sd = unwrap_checkpoint(sd, use_ema)
+    if "tokens_to_token.attention1.attn.qkv.weight" in sd:
+        raise ValueError("tokens_type='transformer' T2T-ViT (t2t_vit_t_*) is not supported: its token attention runs over 3136 "
+                         "tokens, more than EVT_ATTN_MAX_TOKENS; only the performer checkpoints (t2t_vit_*) run here")
+    if "tokens_to_token.attention1.kqv.weight" not in sd or "blocks.0.attn.qkv.weight" not in sd:
+        raise ValueError("not a PyTorch T2T-ViT state dict (no tokens_to_token.attention1.kqv.weight or blocks.0.attn.qkv.weight)")
+    D = sd["cls_token"].shape[-1]
+    if sd["pos_embed"].shape[-2] != 197:
+        raise ValueError(f"pos_embed has {sd['pos_embed'].shape[-2]} rows: only the 224-pixel T2T-ViT (197 tokens) is supported")
+    out: Dict[str, torch.Tensor] = {}
+    for i, (C, k) in ((1, (3, 7)), (2, (64, 3))):
+        s, d = f"tokens_to_token.attention{i}.", f"t2t.performer{i}."
+        out[d + "norm1.gamma"] = _ckk_to_kkc(sd[s + "norm1.weight"], C, k)
+        out[d + "norm1.beta"] = _ckk_to_kkc(sd[s + "norm1.bias"], C, k)
+        out[d + "kqv.kernel"] = _ckk_to_kkc(sd[s + "kqv.weight"], C, k).t().contiguous()
+        out[d + "kqv.bias"] = sd[s + "kqv.bias"]
+        out[d + "w"] = sd[s + "w"]
+        for src, dst in (("proj", "attn_output"), ("mlp.0", "mlp.fc1"), ("mlp.2", "mlp.fc2")):
+            out[d + dst + ".kernel"] = sd[s + src + ".weight"].t().contiguous()
+            out[d + dst + ".bias"] = sd[s + src + ".bias"]
+        out[d + "norm2.gamma"], out[d + "norm2.beta"] = sd[s + "norm2.weight"], sd[s + "norm2.bias"]
+    out["vit.embeddings.patch_embeddings.projection.weight"] = _ckk_to_kkc(sd["tokens_to_token.project.weight"], 64, 3)
+    out["vit.embeddings.patch_embeddings.projection.bias"] = sd["tokens_to_token.project.bias"]
+    out["vit.embeddings.cls_token"] = sd["cls_token"].reshape(1, 1, D)
+    out["vit.embeddings.position_embeddings"] = sd["pos_embed"].reshape(1, -1, D)
+    scale = T2T_TORCH_HEAD_SIZE ** -0.5 if qk_scale is None else float(qk_scale)
+    _timm_blocks_to_canonical(sd, out, D, q_scale=scale * math.sqrt(T2T_TORCH_HEAD_SIZE))
+    out["vit.layernorm.weight"], out["vit.layernorm.bias"] = sd["norm.weight"], sd["norm.bias"]
+    out["classifier.weight"], out["classifier.bias"] = sd["head.weight"], sd["head.bias"]
+    kw = dict(dialect="hf", hidden_act="gelu", layer_norm_eps=1e-5, final_ln=True, head_size=T2T_TORCH_HEAD_SIZE, patch_size=16,
+              image_size=224, embed_k=576, t2t=2)
+    return out, kw

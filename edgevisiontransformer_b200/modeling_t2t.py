@@ -9,17 +9,24 @@ INTEGRATION.md (one entry per Keras variable; Dense kernels ``[in, out]``).  The
 
 and the rest (project + cls + sinusoid position table + 14 TF-dialect encoder blocks + LN + classifier) is the
 model-level C entry point ``evt_model_forward_embedded``.
+
+``B200T2TViTTorch`` and ``t2t_vit_{7,10,12,14,19,24}`` run the published PyTorch checkpoints (yitu-opensource/T2T-ViT,
+``tokens_type='performer'``; the files the reference's tools.py:347-365 loads): NCHW f32 / bf16 / uint8 pixels, the same
+front-end kernels with the stage-1 soft split reading planar pixels (``spec.t2t = 2``), erf-GELU performers and a pre-LN
+(HF-dialect) encoder.  Weights go through ``dialects.t2t_torch_to_canonical``.
 """
 from __future__ import annotations
 
-from typing import Dict, List
+import argparse
+import os
+from typing import Dict, List, Optional
 
 import torch
 import torch.nn as nn
 
 from . import ops
-from .dialects import _encoder_to_canonical
-from .modeling_vit import B200ViTForImageClassification, ImageClassifierOutput
+from .dialects import T2T_TORCH_HEAD_SIZE, _encoder_to_canonical, t2t_torch_to_canonical, unwrap_checkpoint
+from .modeling_vit import B200ViTForImageClassification, ImageClassifierOutput, config_from_state_dict
 
 TF_EPS = 1e-5
 
@@ -160,3 +167,100 @@ def get_t2t_vit_10(sd, **kw):
 
 def get_t2t_vit_7(sd, **kw):
     return B200T2TViT(sd, depth=7, num_heads=4, **kw)
+
+
+# ---------------------------------------------------------------------------------------------- PyTorch T2T-ViT checkpoints
+# upstream factories (models/t2t_vit.py): embed_dim, depth, num_heads, mlp_ratio
+T2T_TORCH = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_12": (256, 12, 4, 2.0),
+             "t2t_vit_14": (384, 14, 6, 3.0), "t2t_vit_19": (448, 19, 7, 3.0), "t2t_vit_24": (512, 24, 8, 3.0)}
+
+
+def load_t2t_checkpoint(path) -> dict:
+    """``torch.load`` of a T2T-ViT ``.pth`` / ``.pth.tar`` with ``weights_only=True``.  timm's checkpoint saver, which wrote the
+    published files, stores the training ``argparse.Namespace`` under ``args``: that one class is allow-listed."""
+    with torch.serialization.safe_globals([argparse.Namespace]):
+        return torch.load(os.fspath(path), map_location="cpu", weights_only=True)
+
+
+class B200T2TViTTorch(B200ViTForImageClassification):
+    """PyTorch ``T2T_ViT`` (``tokens_type='performer'``) on libevt: the whole forward, front-end included, is one C call per
+    chunk.  Input is NCHW ``[B, 3, 224, 224]`` in f32, bf16 or uint8 (uint8 is normalised with ``pixel_mean`` / ``pixel_std``
+    inside the first soft split; the zero padding applies to the normalised image, as upstream pads the normalised tensor).
+
+    ``checkpoint_or_sd``: a file path, a checkpoint dict (``state_dict_ema`` -- used unless ``use_ema=False`` --,
+    ``state_dict`` or ``model``) or a flat state dict.  Depth and embed_dim come from the weights; ``num_heads`` defaults to
+    embed_dim / 64 (the head size of every published config).  ``qk_scale`` defaults to head_dim ** -0.5 as upstream's class
+    does; the ``t2t_vit_*`` factories default it to embed_dim ** -0.5, as upstream's do for ``pretrained=True``."""
+
+    def __init__(self, checkpoint_or_sd, num_heads: Optional[int] = None, qk_scale: Optional[float] = None, device="cuda",
+                 max_batch: int = 1024, precision: str = "bf16", image_size: int = 224, use_ema: bool = True, keep_params: bool = True):
+        if precision != "bf16":
+            raise NotImplementedError("the T2T front-end is implemented for the bf16 mode")
+        if image_size != 224:
+            raise ValueError(f"image_size {image_size}: only the 224-pixel T2T-ViT is supported")
+        sd = load_t2t_checkpoint(checkpoint_or_sd) if isinstance(checkpoint_or_sd, (str, os.PathLike)) else checkpoint_or_sd
+        csd, kw = t2t_torch_to_canonical(sd, qk_scale=qk_scale, use_ema=use_ema)
+        D = csd["vit.embeddings.cls_token"].shape[-1]
+        nh = D // T2T_TORCH_HEAD_SIZE if num_heads is None else int(num_heads)
+        if nh <= 0 or D % nh or D // nh != T2T_TORCH_HEAD_SIZE:
+            raise ValueError(f"embed_dim {D} with num_heads {nh} gives head size {D / max(nh, 1):g}; only head size "
+                             f"{T2T_TORCH_HEAD_SIZE} is implemented")
+        super().__init__(config_from_state_dict(csd, **kw), csd, device=device, max_batch=max_batch, keep_params=keep_params)
+        self.num_heads, self.depth, self.hidden = nh, self.config.num_hidden_layers, D
+
+    @classmethod
+    def from_checkpoint(cls, path, **kw) -> "B200T2TViTTorch":
+        """A published checkpoint file: the factory of its embed_dim (and depth) supplies the defaults."""
+        sd = unwrap_checkpoint(load_t2t_checkpoint(path), kw.get("use_ema", True))
+        name = _factory_of(sd)
+        if name is None and kw.get("qk_scale") is None:
+            raise ValueError("checkpoint shape matches no published t2t_vit_* config; pass qk_scale= explicitly")
+        return globals()[name](sd, **kw) if name is not None else cls(sd, **kw)
+
+
+def _factory_of(sd: Dict[str, torch.Tensor]) -> Optional[str]:
+    if "cls_token" not in sd:
+        return None
+    D, depth = sd["cls_token"].shape[-1], 0
+    while f"blocks.{depth}.attn.qkv.weight" in sd:
+        depth += 1
+    by_dim = [name for name, (d, _, _, _) in T2T_TORCH.items() if d == D]    # same heads, mlp ratio and qk_scale for one D
+    exact = [name for name in by_dim if T2T_TORCH[name][1] == depth]
+    return (exact or by_dim or [None])[0]
+
+
+def _t2t_factory(name: str, checkpoint_or_sd, **kw) -> B200T2TViTTorch:
+    D, _, heads, ratio = T2T_TORCH[name]     # depth comes from the weights
+    sd = load_t2t_checkpoint(checkpoint_or_sd) if isinstance(checkpoint_or_sd, (str, os.PathLike)) else checkpoint_or_sd
+    sd = unwrap_checkpoint(sd, kw.get("use_ema", True))
+    if "cls_token" in sd and "blocks.0.mlp.fc1.weight" in sd:
+        got = (sd["cls_token"].shape[-1], sd["blocks.0.mlp.fc1.weight"].shape[0])
+        if got != (D, int(D * ratio)):
+            raise ValueError(f"{name} is embed_dim {D} with an MLP of {int(D * ratio)}; the weights have {got[0]} and {got[1]}")
+    kw.setdefault("num_heads", heads)
+    kw.setdefault("qk_scale", D ** -0.5)           # upstream's t2t_vit_* with pretrained=True
+    return B200T2TViTTorch(sd, **kw)
+
+
+def t2t_vit_7(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_7", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_10(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_10", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_12(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_12", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_14(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_14", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_19(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_19", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_24(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_24", checkpoint_or_sd, **kw)

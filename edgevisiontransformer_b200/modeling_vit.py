@@ -40,7 +40,8 @@ class B200ViTConfig:
     head_hidden: int = 0
     precision: str = "bf16"           # "bf16" (2e-2 logit tolerance) | "tf32" (1e-3; f32 activations)
     embed_k: int = 0                  # >0: caller-built patch matrix with this K (T2T: 576), see forward_embedded
-    t2t: bool = False                 # tokens-to-token front-end inside the library (NHWC f32 pixels; needs embed_k = 576)
+    t2t: int = 0                      # tokens-to-token front-end inside the library (needs embed_k = 576): 1 / True NHWC f32
+                                      # pixels (TF T2T), 2 NCHW f32 / bf16 / uint8 pixels (PyTorch T2T, modeling_t2t.B200T2TViTTorch)
     head_rows: int = 1                # 2: DeiTForImageClassificationWithTeacher (cls + distillation rows feed ONE folded classifier)
 
     # names the reference's callers read off model.config
@@ -97,7 +98,7 @@ def config_from_state_dict(sd: Dict[str, torch.Tensor], *, layer_norm_eps=1e-12,
                          tokens=sd["vit.embeddings.position_embeddings"].shape[-2], image_size=image_size,
                          patch_size=patch_size, num_labels=sd["classifier.weight"].shape[0],
                          layer_norm_eps=layer_norm_eps, hidden_act=hidden_act, dialect=dialect, final_ln=bool(final_ln),
-                         head_hidden=int(head_hidden), precision=precision, embed_k=int(embed_k), t2t=bool(t2t))
+                         head_hidden=int(head_hidden), precision=precision, embed_k=int(embed_k), t2t=int(t2t))
 
 
 class B200ViTForImageClassification(nn.Module):
@@ -147,7 +148,7 @@ class B200ViTForImageClassification(nn.Module):
             spec.inter[l] = int(config.intermediate[l])
         spec.final_ln = int(config.final_ln)
         spec.head_hidden = int(config.head_hidden)
-        spec.t2t = int(bool(config.t2t))
+        spec.t2t = int(config.t2t)
         spec.embed_k = int(config.embed_k)
         spec.head_rows = int(config.head_rows)
         if config.precision not in ("bf16", "tf32"):

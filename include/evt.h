@@ -301,7 +301,8 @@ typedef struct evt_model_spec {
   int inter[EVT_MAX_LAYERS];   /* FFN width per layer (optimize_model semantics), any int>0  */
   int final_ln;                /* 1: LayerNorm before the head (HF, T2T); 0: TF-dialect DeiT */
   int head_hidden;             /* 0: single Linear head; >0: Dense(head_hidden, gelu)->Dense */
-  int t2t;                     /* 1: T2T front-end (NHWC input) instead of the patch embed   */
+  int t2t;                     /* T2T front-end instead of the patch embed: 1 NHWC f32 pixels (TF T2T); 2 NCHW
+                                  f32 / bf16 / u8 pixels, the PyTorch T2T (stage-1 columns in (kh, kw, c) order); 0 none */
   int precision;               /* evt_precision: 0 bf16 operands, 1 tf32 operands (f32 activations) */
   int embed_k;                 /* 0: 3*patch*patch.  >0: K of the token-embedding GEMM when the caller builds the
                                   patch matrix itself (T2T: 3*3*64 = 576) and calls evt_model_forward_embedded */
