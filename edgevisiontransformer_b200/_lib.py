@@ -97,6 +97,8 @@ SIGNATURES = {
     "evt_performer_fwd": (_i, [_p, _i64, _p, _p, _p, _p, _i, _i, _i, _i, _f, _p]),
     "evt_performer_mlp_fwd": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _f, _p]),
     "evt_performer_block_fwd": (_i, [_p, _i64, _p, _p, _p, _i, _i, _f, _p, _p, _p, _p, _p, _p, _p, _p, _f, _p]),
+    "evt_token_transformer_workspace_bytes": (_i, [_i, _i, C.POINTER(_sz)]),
+    "evt_token_transformer_block_fwd": (_i, [_p, _i64, _p, _p, _i, _i, _f, _p, _p, _p, _p, _p, _p, _p, _p, _f, _p]),
     "evt_model_launches_per_forward": (_i, [_p]),
     "evt_model_profile_begin": (_i, [_p]),
     "evt_model_profile_end": (_i, [_p, C.POINTER(_f), C.POINTER(_i)]),

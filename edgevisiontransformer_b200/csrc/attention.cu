@@ -25,6 +25,7 @@
 #include <math_constants.h>
 
 #include "common.h"
+#include "ops.h"
 #include "ptx.cuh"
 
 namespace evt {
@@ -1008,6 +1009,18 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   if (head_size != kHD) return fail(EVT_ERR_UNSUPPORTED, "attention: only head size 64 is implemented");
   if (S > EVT_ATTN_MAX_TOKENS)
     return fail(EVT_ERR_UNSUPPORTED, "attention: sequence length above " + std::to_string(EVT_ATTN_MAX_TOKENS) + " is not implemented");
+  return attention_any_length_launch(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
+}
+
+// Nothing in attention_long_kernel depends on S beyond the B*S bound checked here: its shared and tensor memory are per
+// 128-key block, its item count B * heads * ceil(Sq / 128) is checked against 2^30 by attention_long_launch, and its TMA
+// coordinates (head column, row within the image, image) stay below 2^31 for any B*S that passes.  The public cap is
+// EVT_ATTN_MAX_TOKENS (attention_launch); the T2T token transformer runs one head over 3136 tokens through here.
+int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
+                                int heads, float scale, cudaStream_t stream) {
+  EVT_CHECK_ARG(qkv && ctx, "attention: null pointer");
+  EVT_CHECK_ARG(B > 0 && S > 0 && heads > 0, "attention: B, S, heads must be positive");
+  EVT_CHECK_ARG(Sq > 0 && Sq <= S, "attention: query rows must be in 1..S");
   EVT_CHECK_ARG(ldq >= 3ll * heads * kHD && ldc >= static_cast<int64_t>(heads) * kHD, "attention: leading dimension too small");
   EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention: ctx must be 16-byte aligned rows");
   EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");

@@ -65,7 +65,8 @@ struct LayerW {
   int a = 0, inter = 0, inter_ld = 0;
 };
 
-// one TokenPerformer of the T2T front-end (modeling/layers/transformer_encoder.py:39-101), emb = 64, m = 32
+// one TokenPerformer of the T2T front-end (modeling/layers/transformer_encoder.py:39-101), emb = 64, m = 32; with spec.t2t = 3 one
+// Token_transformer (PyTorch T2T-ViT, tokens_type='transformer'): wkqv = the bias-free qkv projection (rows q | k | v), no w
 struct PerformerW {
   int in_dim = 0, in_ld = 0;            // 147 / 576, leading dimension of the unfolded rows (multiple of 8)
   float *g1 = nullptr, *b1 = nullptr;   // norm1 over the unfolded row
@@ -149,7 +150,8 @@ Workspace plan_workspace(const evt_model* m, int batch, uint8_t* base) {
       w.t_x[i] = c.take(T * in_ld * 2);
       w.t_kqv[i] = c.take(T * 192 * 2);
       w.t_y[i] = c.take<float>(T * 64 * 4);
-      w.t_ws[i] = c.take(performer_workspace_bytes(batch, t2t_side(s.image, i) * t2t_side(s.image, i)));
+      const int Ti = t2t_side(s.image, i) * t2t_side(s.image, i);
+      w.t_ws[i] = c.take(s.t2t == 3 ? token_transformer_workspace_bytes(batch, Ti) : performer_workspace_bytes(batch, Ti));
     }
     w.t_pm = c.take(Mp * 576 * 2);
   }
@@ -181,7 +183,8 @@ int validate_spec(const evt_model_spec* s) {
                   "head_rows = 2 (two-head distilled DeiT) needs 198 tokens, the final LayerNorm and a single Linear head");
   EVT_CHECK_ARG(s->precision == EVT_PREC_BF16 || s->precision == EVT_PREC_TF32, "precision must be bf16 (0) or tf32 (1)");
   EVT_CHECK_ARG(s->embed_k >= 0 && s->embed_k % 8 == 0, "embed_k must be a non-negative multiple of 8");
-  EVT_CHECK_ARG(s->t2t >= 0 && s->t2t <= 2, "t2t must be 0 (patch embedding), 1 (T2T front-end, NHWC f32 pixels) or 2 (T2T front-end, NCHW pixels)");
+  EVT_CHECK_ARG(s->t2t >= 0 && s->t2t <= 3, "t2t must be 0 (patch embedding), 1 (T2T front-end, NHWC f32 pixels), 2 (T2T front-end, "
+                                            "NCHW pixels) or 3 (T2T front-end with token transformers, NCHW pixels)");
   if (s->t2t) {
     EVT_CHECK_ARG(s->embed_k == 576 && s->precision == EVT_PREC_BF16, "the T2T front-end needs embed_k = 576 (3 x 3 x 64) and the bf16 mode");
     EVT_CHECK_ARG(t2t_side(s->image, 2) * t2t_side(s->image, 2) == patches, "image size does not give image/16 squared T2T tokens");
@@ -361,7 +364,25 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
     EVT_TRY(L.vec(p + "layernorm_after.weight", D, false, &w.ln2_g));
     EVT_TRY(L.vec(p + "layernorm_after.bias", D, false, &w.ln2_b));
   }
-  if (s.t2t) {  // Keras variable names of T2T_module (modeling/models/t2t_vit.py:47-59), Dense kernels [in, out]
+  if (s.t2t == 3) {  // Token_transformer (INTEGRATION.md §3), Dense kernels [in, out]; norm1 / qkv rows in (kh, kw, c) order
+    for (int i = 0; i < 2; ++i) {
+      PerformerW& pw = m->perf[i];
+      const std::string p = "t2t.transformer" + std::to_string(i + 1) + ".";
+      pw.in_dim = i == 0 ? 7 * 7 * 3 : 3 * 3 * 64;
+      pw.in_ld = padn(pw.in_dim, 8);
+      EVT_TRY(L.vec(p + "norm1.gamma", pw.in_dim, false, &pw.g1));
+      EVT_TRY(L.vec(p + "norm1.beta", pw.in_dim, false, &pw.b1));
+      EVT_TRY(L.mat_t(p + "qkv.kernel", 192, pw.in_dim, pw.in_ld, &pw.wkqv));
+      EVT_TRY(L.mat_t(p + "attn_output.kernel", 64, 64, 64, &pw.wo));
+      EVT_TRY(L.vec(p + "attn_output.bias", 64, true, &pw.bo));
+      EVT_TRY(L.vec(p + "norm2.gamma", 64, false, &pw.g2));
+      EVT_TRY(L.vec(p + "norm2.beta", 64, false, &pw.b2));
+      EVT_TRY(L.mat_t(p + "mlp.fc1.kernel", 64, 64, 64, &pw.w1));
+      EVT_TRY(L.vec(p + "mlp.fc1.bias", 64, true, &pw.bb1));
+      EVT_TRY(L.mat_t(p + "mlp.fc2.kernel", 64, 64, 64, &pw.w2));
+      EVT_TRY(L.vec(p + "mlp.fc2.bias", 64, true, &pw.bb2));
+    }
+  } else if (s.t2t) {  // Keras variable names of T2T_module (modeling/models/t2t_vit.py:47-59), Dense kernels [in, out]
     for (int i = 0; i < 2; ++i) {
       PerformerW& pw = m->perf[i];
       const std::string p = "t2t.performer" + std::to_string(i + 1) + ".";
@@ -409,8 +430,9 @@ extern "C" int evt_model_workspace_bytes(const evt_model* m, int batch, size_t* 
 extern "C" int evt_model_launches_per_forward(const evt_model* m) {
   if (!m) return 0;
   const evt_model_spec& s = m->spec;
-  // T2T front-end: per performer unfold+LN, kqv, 3 performer kernels (the last one carries attn_output + MLP); then the last soft split
-  return (s.t2t ? 2 * 5 + 1 : 0) + (s.embed_k > 0 ? 2 : 3) + 7 * s.layers + (s.final_ln && s.head_rows > 1 ? s.head_rows : 1) + (s.head_hidden > 0 ? 2 : 1);
+  // T2T front-end: per performer unfold+LN, kqv, 3 performer kernels (the last one carries attn_output + MLP); per token
+  // transformer (t2t = 3) unfold+LN, qkv, attention, tail; then the last soft split
+  return (s.t2t == 3 ? 2 * 4 + 1 : s.t2t ? 2 * 5 + 1 : 0) + (s.embed_k > 0 ? 2 : 3) + 7 * s.layers + (s.final_ln && s.head_rows > 1 ? s.head_rows : 1) + (s.head_hidden > 0 ? 2 : 1);
 }
 
 static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts* opts, const void* patch_matrix, int64_t patch_ld,
@@ -458,12 +480,15 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   // tokens-to-token front-end (T2T_module.call, modeling/models/t2t_vit.py:63-88).  spec.t2t = 1: NHWC f32 pixels (the TF T2T);
   // 2: NCHW pixels of any evt_pixel_dtype (the PyTorch T2T: nn.Unfold over the image, whose stage-1 columns the first kernel writes
   // in the same (kh, kw, c) order -- the loader permuted the weights).  Stages 2 and 3 read the token-major [B, T, 64] performer
-  // output either way.  The performer MLP's GELU is spec.act (tanh for the TF T2T, erf for the PyTorch one).
+  // output either way.  The performer MLP's GELU is spec.act (tanh for the TF T2T, erf for the PyTorch one).  spec.t2t = 3: the
+  // PyTorch T2T with Token_transformers (tokens_type='transformer') -- the same soft splits; per stage the bias-free qkv GEMM, exact
+  // single-head softmax attention over all T = 3136 / 784 tokens of an image, with Attention.scale = in_dim ** -0.5 (147 / 576)
+  // passed to the kernel, and the tail y = v + proj(ctx); y += mlp(norm2(y)) with erf-GELU (nn.GELU).
   if (s.t2t && patch_matrix == nullptr) {
     const float tf_eps = 1e-5f;   // tf.keras.layers.LayerNormalization(epsilon=1e-5), transformer_encoder.py:49-50; nn.LayerNorm's default
     const void* src = pixels;
     int src_dt = EVT_F32, side = s.image, ch = 3;
-    const bool nchw = s.t2t == 2;
+    const bool nchw = s.t2t >= 2;
     EVT_CHECK_ARG(nchw || o.pixel_dtype == EVT_PIX_F32, "the T2T front-end with spec.t2t = 1 takes f32 NHWC pixels");
     for (int i = 0; i < 2; ++i) {
       const PerformerW& pw = m->perf[i];
@@ -477,6 +502,13 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
         EVT_STAGE(EVT_STAGE_EMBED, unfold_ln_launch(src, src_dt, w.t_x[i], pw.in_ld, pw.g1, pw.b1, tf_eps, batch, side, side, ch, k, st_, pad_, st));
       EVT_STAGE(EVT_STAGE_EMBED, gemm_launch({.A = w.t_x[i], .lda = pw.in_ld, .W = pw.wkqv, .ldw = pw.in_ld, .bias = pw.bkqv, .out = w.t_kqv[i],
                                               .out_dtype = EVT_BF16, .ldo = 192, .M = rows, .N = 192, .K = pw.in_dim}, st));
+      if (s.t2t == 3) {
+        EVT_TRY(token_transformer_block_launch(w.t_kqv[i], 192, w.t_y[i], w.t_ws[i], batch, T, 1.0f / sqrtf(static_cast<float>(pw.in_dim)),
+                                               pw.wo, pw.bo, pw.g2, pw.b2, pw.w1, pw.bb1, pw.w2, pw.bb2, tf_eps, st));
+        EVT_TRY(mark(EVT_STAGE_EMBED));
+        src = w.t_y[i], src_dt = EVT_F32, side = so, ch = 64;
+        continue;
+      }
       // single_attn + attn_output + LayerNorm + MLP (transformer_encoder.py:67-99): the attention contraction's apply kernel carries
       // each tile through the tail, y = the performer's output rows
       EVT_TRY(performer_block_launch(w.t_kqv[i], 192, pw.w, w.t_y[i], w.t_ws[i], batch, T, 1e-8f, pw.wo, pw.bo, pw.g2, pw.b2, pw.w1,

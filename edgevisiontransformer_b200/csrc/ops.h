@@ -46,6 +46,11 @@ int gemm_rowln_launch(const void* A, int64_t lda, const void* W, int64_t ldw, co
 int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                      int heads, int head_size, float scale, cudaStream_t stream);
 
+// attention_launch without the EVT_ATTN_MAX_TOKENS cap (any S with B*S < 2^31 - 512; S > 256 runs attention_long_kernel):
+// the T2T token transformer's single-head attention over 3136 and 784 tokens
+int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
+                                int heads, float scale, cudaStream_t stream);
+
 int attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask, int B, int S,
                           int heads, int head_size, float scale, cudaStream_t stream);
 
@@ -87,6 +92,12 @@ int performer_block_launch(const void* kqv, int64_t ld, const float* w, float* y
 // u8 takes scale3 / bias3) + the performer's norm1 -> bf16 [B*oh*ow, 152], columns in (kh, kw, c) order, 147.. zero
 int unfold773_nchw_launch(const void* pixels, int pixel_dtype, const float* scale3, const float* bias3, void* out, const float* gamma,
                           const float* beta, float eps, int B, int H, int W, cudaStream_t st);
+// T2T Token_transformer after its qkv projection (attention + the performer tail with v from the qkv matrix, erf-GELU): qkv bf16 [B*T, ld],
+// q | k | v in columns [0,64) [64,128) [128,192); y f32 [B*T, 64]; workspace token_transformer_workspace_bytes(B, T) bytes
+size_t token_transformer_workspace_bytes(int B, int T);
+int token_transformer_block_launch(const void* qkv, int64_t ld, float* y, void* workspace, int B, int T, float scale, const void* wo,
+                                   const float* bo, const float* gamma, const float* beta, const void* w1, const float* b1, const void* w2,
+                                   const float* b2, float ln_eps, cudaStream_t st);
 int unfold_launch(const void* x, int x_dtype, void* out, int64_t ldo, int B, int H, int W, int C, int k, int s, int p,
                   cudaStream_t st);
 

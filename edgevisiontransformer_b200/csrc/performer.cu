@@ -642,9 +642,14 @@ __global__ void __launch_bounds__(128) performer_apply_kernel(const __nv_bfloat1
 
 
 
-template <int ACT>
+// The tail as a kernel of its own.  V_QKV = false: y holds v (f32) on entry and is updated in place (evt_performer_mlp_fwd).
+// V_QKV = true (T2T Token_transformer, y = v + proj(ctx), v from qkv columns [128, 192)): the skip input is read straight from
+// the bf16 qkv matrix (row stride ldv) and y is write-only -- no cast launch and no f32 copy of v; the performer path's vout
+// carries the same bf16-rounded v.
+template <int ACT, bool V_QKV = false>
 __global__ void __launch_bounds__(128) performer_mlp_kernel(const __nv_bfloat16* __restrict__ ya, float* __restrict__ y, const TailWeights tw,
-                                                            long long rows) {
+                                                            long long rows, const __nv_bfloat16* __restrict__ vqkv = nullptr,
+                                                            long long ldv = 0) {
   __shared__ TailSmem sm;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, t = lane & 3;
@@ -668,8 +673,13 @@ __global__ void __launch_bounds__(128) performer_mlp_kernel(const __nv_bfloat16*
     for (int nj = 0; nj < 8; ++nj) {
       const int col = nj * 8 + 2 * t;
       float2 vA = make_float2(0.f, 0.f), vB = make_float2(0.f, 0.f);
-      if (okA) vA = *reinterpret_cast<const float2*>(y + (r0 + g) * kEmb + col);
-      if (okB) vB = *reinterpret_cast<const float2*>(y + (r0 + g + 8) * kEmb + col);
+      if constexpr (V_QKV) {
+        if (okA) vA = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(vqkv + (r0 + g) * ldv + 128 + col));
+        if (okB) vB = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(vqkv + (r0 + g + 8) * ldv + 128 + col));
+      } else {
+        if (okA) vA = *reinterpret_cast<const float2*>(y + (r0 + g) * kEmb + col);
+        if (okB) vB = *reinterpret_cast<const float2*>(y + (r0 + g + 8) * kEmb + col);
+      }
       y1[nj][0] = vA.x, y1[nj][1] = vA.y, y1[nj][2] = vB.x, y1[nj][3] = vB.y;
     }
     tail_tile<ACT>(sm, a, y1, g, t, tw.eps);
@@ -796,6 +806,21 @@ extern "C" int evt_performer_block_fwd(const void* kqv, int64_t ld, const float*
                                      static_cast<cudaStream_t>(stream));
 }
 
+extern "C" int evt_token_transformer_workspace_bytes(int B, int T, size_t* out) {
+  EVT_CHECK_ARG(out != nullptr && B > 0 && T > 0, "token_transformer_workspace_bytes: bad arguments");
+  *out = evt::token_transformer_workspace_bytes(B, T);
+  return EVT_OK;
+}
+
+extern "C" int evt_token_transformer_block_fwd(const void* qkv, int64_t ld, float* y, void* workspace, int B, int T, float scale,
+                                               const void* wo, const float* bo, const float* gamma, const float* beta, const void* w1,
+                                               const float* b1, const void* w2, const float* b2, float ln_eps, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::token_transformer_block_launch(qkv, ld, y, workspace, B, T, scale, wo, bo, gamma, beta, w1, b1, w2, b2, ln_eps,
+                                             static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int evt_performer_fwd(const void* kqv, int64_t ld, const float* w, void* yattn, float* vout, void* workspace,
                                  int B, int T, int emb, int m, float eps, evt_stream stream) {
   int rc = evt_device_check();
@@ -880,6 +905,36 @@ int performer_block_launch(const void* kqv, int64_t ld, const float* w, float* y
   else
     performer_apply_kernel<true, EVT_ACT_GELU_TANH><<<grid, 128, 0, st>>>(kqv16, ld, w, stats, nullptr, y, T, eps, tw);
   EVT_LAUNCH_CHECK("performer_apply_tail");
+  return EVT_OK;
+}
+
+// Token_transformer (T2T-ViT, tokens_type='transformer') after its qkv projection, two launches:
+//   ctx = softmax(q k^T * scale) v      one head of 64 over all T tokens of an image (attention_long_kernel for T > 256)
+//   y   = v + proj(ctx);  y += fc2(gelu_erf(fc1(LayerNorm(y))))  the performer tail, v read from qkv columns [128, 192)
+size_t token_transformer_workspace_bytes(int B, int T) { return static_cast<size_t>(B) * T * kEmb * sizeof(__nv_bfloat16); }
+
+int token_transformer_block_launch(const void* qkv, int64_t ld, float* y, void* workspace, int B, int T, float scale, const void* wo,
+                                   const float* bo, const float* gamma, const float* beta, const void* w1, const float* b1, const void* w2,
+                                   const float* b2, float ln_eps, cudaStream_t st) {
+  EVT_CHECK_ARG(qkv && y && workspace && wo && gamma && beta && w1 && w2, "token_transformer_block: null pointer");
+  EVT_CHECK_ARG(B > 0 && T > 0 && B <= 65535, "token_transformer_block: B in 1..65535 and T > 0");
+  EVT_CHECK_ARG(ld >= 3 * kEmb && ld % 8 == 0 && reinterpret_cast<uintptr_t>(qkv) % 16 == 0,
+                "token_transformer_block: qkv rows must be 16-byte aligned with a leading dimension >= 192");
+  for (const void* p : {static_cast<const void*>(workspace), static_cast<const void*>(y), wo, w1, w2})
+    EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(p) % 16 == 0, "token_transformer_block: operands must be 16-byte aligned");
+  EVT_TRY(attention_any_length_launch(qkv, ld, workspace, kEmb, nullptr, B, T, T, 1, scale, st));
+  const long long rows = static_cast<long long>(B) * T;
+  const long long tiles = (rows + kTileTok - 1) / kTileTok;
+  const long long want = (tiles + 3) / 4;
+  const long long cap = static_cast<long long>(num_sms()) * 16;
+  const unsigned grid = static_cast<unsigned>(want < cap ? want : cap);
+  TailWeights tw;
+  tw.wo = reinterpret_cast<const __nv_bfloat16*>(wo), tw.w1 = reinterpret_cast<const __nv_bfloat16*>(w1), tw.w2 = reinterpret_cast<const __nv_bfloat16*>(w2);
+  tw.bo = bo, tw.gamma = gamma, tw.beta = beta, tw.b1 = b1, tw.b2 = b2, tw.eps = ln_eps;
+  const __nv_bfloat16* ctx = reinterpret_cast<const __nv_bfloat16*>(workspace);
+  const __nv_bfloat16* v = reinterpret_cast<const __nv_bfloat16*>(qkv);
+  performer_mlp_kernel<EVT_ACT_GELU_ERF, true><<<grid, 128, 0, st>>>(ctx, y, tw, rows, v, ld);
+  EVT_LAUNCH_CHECK("token_transformer_tail");
   return EVT_OK;
 }
 

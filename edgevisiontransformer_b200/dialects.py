@@ -139,28 +139,40 @@ T2T_TORCH_HEAD_SIZE = 64
 
 def t2t_torch_to_canonical(sd: Dict[str, torch.Tensor], qk_scale: Optional[float] = None, use_ema: bool = True
                            ) -> Tuple[Dict[str, torch.Tensor], dict]:
-    """PyTorch T2T-ViT (``T2T_ViT`` with ``tokens_type='performer'``) state dict or training checkpoint -> (canonical state
-    dict, from_state_dict kwargs).
+    """PyTorch T2T-ViT (``T2T_ViT`` with ``tokens_type='performer'`` or ``'transformer'``) state dict or training checkpoint ->
+    (canonical state dict, from_state_dict kwargs).  The token type is read from the keys.
 
-    * ``tokens_to_token.attention{1,2}.*`` -> ``t2t.performer{1,2}.*`` in the Keras naming the runtime loads (INTEGRATION.md
-      §3): kernels ``[in, out]``; the rows of ``kqv.kernel`` and of ``norm1.{gamma,beta}`` permuted from ``(c, kh, kw)`` to
-      ``(kh, kw, c)`` (stage 1: C = 3, k = 7; stage 2: C = 64, k = 3); ``w`` as stored (already times sqrt(m)).
+    * performer: ``tokens_to_token.attention{1,2}.*`` -> ``t2t.performer{1,2}.*`` in the Keras naming the runtime loads
+      (INTEGRATION.md §3): kernels ``[in, out]``; the rows of ``kqv.kernel`` and of ``norm1.{gamma,beta}`` permuted from
+      ``(c, kh, kw)`` to ``(kh, kw, c)`` (stage 1: C = 3, k = 7; stage 2: C = 64, k = 3); ``w`` as stored (already times
+      sqrt(m)).  ``t2t = 2``.
+    * transformer (``Token_transformer``, one head): -> ``t2t.transformer{1,2}.*``: ``norm1`` and the input rows of
+      ``qkv.kernel`` (from ``attn.qkv.weight``, which has no bias) permuted the same way, ``attn.proj`` -> ``attn_output``,
+      ``mlp.fc{1,2}`` -> ``mlp.fc{1,2}``.  The token attention's scale (in_dim ** -0.5) is the runtime's.  ``t2t = 3``.
     * ``tokens_to_token.project`` -> the token-embedding projection, its 576 input columns permuted the same way (C = 64, k = 3).
     * ``cls_token``, ``pos_embed`` (the sinusoid table stored in the checkpoint) -> the embeddings.
     * ``blocks.*``, ``norm.*``, ``head.*`` as in ``timm_vit_to_canonical``.  ``qk_scale`` (default head_size ** -0.5, the
       scale the runtime applies) is folded into the query rows.
-    Refuses ``tokens_type='transformer'`` checkpoints and any image size other than 224."""
+    Refuses a dict holding both token types, a ``Token_transformer`` with a qkv bias and any image size other than 224."""
     sd = unwrap_checkpoint(sd, use_ema)
-    if "tokens_to_token.attention1.attn.qkv.weight" in sd:
-        raise ValueError("tokens_type='transformer' T2T-ViT (t2t_vit_t_*) is not supported: its token attention runs over 3136 "
-                         "tokens, more than EVT_ATTN_MAX_TOKENS; only the performer checkpoints (t2t_vit_*) run here")
-    if "tokens_to_token.attention1.kqv.weight" not in sd or "blocks.0.attn.qkv.weight" not in sd:
-        raise ValueError("not a PyTorch T2T-ViT state dict (no tokens_to_token.attention1.kqv.weight or blocks.0.attn.qkv.weight)")
+    performer = "tokens_to_token.attention1.kqv.weight" in sd
+    transformer = "tokens_to_token.attention1.attn.qkv.weight" in sd
+    if performer and transformer:
+        raise ValueError("state dict mixes tokens_type='performer' (attention1.kqv) and tokens_type='transformer' (attention1.attn.qkv) "
+                         "token modules: not one T2T-ViT")
+    if not (performer or transformer) or "blocks.0.attn.qkv.weight" not in sd:
+        raise ValueError("not a PyTorch T2T-ViT state dict (no tokens_to_token.attention1.kqv.weight / .attn.qkv.weight or "
+                         "blocks.0.attn.qkv.weight)")
+    if transformer and any(f"tokens_to_token.attention{i}.attn.qkv.bias" in sd for i in (1, 2)):
+        raise ValueError("tokens_type='transformer' with a qkv bias: upstream's Token_transformer has none and it is not implemented")
     D = sd["cls_token"].shape[-1]
     if sd["pos_embed"].shape[-2] != 197:
         raise ValueError(f"pos_embed has {sd['pos_embed'].shape[-2]} rows: only the 224-pixel T2T-ViT (197 tokens) is supported")
     out: Dict[str, torch.Tensor] = {}
     for i, (C, k) in ((1, (3, 7)), (2, (64, 3))):
+        if transformer:
+            _token_transformer_to_canonical(sd, out, i, C, k)
+            continue
         s, d = f"tokens_to_token.attention{i}.", f"t2t.performer{i}."
         out[d + "norm1.gamma"] = _ckk_to_kkc(sd[s + "norm1.weight"], C, k)
         out[d + "norm1.beta"] = _ckk_to_kkc(sd[s + "norm1.bias"], C, k)
@@ -180,5 +192,24 @@ def t2t_torch_to_canonical(sd: Dict[str, torch.Tensor], qk_scale: Optional[float
     out["vit.layernorm.weight"], out["vit.layernorm.bias"] = sd["norm.weight"], sd["norm.bias"]
     out["classifier.weight"], out["classifier.bias"] = sd["head.weight"], sd["head.bias"]
     kw = dict(dialect="hf", hidden_act="gelu", layer_norm_eps=1e-5, final_ln=True, head_size=T2T_TORCH_HEAD_SIZE, patch_size=16,
-              image_size=224, embed_k=576, t2t=2)
+              image_size=224, embed_k=576, t2t=3 if transformer else 2)
     return out, kw
+
+
+T2T_TOKEN_DIM = 64
+
+
+def _token_transformer_to_canonical(sd: Dict[str, torch.Tensor], out: Dict[str, torch.Tensor], i: int, C: int, k: int) -> None:
+    """``tokens_to_token.attention{i}`` (a one-head ``Token_transformer``, token_dim 64) -> ``t2t.transformer{i}.*``."""
+    s, d = f"tokens_to_token.attention{i}.", f"t2t.transformer{i}."
+    w = sd[s + "attn.qkv.weight"]
+    if tuple(w.shape) != (3 * T2T_TOKEN_DIM, C * k * k):
+        raise ValueError(f"{s}attn.qkv.weight is {tuple(w.shape)}, expected ({3 * T2T_TOKEN_DIM}, {C * k * k}): only token_dim "
+                         f"{T2T_TOKEN_DIM} is implemented")
+    out[d + "norm1.gamma"] = _ckk_to_kkc(sd[s + "norm1.weight"], C, k)
+    out[d + "norm1.beta"] = _ckk_to_kkc(sd[s + "norm1.bias"], C, k)
+    out[d + "qkv.kernel"] = _ckk_to_kkc(w, C, k).t().contiguous()
+    for src, dst in (("attn.proj", "attn_output"), ("mlp.fc1", "mlp.fc1"), ("mlp.fc2", "mlp.fc2")):
+        out[d + dst + ".kernel"] = sd[s + src + ".weight"].t().contiguous()
+        out[d + dst + ".bias"] = sd[s + src + ".bias"]
+    out[d + "norm2.gamma"], out[d + "norm2.beta"] = sd[s + "norm2.weight"], sd[s + "norm2.bias"]

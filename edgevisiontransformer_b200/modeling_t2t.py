@@ -13,7 +13,9 @@ model-level C entry point ``evt_model_forward_embedded``.
 ``B200T2TViTTorch`` and ``t2t_vit_{7,10,12,14,19,24}`` run the published PyTorch checkpoints (yitu-opensource/T2T-ViT,
 ``tokens_type='performer'``; the files the reference's tools.py:347-365 loads): NCHW f32 / bf16 / uint8 pixels, the same
 front-end kernels with the stage-1 soft split reading planar pixels (``spec.t2t = 2``), erf-GELU performers and a pre-LN
-(HF-dialect) encoder.  Weights go through ``dialects.t2t_torch_to_canonical``.
+(HF-dialect) encoder.  Weights go through ``dialects.t2t_torch_to_canonical``.  The same class and ``t2t_vit_t_{14,19,24}`` run
+the ``tokens_type='transformer'`` checkpoints (``spec.t2t = 3``): each token stage is a one-head ``Token_transformer`` whose exact
+softmax attention runs over all 3136 (stage 1) or 784 (stage 2) tokens of an image.
 """
 from __future__ import annotations
 
@@ -170,9 +172,15 @@ def get_t2t_vit_7(sd, **kw):
 
 
 # ---------------------------------------------------------------------------------------------- PyTorch T2T-ViT checkpoints
-# upstream factories (models/t2t_vit.py): embed_dim, depth, num_heads, mlp_ratio
+# upstream factories (models/t2t_vit.py): embed_dim, depth, num_heads, mlp_ratio; t2t_vit_t_* are tokens_type='transformer'
 T2T_TORCH = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_12": (256, 12, 4, 2.0),
-             "t2t_vit_14": (384, 14, 6, 3.0), "t2t_vit_19": (448, 19, 7, 3.0), "t2t_vit_24": (512, 24, 8, 3.0)}
+             "t2t_vit_14": (384, 14, 6, 3.0), "t2t_vit_19": (448, 19, 7, 3.0), "t2t_vit_24": (512, 24, 8, 3.0),
+             "t2t_vit_t_14": (384, 14, 6, 3.0), "t2t_vit_t_19": (448, 19, 7, 3.0), "t2t_vit_t_24": (512, 24, 8, 3.0)}
+
+
+def tokens_type_of(sd: Dict[str, torch.Tensor]) -> str:
+    """'transformer' for a state dict with Token_transformer stages (tokens_to_token.attention1.attn.qkv), else 'performer'."""
+    return "transformer" if "tokens_to_token.attention1.attn.qkv.weight" in sd else "performer"
 
 
 def load_t2t_checkpoint(path) -> dict:
@@ -183,8 +191,8 @@ def load_t2t_checkpoint(path) -> dict:
 
 
 class B200T2TViTTorch(B200ViTForImageClassification):
-    """PyTorch ``T2T_ViT`` (``tokens_type='performer'``) on libevt: the whole forward, front-end included, is one C call per
-    chunk.  Input is NCHW ``[B, 3, 224, 224]`` in f32, bf16 or uint8 (uint8 is normalised with ``pixel_mean`` / ``pixel_std``
+    """PyTorch ``T2T_ViT`` (``tokens_type='performer'`` or ``'transformer'``, detected from the keys; ``tokens_type`` says which)
+    on libevt: the whole forward, front-end included, is one C call per chunk.  Input is NCHW ``[B, 3, 224, 224]`` in f32, bf16 or uint8 (uint8 is normalised with ``pixel_mean`` / ``pixel_std``
     inside the first soft split; the zero padding applies to the normalised image, as upstream pads the normalised tensor).
 
     ``checkpoint_or_sd``: a file path, a checkpoint dict (``state_dict_ema`` -- used unless ``use_ema=False`` --,
@@ -207,6 +215,7 @@ class B200T2TViTTorch(B200ViTForImageClassification):
                              f"{T2T_TORCH_HEAD_SIZE} is implemented")
         super().__init__(config_from_state_dict(csd, **kw), csd, device=device, max_batch=max_batch, keep_params=keep_params)
         self.num_heads, self.depth, self.hidden = nh, self.config.num_hidden_layers, D
+        self.tokens_type = "transformer" if kw["t2t"] == 3 else "performer"
 
     @classmethod
     def from_checkpoint(cls, path, **kw) -> "B200T2TViTTorch":
@@ -224,7 +233,9 @@ def _factory_of(sd: Dict[str, torch.Tensor]) -> Optional[str]:
     D, depth = sd["cls_token"].shape[-1], 0
     while f"blocks.{depth}.attn.qkv.weight" in sd:
         depth += 1
-    by_dim = [name for name, (d, _, _, _) in T2T_TORCH.items() if d == D]    # same heads, mlp ratio and qk_scale for one D
+    tt = tokens_type_of(sd) == "transformer"
+    by_dim = [name for name, (d, _, _, _) in T2T_TORCH.items()              # same heads, mlp ratio and qk_scale for one D
+              if d == D and ("_t_" in name) == tt]
     exact = [name for name in by_dim if T2T_TORCH[name][1] == depth]
     return (exact or by_dim or [None])[0]
 
@@ -233,6 +244,10 @@ def _t2t_factory(name: str, checkpoint_or_sd, **kw) -> B200T2TViTTorch:
     D, _, heads, ratio = T2T_TORCH[name]     # depth comes from the weights
     sd = load_t2t_checkpoint(checkpoint_or_sd) if isinstance(checkpoint_or_sd, (str, os.PathLike)) else checkpoint_or_sd
     sd = unwrap_checkpoint(sd, kw.get("use_ema", True))
+    want_tt = "transformer" if "_t_" in name else "performer"
+    if tokens_type_of(sd) != want_tt:
+        raise ValueError(f"{name} is a tokens_type='{want_tt}' T2T-ViT; the weights are tokens_type='{tokens_type_of(sd)}' "
+                         f"({'t2t_vit_t_*' if want_tt == 'performer' else 't2t_vit_*'} runs them)")
     if "cls_token" in sd and "blocks.0.mlp.fc1.weight" in sd:
         got = (sd["cls_token"].shape[-1], sd["blocks.0.mlp.fc1.weight"].shape[0])
         if got != (D, int(D * ratio)):
@@ -264,3 +279,15 @@ def t2t_vit_19(checkpoint_or_sd, **kw):
 
 def t2t_vit_24(checkpoint_or_sd, **kw):
     return _t2t_factory("t2t_vit_24", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_t_14(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_t_14", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_t_19(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_t_19", checkpoint_or_sd, **kw)
+
+
+def t2t_vit_t_24(checkpoint_or_sd, **kw):
+    return _t2t_factory("t2t_vit_t_24", checkpoint_or_sd, **kw)

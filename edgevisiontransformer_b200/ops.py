@@ -411,6 +411,30 @@ def performer_block(kqv: torch.Tensor, w: torch.Tensor, B: int, T: int, wo, bo, 
     return y
 
 
+def token_transformer_block(qkv: torch.Tensor, B: int, T: int, scale: float, wo, bo, gamma, beta, w1, b1, w2, b2,
+                            ln_eps: float) -> torch.Tensor:
+    """T2T-ViT ``Token_transformer`` after its qkv projection, in two launches: ctx = softmax(q k^T * scale) v over all T tokens
+    of an image (one head of 64, any T), y = v + proj(ctx); y += fc2(gelu_erf(fc1(LayerNorm(y)))).
+    qkv bf16 [B*T, >=192] (q | k | v) -> y f32 [B*T, 64]."""
+    _need_cuda(qkv, wo, bo, gamma, beta, w1, b1, w2, b2)
+    if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.shape[0] != B * T or qkv.stride(1) != 1:
+        raise ValueError("token_transformer_block wants a bf16 [B*T, 192] qkv matrix")
+    for m in (wo, w1, w2):
+        if m.dtype != torch.bfloat16 or tuple(m.shape) != (64, 64) or not m.is_contiguous():
+            raise ValueError("token_transformer_block: weights must be contiguous bf16 [64, 64]")
+    import ctypes as C
+    lib = _lib.load()
+    n = C.c_size_t()
+    _lib.check(lib.evt_token_transformer_workspace_bytes(B, T, C.byref(n)), "token_transformer_workspace_bytes")
+    ws = torch.empty(n.value, dtype=torch.uint8, device=qkv.device)
+    y = torch.empty((B * T, 64), dtype=torch.float32, device=qkv.device)
+    _lib.check(lib.evt_token_transformer_block_fwd(qkv.data_ptr(), qkv.stride(0), y.data_ptr(), ws.data_ptr(), B, T, float(scale),
+                                                   wo.data_ptr(), _ptr(bo), gamma.contiguous().data_ptr(), beta.contiguous().data_ptr(),
+                                                   w1.data_ptr(), _ptr(b1), w2.data_ptr(), _ptr(b2), float(ln_eps), _stream()),
+               "token_transformer_block")
+    return y
+
+
 def set_gemm_pair_mode(mode: int) -> None:
     """-1 automatic, 0 single-CTA GEMM kernel only, 1 CTA-pair (cta_group::2) kernel whenever applicable."""
     _lib.load().evt_gemm_set_pair_mode(int(mode))

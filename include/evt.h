@@ -239,6 +239,20 @@ int evt_performer_block_fwd(const void* kqv, int64_t ld, const float* w, float* 
                             const void* wo, const float* bo, const float* gamma, const float* beta, const void* w1,
                             const float* b1, const void* w2, const float* b2, float ln_eps, evt_stream stream);
 
+/* T2T-ViT Token_transformer (tokens_type='transformer', one head, token_dim 64) after its qkv projection, two launches:
+ *   ctx = softmax(q k^T * scale) v   exact attention over all T tokens of an image (any T >= 1, not capped by
+ *                                    EVT_ATTN_MAX_TOKENS: the T2T stages run T = 3136 and 784)
+ *   y   = v + proj(ctx);  y += fc2(gelu_erf(fc1(LayerNorm(y))))
+ *   qkv   : bf16 [B*T, ld], q | k | v in columns [0,64) [64,128) [128,192) (no bias); ld >= 192, multiple of 8
+ *   y     : f32 [B*T, 64] out (token-major: the layout the next soft split reads)
+ *   scale : Attention.scale, upstream in_dim ** -0.5 (147 ** -0.5, 576 ** -0.5)
+ *   wo, w1, w2 : bf16 [64 out, 64 in] dense;  bo, b1, b2 : f32 [64] or NULL;  gamma, beta : f32 [64] (norm2)
+ *   workspace  : evt_token_transformer_workspace_bytes(B, T) bytes (the bf16 context), 16-byte aligned. */
+int evt_token_transformer_workspace_bytes(int B, int T, size_t* out);
+int evt_token_transformer_block_fwd(const void* qkv, int64_t ld, float* y, void* workspace, int B, int T, float scale,
+                                    const void* wo, const float* bo, const float* gamma, const float* beta, const void* w1,
+                                    const float* b1, const void* w2, const float* b2, float ln_eps, evt_stream stream);
+
 /* ---- Swin shifted-window block (tools.py:265-292 export_onnx_swin, utils.py:14-47 get_swin; arithmetic:
  * SITE/models/swin/modeling_swin.py).  Token rows are kept in the window order of the current block, see
  * edgevisiontransformer_b200/modeling_swin.py. */
@@ -302,7 +316,8 @@ typedef struct evt_model_spec {
   int final_ln;                /* 1: LayerNorm before the head (HF, T2T); 0: TF-dialect DeiT */
   int head_hidden;             /* 0: single Linear head; >0: Dense(head_hidden, gelu)->Dense */
   int t2t;                     /* T2T front-end instead of the patch embed: 1 NHWC f32 pixels (TF T2T); 2 NCHW
-                                  f32 / bf16 / u8 pixels, the PyTorch T2T (stage-1 columns in (kh, kw, c) order); 0 none */
+                                  f32 / bf16 / u8 pixels, the PyTorch T2T (stage-1 columns in (kh, kw, c) order); 3 as 2
+                                  with Token_transformers (t2t_vit_t_*) instead of performers; 0 none */
   int precision;               /* evt_precision: 0 bf16 operands, 1 tf32 operands (f32 activations) */
   int embed_k;                 /* 0: 3*patch*patch.  >0: K of the token-embedding GEMM when the caller builds the
                                   patch matrix itself (T2T: 3*3*64 = 576) and calls evt_model_forward_embedded */
