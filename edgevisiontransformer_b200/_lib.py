@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EVT_LIB_PATH") or os.path.join(HERE, "libevt.so")   # EVT_LIB_PATH: A/B a differently built library
 
 EVT_OK, EVT_ERR_INVALID, EVT_ERR_CUDA, EVT_ERR_UNSUPPORTED, EVT_ERR_STATE = 0, -1, -2, -3, -4
-EVT_F32, EVT_BF16 = 0, 1
+EVT_F32, EVT_BF16, EVT_TF32 = 0, 1, 2
 ACT_NONE, ACT_GELU_ERF, ACT_GELU_TANH = 0, 1, 2
 DIALECT_HF, DIALECT_TF = 0, 1
 PREC_BF16, PREC_TF32 = 0, 1
@@ -48,7 +48,7 @@ SWIN_MAX_STAGES = 8
 class SwinSpec(C.Structure):
     _fields_ = [("image", C.c_int), ("patch", C.c_int), ("window", C.c_int), ("embed_dim", C.c_int), ("stages", C.c_int),
                 ("depths", C.c_int * SWIN_MAX_STAGES), ("heads", C.c_int * SWIN_MAX_STAGES), ("num_labels", C.c_int),
-                ("eps", C.c_float)]
+                ("eps", C.c_float), ("precision", C.c_int)]
 
 
 class TensorView(C.Structure):
@@ -71,6 +71,7 @@ SIGNATURES = {
     "evt_layernorm2d_fwd": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _f, _p]),
     "evt_gemm_bias_act": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _i, _p, _i, _i64, _i, _i, _i, _i64, _i, _i, _i, _p]),
     "evt_gemm_bias_act_tf32": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _i, _p, _i64, _i, _i, _i, _i64, _i, _i, _i, _p]),
+    "evt_gemm_bias_act_tf32_ex": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _i, _p, _i, _i64, _i, _i, _i, _i64, _i, _i, _i, _p]),
     "evt_layernorm_gemm": (_i, [_p, _i64, _p, _p, _f, _p, _p, _i64, _p, _p, _i64, _i64, _i, _i, _i, _p]),
     "evt_gemm_residual_layernorm": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _p, _p, _f, _p, _i64, _i64, _i, _i, _p]),
     "evt_gemm_residual_layernorm_ex": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _p, _p, _f, _i, _p, _i64, _i64, _i, _i, _p]),
@@ -78,6 +79,7 @@ SIGNATURES = {
     "evt_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _f, _p]),
     "evt_attention_query_rows_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _i, _f, _p]),
     "evt_im2col_patch": (_i, [_p, _p, _i, _i, _i, _i, _p]),
+    "evt_im2col_patch_ex": (_i, [_p, _p, _i, _i, _i, _i, _i, _p]),
     "evt_patch_embed_workspace_bytes": (_i, [_i, _i, _i, _i, _i, C.POINTER(C.c_size_t)]),
     "evt_patch_embed_fwd": (_i, [_p, _i, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p]),
     "evt_prefix_tokens": (_i, [_p, _p, _p, _i, _i, _i, _i, _p]),
@@ -85,7 +87,9 @@ SIGNATURES = {
     "evt_unfold_nhwc": (_i, [_p, _i, _p, _i64, _i, _i, _i, _i, _i, _i, _i, _p]),
     "evt_gather_layernorm": (_i, [_p, _p, _p, _p, _p, _i, _p, _i64, _i, _i, _i, _i, _f, _p]),
     "evt_window_attention_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i64, _i, _i, _i, _f, _p]),
+    "evt_window_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i64, _i, _i, _i, _f, _p]),
     "evt_layernorm_mean_tokens": (_i, [_p, _p, _p, _p, _i64, _i, _i, _f, _p]),
+    "evt_layernorm_mean_tokens_ex": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _f, _p]),
     "evt_model_create": (_i, [C.POINTER(ModelSpec), C.POINTER(_p)]),
     "evt_model_load_weights": (_i, [_p, C.POINTER(TensorView), _i, _p]),
     "evt_model_workspace_bytes": (_i, [_p, _i, C.POINTER(_sz)]),

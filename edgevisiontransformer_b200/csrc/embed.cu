@@ -188,9 +188,10 @@ int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, cons
   const int in_bytes = pixel_dtype == EVT_PIX_F32 ? 4 : pixel_dtype == EVT_PIX_BF16 ? 2 : 1;
   EVT_CHECK_ARG(pixel_dtype == EVT_PIX_F32 || pixel_dtype == EVT_PIX_BF16 || pixel_dtype == EVT_PIX_U8, "im2col: unknown pixel dtype");
   EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(pixels) % (8 * in_bytes) == 0, "im2col: pixel pointer must be aligned to 8 pixels");
-  if (P % 8 != 0 && P % 4 == 0 && out_dtype == EVT_BF16 && row_off == 0 && pixel_dtype == EVT_PIX_F32)
-    return im2col4_launch(reinterpret_cast<const float*>(pixels), cols, B, H, W, P, st);  // Swin: P = 4
-  EVT_CHECK_ARG(P % 8 == 0 && W % 8 == 0, "im2col: patch width must be a multiple of 8 (f32 pixels, bf16 output: of 4)");
+  // out_dtype: EVT_BF16, or f32 rounded to tf32 (EVT_TF32; EVT_F32 means the same here: the patch matrix feeds a tf32 GEMM)
+  if (P % 8 != 0 && P % 4 == 0 && row_off == 0 && pixel_dtype == EVT_PIX_F32)  // Swin: P = 4
+    return im2col4_launch(reinterpret_cast<const float*>(pixels), cols, out_dtype == EVT_BF16 ? EVT_BF16 : EVT_TF32, B, H, W, P, st);
+  EVT_CHECK_ARG(P % 8 == 0 && W % 8 == 0, "im2col: patch width must be a multiple of 8 (f32 pixels: of 4)");
   PixAffine af = {{1.f, 1.f, 1.f}, {0.f, 0.f, 0.f}};
   if (pixel_dtype == EVT_PIX_U8) {
     EVT_CHECK_ARG(scale3 && bias3, "im2col: u8 pixels need a per-channel scale and bias");
@@ -262,6 +263,12 @@ extern "C" int evt_im2col_patch(const float* pixels, void* cols, int B, int H, i
   int rc = evt_device_check();
   if (rc != EVT_OK) return rc;
   return evt::im2col_launch(pixels, EVT_PIX_F32, nullptr, nullptr, cols, EVT_BF16, B, H, W, P, static_cast<cudaStream_t>(stream));
+}
+extern "C" int evt_im2col_patch_ex(const float* pixels, void* cols, int out_dtype, int B, int H, int W, int P, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  EVT_CHECK_ARG(out_dtype == EVT_BF16 || out_dtype == EVT_TF32, "im2col: out dtype must be bf16 or tf32");
+  return evt::im2col_launch(pixels, EVT_PIX_F32, nullptr, nullptr, cols, out_dtype, B, H, W, P, static_cast<cudaStream_t>(stream));
 }
 // ViTEmbeddings.forward as ONE op-level call (SURVEY.md section 8 rows a1 + a2): the same three launches the model runtime
 // issues -- patch gather with one row per TOKEN (prefix rows zero), residual rows preset to pos + (prefix token | conv bias),

@@ -404,3 +404,17 @@ extern "C" int evt_gemm_bias_act_tf32(const float* A, int64_t lda, const float* 
                            .map = {.res_row_mod = res_row_mod, .res_row_off = res_row_off, .out_group = out_group, .out_group_stride = out_group_stride,
                                     .out_group_off = out_group_off}}, static_cast<cudaStream_t>(stream));
 }
+
+// tf32 flavour with a choice of output: EVT_F32, or EVT_TF32 (f32 rounded to nearest tf32, for an output that feeds another tf32 op).
+extern "C" int evt_gemm_bias_act_tf32_ex(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
+                                         const float* residual, int64_t ldr, int res_row_mod, int res_row_off, float* out, int out_dtype,
+                                         int64_t ldo, int out_group, int out_group_stride, int out_group_off, int64_t M, int N, int K,
+                                         int act, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  EVT_CHECK_ARG(out_dtype == EVT_F32 || out_dtype == EVT_TF32, "gemm_tf32: out dtype must be f32 or tf32");
+  return evt::gemm_launch({.A = A, .lda = lda, .W = W, .ldw = ldw, .in_dtype = EVT_F32, .bias = bias, .residual = residual, .ldr = ldr,
+                           .out = out, .out_dtype = out_dtype, .ldo = ldo, .M = M, .N = N, .K = K, .act = act,
+                           .map = {.res_row_mod = res_row_mod, .res_row_off = res_row_off, .out_group = out_group, .out_group_stride = out_group_stride,
+                                    .out_group_off = out_group_off}}, static_cast<cudaStream_t>(stream));
+}

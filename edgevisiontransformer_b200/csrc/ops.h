@@ -63,14 +63,17 @@ int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, cons
                   int H, int W, int P, cudaStream_t st, int row_stride = 0, int row_off = 0);
 int embed_fill_launch(const float* prefix, const float* pos, const float* bias, float* out, int B, int tokens, int n_prefix, int D,
                       cudaStream_t st);
-int im2col4_launch(const float* pixels, void* cols, int B, int H, int W, int P, cudaStream_t st);  // swin.cu, P % 4 == 0
-// swin.cu: evt_gather_layernorm, evt_window_attention_fwd and evt_layernorm_mean_tokens without the device check
+// swin.cu, P % 4 == 0; out_dtype EVT_BF16 or EVT_TF32
+int im2col4_launch(const float* pixels, void* cols, int out_dtype, int B, int H, int W, int P, cudaStream_t st);
+// swin.cu: evt_gather_layernorm, evt_window_attention_fwd(_tf32) and evt_layernorm_mean_tokens_ex without the device check
 int gather_layernorm_launch(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype, float* copy_f32,
                             int64_t images, int T_in, int T_out, int G, int C, float eps, cudaStream_t st);
 int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
                             int window_tokens, int heads, int head_size, float scale, cudaStream_t st);
-int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
-                                 cudaStream_t st);
+int window_attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                                 int window_tokens, int heads, int head_size, float scale, cudaStream_t st);
+int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T, int D,
+                                 float eps, cudaStream_t st);
 int prefix_tokens_launch(const float* prefix, const float* pos, float* out, int B, int tokens, int n_prefix, int D,
                          cudaStream_t st);
 int cast_launch(const float* x, void* y, int64_t n, cudaStream_t st);

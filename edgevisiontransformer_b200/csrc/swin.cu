@@ -18,6 +18,7 @@
 //                             windows per tile was measured slower, DESIGN.md).
 //   window_attention144_kernel the same for 12 x 12 windows (144 tokens, swin_*_window12_384); K and V fragments are
 //                             re-read from shared memory per query m-tile instead of held in registers.
+//   window_attention_tf32_kernel the tf32 accuracy mode of both (f32 q / k / v / context, mma.sync m16n8k8 tf32).
 //   ln_mean_tokens_kernel     final LayerNorm + average pool over the tokens of an image (SwinModel.layernorm + pooler).
 #include <cuda_bf16.h>
 #include <math_constants.h>
@@ -146,6 +147,9 @@ int launch_gather_ln_sub(const float* x, const int* idx, const float* gamma, con
   if (y_dtype == EVT_BF16)
     EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, EVT_BF16>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
                         T_in, T_out, eps));
+  else if (y_dtype == EVT_TF32)
+    EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, EVT_TF32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
+                        T_in, T_out, eps));
   else
     EVT_CUDA(launch_pdl(gather_ln_sub_kernel<LPR, NV, EVT_F32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out,
                         T_in, T_out, eps));
@@ -160,6 +164,9 @@ int launch_gather_ln(const float* x, const int* idx, const float* gamma, const f
   const bool pdl = pdl_for_work(rows_out, static_cast<long long>(G) * C);
   if (y_dtype == EVT_BF16)
     EVT_CUDA(launch_pdl(gather_ln_kernel<NV, EVT_BF16>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
+                        T_out, G, C, eps));
+  else if (y_dtype == EVT_TF32)
+    EVT_CUDA(launch_pdl(gather_ln_kernel<NV, EVT_TF32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
                         T_out, G, C, eps));
   else
     EVT_CUDA(launch_pdl(gather_ln_kernel<NV, EVT_F32>, dim3(grid), dim3(256), 0, st, pdl, x, idx, gamma, beta, y, copy, rows_out, T_in,
@@ -185,16 +192,24 @@ constexpr int kW12MatBytes = kW12Tok * kWHd * 2;  // 9 KB
 // eight 16-byte rows an ldmatrix phase reads fall into eight different bank groups
 __device__ __forceinline__ uint32_t wofs(int row, int chunk) { return row * 64 + ((chunk ^ ((row >> 1) & 3)) << 4); }
 
+// tf32 kernel: byte offset of (row, 16-byte chunk) in a [rows][128 bytes] f32 matrix: chunk c stored at c ^ f(row),
+// f(row) = (row & 6) ^ ((row & 1) << 2).  The 128-bit loads of window_attention_tf32_kernel run in phases of 8 lanes: Q / K
+// rows R + 2p, R + 2p + 1 (R % 8 == 0) at chunks 4j + t, and V rows 8nt + 2t (or + 1) at chunks 2p, 2p + 1; either way the 8
+// lanes of a phase hit 8 different bank groups.
+__device__ __forceinline__ uint32_t wofs32(int row, int chunk) { return row * 128 + ((chunk ^ (row & 6) ^ ((row & 1) << 2)) << 4); }
+
 // cp.async the q, k and v slices of head h of the window whose first row is row0 (TOK rows each) into the warp's three
-// swizzled matrices at aQ, aQ + MAT, aQ + 2 MAT, and wait for them
-template <int TOK, int MAT>
-__device__ __forceinline__ void stage_window(const __nv_bfloat16* __restrict__ qkv, long long ldq, long long row0, int C, int h,
+// swizzled matrices at aQ, aQ + MAT, aQ + 2 MAT, and wait for them; T = __nv_bfloat16 (wofs layout) or float (wofs32)
+template <typename T, int TOK, int MAT>
+__device__ __forceinline__ void stage_window(const T* __restrict__ qkv, long long ldq, long long row0, int C, int h,
                                              uint32_t aQ, int lane) {
-  for (int c = lane; c < 3 * TOK * 4; c += 32) {
-    const int mat = c / (TOK * 4), rc = c - mat * (TOK * 4);
-    const int row = rc >> 2, ch = rc & 3;
-    const __nv_bfloat16* src = qkv + (row0 + row) * ldq + mat * C + h * kWHd + ch * 8;
-    const uint32_t dst = aQ + mat * MAT + wofs(row, ch);
+  constexpr int CPR = kWHd * static_cast<int>(sizeof(T)) / 16;  // 16-byte chunks per row: 4 (bf16) or 8 (f32)
+  constexpr int LOG = CPR == 4 ? 2 : 3;
+  for (int c = lane; c < 3 * TOK * CPR; c += 32) {
+    const int mat = c / (TOK * CPR), rc = c - mat * (TOK * CPR);
+    const int row = rc >> LOG, ch = rc & (CPR - 1);
+    const T* src = qkv + (row0 + row) * ldq + mat * C + h * kWHd + ch * (16 / static_cast<int>(sizeof(T)));
+    const uint32_t dst = aQ + mat * MAT + (CPR == 4 ? wofs(row, ch) : wofs32(row, ch));
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
   }
   asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
@@ -274,7 +289,7 @@ __global__ void __launch_bounds__(kWWarps * 32) window_attention_kernel(const __
     const int h = static_cast<int>(item - w * heads);
     const long long row0 = w * kWTok;
     __syncwarp();  // every lane is done with the previous item's shared memory
-    stage_window<kWTok, kWMatBytes>(qkv, ldq, row0, C, h, aQ, lane);
+    stage_window<__nv_bfloat16, kWTok, kWMatBytes>(qkv, ldq, row0, C, h, aQ, lane);
     __syncwarp();
     // K fragments (B operand of S = Q K^T): n-tile nt = keys 8 nt .. 8 nt + 7; registers {ks0.b0, ks0.b1, ks1.b0, ks1.b1}
     uint32_t kb[7][4];
@@ -351,7 +366,7 @@ __global__ void __launch_bounds__(kW12Warps * 32) window_attention144_kernel(con
     const int h = static_cast<int>(item - w * heads);
     const long long row0 = w * kW12Tok;
     __syncwarp();  // every lane is done with the previous item's shared memory
-    stage_window<kW12Tok, kW12MatBytes>(qkv, ldq, row0, C, h, aQ, lane);
+    stage_window<__nv_bfloat16, kW12Tok, kW12MatBytes>(qkv, ldq, row0, C, h, aQ, lane);
     __syncwarp();
     const float* tb = tab + ((w % n_tab) * heads + h) * static_cast<long long>(kW12Tok * kW12Tok);
 #pragma unroll 1
@@ -397,12 +412,133 @@ __global__ void __launch_bounds__(kW12Warps * 32) window_attention144_kernel(con
   }
 }
 
+// tf32 accuracy mode of the two kernels above, both window sizes: f32 q / k / v in, f32 context out, one warp per (window,
+// head), mma.sync m16n8k8 tf32 with f32 accumulation, K and V fragments read from shared memory per query m-tile.  The
+// arithmetic is that of attention_tf32_kernel (attention.cu): scores in f32 from the tf32 operands, exp2f (not the approx
+// instruction), every probability rounded to tf32 before P V and the row sum taken over the rounded values, the context
+// divided by that sum and rounded to tf32 on store.  q / k / v are expected tf32-representable (the QKV GEMM rounds its
+// output); the tensor core would truncate the low mantissa bits otherwise.
+// Fragment orders (any consistent permutation of a contraction index is free):
+//   S = Q K^T   k-step 2j reads head dims 16j + 4t + {0, 1} as its columns t / t + 4, k-step 2j + 1 dims 16j + 4t + {2, 3}:
+//               one 128-bit load gives a lane its Q (or K) values of two k-steps.
+//   O = P V     the S accumulator of n-tile nt holds keys 8nt + 2t, 8nt + 2t + 1 in registers 0 / 1 (2 / 3: row g + 8).  Used
+//               as they are as the A fragment of k-step nt, its columns t / t + 4 are those two keys, so the B fragment reads
+//               V rows 8nt + 2t and 8nt + 2t + 1: no shuffles.  Column g of n-tile n of O is head dim 4g + n, so one 128-bit
+//               load gives a lane its B values of all four n-tiles, and it ends up holding dims 8t .. 8t + 3 (register 0 of
+//               n = 0..3) and 8t + 4 .. 8t + 7 (register 1) of its rows: two 16-byte stores per row.
+// TOK = window tokens, ROWS = rows per matrix in shared memory (TOK rounded up to m16; rows TOK.. are zero), NT = key n-tiles;
+// the table is [n_tab, heads, ROWS, 8 NT] (window_table_shape).
+template <int TOK, int ROWS, int NT>
+__global__ void __launch_bounds__(kWWarps * 32) window_attention_tf32_kernel(const float* __restrict__ qkv, long long ldq,
+                                                                             float* __restrict__ ctx, long long ldc,
+                                                                             const float* __restrict__ tab, int n_tab, int heads,
+                                                                             long long n_items, float scale_log2e) {
+  constexpr int MAT = ROWS * kWHd * 4, MT = ROWS / 16, TCOLS = NT * 8;
+  extern __shared__ __align__(128) uint8_t wsm[];
+  ptx::grid_dep_launch();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint8_t* sQ = wsm + warp * 3 * MAT;
+  const uint8_t* sK = sQ + MAT;
+  const uint8_t* sV = sK + MAT;
+  // zero rows TOK..ROWS-1 once (cp.async never touches them): P = 0 there must meet finite V, padded K rows only feed
+  // columns the table masks, padded Q rows are not stored
+  if constexpr (ROWS > TOK) {
+    for (int i = lane; i < 3 * (ROWS - TOK) * 8; i += 32) {
+      const int mat = i / ((ROWS - TOK) * 8), rc = i % ((ROWS - TOK) * 8);
+      *reinterpret_cast<uint4*>(wsm + warp * 3 * MAT + mat * MAT + (TOK + rc / 8) * 128 + (rc % 8) * 16) = make_uint4(0, 0, 0, 0);
+    }
+  }
+  ptx::grid_dep_wait();
+  const int C = heads * kWHd;
+  const int g = lane >> 2, t = lane & 3;
+  const uint32_t aQ = ptx::smem_u32(sQ);
+  auto ld4 = [](const uint8_t* m, int row, int chunk) { return *reinterpret_cast<const float4*>(m + wofs32(row, chunk)); };
+  for (long long item = static_cast<long long>(blockIdx.x) * kWWarps + warp; item < n_items;
+       item += static_cast<long long>(gridDim.x) * kWWarps) {
+    const long long w = item / heads;
+    const int h = static_cast<int>(item - w * heads);
+    const long long row0 = w * TOK;
+    __syncwarp();  // every lane is done with the previous item's shared memory
+    stage_window<float, TOK, MAT>(qkv, ldq, row0, C, h, aQ, lane);
+    __syncwarp();
+    const float* tb = tab + ((w % n_tab) * heads + h) * static_cast<long long>(ROWS * TCOLS);
+#pragma unroll 1
+    for (int mt = 0; mt < MT; ++mt) {
+      uint32_t qa[4][4];  // A fragments of the four k-steps over the 32 head dims
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        const float4 lo = ld4(sQ, mt * 16 + g, 4 * j + t), hi = ld4(sQ, mt * 16 + g + 8, 4 * j + t);
+        qa[2 * j][0] = __float_as_uint(lo.x), qa[2 * j][1] = __float_as_uint(hi.x);
+        qa[2 * j][2] = __float_as_uint(lo.y), qa[2 * j][3] = __float_as_uint(hi.y);
+        qa[2 * j + 1][0] = __float_as_uint(lo.z), qa[2 * j + 1][1] = __float_as_uint(hi.z);
+        qa[2 * j + 1][2] = __float_as_uint(lo.w), qa[2 * j + 1][3] = __float_as_uint(hi.w);
+      }
+      float s[NT][4];
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) {
+        s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const float4 k = ld4(sK, nt * 8 + g, 4 * j + t);
+          ptx::mma_tf32_1688(s[nt], qa[2 * j], __float_as_uint(k.x), __float_as_uint(k.y));
+          ptx::mma_tf32_1688(s[nt], qa[2 * j + 1], __float_as_uint(k.z), __float_as_uint(k.w));
+        }
+      }
+      const float* t0 = tb + (mt * 16 + g) * TCOLS + 2 * t;
+      float m0, m1;
+      scores_rowmax<NT>(s, t0, t0 + 8 * TCOLS, scale_log2e, m0, m1);
+      float l0 = 0.f, l1 = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) {
+        s[nt][0] = ptx::round_tf32(exp2f(s[nt][0] - m0));
+        s[nt][1] = ptx::round_tf32(exp2f(s[nt][1] - m0));
+        s[nt][2] = ptx::round_tf32(exp2f(s[nt][2] - m1));
+        s[nt][3] = ptx::round_tf32(exp2f(s[nt][3] - m1));
+        l0 += s[nt][0] + s[nt][1];
+        l1 += s[nt][2] + s[nt][3];
+      }
+      l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
+      l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+      l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
+      l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+      float o[4][4];
+#pragma unroll
+      for (int n = 0; n < 4; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) {
+        const uint32_t pa[4] = {__float_as_uint(s[nt][0]), __float_as_uint(s[nt][2]), __float_as_uint(s[nt][1]), __float_as_uint(s[nt][3])};
+        const float4 v0 = ld4(sV, nt * 8 + 2 * t, g), v1 = ld4(sV, nt * 8 + 2 * t + 1, g);
+        ptx::mma_tf32_1688(o[0], pa, __float_as_uint(v0.x), __float_as_uint(v1.x));
+        ptx::mma_tf32_1688(o[1], pa, __float_as_uint(v0.y), __float_as_uint(v1.y));
+        ptx::mma_tf32_1688(o[2], pa, __float_as_uint(v0.z), __float_as_uint(v1.z));
+        ptx::mma_tf32_1688(o[3], pa, __float_as_uint(v0.w), __float_as_uint(v1.w));
+      }
+      const float i0 = 1.0f / l0, i1 = 1.0f / l1;  // l >= 1: the row maximum contributes 2^0
+      const int r0 = mt * 16 + g, r1 = r0 + 8;
+      float* d0 = ctx + (row0 + r0) * ldc + h * kWHd + 8 * t;
+      float* d1 = d0 + 8 * ldc;
+      if (ROWS == TOK || r0 < TOK) {
+        *reinterpret_cast<float4*>(d0) = make_float4(ptx::round_tf32(o[0][0] * i0), ptx::round_tf32(o[1][0] * i0),
+                                                     ptx::round_tf32(o[2][0] * i0), ptx::round_tf32(o[3][0] * i0));
+        *reinterpret_cast<float4*>(d0 + 4) = make_float4(ptx::round_tf32(o[0][1] * i0), ptx::round_tf32(o[1][1] * i0),
+                                                         ptx::round_tf32(o[2][1] * i0), ptx::round_tf32(o[3][1] * i0));
+      }
+      if (ROWS == TOK || r1 < TOK) {
+        *reinterpret_cast<float4*>(d1) = make_float4(ptx::round_tf32(o[0][2] * i1), ptx::round_tf32(o[1][2] * i1),
+                                                     ptx::round_tf32(o[2][2] * i1), ptx::round_tf32(o[3][2] * i1));
+        *reinterpret_cast<float4*>(d1 + 4) = make_float4(ptx::round_tf32(o[0][3] * i1), ptx::round_tf32(o[1][3] * i1),
+                                                         ptx::round_tf32(o[2][3] * i1), ptx::round_tf32(o[3][3] * i1));
+      }
+    }
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------- final LN + pool
 // One CTA (8 warps) per image: every warp normalises tokens warp, warp + 8, ... and accumulates them; the warps' sums meet
-// in shared memory.  D % 4 == 0, D <= 128 * NV.
-template <int NV>
+// in shared memory.  D % 4 == 0, D <= 128 * NV.  y: bf16 (OUT = EVT_BF16) or f32 rounded to tf32 (EVT_TF32).
+template <int NV, int OUT>
 __global__ void __launch_bounds__(256) ln_mean_tokens_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                             const float* __restrict__ beta, __nv_bfloat16* __restrict__ y,
+                                                             const float* __restrict__ beta, void* __restrict__ y,
                                                              int T, int D, float eps) {
   __shared__ float acc_s[8][128 * NV];
   ptx::grid_dep_launch();
@@ -453,14 +589,18 @@ __global__ void __launch_bounds__(256) ln_mean_tokens_kernel(const float* __rest
     float s = 0.f;
 #pragma unroll
     for (int w8 = 0; w8 < 8; ++w8) s += acc_s[w8][c];
-    y[static_cast<long long>(blockIdx.x) * D + c] = __float2bfloat16_rn(s * inv_t * gamma[c] + beta[c]);
+    const float o = s * inv_t * gamma[c] + beta[c];
+    if (OUT == EVT_BF16) reinterpret_cast<__nv_bfloat16*>(y)[static_cast<long long>(blockIdx.x) * D + c] = __float2bfloat16_rn(o);
+    else reinterpret_cast<float*>(y)[static_cast<long long>(blockIdx.x) * D + c] = ptx::round_tf32(o);
   }
 }
 
 // ---------------------------------------------------------------------------------------------------- im2col, P % 4 == 0
-// One thread = 4 consecutive pixels of one image row (16 B in, 8 B out); same (c, i, j) K order as im2col_kernel.
-__global__ void __launch_bounds__(256) im2col4_kernel(const float* __restrict__ px, __nv_bfloat16* __restrict__ cols, int H,
-                                                      int W, int P, long long total) {
+// One thread = 4 consecutive pixels of one image row (16 B in, 8 B of bf16 or 16 B of tf32-rounded f32 out); same (c, i, j)
+// K order as im2col_kernel.
+template <bool OUT_BF16>
+__global__ void __launch_bounds__(256) im2col4_kernel(const float* __restrict__ px, void* __restrict__ cols, int H, int W, int P,
+                                                      long long total) {
   ptx::grid_dep_launch();
   ptx::grid_dep_wait();
   const long long tid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -477,18 +617,24 @@ __global__ void __launch_bounds__(256) im2col4_kernel(const float* __restrict__ 
   const int py = y / P, i = y % P, pxi = x / P, j = x % P;
   const long long row = (b * (H / P) + py) * (W / P) + pxi;
   const int k = (c * P + i) * P + j;
-  uint2 o;
-  o.x = ptx::pack_bf16x2(v.x, v.y);
-  o.y = ptx::pack_bf16x2(v.z, v.w);
-  *reinterpret_cast<uint2*>(cols + row * (3ll * P * P) + k) = o;
+  if (OUT_BF16) {
+    uint2 o;
+    o.x = ptx::pack_bf16x2(v.x, v.y);
+    o.y = ptx::pack_bf16x2(v.z, v.w);
+    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(cols) + row * (3ll * P * P) + k) = o;
+  } else {
+    *reinterpret_cast<float4*>(reinterpret_cast<float*>(cols) + row * (3ll * P * P) + k) =
+        make_float4(ptx::round_tf32(v.x), ptx::round_tf32(v.y), ptx::round_tf32(v.z), ptx::round_tf32(v.w));
+  }
 }
 
 }  // namespace
 
-int im2col4_launch(const float* pixels, void* cols, int B, int H, int W, int P, cudaStream_t st) {
+int im2col4_launch(const float* pixels, void* cols, int out_dtype, int B, int H, int W, int P, cudaStream_t st) {
   const long long total = static_cast<long long>(B) * 3 * H * (W / 4);
-  EVT_CUDA(launch_pdl(im2col4_kernel, dim3(static_cast<unsigned>((total + 255) / 256)), dim3(256), 0, st, false, pixels,
-                      reinterpret_cast<__nv_bfloat16*>(cols), H, W, P, total));
+  const dim3 grid(static_cast<unsigned>((total + 255) / 256));
+  if (out_dtype == EVT_BF16) EVT_CUDA(launch_pdl(im2col4_kernel<true>, grid, dim3(256), 0, st, false, pixels, cols, H, W, P, total));
+  else EVT_CUDA(launch_pdl(im2col4_kernel<false>, grid, dim3(256), 0, st, false, pixels, cols, H, W, P, total));
   EVT_LAUNCH_CHECK("im2col4_kernel");
   return EVT_OK;
 }
@@ -500,7 +646,7 @@ int gather_layernorm_launch(const float* x, const int* idx, const float* gamma, 
   EVT_CHECK_ARG(y == nullptr || (gamma && beta), "gather_layernorm: LayerNorm output needs gamma and beta");
   EVT_CHECK_ARG(images > 0 && T_in > 0 && T_out > 0 && (G == 1 || G == 4), "gather_layernorm: bad sizes (G must be 1 or 4)");
   EVT_CHECK_ARG(C > 0 && C % 4 == 0 && G * C <= 3072, "gather_layernorm: C must be a multiple of 4 with G*C <= 3072");
-  EVT_CHECK_ARG(y_dtype == EVT_BF16 || y_dtype == EVT_F32, "gather_layernorm: y dtype must be bf16 or f32");
+  EVT_CHECK_ARG(y_dtype == EVT_BF16 || y_dtype == EVT_F32 || y_dtype == EVT_TF32, "gather_layernorm: y dtype must be bf16, f32 or tf32");
   EVT_CHECK_ARG(eps >= 0.f, "gather_layernorm: negative eps");
   const long long rows = images * T_out;
   const int D = G * C;
@@ -515,14 +661,23 @@ int gather_layernorm_launch(const float* x, const int* idx, const float* gamma, 
   return launch_gather_ln<24>(x, idx, gamma, beta, y, y_dtype, copy_f32, rows, T_in, T_out, G, C, eps, st);
 }
 
-int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
-                            int window_tokens, int heads, int head_size, float scale, cudaStream_t st) {
+namespace {
+// the checks window_attention_launch and window_attention_tf32_launch share (alignment differs by element type)
+int check_window_attention(const void* qkv, int64_t ldq, const void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                           int window_tokens, int heads, int head_size) {
   EVT_CHECK_ARG(qkv && ctx && table, "window_attention: null pointer");
   EVT_CHECK_ARG(n_windows > 0 && heads > 0 && n_tab > 0, "window_attention: sizes must be positive");
   if ((window_tokens != kWTok && window_tokens != kW12Tok) || head_size != kWHd)
     return fail(EVT_ERR_UNSUPPORTED,
                 "window_attention: only 7x7 (49-token) and 12x12 (144-token) windows with head size 32 are implemented");
   EVT_CHECK_ARG(ldq >= 3ll * heads * kWHd && ldc >= static_cast<int64_t>(heads) * kWHd, "window_attention: leading dimension too small");
+  return EVT_OK;
+}
+}  // namespace
+
+int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                            int window_tokens, int heads, int head_size, float scale, cudaStream_t st) {
+  EVT_TRY(check_window_attention(qkv, ldq, ctx, ldc, table, n_tab, n_windows, window_tokens, heads, head_size));
   EVT_CHECK_ARG(ldq % 8 == 0 && reinterpret_cast<uintptr_t>(qkv) % 16 == 0, "window_attention: qkv rows must be 16-byte aligned");
   EVT_CHECK_ARG(ldc % 2 == 0 && reinterpret_cast<uintptr_t>(ctx) % 4 == 0, "window_attention: ctx rows must be 4-byte aligned");
   const long long items = n_windows * heads;
@@ -552,18 +707,53 @@ int window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc
   return EVT_OK;
 }
 
-int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
-                                 cudaStream_t st) {
-  EVT_CHECK_ARG(x && gamma && beta && y, "layernorm_mean_tokens: null pointer");
-  EVT_CHECK_ARG(images > 0 && T > 0 && D > 0 && D % 4 == 0 && D <= 1536, "layernorm_mean_tokens: D must be a multiple of 4, <= 1536");
+int window_attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* table, int n_tab, int64_t n_windows,
+                                 int window_tokens, int heads, int head_size, float scale, cudaStream_t st) {
+  EVT_TRY(check_window_attention(qkv, ldq, ctx, ldc, table, n_tab, n_windows, window_tokens, heads, head_size));
+  EVT_CHECK_ARG(ldq % 4 == 0 && reinterpret_cast<uintptr_t>(qkv) % 16 == 0, "window_attention_tf32: qkv rows must be 16-byte aligned");
+  EVT_CHECK_ARG(ldc % 4 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "window_attention_tf32: ctx rows must be 16-byte aligned");
+  const long long items = n_windows * heads;
+  const long long ctas_needed = (items + kWWarps - 1) / kWWarps;
+  const bool pdl = pdl_for_work(n_windows * window_tokens, static_cast<long long>(heads) * kWHd);
+  const float sl2e = scale * 1.4426950408889634f;
+  if (window_tokens == kW12Tok) {
+    constexpr auto kern = window_attention_tf32_kernel<kW12Tok, kW12Tok, kW12Tok / 8>;
+    const int smem = kWWarps * 3 * kW12Tok * kWHd * 4;  // 216 KB: one CTA per SM, grid-stride over the rest
+    EVT_TRY(opt_in_smem<kern>(smem));
+    const long long cap = num_sms();
+    EVT_CUDA(launch_pdl(kern, dim3(static_cast<unsigned>(ctas_needed < cap ? ctas_needed : cap)), dim3(kWWarps * 32), smem, st, pdl, qkv,
+                        static_cast<long long>(ldq), ctx, static_cast<long long>(ldc), table, n_tab, heads, items, sl2e));
+  } else {
+    constexpr auto kern = window_attention_tf32_kernel<kWTok, kWRows, kWKeyCols / 8>;
+    const int smem = kWWarps * 3 * kWRows * kWHd * 4;  // 96 KB: two CTAs per SM
+    EVT_TRY(opt_in_smem<kern>(smem));
+    const long long cap = static_cast<long long>(num_sms()) * 2;
+    EVT_CUDA(launch_pdl(kern, dim3(static_cast<unsigned>(ctas_needed < cap ? ctas_needed : cap)), dim3(kWWarps * 32), smem, st, pdl, qkv,
+                        static_cast<long long>(ldq), ctx, static_cast<long long>(ldc), table, n_tab, heads, items, sl2e));
+  }
+  EVT_LAUNCH_CHECK("window_attention_tf32_kernel");
+  return EVT_OK;
+}
+
+template <int OUT>
+int launch_ln_mean_tokens(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
+                          cudaStream_t st) {
   const dim3 grid(static_cast<unsigned>(images));
-  __nv_bfloat16* yo = reinterpret_cast<__nv_bfloat16*>(y);
   const int nv = (D + 127) / 128;
-  if (nv <= 3) EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<3>, grid, dim3(256), 0, st, false, x, gamma, beta, yo, T, D, eps));
-  else if (nv <= 6) EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<6>, grid, dim3(256), 0, st, false, x, gamma, beta, yo, T, D, eps));
-  else EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<12>, grid, dim3(256), 0, st, false, x, gamma, beta, yo, T, D, eps));
+  if (nv <= 3) EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<3, OUT>, grid, dim3(256), 0, st, false, x, gamma, beta, y, T, D, eps));
+  else if (nv <= 6) EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<6, OUT>, grid, dim3(256), 0, st, false, x, gamma, beta, y, T, D, eps));
+  else EVT_CUDA(launch_pdl(ln_mean_tokens_kernel<12, OUT>, grid, dim3(256), 0, st, false, x, gamma, beta, y, T, D, eps));
   EVT_LAUNCH_CHECK("ln_mean_tokens_kernel");
   return EVT_OK;
+}
+
+int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T, int D,
+                                 float eps, cudaStream_t st) {
+  EVT_CHECK_ARG(x && gamma && beta && y, "layernorm_mean_tokens: null pointer");
+  EVT_CHECK_ARG(images > 0 && T > 0 && D > 0 && D % 4 == 0 && D <= 1536, "layernorm_mean_tokens: D must be a multiple of 4, <= 1536");
+  EVT_CHECK_ARG(y_dtype == EVT_BF16 || y_dtype == EVT_TF32, "layernorm_mean_tokens: y dtype must be bf16 or tf32");
+  if (y_dtype == EVT_TF32) return launch_ln_mean_tokens<EVT_TF32>(x, gamma, beta, y, images, T, D, eps, st);
+  return launch_ln_mean_tokens<EVT_BF16>(x, gamma, beta, y, images, T, D, eps, st);
 }
 
 }  // namespace evt
@@ -586,9 +776,25 @@ extern "C" int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx,
                                       static_cast<cudaStream_t>(stream));
 }
 
+extern "C" int evt_window_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* table, int n_tab,
+                                             int64_t n_windows, int window_tokens, int heads, int head_size, float scale,
+                                             evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::window_attention_tf32_launch(qkv, ldq, ctx, ldc, table, n_tab, n_windows, window_tokens, heads, head_size, scale,
+                                           static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T,
                                          int D, float eps, evt_stream stream) {
   int rc = evt_device_check();
   if (rc != EVT_OK) return rc;
-  return evt::layernorm_mean_tokens_launch(x, gamma, beta, y, images, T, D, eps, static_cast<cudaStream_t>(stream));
+  return evt::layernorm_mean_tokens_launch(x, gamma, beta, y, EVT_BF16, images, T, D, eps, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int evt_layernorm_mean_tokens_ex(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images,
+                                            int T, int D, float eps, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::layernorm_mean_tokens_launch(x, gamma, beta, y, y_dtype, images, T, D, eps, static_cast<cudaStream_t>(stream));
 }

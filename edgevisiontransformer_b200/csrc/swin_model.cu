@@ -7,7 +7,8 @@
 //
 // Data layout (see modeling_swin.py): inside a stage the f32 residual stream [B*T, C] is kept in the WINDOW ORDER of the
 // current block.  A block whose cyclic shift differs from the previous one starts with a row gather fused into its
-// layernorm_before (gather_layernorm_launch); patch merging is the same kernel with a 4-row gather.
+// layernorm_before (gather_layernorm_launch); patch merging is the same kernel with a 4-row gather.  spec.precision picks the
+// GEMM / attention operand type (bf16, or f32 holding tf32-rounded values); the launch sequence is the same.
 #include <cuda_bf16.h>
 
 #include <cmath>
@@ -84,7 +85,7 @@ std::vector<float> attention_table(const std::vector<float>& bias_table, int hea
 struct SwinBlock {
   int* idx = nullptr;  // nullable: row gather into this block's window order
   float *ln1_g = nullptr, *ln1_b = nullptr, *ln2_g = nullptr, *ln2_b = nullptr;
-  __nv_bfloat16 *wqkv = nullptr, *wo = nullptr, *w1 = nullptr, *w2 = nullptr;
+  uint8_t *wqkv = nullptr, *wo = nullptr, *w1 = nullptr, *w2 = nullptr;  // bf16, or f32 holding tf32 values (tf32 mode)
   float *bqkv = nullptr, *bo = nullptr, *b1 = nullptr, *b2 = nullptr;
   float* table = nullptr;
   int n_tab = 1;
@@ -95,7 +96,7 @@ struct SwinStage {
   bool merge = false;
   int* m_idx = nullptr;
   float *m_g = nullptr, *m_b = nullptr;
-  __nv_bfloat16* m_w = nullptr;
+  uint8_t* m_w = nullptr;
 };
 
 }  // namespace
@@ -105,9 +106,10 @@ struct evt_swin {
   evt_swin_spec spec;
   bool loaded = false;
   int grid = 0, patch_k = 0, patch_ld = 0;
-  __nv_bfloat16* w_patch = nullptr;
+  int es = 2;  // bytes per GEMM operand element: 2 (bf16) or 4 (tf32 mode: f32 storage of tf32-rounded values)
+  uint8_t* w_patch = nullptr;
   float *b_patch = nullptr, *g_embed = nullptr, *b_embed = nullptr, *g_final = nullptr, *b_final = nullptr, *b_cls = nullptr;
-  __nv_bfloat16* w_cls = nullptr;
+  uint8_t* w_cls = nullptr;
   int* idx_embed = nullptr;
   std::vector<evt::SwinStage> stages;
   std::vector<void*> allocs;
@@ -127,17 +129,18 @@ SwinWs plan(const evt_swin* m, int batch, uint8_t* base) {
   const evt_swin_spec& s = m->spec;
   const size_t T0 = static_cast<size_t>(m->grid) * m->grid * batch;
   const size_t C0 = s.embed_dim;
+  const size_t es = m->es;  // the GEMM operands: bf16, or f32 in the tf32 mode
   WorkspaceCarver c{base};
   SwinWs w;
   // T * C is largest in stage 1 and halves with every patch merging
-  w.cols = c.take(T0 * m->patch_ld * 2);
+  w.cols = c.take(T0 * m->patch_ld * es);
   w.ra = c.take<float>(T0 * C0 * 4);
   w.rb = c.take<float>(T0 * C0 * 4);
-  w.xn = c.take(T0 * C0 * 2);
-  w.qkv = c.take(T0 * 3 * C0 * 2);
-  w.ctx = c.take(T0 * C0 * 2);
-  w.h = c.take(T0 * 4 * C0 * 2);
-  w.pooled = c.take(static_cast<size_t>(batch) * C0 * (1u << (s.stages - 1)) * 2);
+  w.xn = c.take(T0 * C0 * es);
+  w.qkv = c.take(T0 * 3 * C0 * es);
+  w.ctx = c.take(T0 * C0 * es);
+  w.h = c.take(T0 * 4 * C0 * es);
+  w.pooled = c.take(static_cast<size_t>(batch) * C0 * (1u << (s.stages - 1)) * es);
   w.bytes = c.bytes;
   return w;
 }
@@ -155,6 +158,7 @@ extern "C" int evt_swin_create(const evt_swin_spec* s, evt_swin** out) {
   const int grid = s->image / s->patch;
   EVT_CHECK_ARG(grid % (s->window << (s->stages - 1)) == 0, "image / patch must be a multiple of window * 2^(stages-1)");
   EVT_CHECK_ARG(s->num_labels > 0 && s->eps > 0.f && s->embed_dim > 0 && s->embed_dim % 32 == 0, "bad num_labels / eps / embed_dim");
+  EVT_CHECK_ARG(s->precision == EVT_PREC_BF16 || s->precision == EVT_PREC_TF32, "precision must be bf16 (0) or tf32 (1)");
   for (int i = 0; i < s->stages; ++i) {
     EVT_CHECK_ARG(s->depths[i] > 0 && s->heads[i] > 0, "depths / heads must be positive");
     if ((s->embed_dim << i) != 32 * s->heads[i]) return fail(EVT_ERR_UNSUPPORTED, "only head size 32 is implemented");
@@ -164,6 +168,7 @@ extern "C" int evt_swin_create(const evt_swin_spec* s, evt_swin** out) {
   m->grid = grid;
   m->patch_k = 3 * s->patch * s->patch;
   m->patch_ld = (m->patch_k + 7) / 8 * 8;
+  m->es = s->precision == EVT_PREC_TF32 ? 4 : 2;
   *out = m;
   return EVT_OK;
 }
@@ -179,12 +184,12 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
   EVT_CHECK_ARG(m != nullptr && tensors != nullptr && n > 0, "evt_swin_load_weights: bad arguments");
   if (m->loaded) return fail(EVT_ERR_STATE, "weights already loaded; create a new model to reload");
   const evt_swin_spec& s = m->spec;
-  Loader L{&m->allocs, static_cast<cudaStream_t>(stream), 2};
+  Loader L{&m->allocs, static_cast<cudaStream_t>(stream), m->es};
   EVT_TRY(L.index(tensors, n));
   const int ws = s.window;
   const std::string e = "swin.embeddings.";
   const int C0 = s.embed_dim;
-  // patch-embedding weight [C0, 3, 4, 4] -> bf16 [C0, patch_ld]
+  // patch-embedding weight [C0, 3, 4, 4] -> operand type [C0, patch_ld]
   EVT_TRY(L.mat(e + "patch_embeddings.projection.weight", C0, m->patch_k, m->patch_ld, &m->w_patch));
   EVT_TRY(L.vec(e + "patch_embeddings.projection.bias", C0, false, &m->b_patch));
   EVT_TRY(L.vec(e + "norm.weight", C0, false, &m->g_embed));
@@ -222,13 +227,13 @@ extern "C" int evt_swin_load_weights(evt_swin* m, const evt_tensor_view* tensors
       EVT_TRY(L.vec(p + "layernorm_before.weight", C, false, &blk.ln1_g));
       EVT_TRY(L.vec(p + "layernorm_before.bias", C, false, &blk.ln1_b));
       void* q;
-      EVT_TRY(L.alloc(static_cast<size_t>(3) * C * C * 2, &q));
-      blk.wqkv = reinterpret_cast<__nv_bfloat16*>(q);
+      EVT_TRY(L.alloc(static_cast<size_t>(3) * C * C * m->es, &q));
+      blk.wqkv = static_cast<uint8_t*>(q);
       EVT_TRY(L.alloc(static_cast<size_t>(3) * C * 4, &q));
       blk.bqkv = reinterpret_cast<float*>(q);
       const char* names[3] = {"query", "key", "value"};
       for (int t = 0; t < 3; ++t) {
-        EVT_TRY(L.mat_into(p + "attention.self." + names[t] + ".weight", C, C, C, blk.wqkv + static_cast<size_t>(t) * C * C));
+        EVT_TRY(L.mat_into(p + "attention.self." + names[t] + ".weight", C, C, C, blk.wqkv + static_cast<size_t>(t) * C * C * m->es));
         EVT_TRY(L.vec_into(p + "attention.self." + names[t] + ".bias", C, false, blk.bqkv + t * C));
       }
       std::vector<float> bias_table;
@@ -311,9 +316,15 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
   const float scale = 1.0f / sqrtf(32.f);
   const int ws2 = s.window * s.window;
   int T = m->grid * m->grid;
+  // Both modes issue the same launches.  tf32: every producer of a GEMM / attention operand writes f32 rounded to nearest tf32
+  // (adt), the GEMMs read f32 (dt) with kind::tf32, the attention is window_attention_tf32_launch; the residual stream is
+  // unrounded f32 in both.
+  const bool tf32 = s.precision == EVT_PREC_TF32;
+  const int dt = tf32 ? EVT_F32 : EVT_BF16;
+  const int adt = tf32 ? EVT_TF32 : EVT_BF16;
   // SwinEmbeddings (:262-301): 4 x 4 patch conv as im2col + GEMM, LayerNorm, rows gathered into the first window order
-  EVT_TRY(im2col4_launch(pixels, w.cols, batch, s.image, s.image, s.patch, st));
-  EVT_TRY(gemm_launch({.A = w.cols, .lda = m->patch_ld, .W = m->w_patch, .ldw = m->patch_ld, .bias = m->b_patch, .out = w.rb,
+  EVT_TRY(im2col4_launch(pixels, w.cols, adt, batch, s.image, s.image, s.patch, st));
+  EVT_TRY(gemm_launch({.A = w.cols, .lda = m->patch_ld, .W = m->w_patch, .ldw = m->patch_ld, .in_dtype = dt, .bias = m->b_patch, .out = w.rb,
                        .out_dtype = EVT_F32, .ldo = s.embed_dim, .M = static_cast<int64_t>(batch) * T, .N = s.embed_dim, .K = m->patch_k}, st));
   EVT_TRY(gather_layernorm_launch(w.rb, m->idx_embed, m->g_embed, m->b_embed, w.ra, EVT_F32, nullptr, batch, T, T, 1, s.embed_dim, eps, st));
   float* resid = w.ra;
@@ -324,34 +335,38 @@ extern "C" int evt_swin_forward(evt_swin* m, const float* pixels, int batch, flo
     const int64_t M = static_cast<int64_t>(batch) * T;
     for (const SwinBlock& blk : stg.blocks) {
       if (blk.idx != nullptr) {  // cyclic shift / reverse shift folded into layernorm_before; the residual stream is re-ordered too
-        EVT_TRY(gather_layernorm_launch(resid, blk.idx, blk.ln1_g, blk.ln1_b, w.xn, EVT_BF16, other, batch, T, T, 1, C, eps, st));
+        EVT_TRY(gather_layernorm_launch(resid, blk.idx, blk.ln1_g, blk.ln1_b, w.xn, adt, other, batch, T, T, 1, C, eps, st));
         std::swap(resid, other);
       } else {
-        EVT_TRY(layernorm_launch(resid, C, blk.ln1_g, blk.ln1_b, w.xn, EVT_BF16, C, nullptr, M, C, eps, st));
+        EVT_TRY(layernorm_launch(resid, C, blk.ln1_g, blk.ln1_b, w.xn, adt, C, nullptr, M, C, eps, st));
       }
-      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.wqkv, .ldw = C, .bias = blk.bqkv, .out = w.qkv, .out_dtype = EVT_BF16, .ldo = 3 * C,
-                           .M = M, .N = 3 * C, .K = C}, st));
-      EVT_TRY(window_attention_launch(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / ws2, ws2, stg.heads, 32, scale, st));
-      EVT_TRY(gemm_launch({.A = w.ctx, .lda = C, .W = blk.wo, .ldw = C, .bias = blk.bo, .residual = resid, .ldr = C, .out = resid,
+      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.wqkv, .ldw = C, .in_dtype = dt, .bias = blk.bqkv, .out = w.qkv, .out_dtype = adt,
+                           .ldo = 3 * C, .M = M, .N = 3 * C, .K = C}, st));
+      if (tf32)
+        EVT_TRY(window_attention_tf32_launch(reinterpret_cast<const float*>(w.qkv), 3 * C, reinterpret_cast<float*>(w.ctx), C, blk.table,
+                                             blk.n_tab, M / ws2, ws2, stg.heads, 32, scale, st));
+      else
+        EVT_TRY(window_attention_launch(w.qkv, 3 * C, w.ctx, C, blk.table, blk.n_tab, M / ws2, ws2, stg.heads, 32, scale, st));
+      EVT_TRY(gemm_launch({.A = w.ctx, .lda = C, .W = blk.wo, .ldw = C, .in_dtype = dt, .bias = blk.bo, .residual = resid, .ldr = C, .out = resid,
                            .out_dtype = EVT_F32, .ldo = C, .M = M, .N = C, .K = C}, st));
-      EVT_TRY(layernorm_launch(resid, C, blk.ln2_g, blk.ln2_b, w.xn, EVT_BF16, C, nullptr, M, C, eps, st));
-      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.w1, .ldw = C, .bias = blk.b1, .out = w.h, .out_dtype = EVT_BF16, .ldo = 4 * C,
+      EVT_TRY(layernorm_launch(resid, C, blk.ln2_g, blk.ln2_b, w.xn, adt, C, nullptr, M, C, eps, st));
+      EVT_TRY(gemm_launch({.A = w.xn, .lda = C, .W = blk.w1, .ldw = C, .in_dtype = dt, .bias = blk.b1, .out = w.h, .out_dtype = adt, .ldo = 4 * C,
                            .M = M, .N = 4 * C, .K = C, .act = EVT_ACT_GELU_ERF}, st));
-      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = blk.w2, .ldw = 4 * C, .bias = blk.b2, .residual = resid, .ldr = C, .out = resid,
+      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = blk.w2, .ldw = 4 * C, .in_dtype = dt, .bias = blk.b2, .residual = resid, .ldr = C, .out = resid,
                            .out_dtype = EVT_F32, .ldo = C, .M = M, .N = C, .K = 4 * C}, st));
     }
     if (stg.merge) {
       // 2 x 2 neighbourhood concat + LayerNorm(4C) as one gather, then the bias-free reduction to 2C
-      EVT_TRY(gather_layernorm_launch(resid, stg.m_idx, stg.m_g, stg.m_b, w.h, EVT_BF16, nullptr, batch, T, T / 4, 4, C, eps, st));
+      EVT_TRY(gather_layernorm_launch(resid, stg.m_idx, stg.m_g, stg.m_b, w.h, adt, nullptr, batch, T, T / 4, 4, C, eps, st));
       T /= 4;
-      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = stg.m_w, .ldw = 4 * C, .out = other, .out_dtype = EVT_F32, .ldo = 2 * C,
+      EVT_TRY(gemm_launch({.A = w.h, .lda = 4 * C, .W = stg.m_w, .ldw = 4 * C, .in_dtype = dt, .out = other, .out_dtype = EVT_F32, .ldo = 2 * C,
                            .M = static_cast<int64_t>(batch) * T, .N = 2 * C, .K = 4 * C}, st));
       std::swap(resid, other);
     }
   }
   const int Cf = s.embed_dim << (s.stages - 1);
-  EVT_TRY(layernorm_mean_tokens_launch(resid, m->g_final, m->b_final, w.pooled, batch, T, Cf, eps, st));
-  EVT_TRY(gemm_launch({.A = w.pooled, .lda = Cf, .W = m->w_cls, .ldw = Cf, .bias = m->b_cls, .out = logits, .out_dtype = EVT_F32,
+  EVT_TRY(layernorm_mean_tokens_launch(resid, m->g_final, m->b_final, w.pooled, adt, batch, T, Cf, eps, st));
+  EVT_TRY(gemm_launch({.A = w.pooled, .lda = Cf, .W = m->w_cls, .ldw = Cf, .in_dtype = dt, .bias = m->b_cls, .out = logits, .out_dtype = EVT_F32,
                        .ldo = s.num_labels, .M = batch, .N = s.num_labels, .K = Cf}, st));
   return EVT_OK;
 }

@@ -10,8 +10,10 @@ Data layout: inside a stage the f32 residual stream ``[B*T, C]`` is kept in the 
 window, token in window).  A block whose cyclic shift differs from the previous one starts with a row gather fused into its
 ``layernorm_before`` (``evt_gather_layernorm``: LN output for the QKV GEMM + the permuted residual copy); patch merging is
 the same kernel with a 4-row gather.  Everything between -- QKV / out-proj / FC1+GELU / FC2 -- is the tcgen05 GEMM of the
-ViT path with its TMA reduce-add epilogue, attention is ``evt_window_attention_fwd``.  bf16 operands, f32 accumulate /
-residual / LayerNorm / softmax; logits within 2e-2 of the f32 reference.  No CPU fallback.
+ViT path with its TMA reduce-add epilogue, attention is ``evt_window_attention_fwd``.  f32 accumulate / residual / LayerNorm /
+softmax.  ``precision="bf16"`` (default): bf16 GEMM and attention operands, logits within 2e-2 of the f32 reference.
+``precision="tf32"``: the same launches with f32 operands rounded to nearest tf32 where they are written (tf32 GEMMs,
+``evt_window_attention_fwd_tf32``), logits within 1e-3.  No CPU fallback.
 """
 from __future__ import annotations
 
@@ -91,11 +93,14 @@ class B200SwinConfig:
 
 class B200SwinForImageClassification(nn.Module):
     """Inference-only.  ``state_dict`` uses HF key names (``swin.embeddings...``, ``swin.encoder.layers.{s}.blocks.{b}...``).
-    ``window`` 7 (224 pixels) or 12 (384 pixels)."""
+    ``window`` 7 (224 pixels) or 12 (384 pixels).  ``precision`` "bf16" or "tf32" (see the module docstring)."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], depths: Sequence[int], num_heads: Sequence[int], embed_dim: int,
-                 window: int = 7, patch: int = 4, image_size: int = 224, eps: float = 1e-5, device="cuda", max_batch: int = 1024):
+                 window: int = 7, patch: int = 4, image_size: int = 224, eps: float = 1e-5, device="cuda", max_batch: int = 1024,
+                 precision: str = "bf16"):
         super().__init__()
+        if precision not in ("bf16", "tf32"):
+            raise ValueError(f"unsupported precision {precision!r}: 'bf16' or 'tf32'")
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("B200SwinForImageClassification runs only on a CUDA (sm_100a) device; no CPU fallback")
@@ -107,18 +112,22 @@ class B200SwinForImageClassification(nn.Module):
             raise ValueError("image_size / patch must be a multiple of window * 2^(stages-1)")
         self.depths, self.num_heads, self.embed_dim = list(depths), list(num_heads), embed_dim
         self.window, self.patch, self.image_size, self.eps = window, patch, image_size, eps
-        self.max_batch, self._device = int(max_batch), dev
+        self.max_batch, self._device, self.precision = int(max_batch), dev, precision
+        tf32 = precision == "tf32"
+        # what each producer of a GEMM / attention operand writes in the op-level composition (_run_impl)
+        self._adt = ops.TF32 if tf32 else torch.bfloat16
         self._graphs: dict = {}
         sd = {k: v.detach() for k, v in state_dict.items()}
 
         def f32(k):
             return sd[k].to(device=dev, dtype=torch.float32).contiguous()
 
-        def bf16(k):
-            return sd[k].to(device=dev, dtype=torch.float32).reshape(sd[k].shape[0], -1).to(torch.bfloat16).contiguous()
+        def mat(k):  # a GEMM weight in the operand type: bf16, or f32 rounded to nearest tf32 (as evt_swin_load_weights packs it)
+            w = sd[k].to(device=dev, dtype=torch.float32).reshape(sd[k].shape[0], -1)
+            return (ops.round_tf32(w) if tf32 else w.to(torch.bfloat16)).contiguous()
 
         e = "swin.embeddings."
-        self.w_patch, self.b_patch = bf16(e + "patch_embeddings.projection.weight"), f32(e + "patch_embeddings.projection.bias")
+        self.w_patch, self.b_patch = mat(e + "patch_embeddings.projection.weight"), f32(e + "patch_embeddings.projection.bias")
         self.g_embed, self.be_embed = f32(e + "norm.weight"), f32(e + "norm.bias")
         self.stages: List[dict] = []
         H = grid
@@ -138,15 +147,15 @@ class B200SwinForImageClassification(nn.Module):
                     blk["idx"] = _inverse(order)[want].to(torch.int32).to(dev)
                     order = want
                 blk["ln1"] = (f32(p + "layernorm_before.weight"), f32(p + "layernorm_before.bias"))
-                blk["wqkv"] = torch.cat([bf16(p + f"attention.self.{n}.weight") for n in ("query", "key", "value")], 0).contiguous()
+                blk["wqkv"] = torch.cat([mat(p + f"attention.self.{n}.weight") for n in ("query", "key", "value")], 0).contiguous()
                 blk["bqkv"] = torch.cat([f32(p + f"attention.self.{n}.bias") for n in ("query", "key", "value")], 0).contiguous()
                 mask = shift_mask(H, H, window, shift) if shift > 0 else None
                 blk["table"] = attention_table(sd[p + "attention.self.relative_position_bias_table"].float().cpu(), heads, window,
                                                mask).to(dev)
-                blk["wo"], blk["bo"] = bf16(p + "attention.output.dense.weight"), f32(p + "attention.output.dense.bias")
+                blk["wo"], blk["bo"] = mat(p + "attention.output.dense.weight"), f32(p + "attention.output.dense.bias")
                 blk["ln2"] = (f32(p + "layernorm_after.weight"), f32(p + "layernorm_after.bias"))
-                blk["w1"], blk["b1"] = bf16(p + "intermediate.dense.weight"), f32(p + "intermediate.dense.bias")
-                blk["w2"], blk["b2"] = bf16(p + "output.dense.weight"), f32(p + "output.dense.bias")
+                blk["w1"], blk["b1"] = mat(p + "intermediate.dense.weight"), f32(p + "intermediate.dense.bias")
+                blk["w2"], blk["b2"] = mat(p + "output.dense.weight"), f32(p + "output.dense.bias")
                 blocks.append(blk)
             st = dict(C=C, heads=heads, H=H, blocks=blocks, merge=None)
             if s + 1 < len(depths):
@@ -157,11 +166,11 @@ class B200SwinForImageClassification(nn.Module):
                 src = torch.stack([(2 * y2) * H + 2 * x2, (2 * y2 + 1) * H + 2 * x2, (2 * y2) * H + 2 * x2 + 1,
                                    (2 * y2 + 1) * H + 2 * x2 + 1], dim=1)                        # :334-343 concat order
                 st["merge"] = dict(idx=_inverse(order)[src].to(torch.int32).contiguous().to(dev),
-                                   ln=(f32(p + "norm.weight"), f32(p + "norm.bias")), w=bf16(p + "reduction.weight"))
+                                   ln=(f32(p + "norm.weight"), f32(p + "norm.bias")), w=mat(p + "reduction.weight"))
                 order, H = nxt, H2
             self.stages.append(st)
         self.g_final, self.b_final = f32("swin.layernorm.weight"), f32("swin.layernorm.bias")
-        self.w_cls, self.b_cls = bf16("classifier.weight"), f32("classifier.bias")
+        self.w_cls, self.b_cls = mat("classifier.weight"), f32("classifier.bias")
         self.num_labels = self.w_cls.shape[0]
         self.config = B200SwinConfig(depths, num_heads, embed_dim, window, patch, image_size, eps, self.num_labels)
         self._param = nn.Parameter(self.b_cls, requires_grad=False)       # next(model.parameters()).device works
@@ -174,6 +183,7 @@ class B200SwinForImageClassification(nn.Module):
         spec = _lib.SwinSpec()
         spec.image, spec.patch, spec.window, spec.embed_dim = image_size, patch, window, embed_dim
         spec.stages, spec.num_labels, spec.eps = len(self.depths), self.num_labels, float(eps)
+        spec.precision = _lib.PREC_TF32 if tf32 else _lib.PREC_BF16
         for i, (d, h) in enumerate(zip(self.depths, self.num_heads)):
             spec.depths[i], spec.heads[i] = int(d), int(h)
         with torch.cuda.device(dev):
@@ -267,8 +277,8 @@ class B200SwinForImageClassification(nn.Module):
 
     def _run_impl(self, x: torch.Tensor) -> torch.Tensor:
         B = x.shape[0]
-        eps, ws2 = self.eps, self.window * self.window
-        cols = ops.im2col_patch(x, self.patch)
+        eps, ws2, adt = self.eps, self.window * self.window, self._adt
+        cols = ops.im2col_patch(x, self.patch, out_dtype=adt)
         y = ops.linear(cols, self.w_patch, self.b_patch, out_dtype=torch.float32)
         T = (self.image_size // self.patch) ** 2
         resid, _ = ops.gather_layernorm(y, self.idx_embed, self.g_embed, self.be_embed, eps, B, T, T, out_dtype=torch.float32)
@@ -276,21 +286,21 @@ class B200SwinForImageClassification(nn.Module):
             C, heads, T = st["C"], st["heads"], st["H"] * st["H"]
             for blk in st["blocks"]:
                 if blk["idx"] is not None:
-                    xn, resid = ops.gather_layernorm(resid, blk["idx"], *blk["ln1"], eps, B, T, T, copy=True)
+                    xn, resid = ops.gather_layernorm(resid, blk["idx"], *blk["ln1"], eps, B, T, T, out_dtype=adt, copy=True)
                 else:
-                    xn = ops.layernorm(resid, *blk["ln1"], eps)
-                qkv = ops.linear(xn, blk["wqkv"], blk["bqkv"])
+                    xn = ops.layernorm(resid, *blk["ln1"], eps, out_dtype=adt)
+                qkv = ops.linear(xn, blk["wqkv"], blk["bqkv"], out_dtype=adt)
                 ctx = ops.window_attention(qkv, blk["table"], B * T // ws2, heads, ws2, 32)
                 ops.linear(ctx, blk["wo"], blk["bo"], residual=resid, out=resid, out_dtype=torch.float32)
-                xn = ops.layernorm(resid, *blk["ln2"], eps)
-                h = ops.linear(xn, blk["w1"], blk["b1"], act="gelu_erf")
+                xn = ops.layernorm(resid, *blk["ln2"], eps, out_dtype=adt)
+                h = ops.linear(xn, blk["w1"], blk["b1"], act="gelu_erf", out_dtype=adt)
                 ops.linear(h, blk["w2"], blk["b2"], residual=resid, out=resid, out_dtype=torch.float32)
             if st["merge"] is not None:
                 mg = st["merge"]
-                xm, _ = ops.gather_layernorm(resid, mg["idx"], *mg["ln"], eps, B, T, T // 4, G=4)
+                xm, _ = ops.gather_layernorm(resid, mg["idx"], *mg["ln"], eps, B, T, T // 4, G=4, out_dtype=adt)
                 resid = ops.linear(xm, mg["w"], None, out_dtype=torch.float32)
         last = self.stages[-1]
-        pooled = ops.layernorm_mean_tokens(resid, self.g_final, self.b_final, eps, B, last["H"] * last["H"])
+        pooled = ops.layernorm_mean_tokens(resid, self.g_final, self.b_final, eps, B, last["H"] * last["H"], out_dtype=adt)
         return ops.linear(pooled, self.w_cls, self.b_cls, out_dtype=torch.float32)
 
     @torch.no_grad()

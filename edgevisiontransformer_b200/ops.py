@@ -9,7 +9,11 @@ from typing import Optional
 import torch
 
 from . import _lib
-from ._lib import ACT_GELU_ERF, ACT_GELU_TANH, ACT_NONE, EVT_BF16, EVT_F32  # noqa: F401
+from ._lib import ACT_GELU_ERF, ACT_GELU_TANH, ACT_NONE, EVT_BF16, EVT_F32, EVT_TF32  # noqa: F401
+
+# out_dtype of layernorm / linear / gather_layernorm / layernorm_mean_tokens / im2col_patch: an f32 tensor whose values are
+# rounded to nearest tf32 when written (the operand of a tf32 GEMM or attention, whose tensor cores would truncate).
+TF32 = "tf32"
 
 ACTS = {None: ACT_NONE, "none": ACT_NONE, "gelu": ACT_GELU_ERF, "gelu_erf": ACT_GELU_ERF, "erf": ACT_GELU_ERF,
         "gelu_tanh": ACT_GELU_TANH, "gelu_new": ACT_GELU_TANH, "gelu_pytorch_tanh": ACT_GELU_TANH}
@@ -27,7 +31,13 @@ def _need_cuda(*ts: Optional[torch.Tensor]) -> None:
                                "there is no CPU fallback")
 
 
-def _dt(t: torch.Tensor) -> int:
+def _storage(out_dtype) -> torch.dtype:
+    return torch.float32 if out_dtype == TF32 else out_dtype
+
+
+def _dt(t: torch.Tensor, out_dtype=None) -> int:
+    if out_dtype == TF32:
+        return EVT_TF32
     if t.dtype == torch.float32:
         return EVT_F32
     if t.dtype == torch.bfloat16:
@@ -39,9 +49,17 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def round_tf32(x: torch.Tensor) -> torch.Tensor:
+    """f32 -> the nearest tf32 value (ties away from zero), as f32: what ``cvt.rna.tf32.f32`` gives, i.e. what the tf32 mode's
+    kernels write.  Finite inputs; any device."""
+    b = x.float().contiguous().view(torch.int32)
+    return ((b + 0x1000) & ~0x1FFF).view(torch.float32)
+
+
 def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float,
               out_dtype: torch.dtype = torch.bfloat16, write_back: bool = False) -> torch.Tensor:
-    """LayerNorm over the last dim of an f32 tensor whose rows are contiguous. write_back: x <- LN(x) too."""
+    """LayerNorm over the last dim of an f32 tensor whose rows are contiguous (out_dtype bf16, f32 or TF32).
+    write_back: x <- LN(x) too."""
     _need_cuda(x, gamma, beta)
     if x.dtype != torch.float32 or x.stride(-1) != 1:
         raise ValueError("layernorm wants an f32 tensor with unit inner stride")
@@ -49,9 +67,9 @@ def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: flo
     x2 = x.reshape(-1, D)
     if x2.data_ptr() != x.data_ptr():
         raise ValueError("layernorm wants a tensor viewable as [rows, D]")
-    y = torch.empty(x2.shape, dtype=out_dtype, device=x.device)
+    y = torch.empty(x2.shape, dtype=_storage(out_dtype), device=x.device)
     lib = _lib.load()
-    _lib.check(lib.evt_layernorm_fwd(x2.data_ptr(), x2.stride(0), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), _dt(y),
+    _lib.check(lib.evt_layernorm_fwd(x2.data_ptr(), x2.stride(0), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), _dt(y, out_dtype),
                                      y.stride(0), x2.data_ptr() if write_back else None, x2.shape[0], D, float(eps),
                                      _stream()), "layernorm")
     return y.view(*x.shape)
@@ -90,7 +108,7 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
            residual: Optional[torch.Tensor] = None, out_dtype: torch.dtype = torch.bfloat16,
            out: Optional[torch.Tensor] = None, n: Optional[int] = None, k: Optional[int] = None) -> torch.Tensor:
     """out[M,N] = act(a[M,K] @ w[N,K]^T + bias) (+ residual).  a, w bf16 (tensor cores, f32 accumulate) or
-    both f32 (tf32 mode).  Row strides may exceed the logical K / N (padded leading dimensions)."""
+    both f32 (tf32 mode; out_dtype f32 or TF32).  Row strides may exceed the logical K / N (padded leading dimensions)."""
     _need_cuda(a, w, bias, residual, out)
     if a.dim() != 2 or w.dim() != 2 or a.stride(1) != 1 or w.stride(1) != 1:
         raise ValueError("linear wants 2-D operands with unit inner stride")
@@ -101,22 +119,30 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
     N = n if n is not None else w.shape[0]
     if w.shape[1] < K or a.shape[1] < K:
         raise ValueError("linear: K exceeds operand width")
+    rounded = out_dtype == TF32
     if out is None:
-        out = torch.empty((M, N), dtype=out_dtype, device=a.device)
+        out = torch.empty((M, N), dtype=_storage(out_dtype), device=a.device)
     if residual is not None and (residual.dtype != torch.float32 or residual.stride(1) != 1):
         raise ValueError("linear: residual must be f32 with unit inner stride")
     lib = _lib.load()
     act_id = ACTS[act] if not isinstance(act, int) else act
     if a.dtype == torch.bfloat16:
+        if rounded:
+            raise ValueError("linear: a TF32 output needs f32 (tf32-mode) operands")
         rc = lib.evt_gemm_bias_act(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(residual),
                                    residual.stride(0) if residual is not None else 0, 0, 0, out.data_ptr(), _dt(out),
                                    out.stride(0), 0, 0, 0, M, N, K, act_id, _stream())
     elif a.dtype == torch.float32:
         if out.dtype != torch.float32:
             raise ValueError("linear: tf32 mode writes f32")
-        rc = lib.evt_gemm_bias_act_tf32(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(residual),
-                                        residual.stride(0) if residual is not None else 0, 0, 0, out.data_ptr(),
-                                        out.stride(0), 0, 0, 0, M, N, K, act_id, _stream())
+        if rounded:
+            rc = lib.evt_gemm_bias_act_tf32_ex(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(residual),
+                                               residual.stride(0) if residual is not None else 0, 0, 0, out.data_ptr(), EVT_TF32,
+                                               out.stride(0), 0, 0, 0, M, N, K, act_id, _stream())
+        else:
+            rc = lib.evt_gemm_bias_act_tf32(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(residual),
+                                            residual.stride(0) if residual is not None else 0, 0, 0, out.data_ptr(),
+                                            out.stride(0), 0, 0, 0, M, N, K, act_id, _stream())
     else:
         raise ValueError(f"linear: unsupported dtype {a.dtype}")
     _lib.check(rc, "gemm")
@@ -202,18 +228,19 @@ def gather_layernorm(x: torch.Tensor, idx: torch.Tensor, gamma: Optional[torch.T
                      images: int, T_in: int, T_out: int, G: int = 1, out_dtype: Optional[torch.dtype] = torch.bfloat16,
                      copy: bool = False):
     """Row gather fused with LayerNorm (Swin window partition / shift / patch merging, include/evt.h).
-    x f32 [images*T_in, C]; idx int32 [T_out*G] -> (LN output [images*T_out, G*C] or None, raw gathered f32 copy or None)."""
+    x f32 [images*T_in, C]; idx int32 [T_out*G] -> (LN output [images*T_out, G*C] (out_dtype bf16, f32 or TF32) or None, raw
+    gathered f32 copy or None)."""
     _need_cuda(x, idx, gamma, beta)
     if x.dtype != torch.float32 or x.dim() != 2 or not x.is_contiguous() or x.shape[0] != images * T_in:
         raise ValueError("gather_layernorm wants a contiguous f32 [images*T_in, C] matrix")
     if idx.dtype != torch.int32 or idx.numel() != T_out * G or not idx.is_contiguous():
         raise ValueError("gather_layernorm: idx must be a contiguous int32 [T_out*G] tensor")
     C = x.shape[1]
-    y = torch.empty((images * T_out, G * C), dtype=out_dtype, device=x.device) if out_dtype is not None else None
+    y = torch.empty((images * T_out, G * C), dtype=_storage(out_dtype), device=x.device) if out_dtype is not None else None
     cp = torch.empty((images * T_out, G * C), dtype=torch.float32, device=x.device) if copy else None
     lib = _lib.load()
     _lib.check(lib.evt_gather_layernorm(x.data_ptr(), idx.data_ptr(), _ptr(gamma), _ptr(beta), _ptr(y),
-                                        _dt(y) if y is not None else EVT_BF16, _ptr(cp), images, T_in, T_out, G, C, float(eps),
+                                        _dt(y, out_dtype) if y is not None else EVT_BF16, _ptr(cp), images, T_in, T_out, G, C, float(eps),
                                         _stream()), "gather_layernorm")
     return y, cp
 
@@ -227,43 +254,51 @@ def window_table_shape(window_tokens: int):
 def window_attention(qkv: torch.Tensor, table: torch.Tensor, n_windows: int, heads: int, window_tokens: int = 49,
                      head_size: int = 32, scale: Optional[float] = None) -> torch.Tensor:
     """qkv bf16 [n_windows*N, 3*heads*32] in window order (N = window_tokens, 49 or 144), table f32
-    [n_tab, heads, *window_table_shape(N)] (log2 domain, include/evt.h) -> ctx bf16 [n_windows*N, heads*32]."""
+    [n_tab, heads, *window_table_shape(N)] (log2 domain, include/evt.h) -> ctx bf16 [n_windows*N, heads*32].
+    f32 qkv (tf32-representable values, e.g. from a TF32 linear) runs the tf32 kernel -> ctx f32, rounded to tf32."""
     _need_cuda(qkv, table)
-    if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.stride(1) != 1 or qkv.shape[0] != n_windows * window_tokens:
-        raise ValueError("window_attention wants a bf16 [n_windows*tokens, 3*heads*head_size] matrix")
+    if qkv.dtype not in (torch.bfloat16, torch.float32) or qkv.dim() != 2 or qkv.stride(1) != 1 or qkv.shape[0] != n_windows * window_tokens:
+        raise ValueError("window_attention wants a bf16 (or f32 for the tf32 mode) [n_windows*tokens, 3*heads*head_size] matrix")
     want = (heads, *window_table_shape(window_tokens))
     if table.dtype != torch.float32 or table.dim() != 4 or tuple(table.shape[1:]) != want or not table.is_contiguous():
         raise ValueError(f"window_attention: table must be a contiguous f32 [n_tab, {want[0]}, {want[1]}, {want[2]}] tensor")
-    ctx = torch.empty((qkv.shape[0], heads * head_size), dtype=torch.bfloat16, device=qkv.device)
+    ctx = torch.empty((qkv.shape[0], heads * head_size), dtype=qkv.dtype, device=qkv.device)
     scale = float(head_size ** -0.5 if scale is None else scale)
     lib = _lib.load()
-    _lib.check(lib.evt_window_attention_fwd(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), table.data_ptr(),
+    fn = lib.evt_window_attention_fwd if qkv.dtype == torch.bfloat16 else lib.evt_window_attention_fwd_tf32
+    _lib.check(fn(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), table.data_ptr(),
                                             table.shape[0], n_windows, window_tokens, heads, head_size, scale, _stream()),
                "window_attention")
     return ctx
 
 
-def layernorm_mean_tokens(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, images: int, T: int) -> torch.Tensor:
-    """mean over tokens of LayerNorm(x): x f32 [images*T, D] -> bf16 [images, D] (Swin final norm + pooler)."""
+def layernorm_mean_tokens(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, images: int, T: int,
+                          out_dtype=torch.bfloat16) -> torch.Tensor:
+    """mean over tokens of LayerNorm(x): x f32 [images*T, D] -> [images, D] bf16 or TF32 (Swin final norm + pooler)."""
     _need_cuda(x, gamma, beta)
     if x.dtype != torch.float32 or x.dim() != 2 or not x.is_contiguous() or x.shape[0] != images * T:
         raise ValueError("layernorm_mean_tokens wants a contiguous f32 [images*T, D] matrix")
-    y = torch.empty((images, x.shape[1]), dtype=torch.bfloat16, device=x.device)
+    if out_dtype not in (torch.bfloat16, TF32):
+        raise ValueError("layernorm_mean_tokens: out_dtype must be bf16 or TF32")
+    y = torch.empty((images, x.shape[1]), dtype=_storage(out_dtype), device=x.device)
     lib = _lib.load()
-    _lib.check(lib.evt_layernorm_mean_tokens(x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), images, T, x.shape[1],
-                                             float(eps), _stream()), "layernorm_mean_tokens")
+    _lib.check(lib.evt_layernorm_mean_tokens_ex(x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), _dt(y, out_dtype), images,
+                                                T, x.shape[1], float(eps), _stream()), "layernorm_mean_tokens")
     return y
 
 
-def im2col_patch(pixels: torch.Tensor, patch: int = 16) -> torch.Tensor:
+def im2col_patch(pixels: torch.Tensor, patch: int = 16, out_dtype=torch.bfloat16) -> torch.Tensor:
+    """f32 NCHW pixels -> the patch matrix [B*(H/P)*(W/P), 3*P*P] in (c, i, j) order, bf16 or TF32."""
     _need_cuda(pixels)
+    if out_dtype not in (torch.bfloat16, TF32):
+        raise ValueError("im2col_patch: out_dtype must be bf16 or TF32")
     if pixels.dtype != torch.float32 or pixels.dim() != 4 or pixels.shape[1] != 3:
         raise ValueError("im2col_patch wants f32 NCHW pixels with 3 channels")
     pixels = pixels.contiguous()
     B, _, H, W = pixels.shape
-    cols = torch.empty((B * (H // patch) * (W // patch), 3 * patch * patch), dtype=torch.bfloat16, device=pixels.device)
+    cols = torch.empty((B * (H // patch) * (W // patch), 3 * patch * patch), dtype=_storage(out_dtype), device=pixels.device)
     lib = _lib.load()
-    _lib.check(lib.evt_im2col_patch(pixels.data_ptr(), cols.data_ptr(), B, H, W, patch, _stream()), "im2col")
+    _lib.check(lib.evt_im2col_patch_ex(pixels.data_ptr(), cols.data_ptr(), _dt(cols, out_dtype), B, H, W, patch, _stream()), "im2col")
     return cols
 
 

@@ -116,6 +116,13 @@ int evt_gemm_bias_act_tf32(const float* A, int64_t lda, const float* W, int64_t 
                            float* out, int64_t ldo, int out_group, int out_group_stride, int out_group_off,
                            int64_t M, int N, int K, int act, evt_stream stream);
 
+/* evt_gemm_bias_act_tf32 with a choice of output type: out_dtype EVT_F32, or EVT_TF32 (f32 rounded to nearest tf32: an output
+ * that feeds another tf32 GEMM or attention, as the QKV and FC1 outputs of the tf32 Swin forward; no residual then). */
+int evt_gemm_bias_act_tf32_ex(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
+                              const float* residual, int64_t ldr, int res_row_mod, int res_row_off,
+                              float* out, int out_dtype, int64_t ldo, int out_group, int out_group_stride, int out_group_off,
+                              int64_t M, int N, int K, int act, evt_stream stream);
+
 /* out[M,N] (bf16) = act( LayerNorm(x)[M,K] W[N,K]^T + bias ) -- the LayerNorm that precedes a projection, run inside
  * the GEMM as the producer of its A operand: layernorm_before -> query|key|value and layernorm_after ->
  * intermediate.dense of a ViT layer (SITE/models/vit/modeling_vit.py:333-340) for narrow residual streams, where the
@@ -177,6 +184,9 @@ int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ld
  * K order (c, i, j) -- the im2col of Conv2d(3,D,P,P) (SITE/models/vit/modeling_vit.py:151-167).  P a multiple of 4
  * (ViT / DeiT: 16; Swin: 4). */
 int evt_im2col_patch(const float* pixels, void* cols, int B, int H, int W, int P, evt_stream stream);
+/* evt_im2col_patch with a choice of output: out_dtype EVT_BF16 (as above) or EVT_TF32 (f32 [.., 3*P*P] rounded to nearest
+ * tf32: the A operand of a tf32 GEMM). */
+int evt_im2col_patch_ex(const float* pixels, void* cols, int out_dtype, int B, int H, int W, int P, evt_stream stream);
 
 /* ViTEmbeddings.forward as one op-level call (SITE/models/vit/modeling_vit.py:95-126 = cls / distillation token,
  * position embeddings; :151-167 = ViTPatchEmbeddings, Conv2d(3, D, P, P) as an im2col GEMM):
@@ -262,7 +272,8 @@ int evt_token_transformer_block_fwd(const void* qkv, int64_t ld, float* y, void*
  *   G = 1: window partition / cyclic shift / reverse (SwinLayer.forward :606-637) folded into layernorm_before;
  *          copy_f32 (nullable) receives the gathered, un-normalised rows = the residual stream in the new order
  *   G = 4: SwinPatchMerging (:326-349): 2x2 neighbourhood concat + LayerNorm(4C)
- *   y (nullable when copy_f32 is given): bf16 or f32 [images * T_out, G*C]; idx: int32 [T_out * G] (device). */
+ *   y (nullable when copy_f32 is given): y_dtype bf16, f32 or tf32 (f32 rounded to nearest tf32) [images * T_out, G*C];
+ *   idx: int32 [T_out * G] (device). */
 int evt_gather_layernorm(const float* x, const int* idx, const float* gamma, const float* beta, void* y, int y_dtype,
                          float* copy_f32, int64_t images, int T_in, int T_out, int G, int C, float eps, evt_stream stream);
 
@@ -278,10 +289,21 @@ int evt_gather_layernorm(const float* x, const int* idx, const float* gamma, con
 int evt_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, int n_tab,
                              int64_t n_windows, int window_tokens, int heads, int head_size, float scale, evt_stream stream);
 
+/* tf32 flavour of evt_window_attention_fwd (the Swin tf32 mode), same windows, table and checks:
+ *   qkv : f32 [n_windows * N, ldq], values tf32-representable (the tensor core reads them as tf32); ldq % 4 == 0, 16-byte aligned
+ *   ctx : f32 [n_windows * N, ldc], rounded to nearest tf32; ldc % 4 == 0, 16-byte aligned
+ * Scores accumulate in f32; each probability exp2(s - max) is rounded to tf32 before P V, and the row sum is taken over the
+ * rounded values (the arithmetic of evt_attention_fwd_tf32). */
+int evt_window_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* table, int n_tab,
+                                  int64_t n_windows, int window_tokens, int heads, int head_size, float scale, evt_stream stream);
+
 /* y[image, :] (bf16) = mean over the T tokens of LayerNorm(x[image, t, :]) -- SwinModel.layernorm + AdaptiveAvgPool1d
  * (:899-904).  x f32 [images, T, D]. */
 int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D,
                               float eps, evt_stream stream);
+/* The same with y_dtype EVT_BF16 or EVT_TF32 (f32 rounded to nearest tf32). */
+int evt_layernorm_mean_tokens_ex(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T,
+                                 int D, float eps, evt_stream stream);
 
 /* ------------------------------------------------------------------ model level ---------- */
 
@@ -400,8 +422,8 @@ int evt_model_destroy(evt_model* m);
 /* The shifted-window classifier the reference builds with utils.get_swin (utils.py:14-47) and exports / benchmarks in
  * tools.py:265-292 (swin_{tiny,small,base}_patch4_window7_224), arithmetic as in SITE/models/swin/modeling_swin.py;
  * also the 384-pixel swin_{base,large}_patch4_window12_384 (12 x 12 windows).
- * One call = the whole forward as a fixed launch sequence on `stream` (CUDA-graph capturable).  bf16 operands, f32
- * accumulate / residual stream / LayerNorm / softmax. */
+ * One call = the whole forward as a fixed launch sequence on `stream` (CUDA-graph capturable).  f32 accumulate / residual
+ * stream / LayerNorm / softmax; GEMM and attention operands bf16 or tf32 (spec.precision, the same launches either way). */
 typedef struct evt_swin evt_swin;
 
 #define EVT_SWIN_MAX_STAGES 8
@@ -414,6 +436,8 @@ typedef struct evt_swin_spec {
   int heads[EVT_SWIN_MAX_STAGES];    /* heads per stage, e.g. 3, 6, 12, 24 */
   int num_labels;
   float eps;                         /* LayerNorm epsilon (1e-5) */
+  int precision;                     /* evt_precision: 0 bf16 operands (logits within 2e-2 of fp32), 1 tf32 operands (f32
+                                        activations rounded to tf32, logits within 1e-3); last, so a zeroed spec is bf16 */
 } evt_swin_spec;
 
 int evt_swin_create(const evt_swin_spec* spec, evt_swin** out);
