@@ -79,6 +79,26 @@ def _random_t2t_weights(hidden, depth, heads, mlp_ratio, seed=0):
     return sd
 
 
+def _random_deit3(name: str, seed: int = 0):
+    """A models_v2-layout DeiT III state dict of the named shape: N(0, 0.02) weights, LayerScale gamma 0.1, unit norms."""
+    from ..modeling_vit import DEIT3
+    D, _, P, image = DEIT3[name]
+    depth = {384: 12, 512: 12, 768: 12, 1024: 24, 1280: 32}[D]
+    g = torch.Generator().manual_seed(seed)
+    r = lambda *s: torch.randn(*s, generator=g) * 0.02  # noqa: E731
+    sd = {"cls_token": r(1, 1, D), "pos_embed": r(1, (image // P) ** 2, D), "patch_embed.proj.weight": r(D, 3, P, P),
+          "patch_embed.proj.bias": r(D), "norm.weight": torch.ones(D), "norm.bias": torch.zeros(D), "head.weight": r(1000, D),
+          "head.bias": torch.zeros(1000)}
+    for l in range(depth):
+        p = f"blocks.{l}."
+        sd.update({p + "norm1.weight": torch.ones(D), p + "norm1.bias": torch.zeros(D), p + "attn.qkv.weight": r(3 * D, D),
+                   p + "attn.qkv.bias": r(3 * D), p + "attn.proj.weight": r(D, D), p + "attn.proj.bias": r(D),
+                   p + "norm2.weight": torch.ones(D), p + "norm2.bias": torch.zeros(D), p + "mlp.fc1.weight": r(4 * D, D),
+                   p + "mlp.fc1.bias": r(4 * D), p + "mlp.fc2.weight": r(D, 4 * D), p + "mlp.fc2.bias": r(D),
+                   p + "gamma_1": torch.full((D,), 0.1), p + "gamma_2": torch.full((D,), 0.1)})
+    return sd
+
+
 def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", image_size: int = 224, **op_kw):
     """-> (callable taking one CUDA tensor, input shape without batch, description).  image_size: deit_* and swin_* (224 or
     384: deit_*_patch16_{224,384}, swin_*_patch4_window7_224 / swin_*_patch4_window12_384)."""
@@ -87,6 +107,11 @@ def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device
         m = B200ViTForImageClassification.from_hf(_random_hf(name, image_size=image_size), device=device, max_batch=max_batch,
                                                   precision=precision, keep_params=False)
         return m, (3, image_size, image_size), f"{name} random-init ({precision}, {image_size} px)"
+    from ..modeling_vit import DEIT3
+    if name in DEIT3:
+        from .. import modeling_vit
+        m = getattr(modeling_vit, name)(_random_deit3(name), device=device, max_batch=max_batch, precision=precision, keep_params=False)
+        return m, (3, m.config.image_size, m.config.image_size), f"{name} random-init ({precision})"
     if name in T2T:
         from ..modeling_t2t import B200T2TViT
         hidden, depth, heads, ratio = T2T[name]
@@ -148,7 +173,7 @@ def b200_benchmark(model, input_shape: Sequence[int], num_runs: int = 50, warmup
 
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="b200_benchmark", description=__doc__.split("\n")[0])
-    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir | T2T-ViT .pth[.tar]")
+    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | deit3_* (modeling_vit.DEIT3) | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir | T2T-ViT .pth[.tar]")
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--precision", default="bf16", choices=["bf16", "tf32"])
     ap.add_argument("--num_runs", type=int, default=50)

@@ -19,7 +19,8 @@
 // SK = S rounded up to 16; key columns >= S are masked to probability 0, so the extra K/V rows the TMA box
 // picks up (next image's tokens, or zero fill past the end of the matrix) never contribute.
 // TMEM: 2 slots x 256 columns (S at [0,SK), P overlaid at [0,SK/2), O overlaid at [128,192)).
-// Longer sequences (257 .. EVT_ATTN_MAX_TOKENS) run attention_long_kernel below; attention_launch picks by S.
+// Longer sequences (257 .. EVT_ATTN_MAX_TOKENS) run attention_long_kernel below; attention_launch picks by S.  Head size 80
+// runs attention_long_kernel<80> at every S.
 #include <cuda_bf16.h>
 
 #include <math_constants.h>
@@ -262,12 +263,12 @@ struct AttnSmem {
   uint64_t* slot_free;  // [2] softmax group (4 warps, O read out) -> QK issuer
   uint32_t* tmem_ptr;
 };
-__device__ __forceinline__ AttnSmem attn_smem(uint8_t* smem_raw, int kv_ring_bytes) {
+__device__ __forceinline__ AttnSmem attn_smem(uint8_t* smem_raw, int kv_ring_bytes, int q_tile_bytes = kQTileBytes) {
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   AttnSmem m;
   m.kv_ring = smem;
   m.q_ring = smem + kv_ring_bytes;
-  m.staging = m.q_ring + 2 * kQTileBytes;
+  m.staging = m.q_ring + 2 * q_tile_bytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(m.staging + kSoftmaxWarps * kStgWarpBytes);
   m.kv_full = bars;
   m.kv_empty = bars + kMaxKV;
@@ -317,14 +318,31 @@ __device__ __forceinline__ uint32_t attn_prologue(int warp, const AttnSmem& sm, 
 // warp's 32 rows of O (TMEM lane row t_row), release the slot (slot_free), then O * hm / sum -> bf16, row per thread, into
 // the warp's 128B-swizzled staging tile (16-byte piece i of row r at piece i ^ (r & 7)) and a 3-D TMA store of the tile at
 // (col, row, img); rows past the end of the tensor map are clipped.  A warp with no live row only takes part in the barriers.
+// HD = 80: O columns 64..79 go straight from registers to `tail` (this thread's row, 32 bytes; null for a row past Sq).
+template <int HD = 64>
 __device__ __forceinline__ void store_context(float sum, float hm, bool warp_live, uint64_t* pv_done, uint32_t phase,
                                               uint64_t* slot_free, uint32_t t_row, uint8_t* stg, const CUtensorMap* tmO, int col,
-                                              int row, int img) {
+                                              int row, int img, __nv_bfloat16* tail = nullptr) {
+  static_assert(HD == 64 || HD == 80, "head size 64 or 80");
   const int lane = threadIdx.x & 31;
   const float inv = ptx::rcp_approx(sum) * hm;  // sum >= 1 (the maximum contributes 2^0)
   if (warp_live && ptx::elect_one()) ptx::bulk_wait_read<0>();  // the previous context tile has left the staging buffer
   ptx::mbar_wait(pv_done, phase);
   ptx::tc_fence_after();
+  if constexpr (HD == 80) {  // columns 64..79 first, so that they are never live beside the other 64
+    if (warp_live) {
+      uint32_t o2[16];
+      ptx::tmem_ld_x16(t_row + kOCol + 64, o2);
+      ptx::tmem_ld_wait();
+      if (tail != nullptr) {
+        uint32_t w[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) w[j] = ptx::pack_bf16x2(__uint_as_float(o2[2 * j]) * inv, __uint_as_float(o2[2 * j + 1]) * inv);
+        reinterpret_cast<uint4*>(tail)[0] = make_uint4(w[0], w[1], w[2], w[3]);
+        reinterpret_cast<uint4*>(tail)[1] = make_uint4(w[4], w[5], w[6], w[7]);
+      }
+    }
+  }
   uint32_t o0[32], o1[32];
   if (warp_live) {
     ptx::tmem_ld_x32(t_row + kOCol, o0);
@@ -540,8 +558,14 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
 //                      kRescaleLog2 (log2 units); only then are O and the sum multiplied by 2^(mu - mu_new).  In between
 //                      P <= 2^kRescaleLog2, and O and the sum share the same stale maximum, so the quotient is exact.
 //                      Every decision is per row: a row comes out the same whatever Sq is and whatever its neighbours hold.
+//
+// Head size 80 (attention_long_kernel<80>, every S from 1 to EVT_ATTN_MAX_TOKENS): a 160-byte bf16 row is wider than one
+// 128-byte swizzle atom, so every Q tile and K / V block is two operands: columns 0..63 as before (SW128, tmQ / tmKV) and
+// columns 64..79 as a 32-byte-swizzled one (SW32, tmQ32 / tmKV32).  S = Q K^T is four SW128 K-steps plus one SW32 K-step;
+// O = P V is N = 64 from the SW128 V plus N = 16 from the SW32 V (both MN-major) into TMEM columns [128, 208).  A ring stage
+// is 40 KB, so the ring has 3 stages instead of 4.  O columns 64..79 leave by direct 32-byte stores beside the TMA store.
 constexpr int kKeyBlock = 128;
-constexpr int kKeyBlockBytes = kKeyBlock * 128;  // one K or V block, 128 keys x 64 bf16
+constexpr int kKeyBlockBytes = kKeyBlock * 128;  // 128 keys (or query rows) x 64 bf16: the SW128 part of a block or Q tile
 constexpr int kLongStages = 4;
 static_assert(kLongStages == kMaxKV, "attn_prologue initialises kMaxKV K/V stages");
 constexpr float kRescaleLog2 = 8.f;
@@ -553,6 +577,14 @@ struct AttnLongParams {
   int q_tiles;   // query tiles per (image, head)
   int n_items;   // B * heads * q_tiles
   float scale_log2e;
+  __nv_bfloat16* ctx;  // head size 80: context columns 64..79 are stored through this ([B*Sq, ldc])
+  long long ldc;
+};
+template <int HD>
+struct LongShape {
+  static constexpr int kStages = HD == 64 ? kLongStages : 3;
+  static constexpr int kBlockBytes = kKeyBlock * HD * 2;  // one K or V block: the SW128 part, then (HD = 80) the SW32 part
+  static constexpr int kQBytes = kQRows * HD * 2;
 };
 
 struct LongItem {
@@ -575,9 +607,9 @@ __device__ __forceinline__ int groups_of(const AttnLongParams& p, int ql) { retu
 
 // One 128-key block of the online softmax for the query row at t_row (nvalid: valid keys in the block, 1..128).  mu is
 // the row's current maximum times scale * log2(e), sum its running sum; both are updated, and O (TMEM columns
-// [kOCol, kOCol + 64)) is rescaled with them when the maximum moves (has_o: O already holds earlier blocks).
+// [kOCol, kOCol + HD)) is rescaled with them when the maximum moves (has_o: O already holds earlier blocks).
 // bf16 P is written over the consumed S columns; the caller issues tcgen05.wait::st.
-template <bool MASKED>
+template <int HD, bool MASKED>
 __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool has_o, float scale_log2e, float& mu, float& sum) {
   const uint64_t scale2 = ptx::pk2(scale_log2e, scale_log2e);
   uint32_t ra[16], rb[16];
@@ -601,8 +633,15 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
     sum *= alpha;
   }
   if (has_o && __any_sync(0xffffffffu, grow)) {
+    if constexpr (HD % 32 != 0) {  // O columns [64, 80)
+      ptx::tmem_ld_x16(t_row + kOCol + HD - 16, ra);
+      ptx::tmem_ld_wait();
 #pragma unroll
-    for (int c = 0; c < kHD / 16; c += 2) {
+      for (int j = 0; j < 16; ++j) ra[j] = __float_as_uint(__uint_as_float(ra[j]) * alpha);
+      ptx::tmem_st_x16(t_row + kOCol + HD - 16, ra);
+    }
+#pragma unroll
+    for (int c = 0; c + 1 < HD / 16; c += 2) {
       ptx::tmem_ld_x16(t_row + kOCol + c * 16, ra);
       ptx::tmem_ld_x16(t_row + kOCol + (c + 1) * 16, rb);
       ptx::tmem_ld_wait();
@@ -636,14 +675,17 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
   sum += (s0 + s1) + (s2 + s3);
 }
 
+template <int HD>
 __global__ void __launch_bounds__(kThreads2, 1)
 attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
-                      const __grid_constant__ CUtensorMap tmO, const AttnLongParams p) {
+                      const __grid_constant__ CUtensorMap tmO, const AttnLongParams p, const __grid_constant__ CUtensorMap tmQ32,
+                      const __grid_constant__ CUtensorMap tmKV32) {
+  using LS = LongShape<HD>;
   extern __shared__ uint8_t smem_raw[];
-  const AttnSmem sm = attn_smem(smem_raw, kLongStages * 2 * kKeyBlockBytes);  // ring: kLongStages x (K | V) blocks
+  const AttnSmem sm = attn_smem(smem_raw, LS::kStages * 2 * LS::kBlockBytes, LS::kQBytes);  // ring: kStages x (K | V) blocks
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int a = p.heads * kHD;
+  const int a = p.heads * HD;
   const int n_units = (p.n_items + 1) / 2;
   const int my_units = (n_units - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
   const uint32_t tmem_base = attn_prologue(warp, sm, &tmQ, &tmKV, &tmO, 1);
@@ -659,20 +701,26 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         for (int g = 0; g < n_g; ++g) {
           const LongItem it = long_item(p, item_index(ql, g));
           ptx::mbar_wait(&sm.q_empty[g], (ql & 1) ^ 1);
-          ptx::mbar_arrive_expect_tx(&sm.q_full[g], kQTileBytes);
+          ptx::mbar_arrive_expect_tx(&sm.q_full[g], LS::kQBytes);
 #pragma unroll
           for (int q = 0; q < 4; ++q)  // rows past Sq arrive as zeros
-            ptx::tma_load_3d(sm.q_ring + g * kQTileBytes + q * kStgWarpBytes, &tmQ, &sm.q_full[g], it.h * kHD, it.mt * kQRows + 32 * q, it.b);
+            ptx::tma_load_3d(sm.q_ring + g * LS::kQBytes + q * kStgWarpBytes, &tmQ, &sm.q_full[g], it.h * HD, it.mt * kQRows + 32 * q, it.b);
+          if constexpr (HD == 80)
+            ptx::tma_load_3d(sm.q_ring + g * LS::kQBytes + kKeyBlockBytes, &tmQ32, &sm.q_full[g], it.h * HD + 64, it.mt * kQRows, it.b);
         }
         for (int kb = 0; kb < p.n_kb; ++kb) {
           for (int g = 0; g < n_g; ++g) {
             const LongItem it = long_item(p, item_index(ql, g));
             ptx::mbar_wait(&sm.kv_empty[t], kph ^ 1);
-            uint8_t* sK = sm.kv_ring + t * 2 * kKeyBlockBytes;
-            ptx::mbar_arrive_expect_tx(&sm.kv_full[t], 2 * kKeyBlockBytes);
-            ptx::tma_load_3d(sK, &tmKV, &sm.kv_full[t], a + it.h * kHD, kb * kKeyBlock, it.b);
-            ptx::tma_load_3d(sK + kKeyBlockBytes, &tmKV, &sm.kv_full[t], 2 * a + it.h * kHD, kb * kKeyBlock, it.b);
-            if (++t == kLongStages) {
+            uint8_t* sK = sm.kv_ring + t * 2 * LS::kBlockBytes;
+            ptx::mbar_arrive_expect_tx(&sm.kv_full[t], 2 * LS::kBlockBytes);
+            ptx::tma_load_3d(sK, &tmKV, &sm.kv_full[t], a + it.h * HD, kb * kKeyBlock, it.b);
+            ptx::tma_load_3d(sK + LS::kBlockBytes, &tmKV, &sm.kv_full[t], 2 * a + it.h * HD, kb * kKeyBlock, it.b);
+            if constexpr (HD == 80) {
+              ptx::tma_load_3d(sK + kKeyBlockBytes, &tmKV32, &sm.kv_full[t], a + it.h * HD + 64, kb * kKeyBlock, it.b);
+              ptx::tma_load_3d(sK + LS::kBlockBytes + kKeyBlockBytes, &tmKV32, &sm.kv_full[t], 2 * a + it.h * HD + 64, kb * kKeyBlock, it.b);
+            }
+            if (++t == LS::kStages) {
               t = 0;
               kph ^= 1;
             }
@@ -698,14 +746,17 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
               ptx::mbar_wait(&sm.pv_done[g], (ql * p.n_kb + kb - 1) & 1);  // the previous block's P has been read
             }
             ptx::tc_fence_after();
-            const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(sm.q_ring + g * kQTileBytes));
-            const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + t * 2 * kKeyBlockBytes));
+            const uint64_t qd = ptx::smem_desc_sw128(ptx::smem_u32(sm.q_ring + g * LS::kQBytes));
+            const uint64_t kd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + t * 2 * LS::kBlockBytes));
             const uint32_t slot = tmem_base + g * kSlotCols;
 #pragma unroll
-            for (int k = 0; k < kHD / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
+            for (int k = 0; k < 64 / 16; ++k) ptx::mma_f16_ss(slot, qd + 2 * k, kd + 2 * k, idesc_qk, k != 0 ? 1u : 0u);
+            if constexpr (HD == 80)
+              ptx::mma_f16_ss(slot, ptx::smem_desc_sw32(ptx::smem_u32(sm.q_ring + g * LS::kQBytes + kKeyBlockBytes)),
+                              ptx::smem_desc_sw32(ptx::smem_u32(sm.kv_ring + t * 2 * LS::kBlockBytes + kKeyBlockBytes)), idesc_qk, 1u);
             ptx::mma_commit(&sm.s_ready[g]);
             if (kb == p.n_kb - 1) ptx::mma_commit(&sm.q_empty[g]);
-            if (++t == kLongStages) {
+            if (++t == LS::kStages) {
               t = 0;
               kph ^= 1;
             }
@@ -716,7 +767,8 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   } else if (warp == kPVWarp) {
     // ------------------------------------------------------------ O += P V issuer
     if (ptx::elect_one()) {
-      const uint32_t idesc_pv = ptx::make_idesc(kQRows, kHD, 1, 0, 1);
+      const uint32_t idesc_pv = ptx::make_idesc(kQRows, 64, 1, 0, 1);
+      const uint32_t idesc_pv16 = ptx::make_idesc(kQRows, 16, 1, 0, 1);
       int t = 0;
       uint32_t kph = 0;
       for (int ql = 0; ql < my_units; ++ql) {
@@ -726,14 +778,19 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
             ptx::mbar_wait(&sm.kv_full[t], kph);  // complete long ago (S of this block exists); taken for the memory ordering
             ptx::mbar_wait(&sm.p_ready[g], (ql * p.n_kb + kb) & 1);
             ptx::tc_fence_after();
-            const uint64_t vd = ptx::smem_desc_sw128(ptx::smem_u32(sm.kv_ring + t * 2 * kKeyBlockBytes + kKeyBlockBytes));
+            const uint32_t v_addr = ptx::smem_u32(sm.kv_ring + t * 2 * LS::kBlockBytes + LS::kBlockBytes);
+            const uint64_t vd = ptx::smem_desc_sw128(v_addr);
             const uint32_t slot = tmem_base + g * kSlotCols;
 #pragma unroll
-            for (int k = 0; k < kKeyBlock / 16; ++k)
+            for (int k = 0; k < kKeyBlock / 16; ++k) {
               ptx::mma_f16_ts(slot + kOCol, slot + 8 * k, vd + static_cast<uint64_t>(128 * k), idesc_pv, (kb | k) != 0 ? 1u : 0u);
+              if constexpr (HD == 80)  // 16 keys x 32 B = 512 B per K-step
+                ptx::mma_f16_ts(slot + kOCol + 64, slot + 8 * k, ptx::smem_desc_sw32(v_addr + kKeyBlockBytes) + static_cast<uint64_t>(32 * k),
+                                idesc_pv16, (kb | k) != 0 ? 1u : 0u);
+            }
             ptx::mma_commit(&sm.pv_done[g]);
             ptx::mma_commit(&sm.kv_empty[t]);
-            if (++t == kLongStages) {
+            if (++t == LS::kStages) {
               t = 0;
               kph ^= 1;
             }
@@ -765,16 +822,20 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         if (kb != 0) ptx::mbar_wait(&sm.pv_done[grp], (c0 + kb - 1) & 1);  // O may be rescaled below
         ptx::tc_fence_after();
         if (warp_live) {
-          if (kb != p.n_kb - 1) softmax_block<false>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum);
-          else softmax_block<true>(t_row, last_valid, kb != 0, p.scale_log2e, mu, sum);
+          if (kb != p.n_kb - 1) softmax_block<HD, false>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum);
+          else softmax_block<HD, true>(t_row, last_valid, kb != 0, p.scale_log2e, mu, sum);
           ptx::tmem_st_wait();
         }
         ptx::tc_fence_before();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&sm.p_ready[grp]);
       }
-      store_context(sum, hm, warp_live, &sm.pv_done[grp], (c0 + p.n_kb - 1) & 1, &sm.slot_free[grp], t_row, stg, &tmO, u.h * kHD,
-                    qrow0, u.b);
+      __nv_bfloat16* tail = nullptr;
+      if constexpr (HD == 80) {
+        if (qrow0 + lane < p.Sq) tail = p.ctx + (static_cast<long long>(u.b) * p.Sq + qrow0 + lane) * p.ldc + u.h * HD + 64;
+      }
+      store_context<HD>(sum, hm, warp_live, &sm.pv_done[grp], (c0 + p.n_kb - 1) & 1, &sm.slot_free[grp], t_row, stg, &tmO, u.h * HD,
+                        qrow0, u.b, tail);
     }
     if (ptx::elect_one()) ptx::bulk_wait<0>();
   }
@@ -963,9 +1024,11 @@ attention_tf32_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   }
 }
 
-// S > 256: attention_long_kernel.  Argument checks are the caller's (attention_launch).
+// S > 256 (head size 64) or any S (head size 80): attention_long_kernel.  Argument checks are the caller's.
+template <int HD>
 int attention_long_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                           int heads, float scale, cudaStream_t stream) {
+  using LS = LongShape<HD>;
   AttnLongParams q;
   q.head_mask = head_mask;
   q.S = S;
@@ -977,24 +1040,37 @@ int attention_long_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, 
   EVT_CHECK_ARG(n_items < (1ll << 30), "attention: B * heads * query tiles too large");
   q.n_items = static_cast<int>(n_items);
   q.scale_log2e = scale * 1.4426950408889634f;
-  CUtensorMap tmQ, tmKV, tmO;
+  q.ctx = static_cast<__nv_bfloat16*>(ctx);
+  q.ldc = ldc;
+  CUtensorMap tmQ, tmKV, tmO, tmQ32, tmKV32;
   // K / V: 128-key blocks of one image (keys past S arrive as zeros); Q: the first Sq rows of every image; context packed
-  int rc = make_tmap_3d_rows(&tmKV, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
-                             static_cast<uint64_t>(ldq), kKeyBlock, kHD, static_cast<uint64_t>(S));
+  int rc = make_tmap_3d_rows(&tmKV, qkv, 2, 3ull * heads * HD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
+                             static_cast<uint64_t>(ldq), kKeyBlock, 64, static_cast<uint64_t>(S));
   if (rc != EVT_OK) return rc;
-  rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
-                         static_cast<uint64_t>(ldq), 32, kHD, static_cast<uint64_t>(S));
+  rc = make_tmap_3d_rows(&tmQ, qkv, 2, 3ull * heads * HD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                         static_cast<uint64_t>(ldq), 32, 64, static_cast<uint64_t>(S));
   if (rc != EVT_OK) return rc;
-  rc = make_tmap_3d_rows(&tmO, ctx, 2, static_cast<uint64_t>(heads) * kHD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
-                         static_cast<uint64_t>(ldc), 32, kHD);
+  rc = make_tmap_3d_rows(&tmO, ctx, 2, static_cast<uint64_t>(heads) * HD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                         static_cast<uint64_t>(ldc), 32, 64);
   if (rc != EVT_OK) return rc;
+  if (HD == 80) {  // the SW32 parts: head columns 64..79
+    rc = make_tmap_3d_rows_sw32(&tmKV32, qkv, 3ull * heads * HD, static_cast<uint64_t>(S), static_cast<uint64_t>(B),
+                                static_cast<uint64_t>(ldq), kKeyBlock, static_cast<uint64_t>(S));
+    if (rc != EVT_OK) return rc;
+    rc = make_tmap_3d_rows_sw32(&tmQ32, qkv, 3ull * heads * HD, static_cast<uint64_t>(Sq), static_cast<uint64_t>(B),
+                                static_cast<uint64_t>(ldq), kQRows, static_cast<uint64_t>(S));
+    if (rc != EVT_OK) return rc;
+  } else {
+    tmQ32 = tmQ;  // not read
+    tmKV32 = tmKV;
+  }
   const long long units = (n_items + 1) / 2;
   const int grid = units < num_sms() ? static_cast<int>(units) : num_sms();
-  const int smem = 1024 + kLongStages * 2 * kKeyBlockBytes + 2 * kQTileBytes + kSoftmaxWarps * kStgWarpBytes +
-                   (2 * kLongStages + 12) * 8 + 16;
-  EVT_TRY(opt_in_smem<attention_long_kernel>(smem));
-  const bool pdl = pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * kHD);
-  EVT_CUDA(launch_pdl(attention_long_kernel, dim3(grid), dim3(kThreads2), smem, stream, pdl, tmQ, tmKV, tmO, q));
+  const int smem = 1024 + LS::kStages * 2 * LS::kBlockBytes + 2 * LS::kQBytes + kSoftmaxWarps * kStgWarpBytes +
+                   (2 * kMaxKV + 12) * 8 + 16;
+  EVT_TRY(opt_in_smem<attention_long_kernel<HD>>(smem));
+  const bool pdl = pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * HD);
+  EVT_CUDA(launch_pdl(attention_long_kernel<HD>, dim3(grid), dim3(kThreads2), smem, stream, pdl, tmQ, tmKV, tmO, q, tmQ32, tmKV32));
   EVT_LAUNCH_CHECK("attention_long_kernel");
   return EVT_OK;
 }
@@ -1006,9 +1082,15 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
   EVT_CHECK_ARG(qkv && ctx, "attention: null pointer");
   EVT_CHECK_ARG(B > 0 && S > 0 && heads > 0, "attention: B, S, heads must be positive");
   EVT_CHECK_ARG(Sq > 0 && Sq <= S, "attention: query rows must be in 1..S");
-  if (head_size != kHD) return fail(EVT_ERR_UNSUPPORTED, "attention: only head size 64 is implemented");
+  if (head_size != kHD && head_size != 80) return fail(EVT_ERR_UNSUPPORTED, "attention: only head sizes 64 and 80 are implemented");
   if (S > EVT_ATTN_MAX_TOKENS)
     return fail(EVT_ERR_UNSUPPORTED, "attention: sequence length above " + std::to_string(EVT_ATTN_MAX_TOKENS) + " is not implemented");
+  if (head_size == 80) {  // the key-blocked kernel at every S
+    EVT_CHECK_ARG(ldq >= 3ll * heads * 80 && ldc >= static_cast<int64_t>(heads) * 80, "attention: leading dimension too small");
+    EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention: ctx must be 16-byte aligned rows");
+    EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");
+    return attention_long_launch<80>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
+  }
   return attention_any_length_launch(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
 }
 
@@ -1024,7 +1106,7 @@ int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t
   EVT_CHECK_ARG(ldq >= 3ll * heads * kHD && ldc >= static_cast<int64_t>(heads) * kHD, "attention: leading dimension too small");
   EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention: ctx must be 16-byte aligned rows");
   EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");
-  if (S > 256) return attention_long_launch(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
+  if (S > 256) return attention_long_launch<kHD>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
   const int SK = (S + 15) / 16 * 16;
   const uint64_t rows = static_cast<uint64_t>(B) * S;
   const int q_tiles = (Sq + kQRows - 1) / kQRows;

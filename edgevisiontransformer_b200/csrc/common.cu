@@ -101,7 +101,8 @@ static int encode_tmap(CUtensorMap* out, const void* base, int elem_bytes, int r
   const cuuint32_t estr[3] = {1, 1, 1};
   CUresult r = enc(out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, const_cast<void*>(base),
                    dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(EVT_ERR_CUDA, std::string("cuTensorMapEncodeTiled") + what + " failed with CUresult " + std::to_string((int)r));
   return EVT_OK;
@@ -132,6 +133,13 @@ int make_tmap_3d_rows(CUtensorMap* out, const void* base, int elem_bytes, uint64
   if (!err && elem_bytes != 2) err = "3-D TMA map: bf16 only";
   if (!err && batch_rows != 0 && batch_rows < rows) err = "3-D TMA map: batch entries closer than their row count";
   return encode_tmap(out, base, elem_bytes, 3, cols, rows, batch, ld, box_rows, box_cols, 128, err, " (3-D)", batch_rows);
+}
+
+int make_tmap_3d_rows_sw32(CUtensorMap* out, const void* base, uint64_t cols, uint64_t rows, uint64_t batch, uint64_t ld,
+                           uint32_t box_rows, uint64_t batch_rows) {
+  const char* err = box_rows > 256 || box_rows == 0 ? "TMA box must be at most 256 rows" : nullptr;
+  if (!err && batch_rows != 0 && batch_rows < rows) err = "3-D TMA map: batch entries closer than their row count";
+  return encode_tmap(out, base, 2, 3, cols, rows, batch, ld, box_rows, 16, 32, err, " (3-D, 32B swizzle)", batch_rows);
 }
 
 }  // namespace evt

@@ -146,5 +146,8 @@ int make_tmap_2d_sw(CUtensorMap* out, const void* base, int elem_bytes, uint64_t
 // batch_rows: matrix rows from one batch entry to the next (0 = rows; more: only the first `rows` of each entry are in view).
 int make_tmap_3d_rows(CUtensorMap* out, const void* base, int elem_bytes, uint64_t cols, uint64_t rows, uint64_t batch,
                       uint64_t ld, uint32_t box_rows, uint32_t box_cols, uint64_t batch_rows = 0);
+// make_tmap_3d_rows for bf16 boxes 16 columns (32 bytes) wide, 32-byte swizzle: the columns of a head past its first 64.
+int make_tmap_3d_rows_sw32(CUtensorMap* out, const void* base, uint64_t cols, uint64_t rows, uint64_t batch, uint64_t ld,
+                           uint32_t box_rows, uint64_t batch_rows);
 
 }  // namespace evt

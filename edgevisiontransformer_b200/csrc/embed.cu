@@ -82,6 +82,54 @@ __global__ void __launch_bounds__(256) im2col_kernel(const TIN* __restrict__ px,
   }
 }
 
+// P = 14 (deit_huge_patch14): an 8-pixel run of an image row crosses patch borders, so this gather is organised by output
+// instead: one thread = 8 consecutive columns of one patch row (16 B of bf16 or 32 B of tf32-rounded f32 out), each read
+// from its (c, i, j) pixel.  The row is kPatchLd14 = 592 wide (588 = 3 * 14 * 14 rounded up to 16-byte TMA rows); columns
+// 588..591 are written as zeros.  Consecutive threads walk one patch row, so a warp reads a few 56-byte pixel runs.
+__device__ __forceinline__ float ld1(const float* p) { return *p; }
+__device__ __forceinline__ float ld1(const __nv_bfloat16* p) { return __bfloat162float(*p); }
+__device__ __forceinline__ float ld1(const uint8_t* p) { return static_cast<float>(*p); }
+template <typename TIN, bool OUT_BF16, bool AFFINE>
+__global__ void __launch_bounds__(256) im2col14_kernel(const TIN* __restrict__ px, void* __restrict__ cols_, int H, int W,
+                                                       long long total, int row_stride, int row_off, const PixAffine af) {
+  constexpr int P = 14, K = 3 * P * P, Q = kPatchLd14 / 8;
+  ptx::grid_dep_launch();
+  ptx::grid_dep_wait();
+  const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  const int q = static_cast<int>(t % Q);
+  const long long r = t / Q;  // b * patches + patch
+  const int gw = W / P, patches = (H / P) * gw;
+  const int patch = static_cast<int>(r % patches);
+  const long long b = r / patches;
+  const int y0 = (patch / gw) * P, x0 = (patch % gw) * P;
+  float v[8];
+#pragma unroll
+  for (int e = 0; e < 8; ++e) {
+    const int k = q * 8 + e;
+    v[e] = 0.f;
+    if (k < K) {
+      const int c = k / (P * P), i = (k / P) % P, j = k % P;
+      v[e] = ld1(px + ((b * 3 + c) * H + y0 + i) * static_cast<long long>(W) + x0 + j);
+      if (AFFINE) v[e] = fmaf(v[e], c == 0 ? af.scale[0] : c == 1 ? af.scale[1] : af.scale[2],
+                              c == 0 ? af.bias[0] : c == 1 ? af.bias[1] : af.bias[2]);
+    }
+  }
+  const long long row = b * row_stride + row_off + patch;
+  if (OUT_BF16) {
+    uint4 o;
+    o.x = ptx::pack_bf16x2(v[0], v[1]);
+    o.y = ptx::pack_bf16x2(v[2], v[3]);
+    o.z = ptx::pack_bf16x2(v[4], v[5]);
+    o.w = ptx::pack_bf16x2(v[6], v[7]);
+    *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(cols_) + row * kPatchLd14 + q * 8) = o;
+  } else {
+    float* dst = reinterpret_cast<float*>(cols_) + row * kPatchLd14 + q * 8;
+    *reinterpret_cast<float4*>(dst) = make_float4(ptx::round_tf32(v[0]), ptx::round_tf32(v[1]), ptx::round_tf32(v[2]), ptx::round_tf32(v[3]));
+    *reinterpret_cast<float4*>(dst + 4) = make_float4(ptx::round_tf32(v[4]), ptx::round_tf32(v[5]), ptx::round_tf32(v[6]), ptx::round_tf32(v[7]));
+  }
+}
+
 __global__ void __launch_bounds__(256) prefix_tokens_kernel(const float* __restrict__ prefix,
                                                             const float* __restrict__ pos, float* __restrict__ out,
                                                             int B, int tokens, int n_prefix, int D) {
@@ -176,6 +224,21 @@ int im2col_typed(const void* pixels, void* cols, int out_dtype, int B, int H, in
   return EVT_OK;
 }
 
+template <typename TIN, bool AFFINE>
+int im2col14_typed(const void* pixels, void* cols, int out_dtype, int B, int H, int W, cudaStream_t st, int row_stride, int row_off,
+                   const PixAffine& af) {
+  const long long total = static_cast<long long>(B) * (H / 14) * (W / 14) * (kPatchLd14 / 8);
+  const dim3 grid(static_cast<unsigned>((total + 255) / 256));
+  const bool pdl = pdl_for_rows(static_cast<long long>(B) * 256);
+  const TIN* px = reinterpret_cast<const TIN*>(pixels);
+  if (out_dtype == EVT_BF16)
+    EVT_CUDA(launch_pdl(im2col14_kernel<TIN, true, AFFINE>, grid, dim3(256), 0, st, pdl, px, cols, H, W, total, row_stride, row_off, af));
+  else
+    EVT_CUDA(launch_pdl(im2col14_kernel<TIN, false, AFFINE>, grid, dim3(256), 0, st, pdl, px, cols, H, W, total, row_stride, row_off, af));
+  EVT_LAUNCH_CHECK("im2col14");
+  return EVT_OK;
+}
+
 }  // namespace
 
 int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, const float* bias3, void* cols, int out_dtype, int B,
@@ -189,6 +252,16 @@ int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, cons
   EVT_CHECK_ARG(pixel_dtype == EVT_PIX_F32 || pixel_dtype == EVT_PIX_BF16 || pixel_dtype == EVT_PIX_U8, "im2col: unknown pixel dtype");
   EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(pixels) % (8 * in_bytes) == 0, "im2col: pixel pointer must be aligned to 8 pixels");
   // out_dtype: EVT_BF16, or f32 rounded to tf32 (EVT_TF32; EVT_F32 means the same here: the patch matrix feeds a tf32 GEMM)
+  if (P == 14) {  // rows of kPatchLd14 columns, see im2col14_kernel
+    PixAffine af = {{1.f, 1.f, 1.f}, {0.f, 0.f, 0.f}};
+    if (pixel_dtype == EVT_PIX_U8) {
+      EVT_CHECK_ARG(scale3 && bias3, "im2col: u8 pixels need a per-channel scale and bias");
+      for (int c = 0; c < 3; ++c) af.scale[c] = scale3[c], af.bias[c] = bias3[c];
+      return im2col14_typed<uint8_t, true>(pixels, cols, out_dtype, B, H, W, st, row_stride, row_off, af);
+    }
+    if (pixel_dtype == EVT_PIX_BF16) return im2col14_typed<__nv_bfloat16, false>(pixels, cols, out_dtype, B, H, W, st, row_stride, row_off, af);
+    return im2col14_typed<float, false>(pixels, cols, out_dtype, B, H, W, st, row_stride, row_off, af);
+  }
   if (P % 8 != 0 && P % 4 == 0 && row_off == 0 && pixel_dtype == EVT_PIX_F32)  // Swin: P = 4
     return im2col4_launch(reinterpret_cast<const float*>(pixels), cols, out_dtype == EVT_BF16 ? EVT_BF16 : EVT_TF32, B, H, W, P, st);
   EVT_CHECK_ARG(P % 8 == 0 && W % 8 == 0, "im2col: patch width must be a multiple of 8 (f32 pixels: of 4)");
@@ -277,7 +350,7 @@ extern "C" int evt_patch_embed_workspace_bytes(int B, int H, int W, int P, int n
   EVT_CHECK_ARG(out != nullptr, "patch_embed: null out");
   EVT_CHECK_ARG(B > 0 && H > 0 && W > 0 && P > 0 && n_prefix > 0 && H % P == 0 && W % P == 0, "patch_embed: bad sizes");
   const size_t tokens = static_cast<size_t>(n_prefix) + static_cast<size_t>(H / P) * (W / P);
-  *out = static_cast<size_t>(B) * tokens * 3 * P * P * 2;
+  *out = static_cast<size_t>(B) * tokens * evt::patch_k(P) * 2;
   return EVT_OK;
 }
 extern "C" int evt_patch_embed_fwd(const void* pixels, int pixel_dtype, const float* pixel_scale, const float* pixel_bias,
@@ -289,8 +362,9 @@ extern "C" int evt_patch_embed_fwd(const void* pixels, int pixel_dtype, const fl
   EVT_CHECK_ARG(pixels && W && bias && prefix && pos && out && workspace, "patch_embed: null pointer");
   EVT_CHECK_ARG(B > 0 && H > 0 && Wd > 0 && P > 0 && D > 0 && n_prefix > 0, "patch_embed: sizes must be positive");
   EVT_CHECK_ARG(H % P == 0 && Wd % P == 0, "patch_embed: image size must be a multiple of the patch size");
-  const int K = 3 * P * P;
-  EVT_CHECK_ARG(D % 4 == 0 && ldw >= K && ldw % 8 == 0, "patch_embed: D must be a multiple of 4, ldw a multiple of 8 and >= 3*P*P");
+  const int K = evt::patch_k(P);
+  EVT_CHECK_ARG(D % 4 == 0 && ldw >= K && ldw % 8 == 0,
+                "patch_embed: D must be a multiple of 4, ldw a multiple of 8 and >= 3*P*P (P = 14: >= 592, pad columns zero)");
   EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 1024 == 0, "patch_embed: workspace must be 1 KiB aligned");
   const int tokens = n_prefix + (H / P) * (Wd / P);
   const long long M = static_cast<long long>(B) * tokens;

@@ -165,14 +165,16 @@ int validate_spec(const evt_model_spec* s) {
   EVT_CHECK_ARG(s->hidden > 0 && s->hidden % 8 == 0, "hidden size must be a positive multiple of 8");
   EVT_CHECK_ARG(s->layers > 0 && s->layers <= EVT_MAX_LAYERS, "layer count out of range");
   EVT_CHECK_ARG(s->patch > 0 && s->image > 0 && s->image % s->patch == 0, "image size must be a multiple of the patch size");
-  EVT_CHECK_ARG(s->patch % 8 == 0, "patch size must be a multiple of 8");
+  EVT_CHECK_ARG(s->patch % 8 == 0 || s->patch == 14, "patch size must be a multiple of 8, or 14");
   const int patches = (s->image / s->patch) * (s->image / s->patch);
   EVT_CHECK_ARG(s->tokens == patches + 1 || s->tokens == patches + 2, "tokens must be patches + 1 (cls) or + 2 (cls, distillation)");
   if (s->tokens > EVT_ATTN_MAX_TOKENS)
     return fail(EVT_ERR_UNSUPPORTED, "more than " + std::to_string(EVT_ATTN_MAX_TOKENS) + " tokens per image is not implemented");
   if (s->tokens > 256 && s->precision == EVT_PREC_TF32)  // its attention keeps every key of a head on chip
     return fail(EVT_ERR_UNSUPPORTED, "the tf32 mode supports at most 256 tokens per image; use the bf16 mode");
-  if (s->head_size != 64) return fail(EVT_ERR_UNSUPPORTED, "only head size 64 is implemented");
+  if (s->head_size != 64 && s->head_size != 80) return fail(EVT_ERR_UNSUPPORTED, "only head sizes 64 and 80 are implemented");
+  if (s->head_size == 80 && s->precision != EVT_PREC_BF16)
+    return fail(EVT_ERR_UNSUPPORTED, "head size 80 is implemented in the bf16 mode only");
   EVT_CHECK_ARG(s->num_labels > 0, "num_labels must be positive");
   EVT_CHECK_ARG(s->act == EVT_ACT_GELU_ERF || s->act == EVT_ACT_GELU_TANH, "FFN activation must be erf- or tanh-GELU");
   EVT_CHECK_ARG(s->eps > 0.f, "LayerNorm eps must be positive");
@@ -302,7 +304,7 @@ extern "C" int evt_model_create(const evt_model_spec* spec, evt_model** out) {
   cudaGetDevice(&m->device);
   m->patches = (spec->image / spec->patch) * (spec->image / spec->patch);
   m->n_prefix = spec->tokens - m->patches;
-  m->patch_k = spec->embed_k > 0 ? spec->embed_k : 3 * spec->patch * spec->patch;
+  m->patch_k = spec->embed_k > 0 ? spec->embed_k : patch_k(spec->patch);  // P = 14: 588 columns + 4 zero ones
   m->es = spec->precision == EVT_PREC_TF32 ? 4 : 2;
   m->pad = 16 / m->es;
   m->layers.resize(spec->layers);
@@ -326,7 +328,7 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
   EVT_TRY(L.index(tensors, n));
   const int D = s.hidden;
   const std::string e = "vit.embeddings.";
-  EVT_TRY(L.mat(e + "patch_embeddings.projection.weight", D, m->patch_k, m->patch_k, &m->w_patch));
+  EVT_TRY(L.mat(e + "patch_embeddings.projection.weight", D, s.embed_k > 0 ? m->patch_k : 3 * s.patch * s.patch, m->patch_k, &m->w_patch));
   EVT_TRY(L.vec(e + "patch_embeddings.projection.bias", D, false, &m->b_patch));
   EVT_TRY(L.vec(e + "position_embeddings", static_cast<int64_t>(s.tokens) * D, false, &m->pos));
   {

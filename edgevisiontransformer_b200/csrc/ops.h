@@ -59,6 +59,9 @@ int layernorm_launch(const float* x, int64_t x_stride, const float* gamma, const
 
 // row_stride > 0: patch p of image b is written to row b * row_stride + row_off + p (one row per token); 0 = dense patch matrix
 // pixel_dtype: evt_pixel_dtype; scale3 / bias3 (host, 3 floats each): per-channel affine applied to u8 pixels
+// Columns of a patch-matrix row: 3 * P * P, except P = 14, whose 588 are padded with zero columns to kPatchLd14 (16-byte rows).
+constexpr int kPatchLd14 = 592;
+inline int patch_k(int P) { return P == 14 ? kPatchLd14 : 3 * P * P; }
 int im2col_launch(const void* pixels, int pixel_dtype, const float* scale3, const float* bias3, void* cols, int out_dtype, int B,
                   int H, int W, int P, cudaStream_t st, int row_stride = 0, int row_off = 0);
 int embed_fill_launch(const float* prefix, const float* pos, const float* bias, float* out, int B, int tokens, int n_prefix, int D,

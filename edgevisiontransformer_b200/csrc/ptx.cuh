@@ -465,6 +465,18 @@ __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t smem_addr) {
   return d;
 }
 
+// The same for SWIZZLE_32B: 32-byte rows, 8-row groups 256 bytes apart.  K-major: 16 bf16 of K per row (one K = 16 step);
+// MN-major B operand: 16 bf16 of N per row.
+__device__ __forceinline__ uint64_t smem_desc_sw32(uint32_t smem_addr) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>(256 >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(6) << 61;                     // SWIZZLE_32B
+  return d;
+}
+
 // Instruction descriptor for kind::f16 / kind::tf32 with f32 accumulation.
 //   ab_fmt: 0 f16, 1 bf16, 2 tf32;  *_mn_major: 0 = K-major operand, 1 = MN-major
 __host__ __device__ constexpr uint32_t make_idesc(int M, int N, int ab_fmt, int a_mn_major, int b_mn_major) {

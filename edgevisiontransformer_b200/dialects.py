@@ -12,6 +12,12 @@ timm / facebookresearch-deit dialect (``torch.hub.load('facebookresearch/deit:ma
 utils.py:52-62, tools.py:244-263): same function as HF ViT with a fused ``attn.qkv`` Linear (rows q | k | v, head-major
 inside each), LayerNorm eps 1e-6 and flat key names -> pure renaming + split, see ``timm_vit_to_canonical``.
 
+DeiT III (facebookresearch-deit ``models_v2``: ``deit_{small,medium,base,large}_patch16_LS``, ``deit_huge_patch14_LS``; timm
+``deit3_*``): the same blocks with LayerScale, ``x + gamma_1 * attn(norm1(x))`` and ``x + gamma_2 * mlp(norm2(x))`` (keys
+``blocks.{l}.gamma_{1,2}`` or timm's ``blocks.{l}.ls{1,2}.gamma``), and a position embedding of the patches only (no cls row).
+LayerScale is folded into the two residual projections, ``W' = diag(gamma) W``, ``b' = gamma * b``; the cls token gets a zero
+position row.  See ``timm_vit_to_canonical``.
+
 PyTorch T2T-ViT (yitu-opensource/T2T-ViT, ``tokens_type='performer'``; the reference's tools.py:347-365 loads these files):
 timm-layout encoder blocks without qkv bias, plus the tokens-to-token module, whose ``nn.Unfold`` soft splits order their
 columns ``(c, kh, kw)`` -> permuted to the ``(kh, kw, c)`` order of the library's soft splits, see ``t2t_torch_to_canonical``.
@@ -19,6 +25,7 @@ columns ``(c, kh, kw)`` -> permuted to the ``(kh, kw, c)`` order of the library'
 from __future__ import annotations
 
 import math
+import re
 from typing import Dict, List, Optional, Tuple
 
 import torch
@@ -73,13 +80,18 @@ def timm_vit_to_canonical(sd: Dict[str, torch.Tensor], patch: int = 16) -> Tuple
     ``modeling_vit.normalise_keys`` folds into one classifier.  Half of that layout is refused."""
     if "model" in sd and isinstance(sd["model"], dict):
         sd = sd["model"]
+    _refuse_deit3_variants(sd)
     distilled = "dist_token" in sd
     if distilled != ("head_dist.weight" in sd):
         raise ValueError("distilled DeiT checkpoint needs both dist_token and head_dist")
     D = sd["cls_token"].shape[-1]
+    pos = sd["pos_embed"].reshape(1, -1, D)
+    n_prefix = 2 if distilled else 1
+    if math.isqrt(pos.shape[1]) ** 2 == pos.shape[1]:   # patches only (DeiT III): the prefix tokens get no position row
+        pos = torch.cat((pos.new_zeros(1, n_prefix, D), pos), dim=1)
     out: Dict[str, torch.Tensor] = {
         "vit.embeddings.cls_token": sd["cls_token"].reshape(1, 1, D),
-        "vit.embeddings.position_embeddings": sd["pos_embed"].reshape(1, -1, D),
+        "vit.embeddings.position_embeddings": pos,
         "vit.embeddings.patch_embeddings.projection.weight": sd["patch_embed.proj.weight"],
         "vit.embeddings.patch_embeddings.projection.bias": sd["patch_embed.proj.bias"],
         "vit.layernorm.weight": sd["norm.weight"], "vit.layernorm.bias": sd["norm.bias"],
@@ -90,14 +102,48 @@ def timm_vit_to_canonical(sd: Dict[str, torch.Tensor], patch: int = 16) -> Tuple
         out["distillation_classifier.weight"], out["distillation_classifier.bias"] = sd["head_dist.weight"], sd["head_dist.bias"]
     else:
         out["classifier.weight"], out["classifier.bias"] = sd["head.weight"], sd["head.bias"]
-    if _timm_blocks_to_canonical(sd, out, D) == 0:
+    depth = _timm_blocks_to_canonical(sd, out, D)
+    if depth == 0:
         raise ValueError("not a timm VisionTransformer state dict (no blocks.0.attn.qkv.weight)")
+    stray = [k for k in sd if _LAYERSCALE.search(k) and int(k.split(".")[1]) >= depth]
+    if stray:
+        raise ValueError(f"LayerScale parameters of blocks the state dict does not have: {stray[:4]}")
     return out, dict(layer_norm_eps=1e-6, hidden_act="gelu", patch_size=patch)
+
+
+_LAYERSCALE = re.compile(r"^blocks\.\d+\.(gamma_[12]|ls[12]\.gamma)$")
+DEIT3_HUGE_DIM, DEIT3_GIANT_DIM = 1280, 1408
+
+
+def _refuse_deit3_variants(sd: Dict[str, torch.Tensor]) -> None:
+    """The DeiT III variants this library does not run, refused by name rather than loaded wrong."""
+    if any(re.match(r"^blocks\.\d+\.(attn1|mlp1|norm11|norm21|gamma_1_1|gamma_2_1)\.?", k) for k in sd):
+        raise ValueError("parallel-block DeiT III (deit_huge_patch14_26x2_LS: two attention and two MLP branches per block) "
+                         "is not implemented")
+    if "cls_token" in sd and sd["cls_token"].shape[-1] == DEIT3_GIANT_DIM and any(_LAYERSCALE.search(k) for k in sd):
+        raise ValueError("DeiT III Giant (deit_giant_patch14_LS, embed dim 1408, head size 88) is not implemented")
+
+
+def deit3_head_size(sd: Dict[str, torch.Tensor]) -> int:
+    """Head size of a DeiT III state dict (80 for Huge, embed dim 1280; 64 for every smaller model), else 64."""
+    if "model" in sd and isinstance(sd["model"], dict):
+        sd = sd["model"]
+    layerscale = any(_LAYERSCALE.search(k) for k in sd)
+    return 80 if layerscale and "cls_token" in sd and sd["cls_token"].shape[-1] == DEIT3_HUGE_DIM else 64
+
+
+def _layerscale(sd: Dict[str, torch.Tensor], l: int, i: int) -> Optional[torch.Tensor]:
+    """gamma_i of block l in either key layout (None without LayerScale); both layouts at once are refused."""
+    a, b = sd.get(f"blocks.{l}.gamma_{i}"), sd.get(f"blocks.{l}.ls{i}.gamma")
+    if a is not None and b is not None:
+        raise ValueError(f"block {l} has both blocks.{l}.gamma_{i} and blocks.{l}.ls{i}.gamma")
+    return a if a is not None else b
 
 
 def _timm_blocks_to_canonical(sd: Dict[str, torch.Tensor], out: Dict[str, torch.Tensor], D: int, q_scale: float = 1.0) -> int:
     """timm ``Block`` s ``blocks.{l}.*`` (fused ``attn.qkv``, rows q | k | v) -> ``vit.encoder.layer.{l}.*``; returns the depth.
-    ``q_scale`` multiplies the query rows (weight and bias): how a softmax scale other than head_size ** -0.5 is folded in."""
+    ``q_scale`` multiplies the query rows (weight and bias): how a softmax scale other than head_size ** -0.5 is folded in.
+    LayerScale (DeiT III) is folded in f32 into the rows of ``attn.proj`` (gamma_1) and ``mlp.fc2`` (gamma_2)."""
     l = 0
     while f"blocks.{l}.attn.qkv.weight" in sd:
         p, q = f"blocks.{l}.", f"vit.encoder.layer.{l}."
@@ -114,6 +160,18 @@ def _timm_blocks_to_canonical(sd: Dict[str, torch.Tensor], out: Dict[str, torch.
                          ("norm1", "layernorm_before"), ("norm2", "layernorm_after")):
             out[q + dst + ".weight"] = sd[p + src + ".weight"]
             out[q + dst + ".bias"] = sd[p + src + ".bias"]
+        g1, g2 = _layerscale(sd, l, 1), _layerscale(sd, l, 2)
+        if (g1 is None) != (g2 is None):
+            raise ValueError(f"block {l} has LayerScale on one residual branch only")
+        for g, dst in ((g1, "attention.output.dense"), (g2, "output.dense")):
+            if g is not None:
+                w, b = out[q + dst + ".weight"], out[q + dst + ".bias"]
+                dt = torch.promote_types(w.dtype, torch.float32)        # f32 at least (f64 weights stay f64)
+                g = g.to(dt).reshape(-1)
+                if g.numel() != D:
+                    raise ValueError(f"block {l}: LayerScale has {g.numel()} entries, expected {D}")
+                out[q + dst + ".weight"] = w.to(dt) * g[:, None]
+                out[q + dst + ".bias"] = b.to(dt) * g
         l += 1
     return l
 

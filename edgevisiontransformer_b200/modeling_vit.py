@@ -205,11 +205,20 @@ class B200ViTForImageClassification(nn.Module):
     @classmethod
     def from_timm(cls, model_or_state_dict, **kw):
         """Build from a timm / facebookresearch-deit ``VisionTransformer`` (the model ``utils.get_torch_deit`` returns,
-        utils.py:52-62) or its state dict: fused qkv, LayerNorm eps 1e-6 (dialects.timm_vit_to_canonical)."""
-        from .dialects import timm_vit_to_canonical
+        utils.py:52-62) or its state dict: fused qkv, LayerNorm eps 1e-6 (dialects.timm_vit_to_canonical).  DeiT III
+        (``models_v2`` / timm ``deit3_*``, LayerScale) loads too.  The patch size is read from the patch projection; the head
+        size (not in the weights) defaults to 64, or to 80 for a DeiT III of embed dim 1280 (Huge); ``head_size=`` overrides."""
+        from .dialects import deit3_head_size, timm_vit_to_canonical
         sd = model_or_state_dict.state_dict() if hasattr(model_or_state_dict, "state_dict") else model_or_state_dict
+        sd = {k: v for k, v in sd.items()}
         image = kw.pop("image_size", None)
-        csd, cfg_kw = timm_vit_to_canonical({k: v for k, v in sd.items()}, patch=kw.pop("patch_size", 16))
+        head_size = kw.pop("head_size", None)
+        inner = sd["model"] if isinstance(sd.get("model"), dict) else sd
+        patch = kw.pop("patch_size", None)
+        if patch is None:
+            patch = inner["patch_embed.proj.weight"].shape[-1] if "patch_embed.proj.weight" in inner else 16
+        csd, cfg_kw = timm_vit_to_canonical(sd, patch=patch)
+        cfg_kw["head_size"] = deit3_head_size(sd) if head_size is None else int(head_size)
         if image is None:                       # from the position rows: 197 / 198 -> 224, 577 / 578 -> 384
             n_prefix = 2 if "vit.embeddings.distillation_token" in csd else 1
             image = int(round((csd["vit.embeddings.position_embeddings"].shape[1] - n_prefix) ** 0.5)) * cfg_kw["patch_size"]
@@ -470,6 +479,74 @@ class B200ViTForImageClassification(nn.Module):
         self._profiling = False
         _lib.check(self._lib.evt_model_profile_end(self._handle, ms, cnt), "profile_end")
         return {name: (float(ms[i]), int(cnt[i])) for i, name in enumerate(_lib.STAGES)}
+
+
+# DeiT III (facebookresearch-deit models_v2 ``deit_*_LS``, timm ``deit3_*``): name -> (embed dim, heads, patch, image size).
+# Depth comes from the weights.
+DEIT3 = {
+    "deit3_small_patch16_224": (384, 6, 16, 224), "deit3_small_patch16_384": (384, 6, 16, 384),
+    "deit3_medium_patch16_224": (512, 8, 16, 224), "deit3_medium_patch16_384": (512, 8, 16, 384),
+    "deit3_base_patch16_224": (768, 12, 16, 224), "deit3_base_patch16_384": (768, 12, 16, 384),
+    "deit3_large_patch16_224": (1024, 16, 16, 224), "deit3_large_patch16_384": (1024, 16, 16, 384),
+    "deit3_huge_patch14_224": (1280, 16, 14, 224),
+}
+
+
+def _deit3_factory(name: str, checkpoint_or_sd, **kw) -> B200ViTForImageClassification:
+    """A DeiT III checkpoint (file or state dict, either key layout) as the named model: its shapes must match the name."""
+    from .dialects import _LAYERSCALE, _refuse_deit3_variants, unwrap_checkpoint
+    D, heads, patch, image = DEIT3[name]
+    sd = checkpoint_or_sd
+    if isinstance(sd, (str, os.PathLike)):
+        sd = torch.load(sd, map_location="cpu", weights_only=True)
+    sd = unwrap_checkpoint(sd)
+    _refuse_deit3_variants(sd)
+    if not any(_LAYERSCALE.search(k) for k in sd):
+        raise ValueError(f"{name} is a DeiT III (LayerScale) model; the weights have no blocks.*.gamma_1 / ls1.gamma")
+    got = (sd["cls_token"].shape[-1], sd["patch_embed.proj.weight"].shape[-1], sd["blocks.0.mlp.fc1.weight"].shape[0])
+    if got != (D, patch, 4 * D):
+        raise ValueError(f"{name} is embed dim {D}, patch {patch}, MLP {4 * D}; the weights have {got[0]}, {got[1]} and {got[2]}")
+    n, patches = sd["pos_embed"].shape[-2], (image // patch) ** 2
+    if n not in (patches, patches + 1):
+        raise ValueError(f"{name} has {patches} patches; the weights have {n} position rows")
+    kw.setdefault("image_size", image)
+    return B200ViTForImageClassification.from_timm(sd, patch_size=patch, head_size=D // heads, **kw)
+
+
+def deit3_small_patch16_224(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_small_patch16_224", checkpoint_or_sd, **kw)
+
+
+def deit3_small_patch16_384(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_small_patch16_384", checkpoint_or_sd, **kw)
+
+
+def deit3_medium_patch16_224(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_medium_patch16_224", checkpoint_or_sd, **kw)
+
+
+def deit3_medium_patch16_384(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_medium_patch16_384", checkpoint_or_sd, **kw)
+
+
+def deit3_base_patch16_224(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_base_patch16_224", checkpoint_or_sd, **kw)
+
+
+def deit3_base_patch16_384(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_base_patch16_384", checkpoint_or_sd, **kw)
+
+
+def deit3_large_patch16_224(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_large_patch16_224", checkpoint_or_sd, **kw)
+
+
+def deit3_large_patch16_384(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_large_patch16_384", checkpoint_or_sd, **kw)
+
+
+def deit3_huge_patch14_224(checkpoint_or_sd, **kw):
+    return _deit3_factory("deit3_huge_patch14_224", checkpoint_or_sd, **kw)
 
 
 def _first(v):

@@ -322,7 +322,10 @@ def patch_embed(pixels: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, 
     w = weight.reshape(D, -1)
     if w.shape[1] != K:
         raise ValueError(f"patch_embed: weight has {w.shape[1]} inputs per filter, expected {K}")
-    w = w.to(torch.bfloat16).contiguous()
+    w = w.to(torch.bfloat16)
+    if patch == 14:   # the library's P = 14 patch rows are 592 wide: 588 columns and 4 zero ones
+        w = torch.nn.functional.pad(w, (0, 592 - K))
+    w = w.contiguous()
     prefix = prefix.reshape(-1, D).float().contiguous()
     tokens = prefix.shape[0] + (H // patch) * (W // patch)
     pos = pos.reshape(-1, D).float().contiguous()
@@ -340,7 +343,7 @@ def patch_embed(pixels: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, 
     ws = torch.empty(n.value + 1024, dtype=torch.uint8, device=pixels.device)
     ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
     out = torch.empty((B, tokens, D), dtype=torch.float32, device=pixels.device)
-    _lib.check(lib.evt_patch_embed_fwd(pixels.data_ptr(), pix, scale, shift, w.data_ptr(), K, bias.float().contiguous().data_ptr(),
+    _lib.check(lib.evt_patch_embed_fwd(pixels.data_ptr(), pix, scale, shift, w.data_ptr(), w.shape[1], bias.float().contiguous().data_ptr(),
                                        prefix.data_ptr(), pos.data_ptr(), out.data_ptr(), ws_ptr, B, H, W, patch, D,
                                        prefix.shape[0], _stream()), "patch_embed")
     return out

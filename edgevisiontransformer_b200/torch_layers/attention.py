@@ -44,8 +44,9 @@ class Attention(nn.Module):
     def forward(self, x, residual=None):
         if not x.is_cuda:
             raise RuntimeError("edgevisiontransformer_b200.torch_layers.Attention needs CUDA tensors (no CPU fallback)")
-        if self.head_size != 64:
-            raise NotImplementedError("the fused attention kernel implements head_size 64 (every DeiT / T2T configuration)")
+        if self.head_size not in (64, 80):
+            raise NotImplementedError("the fused attention kernel implements head_size 64 (every DeiT / T2T configuration) and 80 "
+                                      "(DeiT III Huge)")
         B, n, h = x.shape
         wqkv, bqkv, wo, bo = self._weights()
         xb = ops.cast_bf16(x.float().reshape(B * n, h))

@@ -159,8 +159,9 @@ int evt_gemm_residual_layernorm_ex(const void* A, int64_t lda, const void* W, in
  * (32 * 32 + 2 tokens). */
 #define EVT_ATTN_MAX_TOKENS 1026
 
-/* Fused softmax(Q K^T * scale) V, head size 64, any S from 1 to EVT_ATTN_MAX_TOKENS.  S <= 256 keeps every key of a head
- * on chip; longer sequences run query tiles against 128-key blocks with an online softmax (no score tensor in HBM either way):
+/* Fused softmax(Q K^T * scale) V, head size 64 or 80, any S from 1 to EVT_ATTN_MAX_TOKENS.  Head size 64 with S <= 256 keeps
+ * every key of a head on chip; longer sequences, and head size 80 (DeiT III Huge) at every S, run query tiles against 128-key
+ * blocks with an online softmax (no score tensor in HBM either way):
  * eager_attention_forward SITE/models/vit/modeling_vit.py:171-196 ==
  * modeling/torch_layers/attention.py:36-45 == modeling/layers/attention.py:30-33.
  *   qkv : bf16 [B*S, ldq]; q of head h at columns [h*64, h*64+64), k at [heads*64 + h*64, ...),
@@ -182,7 +183,8 @@ int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ld
 
 /* Non-overlapping patch gather: pixels f32 NCHW [B,3,H,W] -> bf16 [B*(H/P)*(W/P), 3*P*P] with
  * K order (c, i, j) -- the im2col of Conv2d(3,D,P,P) (SITE/models/vit/modeling_vit.py:151-167).  P a multiple of 4
- * (ViT / DeiT: 16; Swin: 4). */
+ * (ViT / DeiT: 16; Swin: 4) or 14 (DeiT III Huge), whose rows are 592 wide: 588 columns, then 4 zero columns
+ * (16-byte rows for TMA). */
 int evt_im2col_patch(const float* pixels, void* cols, int B, int H, int W, int P, evt_stream stream);
 /* evt_im2col_patch with a choice of output: out_dtype EVT_BF16 (as above) or EVT_TF32 (f32 [.., 3*P*P] rounded to nearest
  * tf32: the A operand of a tf32 GEMM). */
@@ -194,10 +196,11 @@ int evt_im2col_patch_ex(const float* pixels, void* cols, int out_dtype, int B, i
  * pixels    NCHW [B,3,H,W] of pixel_dtype (evt_pixel_dtype: f32, bf16 or raw u8; u8 takes pixel_scale / pixel_bias,
  *           3 HOST floats each, applied as x * scale[c] + bias[c] inside the patch gather; NULL otherwise)
  * W         bf16 [D, ldw], K order (c, i, j) = conv.weight.reshape(D, -1); ldw >= 3*P*P, multiple of 8
+ *           (P = 14: ldw >= 592, columns 588..591 zero)
  * bias      f32 [D]; prefix f32 [n_prefix, D] (cls, or cls + distillation token); pos f32 [tokens, D]
  * out       f32 [B * tokens, D], tokens = n_prefix + (H/P)*(W/P)
  * workspace evt_patch_embed_workspace_bytes bytes, 1 KiB aligned (the bf16 patch matrix, one row per token)
- * P a multiple of 8.  Three launches (patch gather, row preset, tcgen05 GEMM with a TMA reduce-add epilogue). */
+ * P a multiple of 8, or 14.  Three launches (patch gather, row preset, tcgen05 GEMM with a TMA reduce-add epilogue). */
 int evt_patch_embed_workspace_bytes(int B, int H, int W, int P, int n_prefix, size_t* out);
 int evt_patch_embed_fwd(const void* pixels, int pixel_dtype, const float* pixel_scale, const float* pixel_bias,
                         const void* W, int64_t ldw, const float* bias, const float* prefix, const float* pos,
