@@ -48,7 +48,8 @@ SWIN_MAX_STAGES = 8
 class SwinSpec(C.Structure):
     _fields_ = [("image", C.c_int), ("patch", C.c_int), ("window", C.c_int), ("embed_dim", C.c_int), ("stages", C.c_int),
                 ("depths", C.c_int * SWIN_MAX_STAGES), ("heads", C.c_int * SWIN_MAX_STAGES), ("num_labels", C.c_int),
-                ("eps", C.c_float), ("precision", C.c_int)]
+                ("eps", C.c_float), ("precision", C.c_int), ("version", C.c_int),
+                ("pretrained_window", C.c_int * SWIN_MAX_STAGES), ("mask_adds", C.c_int)]
 
 
 class TensorView(C.Structure):
@@ -90,6 +91,10 @@ SIGNATURES = {
     "evt_window_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i64, _i, _i, _i, _f, _p]),
     "evt_layernorm_mean_tokens": (_i, [_p, _p, _p, _p, _i64, _i, _i, _f, _p]),
     "evt_layernorm_mean_tokens_ex": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _f, _p]),
+    "evt_cosine_window_attention_fwd": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _i, _i, _i, _i, _f, _p]),
+    "evt_postnorm_residual": (_i, [_p, _p, _p, _p, _p, _p, _p, _i64, _i, _i, _i, _i, _f, _p]),
+    "evt_swinv2_cpb_table": (_i, [_p, _p, _p, _i, _i, _i, _p]),
+    "evt_swinv2_score_bias": (_i, [_p, _i, _i, _i, _i, _f, _p]),
     "evt_model_create": (_i, [C.POINTER(ModelSpec), C.POINTER(_p)]),
     "evt_model_load_weights": (_i, [_p, C.POINTER(TensorView), _i, _p]),
     "evt_model_workspace_bytes": (_i, [_p, _i, C.POINTER(_sz)]),

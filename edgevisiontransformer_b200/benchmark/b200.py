@@ -29,6 +29,8 @@ SWIN = {"swin_tiny": (96, [2, 2, 6, 2], [3, 6, 12, 24]), "swin_small": (96, [2, 
 # swin_*_patch4_window7_224 (tools.py:280); --image-size 384 takes the window12_384 geometry (published for base / large;
 # tiny / small run the same geometry)
 SWIN_WINDOW = {224: 7, 384: 12}
+# swinv2_*_patch4_window{8,16}_256 (modeling_swinv2.SWINV2): --window picks 8 (default) or 16, always 256 pixels
+SWINV2 = ("swinv2_tiny", "swinv2_small", "swinv2_base")
 T2T = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_12": (256, 12, 4, 2.0),
        "t2t_vit_14": (384, 14, 6, 3.0)}
 
@@ -99,7 +101,8 @@ def _random_deit3(name: str, seed: int = 0):
     return sd
 
 
-def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", image_size: int = 224, **op_kw):
+def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device="cuda", image_size: int = 224, window: int = 8,
+                **op_kw):
     """-> (callable taking one CUDA tensor, input shape without batch, description).  image_size: deit_* and swin_* (224 or
     384: deit_*_patch16_{224,384}, swin_*_patch4_window7_224 / swin_*_patch4_window12_384)."""
     from .. import B200ViTForImageClassification
@@ -128,6 +131,15 @@ def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device
                                                    depths=depths, num_heads=heads, num_labels=1000)).eval()
         m = B200SwinForImageClassification.from_hf(hf, device=device, max_batch=min(max_batch, 1024))
         return m, (3, image_size, image_size), f"{name} random-init (bf16, {image_size} px, window {window})"
+    if name in SWINV2:
+        from ..modeling_swinv2 import SWINV2 as V2, B200Swinv2ForImageClassification
+        from transformers import Swinv2Config, Swinv2ForImageClassification
+        dim, depths, heads, _, pws = V2[f"{name}_patch4_window{window}_256"]
+        torch.manual_seed(0)
+        hf = Swinv2ForImageClassification(Swinv2Config(image_size=256, patch_size=4, window_size=window, embed_dim=dim, depths=depths,
+                                                        num_heads=heads, pretrained_window_sizes=pws, num_labels=1000)).eval()
+        m = B200Swinv2ForImageClassification.from_hf(hf, device=device, max_batch=min(max_batch, 1024), precision=precision)
+        return m, (3, 256, 256), f"{name}_patch4_window{window}_256 random-init ({precision})"
     if name in ("attention", "ffn"):
         from .. import torch_layers as tl
         h, n = op_kw.get("h", 768), op_kw.get("n", 128)
@@ -180,6 +192,7 @@ def main(argv=None) -> int:
     ap.add_argument("--warmup_runs", type=int, default=20)
     ap.add_argument("--topk", type=int, default=None)
     ap.add_argument("--graph", action="store_true", help="CUDA-graph replay (small-batch latency path)")
+    ap.add_argument("--window", type=int, default=None, choices=[8, 16], help="swinv2_{tiny,small,base}: window 8 (default) or 16, 256 px")
     ap.add_argument("--image-size", type=int, default=224,
                     help="deit_* / swin_* input resolution (384: deit_*_patch16_384, 577 tokens; swin_*_patch4_window12_384)")
     for k, d in (("h", 768), ("a", 12), ("i", 3072), ("n", 128)):
@@ -189,11 +202,17 @@ def main(argv=None) -> int:
     if not torch.cuda.is_available():
         print("b200_benchmark needs a B200 (sm_100a): the backend has no CPU path")
         return 2
-    if a.image_size != 224 and a.model not in DEIT and a.model not in SWIN:
+    if a.window is not None and a.model not in SWINV2:
+        ap.error("--window applies to the swinv2_* models only")
+    if a.model in SWINV2:
+        if a.image_size not in (224, 256):
+            ap.error("swinv2_* runs at 256 pixels")
+        a.image_size = 256
+    if a.image_size != 224 and a.model not in DEIT and a.model not in SWIN and a.model not in SWINV2:
         ap.error("--image-size applies to the deit_* and swin_* models only")
     if a.model in SWIN and a.image_size not in SWIN_WINDOW:
         ap.error("swin_* runs at --image-size 224 (window 7) or 384 (window 12)")
-    model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), image_size=a.image_size, h=a.h, a=a.a, i=a.i,
+    model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), image_size=a.image_size, window=a.window or 8, h=a.h, a=a.a, i=a.i,
                                      n=a.n, h_k=a.h_k)
     avg, std, times = b200_benchmark(model, (a.batch, *shape), a.num_runs, a.warmup_runs, a.topk, graph=a.graph)
     print(f"{desc}: batch {a.batch}")

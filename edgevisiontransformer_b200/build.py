@@ -20,7 +20,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, os.environ.get("EVT_BUILD_OUT", "libevt.so"))
 OBJ_DIR = os.path.join(CSRC, "build" + ("_" + os.path.splitext(os.path.basename(OUT))[0] if "EVT_BUILD_OUT" in os.environ else ""))
 
-SOURCES = ["common.cu", "gemm.cu", "gemm2.cu", "gemm_ln.cu", "gemm_rowln.cu", "attention.cu", "layernorm.cu", "embed.cu", "performer.cu", "swin.cu", "swin_model.cu", "model.cu"]
+SOURCES = ["common.cu", "gemm.cu", "gemm2.cu", "gemm_ln.cu", "gemm_rowln.cu", "attention.cu", "layernorm.cu", "embed.cu", "performer.cu", "swin.cu", "swinv2.cu", "swin_model.cu", "model.cu"]
 # Kernels that lost their A/B tests are not kept in the tree: DESIGN.md records each result and the commit its source is at.
 
 NVCC_FLAGS = [

@@ -77,6 +77,13 @@ int window_attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int6
                                  int window_tokens, int heads, int head_size, float scale, cudaStream_t st);
 int layernorm_mean_tokens_launch(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T, int D,
                                  float eps, cudaStream_t st);
+// swinv2.cu: evt_cosine_window_attention_fwd and evt_postnorm_residual without the device check; the host CPB evaluation
+// (out [heads, (2 ws - 1)^2] = 16 sigmoid(cpb_mlp(coords)), host pointers)
+int cosine_window_attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table, const float* head_scale,
+                                   int64_t n_windows, int window, int heads, int head_size, int grid, int shift, float mask, cudaStream_t st);
+int postnorm_residual_launch(const float* y, const float* resid, const int* idx, const float* gamma, const float* beta, float* out_f32,
+                             void* out_bf16, int64_t images, int T_in, int T_out, int G, int C, float eps, cudaStream_t st);
+int swinv2_cpb_table(const float* w1, const float* b1, const float* w2, int heads, int ws, int pws, float* out);
 int prefix_tokens_launch(const float* prefix, const float* pos, float* out, int B, int tokens, int n_prefix, int D,
                          cudaStream_t st);
 int cast_launch(const float* x, void* y, int64_t n, cudaStream_t st);

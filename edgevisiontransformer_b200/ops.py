@@ -287,6 +287,75 @@ def layernorm_mean_tokens(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tens
     return y
 
 
+def cosine_window_attention(qkv: torch.Tensor, table: torch.Tensor, head_scale: torch.Tensor, n_windows: int, heads: int,
+                            window: int, grid: int, shift: int = 0, mask: float = -100.0) -> torch.Tensor:
+    """Swin V2 cosine window attention (include/evt.h evt_cosine_window_attention_fwd): qkv bf16 [n_windows*window^2, 3*heads*32]
+    in window order, table f32 [heads, (2*window-1)^2] = 16 sigmoid(cpb) * log2(e), head_scale f32 [heads] =
+    exp(min(logit_scale, ln 100)) * log2(e); grid = tokens per image side, shift = the block's cyclic shift (0: no mask), mask =
+    what a masked score gets added -> ctx bf16 [n_windows*window^2, heads*32]."""
+    _need_cuda(qkv, table, head_scale)
+    N = window * window
+    if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.stride(1) != 1 or qkv.shape[0] != n_windows * N:
+        raise ValueError("cosine_window_attention wants a bf16 [n_windows*window^2, 3*heads*32] matrix")
+    nt = (2 * window - 1) ** 2
+    if table.dtype != torch.float32 or tuple(table.shape) != (heads, nt) or not table.is_contiguous():
+        raise ValueError(f"cosine_window_attention: table must be a contiguous f32 [{heads}, {nt}] tensor")
+    if head_scale.dtype != torch.float32 or head_scale.numel() != heads or not head_scale.is_contiguous():
+        raise ValueError(f"cosine_window_attention: head_scale must be a contiguous f32 [{heads}] tensor")
+    ctx = torch.empty((qkv.shape[0], heads * 32), dtype=torch.bfloat16, device=qkv.device)
+    lib = _lib.load()
+    _lib.check(lib.evt_cosine_window_attention_fwd(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), table.data_ptr(),
+                                                   head_scale.data_ptr(), n_windows, window, heads, 32, grid, shift, float(mask),
+                                                   _stream()), "cosine_window_attention")
+    return ctx
+
+
+def postnorm_residual(y: torch.Tensor, resid: Optional[torch.Tensor], idx: Optional[torch.Tensor], gamma: torch.Tensor,
+                      beta: torch.Tensor, eps: float, images: int, T_out: int, G: int = 1, f32: bool = True, bf16: bool = True):
+    """Post-norm residual update (include/evt.h evt_postnorm_residual): row r, group g of the output =
+    (resid[s] if resid is given else 0) + LayerNorm(y[s]), s = image * T_in + (idx[t * G + g] if idx is given else t).
+    y / resid f32 [images*T_in, C] -> (f32 [images*T_out, G*C] or None, bf16 [images*T_out, G*C] or None)."""
+    _need_cuda(y, resid, idx, gamma, beta)
+    if y.dtype != torch.float32 or y.dim() != 2 or not y.is_contiguous() or y.shape[0] % images:
+        raise ValueError("postnorm_residual wants a contiguous f32 [images*T_in, C] matrix")
+    if resid is not None and (resid.dtype != torch.float32 or resid.shape != y.shape or not resid.is_contiguous()):
+        raise ValueError("postnorm_residual: resid must be a contiguous f32 tensor shaped like y")
+    if idx is not None and (idx.dtype != torch.int32 or idx.numel() != T_out * G or not idx.is_contiguous()):
+        raise ValueError("postnorm_residual: idx must be a contiguous int32 [T_out*G] tensor")
+    T_in, C = y.shape[0] // images, y.shape[1]
+    o32 = torch.empty((images * T_out, G * C), dtype=torch.float32, device=y.device) if f32 else None
+    o16 = torch.empty((images * T_out, G * C), dtype=torch.bfloat16, device=y.device) if bf16 else None
+    lib = _lib.load()
+    _lib.check(lib.evt_postnorm_residual(y.data_ptr(), _ptr(resid), _ptr(idx), gamma.data_ptr(), beta.data_ptr(), _ptr(o32), _ptr(o16),
+                                         images, T_in, T_out, G, C, float(eps), _stream()), "postnorm_residual")
+    return o32, o16
+
+
+def swinv2_cpb_table(w1: torch.Tensor, b1: torch.Tensor, w2: torch.Tensor, window: int, pretrained_window: int = 0) -> torch.Tensor:
+    """16 sigmoid(cpb_mlp(relative_coords_table)) as the Swin V2 load computes it on the host: CPU f32 [heads, (2*window-1)^2]
+    from continuous_position_bias_mlp.{0.weight [512, 2], 0.bias [512], 2.weight [heads, 512]}.  Needs no GPU."""
+    w1, b1, w2 = (t.detach().float().cpu().contiguous() for t in (w1, b1, w2))
+    if tuple(w1.shape) != (512, 2) or tuple(b1.shape) != (512,) or w2.dim() != 2 or w2.shape[1] != 512:
+        raise ValueError("swinv2_cpb_table wants w1 [512, 2], b1 [512], w2 [heads, 512]")
+    out = torch.empty((w2.shape[0], (2 * window - 1) ** 2), dtype=torch.float32)
+    _lib.check(_lib.load().evt_swinv2_cpb_table(w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), w2.shape[0], window, pretrained_window,
+                                                out.data_ptr()), "swinv2_cpb_table")
+    return out
+
+
+def swinv2_score_bias(table: torch.Tensor, window: int, grid: int, shift: int, mask: float = -100.0) -> torch.Tensor:
+    """Dense [(grid/window)^2, heads, N, N] form of what evt_cosine_window_attention_fwd adds to the scores (bias from the compact
+    CPU f32 table [heads, (2*window-1)^2], plus `mask` between shift regions), from the kernel's index arithmetic.  No GPU."""
+    table = table.detach().float().cpu().contiguous()
+    heads, N = table.shape[0], window * window
+    if table.dim() != 2 or table.shape[1] != (2 * window - 1) ** 2:
+        raise ValueError("swinv2_score_bias: table must be [heads, (2*window-1)^2]")
+    out = torch.empty(((grid // window) ** 2, heads, N, N), dtype=torch.float32)
+    _lib.check(_lib.load().evt_swinv2_score_bias(table.data_ptr(), heads, window, grid, shift, float(mask), out.data_ptr()),
+               "swinv2_score_bias")
+    return out
+
+
 def im2col_patch(pixels: torch.Tensor, patch: int = 16, out_dtype=torch.bfloat16) -> torch.Tensor:
     """f32 NCHW pixels -> the patch matrix [B*(H/P)*(W/P), 3*P*P] in (c, i, j) order, bf16 or TF32."""
     _need_cuda(pixels)

@@ -308,6 +308,46 @@ int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* b
 int evt_layernorm_mean_tokens_ex(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T,
                                  int D, float eps, evt_stream stream);
 
+/* ---- Swin V2 block (SITE/models/swinv2/modeling_swinv2.py, microsoft/Swin-Transformer swin_transformer_v2.py).  Same window
+ * order of the token rows as the V1 ops above. */
+
+/* Cosine window attention (Swinv2SelfAttention.forward :421-470) for 8x8 (window = 8) or 16x16 (window = 16) windows, head
+ * size 32; anything else is EVT_ERR_UNSUPPORTED:
+ *   ctx = softmax(normalize(q) normalize(k)^T * exp(min(logit_scale_h, ln 100)) + bias_h[rel(a, b)] + shift mask) v
+ *   qkv        : bf16 [n_windows * N, ldq] (N = window^2), columns q | k | v (heads*32 each), rows in window order
+ *   table      : f32 [heads, (2 window - 1)^2] = 16 sigmoid(cpb_mlp(relative_coords_table)) * log2(e), rows in
+ *                relative_position_index order (evt_swinv2_cpb_table times log2(e))
+ *   head_scale : f32 [heads] = exp(min(logit_scale_h, ln 100)) * log2(e)
+ *   grid       : tokens per image side at this stage; window w of the call is window w % (grid / window)^2 of its image
+ *   shift      : the block's cyclic shift (0: no mask); pairs in different regions of a shifted window get `mask` added
+ *                (natural-log units: -100 once as microsoft/Swin-Transformer adds it, -200 as the HF forward adds it twice)
+ *   ctx        : bf16 [n_windows * N, ldc].
+ * q and k rows are normalised in f32 and rounded to f16 for the score product; P V in bf16; softmax in f32. */
+int evt_cosine_window_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* table,
+                                    const float* head_scale, int64_t n_windows, int window, int heads, int head_size, int grid,
+                                    int shift, float mask, evt_stream stream);
+
+/* Post-norm residual update (Swinv2Layer.forward :700-716, Swinv2PatchMerging :384-386):
+ *   output row r (image r / T_out, token t = r % T_out), group g = 0..G-1 reads source row
+ *   s = image * T_in + (idx ? idx[t * G + g] : t) and writes  (resid ? resid[s] : 0) + LayerNorm(y[s])  (C floats) to
+ *   columns [g C, g C + C) of row r of out_f32 (f32) and / or out_bf16 (bf16), both [images * T_out, G * C], nullable.
+ *   y, resid : f32 [images * T_in, C]; idx : int32 [T_out * G] (device) or NULL (then G = 1, T_in = T_out, and out_f32 may
+ *   alias resid).  G = 1 with idx: the next block's window order; G = 4: patch merging's 2x2 concat. */
+int evt_postnorm_residual(const float* y, const float* resid, const int* idx, const float* gamma, const float* beta,
+                          float* out_f32, void* out_bf16, int64_t images, int T_in, int T_out, int G, int C, float eps,
+                          evt_stream stream);
+
+/* HOST computations of the Swin V2 load (no device needed), exposed so that they can be checked against a reference:
+ * evt_swinv2_cpb_table: out [heads, (2 window - 1)^2] = 16 sigmoid(cpb_mlp(relative_coords_table)) evaluated in f64
+ *   (:490-524; coordinates divided by pretrained_window - 1 when pretrained_window > 0, by window - 1 otherwise);
+ *   w1 f32 [512, 2], b1 f32 [512], w2 f32 [heads, 512] = continuous_position_bias_mlp.{0.weight, 0.bias, 2.weight}.
+ * evt_swinv2_score_bias: out [(grid / window)^2, heads, N, N] = table[h, rel(a, b)] (+ mask where a and b lie in different
+ *   shift regions) -- the dense form of what evt_cosine_window_attention_fwd adds to the scores, from the same index and
+ *   region arithmetic. */
+int evt_swinv2_cpb_table(const float* w1, const float* b1, const float* w2, int heads, int window, int pretrained_window,
+                         float* out);
+int evt_swinv2_score_bias(const float* table, int heads, int window, int grid, int shift, float mask, float* out);
+
 /* ------------------------------------------------------------------ model level ---------- */
 
 typedef struct evt_model evt_model;
@@ -439,8 +479,19 @@ typedef struct evt_swin_spec {
   int heads[EVT_SWIN_MAX_STAGES];    /* heads per stage, e.g. 3, 6, 12, 24 */
   int num_labels;
   float eps;                         /* LayerNorm epsilon (1e-5) */
-  int precision;                     /* evt_precision: 0 bf16 operands (logits within 2e-2 of fp32), 1 tf32 operands (f32
-                                        activations rounded to tf32, logits within 1e-3); last, so a zeroed spec is bf16 */
+  int precision;                     /* evt_precision: 0 bf16 operands (V1 logits within 2e-2 of fp32; V2 see below), 1 tf32
+                                        operands (f32 activations rounded to tf32, logits within 1e-3); a zeroed spec is bf16 */
+  /* Swin V2 (version = 2): the 256-pixel swinv2_{tiny,small,base}_patch4_window{8,16}_256 and
+   * swinv2_{base,large}_patch4_window12to16_192to256_22kto1k_ft.  Post-norm blocks, cosine attention, continuous position
+   * bias; weights under HF Swinv2ForImageClassification names (swinv2.*).  Stage s runs window min(grid_s, window) (8 or 16),
+   * shifted by window / 2 in odd blocks unless grid_s <= window.  bf16 precision only: logits within 2e-2 of fp32 for tiny
+   * and for reduced depths; full-depth base / large reach 2.1e-2 / 2.8e-2, of which bf16-rounded weights alone cause
+   * 1.9e-2 / 2.5e-2 (post-norm blocks carry each branch's relative rounding error into the stream at full scale).  0 or 1 =
+   * V1 exactly as above. */
+  int version;
+  int pretrained_window[EVT_SWIN_MAX_STAGES];  /* V2: pretrained_window_sizes (0: the CPB coordinates are scaled by the window) */
+  int mask_adds;                               /* V2: times the -100 shift mask is added: 1 (microsoft/Swin-Transformer, 0 = 1) or
+                                                  2 (the installed HF forward adds it twice) */
 } evt_swin_spec;
 
 int evt_swin_create(const evt_swin_spec* spec, evt_swin** out);
