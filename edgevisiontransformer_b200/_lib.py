@@ -79,6 +79,8 @@ SIGNATURES = {
     "evt_attention_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _f, _p]),
     "evt_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _f, _p]),
     "evt_attention_query_rows_fwd": (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _i, _f, _p]),
+    "evt_attention_rel_bias_fwd": (_i, [_p, _i64, _p, _i64, _p, _p, _i, _i, _i, _i, _i, _i, _f, _p]),
+    "evt_beit_score_bias": (_i, [_p, _i, _i, _p]),
     "evt_im2col_patch": (_i, [_p, _p, _i, _i, _i, _i, _p]),
     "evt_im2col_patch_ex": (_i, [_p, _p, _i, _i, _i, _i, _i, _p]),
     "evt_patch_embed_workspace_bytes": (_i, [_i, _i, _i, _i, _i, C.POINTER(C.c_size_t)]),
@@ -91,6 +93,7 @@ SIGNATURES = {
     "evt_window_attention_fwd_tf32": (_i, [_p, _i64, _p, _i64, _p, _i, _i64, _i, _i, _i, _f, _p]),
     "evt_layernorm_mean_tokens": (_i, [_p, _p, _p, _p, _i64, _i, _i, _f, _p]),
     "evt_layernorm_mean_tokens_ex": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _f, _p]),
+    "evt_layernorm_patch_mean": (_i, [_p, _p, _p, _p, _i64, _i, _i, _f, _p]),
     "evt_cosine_window_attention_fwd": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _i, _i, _i, _i, _f, _p]),
     "evt_postnorm_residual": (_i, [_p, _p, _p, _p, _p, _p, _p, _i64, _i, _i, _i, _i, _f, _p]),
     "evt_swinv2_cpb_table": (_i, [_p, _p, _p, _i, _i, _i, _p]),

@@ -31,6 +31,8 @@ SWIN = {"swin_tiny": (96, [2, 2, 6, 2], [3, 6, 12, 24]), "swin_small": (96, [2, 
 SWIN_WINDOW = {224: 7, 384: 12}
 # swinv2_*_patch4_window{8,16}_256 (modeling_swinv2.SWINV2): --window picks 8 (default) or 16, always 256 pixels
 SWINV2 = ("swinv2_tiny", "swinv2_small", "swinv2_base")
+# beit_{base,large}_patch16_{224,384,512} (modeling_beit): --image-size 224, 384 or 512
+BEIT = {"beit_base": (768, 12, 12), "beit_large": (1024, 24, 16)}   # hidden, layers, heads
 T2T = {"t2t_vit_7": (256, 7, 4, 2.0), "t2t_vit_10": (256, 10, 4, 2.0), "t2t_vit_12": (256, 12, 4, 2.0),
        "t2t_vit_14": (384, 14, 6, 3.0)}
 
@@ -131,6 +133,15 @@ def build_model(name: str, precision: str = "bf16", max_batch: int = 512, device
                                                    depths=depths, num_heads=heads, num_labels=1000)).eval()
         m = B200SwinForImageClassification.from_hf(hf, device=device, max_batch=min(max_batch, 1024))
         return m, (3, image_size, image_size), f"{name} random-init (bf16, {image_size} px, window {window})"
+    if name in BEIT:
+        from transformers import BeitConfig, BeitForImageClassification
+        from ..modeling_beit import B200BeitForImageClassification
+        D, L, heads = BEIT[name]
+        torch.manual_seed(0)
+        hf = BeitForImageClassification(BeitConfig(hidden_size=D, num_hidden_layers=L, num_attention_heads=heads, intermediate_size=4 * D,
+                                                   image_size=image_size, use_relative_position_bias=True, num_labels=1000)).eval()
+        m = B200BeitForImageClassification.from_hf(hf, device=device, max_batch=max_batch, precision=precision, keep_params=False)
+        return m, (3, image_size, image_size), f"{name}_patch16_{image_size} random-init ({precision})"
     if name in SWINV2:
         from ..modeling_swinv2 import SWINV2 as V2, B200Swinv2ForImageClassification
         from transformers import Swinv2Config, Swinv2ForImageClassification
@@ -185,7 +196,7 @@ def b200_benchmark(model, input_shape: Sequence[int], num_runs: int = 50, warmup
 
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="b200_benchmark", description=__doc__.split("\n")[0])
-    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | deit3_* (modeling_vit.DEIT3) | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir | T2T-ViT .pth[.tar]")
+    ap.add_argument("--model", required=True, help="deit_{tiny,small,base} | deit3_* (modeling_vit.DEIT3) | beit_{base,large} | swin_{tiny,small,base,large} | t2t_vit_{7,10,12,14} | attention | ffn | checkpoint dir | T2T-ViT .pth[.tar]")
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--precision", default="bf16", choices=["bf16", "tf32"])
     ap.add_argument("--num_runs", type=int, default=50)
@@ -194,7 +205,8 @@ def main(argv=None) -> int:
     ap.add_argument("--graph", action="store_true", help="CUDA-graph replay (small-batch latency path)")
     ap.add_argument("--window", type=int, default=None, choices=[8, 16], help="swinv2_{tiny,small,base}: window 8 (default) or 16, 256 px")
     ap.add_argument("--image-size", type=int, default=224,
-                    help="deit_* / swin_* input resolution (384: deit_*_patch16_384, 577 tokens; swin_*_patch4_window12_384)")
+                    help="deit_* / swin_* / beit_* input resolution (384: deit_*_patch16_384, 577 tokens; swin_*_patch4_window12_384; "
+                         "beit_*: 224, 384 or 512)")
     for k, d in (("h", 768), ("a", 12), ("i", 3072), ("n", 128)):
         ap.add_argument(f"--{k}", type=int, default=d)
     ap.add_argument("--h_k", type=int, default=None)
@@ -208,8 +220,10 @@ def main(argv=None) -> int:
         if a.image_size not in (224, 256):
             ap.error("swinv2_* runs at 256 pixels")
         a.image_size = 256
-    if a.image_size != 224 and a.model not in DEIT and a.model not in SWIN and a.model not in SWINV2:
-        ap.error("--image-size applies to the deit_* and swin_* models only")
+    if a.image_size != 224 and a.model not in DEIT and a.model not in SWIN and a.model not in SWINV2 and a.model not in BEIT:
+        ap.error("--image-size applies to the deit_*, beit_* and swin_* models only")
+    if a.model in BEIT and a.image_size not in (224, 384, 512):
+        ap.error("beit_* runs at --image-size 224, 384 or 512")
     if a.model in SWIN and a.image_size not in SWIN_WINDOW:
         ap.error("swin_* runs at --image-size 224 (window 7) or 384 (window 12)")
     model, shape, desc = build_model(a.model, a.precision, max_batch=max(a.batch, 1), image_size=a.image_size, window=a.window or 8, h=a.h, a=a.a, i=a.i,

@@ -108,10 +108,120 @@ __device__ __forceinline__ void chunk_exp(const uint32_t (&r)[W], int nvalid, ui
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// BEiT relative position bias (attention2_kernel<true>, attention_long_kernel<64, true>): the scores of head h become
+// s * scale * log2(e) + table[h][rel(q, k)], table = the checkpoint's [(2W-1)^2 + 3] entries of the head times log2(e), for an
+// image of W x W patches behind one cls token (S = W^2 + 1).  rel is generate_relative_position_index of
+// SITE/models/beit/modeling_beit.py:521-544.  For two patch tokens it is a query part minus a key part, so a softmax thread adds
+// a per-row constant to a per-key value read as a shared-memory broadcast, and each score costs one gathered table read.
+struct RelBias {
+  const float* table;  // f32 [heads, n] (16-byte aligned), n = (2 grid - 1)^2 + 3, times log2(e)
+  int grid;            // W: patches per image side
+  int n;
+};
+__host__ __device__ __forceinline__ int beit_query_part(int t, int W) {  // patch token t >= 1
+  return ((t - 1) / W + W - 1) * (2 * W - 1) + (t - 1) % W + W - 1;
+}
+__host__ __device__ __forceinline__ int beit_key_part(int t, int W) { return (t - 1) / W * (2 * W - 1) + (t - 1) % W; }
+// Index into the table of the bias between query token q and key token k (token 0 = cls).
+__host__ __device__ __forceinline__ int beit_rel_index(int q, int k, int W) {
+  const int n = (2 * W - 1) * (2 * W - 1) + 3;
+  if (q == 0) return k == 0 ? n - 1 : n - 3;
+  if (k == 0) return n - 2;
+  return beit_query_part(q, W) - beit_key_part(k, W);
+}
+
+// One softmax thread's view of the bias: the head's table (shared address `tab`), the key parts (`ko`: uint16 per key column,
+// 0 for the cls column and for columns >= S), the row constant qb and the bias of the cls column b0.  The cls query row (and a
+// row past S) has kmask = 0: every key column then reads table[n - 3].
+struct RowBias {
+  uint32_t ko, tab;
+  int qb, kmask;
+  float b0;
+};
+__device__ __forceinline__ RowBias row_bias(const RelBias& rb, uint32_t ko, uint32_t tab, int q) {
+  const bool patch = q >= 1 && q <= rb.grid * rb.grid;
+  RowBias r;
+  r.ko = ko;
+  r.tab = tab;
+  r.qb = patch ? beit_query_part(q, rb.grid) : rb.n - 3;
+  r.kmask = patch ? -1 : 0;
+  r.b0 = ptx::lds_f1(tab + 4 * (patch ? rb.n - 2 : rb.n - 1));
+  return r;
+}
+// Bias (log2 units) of the 16 key columns col0 .. col0 + 15.
+__device__ __forceinline__ void chunk_bias(const RowBias& r, int col0, float (&b)[16]) {
+  const float4 k0 = ptx::lds_f4(r.ko + 2 * col0), k1 = ptx::lds_f4(r.ko + 2 * col0 + 16);
+  const uint32_t kw[8] = {__float_as_uint(k0.x), __float_as_uint(k0.y), __float_as_uint(k0.z), __float_as_uint(k0.w),
+                          __float_as_uint(k1.x), __float_as_uint(k1.y), __float_as_uint(k1.z), __float_as_uint(k1.w)};
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    b[2 * j] = ptx::lds_f1(r.tab + 4 * (r.qb - (static_cast<int>(kw[j] & 0xffffu) & r.kmask)));
+    b[2 * j + 1] = ptx::lds_f1(r.tab + 4 * (r.qb - (static_cast<int>(kw[j] >> 16) & r.kmask)));
+  }
+  if (col0 == 0) b[0] = r.b0;
+}
+// The biased score t = s * scale_log2e + b of a column pair, one packed FMA: the max pass and the exponential pass both call
+// this, so the maximum is one of the values the exponentials subtract it from.
+__device__ __forceinline__ uint64_t biased_pair(uint32_t s0, uint32_t s1, uint64_t scale2, float b0, float b1) {
+  return ptx::fma2(ptx::pk2(__uint_as_float(s0), __uint_as_float(s1)), scale2, ptx::pk2(b0, b1));
+}
+// chunk_max / chunk_exp of 16 columns with the bias: the maximum is taken over t (log2 units); p = 2^(t + negm).
+template <bool MASKED>
+__device__ __forceinline__ void chunk_max_bias(const uint32_t (&r)[16], int nvalid, uint64_t scale2, const RowBias& rb, int col0,
+                                               float (&m)[4]) {
+  float b[16];
+  chunk_bias(rb, col0, b);
+#pragma unroll
+  for (int j = 0; j < 16; j += 2) {
+    float t0, t1;
+    ptx::upk2(biased_pair(r[j], r[j + 1], scale2, b[j], b[j + 1]), t0, t1);
+    if (!MASKED || j < nvalid) m[j & 3] = fmaxf(m[j & 3], t0);
+    if (!MASKED || j + 1 < nvalid) m[(j + 1) & 3] = fmaxf(m[(j + 1) & 3], t1);
+  }
+}
+template <bool MASKED>
+__device__ __forceinline__ void chunk_exp_bias(const uint32_t (&r)[16], int nvalid, uint64_t scale2, uint64_t negm2, const RowBias& rb,
+                                               int col0, uint64_t (&sum2)[2], uint32_t (&pk)[8]) {
+  float b[16];
+  chunk_bias(rb, col0, b);
+#pragma unroll
+  for (int j = 0; j < 16; j += 2) {
+    float t0, t1;
+    ptx::upk2(ptx::add2(biased_pair(r[j], r[j + 1], scale2, b[j], b[j + 1]), negm2), t0, t1);
+    float p0, p1;
+    if (((j >> 1) & 3) >= 4 - kPolyPairs) {
+      ex2_poly_pair(t0, t1, p0, p1);
+    } else {
+      p0 = ptx::ex2_approx(t0);
+      p1 = ptx::ex2_approx(t1);
+    }
+    if (MASKED) {
+      if (j >= nvalid) p0 = 0.f;
+      if (j + 1 >= nvalid) p1 = 0.f;
+    }
+    sum2[(j >> 1) & 1] = ptx::add2(sum2[(j >> 1) & 1], ptx::pk2(p0, p1));
+    pk[j >> 1] = ptx::pack_bf16x2(p0, p1);
+  }
+}
+// The per-chunk steps of the two softmax passes, with or without the bias (col0: the chunk's first key column).
+template <bool BIAS, bool MASKED>
+__device__ __forceinline__ void row_max_step(const uint32_t (&r)[16], int nvalid, uint64_t scale2, const RowBias& rb, int col0, float (&m)[4]) {
+  if constexpr (BIAS) chunk_max_bias<MASKED>(r, nvalid, scale2, rb, col0, m);
+  else chunk_max<16, MASKED>(r, nvalid, m);
+}
+template <bool BIAS, bool MASKED>
+__device__ __forceinline__ void row_exp_step(const uint32_t (&r)[16], int nvalid, uint64_t scale2, uint64_t negm2, const RowBias& rb, int col0,
+                                             uint64_t (&sum2)[2], uint32_t (&pk)[8]) {
+  if constexpr (BIAS) chunk_exp_bias<MASKED>(r, nvalid, scale2, negm2, rb, col0, sum2, pk);
+  else chunk_exp<16, MASKED>(r, nvalid, scale2, negm2, sum2, pk);
+}
+
 // One query row per thread: row maximum, exponentials, bf16 P written over the consumed S columns of the slot at t_row,
 // f32 row sum returned (the caller issues tcgen05.wait::st).  n16 = score chunks of 16 columns, last_valid = valid columns
-// in the last one.
-__device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_valid, float scale_log2e) {
+// in the last one.  BIAS: the relative position bias of `bias` is added to every score.
+template <bool BIAS = false>
+__device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_valid, float scale_log2e, const RowBias& bias = {}) {
   const uint64_t scale2 = ptx::pk2(scale_log2e, scale_log2e);
   float sum;
   {
@@ -127,24 +237,24 @@ __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_v
       for (; c + 2 <= n16 - 1; c += 2) {
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-        chunk_max<16, false>(ra, 16, m);
+        row_max_step<BIAS, false>(ra, 16, scale2, bias, c * 16, m);
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
-        chunk_max<16, false>(rb, 16, m);
+        row_max_step<BIAS, false>(rb, 16, scale2, bias, (c + 1) * 16, m);
       }
       if (c + 1 < n16) {
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-        chunk_max<16, false>(ra, 16, m);
+        row_max_step<BIAS, false>(ra, 16, scale2, bias, c * 16, m);
         ptx::tmem_ld_wait();
-        chunk_max<16, true>(rb, last_valid, m);
+        row_max_step<BIAS, true>(rb, last_valid, scale2, bias, (c + 1) * 16, m);
       } else {
         ptx::tmem_ld_wait();
-        chunk_max<16, true>(ra, last_valid, m);
+        row_max_step<BIAS, true>(ra, last_valid, scale2, bias, c * 16, m);
       }
     }
     const float mx = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3]));
-    const float nm = -mx * scale_log2e;
+    const float nm = BIAS ? -mx : -mx * scale_log2e;  // with the bias, the maximum is already in log2 units
     const uint64_t negm2 = ptx::pk2(nm, nm);
     // pass 2: probabilities (bf16) written over the S columns already consumed; fp32 row sum
     uint64_t sum2[2] = {0ull, 0ull};
@@ -156,24 +266,24 @@ __device__ __forceinline__ float softmax_row(uint32_t t_row, int n16, int last_v
       for (; c + 2 <= n16 - 1; c += 2) {
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-        chunk_exp<16, false>(ra, 16, scale2, negm2, sum2, pk);
+        row_exp_step<BIAS, false>(ra, 16, scale2, negm2, bias, c * 16, sum2, pk);
         ptx::tmem_st_x8(t_row + c * 8, pk);
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
-        chunk_exp<16, false>(rb, 16, scale2, negm2, sum2, pk);
+        row_exp_step<BIAS, false>(rb, 16, scale2, negm2, bias, (c + 1) * 16, sum2, pk);
         ptx::tmem_st_x8(t_row + (c + 1) * 8, pk);
       }
       if (c + 1 < n16) {
         ptx::tmem_ld_wait();
         ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-        chunk_exp<16, false>(ra, 16, scale2, negm2, sum2, pk);
+        row_exp_step<BIAS, false>(ra, 16, scale2, negm2, bias, c * 16, sum2, pk);
         ptx::tmem_st_x8(t_row + c * 8, pk);
         ptx::tmem_ld_wait();
-        chunk_exp<16, true>(rb, last_valid, scale2, negm2, sum2, pk);
+        row_exp_step<BIAS, true>(rb, last_valid, scale2, negm2, bias, (c + 1) * 16, sum2, pk);
         ptx::tmem_st_x8(t_row + (c + 1) * 8, pk);
       } else {
         ptx::tmem_ld_wait();
-        chunk_exp<16, true>(ra, last_valid, scale2, negm2, sum2, pk);
+        row_exp_step<BIAS, true>(ra, last_valid, scale2, negm2, bias, c * 16, sum2, pk);
         ptx::tmem_st_x8(t_row + c * 8, pk);
       }
     }
@@ -376,6 +486,25 @@ __device__ __forceinline__ void store_context(float sum, float hm, bool warp_liv
   }
 }
 
+// Relative position bias in shared memory, after the AttnSmem fields: the uint16 key parts of kc key columns (filled once per
+// CTA, before the prologue's __syncthreads), then one table of n floats per softmax group.  A group's table is reloaded when its
+// next item has another head: once any warp of the group has passed pv_done of its previous item, all four warps have handed
+// over that item's P, so nobody reads the old table any more; the group's named barrier publishes the new one.
+__device__ __forceinline__ uint32_t bias_smem(const AttnSmem& sm) { return ptx::smem_u32(sm.tmem_ptr) + 16; }
+__host__ __device__ constexpr int bias_smem_bytes(int kc, int n) { return 2 * kc + 2 * 4 * n; }
+__device__ __forceinline__ void fill_key_parts(const AttnSmem& sm, const RelBias& rb, int S, int kc) {
+  uint16_t* ko = reinterpret_cast<uint16_t*>(reinterpret_cast<uint8_t*>(sm.tmem_ptr) + 16);
+  for (int k = threadIdx.x; k < kc; k += blockDim.x) ko[k] = static_cast<uint16_t>(k >= 1 && k < S ? beit_key_part(k, rb.grid) : 0);
+}
+__device__ __forceinline__ void stage_table(const RelBias& rb, int h, uint32_t tab, int grp) {
+  const float4* src = reinterpret_cast<const float4*>(rb.table + static_cast<size_t>(h) * rb.n);
+  for (int i = threadIdx.x & 127; i < rb.n / 4; i += 128) {
+    const float4 v = __ldg(src + i);
+    ptx::sts_f4(tab + 16 * i, v.x, v.y, v.z, v.w);
+  }
+  ptx::named_bar_sync(1 + grp, 128);
+}
+
 __device__ __forceinline__ void attn_teardown(int warp, uint32_t tmem_base) {
   ptx::tc_fence_before();
   __syncthreads();
@@ -385,12 +514,14 @@ __device__ __forceinline__ void attn_teardown(int warp, uint32_t tmem_base) {
   }
 }
 
+template <bool BIAS>
 __global__ void __launch_bounds__(kThreads2, 1)
 attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
-                  const __grid_constant__ CUtensorMap tmO, const Attn2Params p) {
+                  const __grid_constant__ CUtensorMap tmO, const Attn2Params p, const RelBias rbp) {
   extern __shared__ uint8_t smem_raw[];
   const int kv_bytes = p.SK * 128;
   const AttnSmem sm = attn_smem(smem_raw, p.n_kv * 2 * kv_bytes);  // ring: n_kv x (K | V)
+  if constexpr (BIAS) fill_key_parts(sm, rbp, p.S, p.SK);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int a = p.heads * kHD;
@@ -501,6 +632,9 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     const bool split = p.n_mt != p.q_tiles;
     int ql = p.n_mt == 2 ? 0 : grp;
     Unit u = unit_of(p, ql);
+    const uint32_t ko = BIAS ? bias_smem(sm) : 0u;
+    const uint32_t tab = ko + 2 * p.SK + grp * 4 * rbp.n;
+    int tab_h = -1;  // head whose table the group holds
 #pragma unroll 1
     for (int j = grp; j < n_items; j += 2, ql += dql) {
       const uint32_t ph = (j >> 1) & 1;
@@ -521,11 +655,19 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       const bool warp_live = qrow0 < p.Sq;  // block 7 (rows 224..255) when S = 197, or a block past Sq: nothing to do
       float hm = 1.f;
       if (p.head_mask != nullptr) hm = p.head_mask[u.h];
+      RowBias bias{};
+      if constexpr (BIAS) {
+        if (u.h != tab_h) {
+          stage_table(rbp, u.h, tab, grp);
+          tab_h = u.h;
+        }
+        bias = row_bias(rbp, ko, tab, qrow0 + lane);
+      }
       ptx::mbar_wait(&sm.s_ready[grp], ph);
       ptx::tc_fence_after();
       float sum = 1.f;
       if (warp_live) {
-        sum = softmax_row(t_row, n16, last_valid, p.scale_log2e);
+        sum = softmax_row<BIAS>(t_row, n16, last_valid, p.scale_log2e, bias);
         ptx::tmem_st_wait();
       }
       ptx::tc_fence_before();
@@ -608,9 +750,11 @@ __device__ __forceinline__ int groups_of(const AttnLongParams& p, int ql) { retu
 // One 128-key block of the online softmax for the query row at t_row (nvalid: valid keys in the block, 1..128).  mu is
 // the row's current maximum times scale * log2(e), sum its running sum; both are updated, and O (TMEM columns
 // [kOCol, kOCol + HD)) is rescaled with them when the maximum moves (has_o: O already holds earlier blocks).
-// bf16 P is written over the consumed S columns; the caller issues tcgen05.wait::st.
-template <int HD, bool MASKED>
-__device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool has_o, float scale_log2e, float& mu, float& sum) {
+// bf16 P is written over the consumed S columns; the caller issues tcgen05.wait::st.  BIAS: the relative position bias of
+// `bias` is added to every score (col0: the block's first key column); bm and mu are maxima of the biased scores.
+template <int HD, bool MASKED, bool BIAS = false>
+__device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool has_o, float scale_log2e, float& mu, float& sum,
+                                              const RowBias& bias = {}, int col0 = 0) {
   const uint64_t scale2 = ptx::pk2(scale_log2e, scale_log2e);
   uint32_t ra[16], rb[16];
   float m[4] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
@@ -619,12 +763,12 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
   for (int c = 0; c < kKeyBlock / 16; c += 2) {
     ptx::tmem_ld_wait();
     ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-    chunk_max<16, MASKED>(ra, nvalid - c * 16, m);
+    row_max_step<BIAS, MASKED>(ra, nvalid - c * 16, scale2, bias, col0 + c * 16, m);
     ptx::tmem_ld_wait();
     if (c + 2 < kKeyBlock / 16) ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
-    chunk_max<16, MASKED>(rb, nvalid - (c + 1) * 16, m);
+    row_max_step<BIAS, MASKED>(rb, nvalid - (c + 1) * 16, scale2, bias, col0 + (c + 1) * 16, m);
   }
-  const float bm = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3])) * scale_log2e;
+  const float bm = fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3])) * (BIAS ? 1.f : scale_log2e);
   const bool grow = bm > mu + kRescaleLog2;  // always on the first block (mu = -inf)
   float alpha = 1.f;
   if (grow) {
@@ -662,11 +806,11 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
   for (int c = 0; c < kKeyBlock / 16; c += 2) {
     ptx::tmem_ld_wait();
     ptx::tmem_ld_x16(t_row + (c + 1) * 16, rb);
-    chunk_exp<16, MASKED>(ra, nvalid - c * 16, scale2, negm2, sum2, pk);
+    row_exp_step<BIAS, MASKED>(ra, nvalid - c * 16, scale2, negm2, bias, col0 + c * 16, sum2, pk);
     ptx::tmem_st_x8(t_row + c * 8, pk);
     ptx::tmem_ld_wait();
     if (c + 2 < kKeyBlock / 16) ptx::tmem_ld_x16(t_row + (c + 2) * 16, ra);
-    chunk_exp<16, MASKED>(rb, nvalid - (c + 1) * 16, scale2, negm2, sum2, pk);
+    row_exp_step<BIAS, MASKED>(rb, nvalid - (c + 1) * 16, scale2, negm2, bias, col0 + (c + 1) * 16, sum2, pk);
     ptx::tmem_st_x8(t_row + (c + 1) * 8, pk);
   }
   float s0, s1, s2, s3;
@@ -675,14 +819,16 @@ __device__ __forceinline__ void softmax_block(uint32_t t_row, int nvalid, bool h
   sum += (s0 + s1) + (s2 + s3);
 }
 
-template <int HD>
+template <int HD, bool BIAS = false>
 __global__ void __launch_bounds__(kThreads2, 1)
 attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                       const __grid_constant__ CUtensorMap tmO, const AttnLongParams p, const __grid_constant__ CUtensorMap tmQ32,
-                      const __grid_constant__ CUtensorMap tmKV32) {
+                      const __grid_constant__ CUtensorMap tmKV32, const RelBias rbp) {
+  static_assert(!BIAS || HD == 64, "the relative position bias is implemented for head size 64");
   using LS = LongShape<HD>;
   extern __shared__ uint8_t smem_raw[];
   const AttnSmem sm = attn_smem(smem_raw, LS::kStages * 2 * LS::kBlockBytes, LS::kQBytes);  // ring: kStages x (K | V) blocks
+  if constexpr (BIAS) fill_key_parts(sm, rbp, p.S, p.n_kb * kKeyBlock);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int a = p.heads * HD;
@@ -805,6 +951,9 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + grp * kSlotCols;
     const int last_valid = p.S - (p.n_kb - 1) * kKeyBlock;  // valid keys in the last block (1..128)
     uint8_t* stg = sm.staging + warp * kStgWarpBytes;
+    const uint32_t ko = BIAS ? bias_smem(sm) : 0u;
+    const uint32_t tab = ko + 2 * p.n_kb * kKeyBlock + grp * 4 * rbp.n;
+    int tab_h = -1;  // head whose table the group holds
 #pragma unroll 1
     for (int ql = 0; ql < my_units; ++ql) {
       const int idx = item_index(ql, grp);
@@ -814,6 +963,14 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       const bool warp_live = qrow0 < p.Sq;  // rows past Sq (or past S in the last tile): nothing to compute
       float hm = 1.f;
       if (p.head_mask != nullptr) hm = p.head_mask[u.h];
+      RowBias bias{};
+      if constexpr (BIAS) {
+        if (u.h != tab_h) {
+          stage_table(rbp, u.h, tab, grp);
+          tab_h = u.h;
+        }
+        bias = row_bias(rbp, ko, tab, qrow0 + lane);
+      }
       const int c0 = ql * p.n_kb;  // this group's block count before the item: the barrier phases below
       float mu = -CUDART_INF_F, sum = 0.f;
 #pragma unroll 1
@@ -822,8 +979,8 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         if (kb != 0) ptx::mbar_wait(&sm.pv_done[grp], (c0 + kb - 1) & 1);  // O may be rescaled below
         ptx::tc_fence_after();
         if (warp_live) {
-          if (kb != p.n_kb - 1) softmax_block<HD, false>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum);
-          else softmax_block<HD, true>(t_row, last_valid, kb != 0, p.scale_log2e, mu, sum);
+          if (kb != p.n_kb - 1) softmax_block<HD, false, BIAS>(t_row, kKeyBlock, kb != 0, p.scale_log2e, mu, sum, bias, kb * kKeyBlock);
+          else softmax_block<HD, true, BIAS>(t_row, last_valid, kb != 0, p.scale_log2e, mu, sum, bias, kb * kKeyBlock);
           ptx::tmem_st_wait();
         }
         ptx::tc_fence_before();
@@ -1025,9 +1182,9 @@ attention_tf32_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 }
 
 // S > 256 (head size 64) or any S (head size 80): attention_long_kernel.  Argument checks are the caller's.
-template <int HD>
+template <int HD, bool BIAS = false>
 int attention_long_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
-                          int heads, float scale, cudaStream_t stream) {
+                          int heads, float scale, cudaStream_t stream, const RelBias& rb = {}) {
   using LS = LongShape<HD>;
   AttnLongParams q;
   q.head_mask = head_mask;
@@ -1067,15 +1224,20 @@ int attention_long_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, 
   const long long units = (n_items + 1) / 2;
   const int grid = units < num_sms() ? static_cast<int>(units) : num_sms();
   const int smem = 1024 + LS::kStages * 2 * LS::kBlockBytes + 2 * LS::kQBytes + kSoftmaxWarps * kStgWarpBytes +
-                   (2 * kMaxKV + 12) * 8 + 16;
-  EVT_TRY(opt_in_smem<attention_long_kernel<HD>>(smem));
+                   (2 * kMaxKV + 12) * 8 + 16 + (BIAS ? bias_smem_bytes(q.n_kb * kKeyBlock, rb.n) : 0);
+  // opt_in_smem sets the limit once per kernel: the biased kernel's size depends on the grid, so it asks for the maximum
+  EVT_TRY((opt_in_smem<attention_long_kernel<HD, BIAS>>(BIAS ? 232448 : smem)));
   const bool pdl = pdl_for_work(static_cast<long long>(B) * S, static_cast<long long>(heads) * HD);
-  EVT_CUDA(launch_pdl(attention_long_kernel<HD>, dim3(grid), dim3(kThreads2), smem, stream, pdl, tmQ, tmKV, tmO, q, tmQ32, tmKV32));
+  EVT_CUDA(launch_pdl(attention_long_kernel<HD, BIAS>, dim3(grid), dim3(kThreads2), smem, stream, pdl, tmQ, tmKV, tmO, q, tmQ32, tmKV32, rb));
   EVT_LAUNCH_CHECK("attention_long_kernel");
   return EVT_OK;
 }
 
 }  // namespace
+
+template <bool BIAS>
+int attention_short_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
+                           int heads, float scale, cudaStream_t stream, const RelBias& rb = {});
 
 int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                      int heads, int head_size, float scale, cudaStream_t stream) {
@@ -1107,6 +1269,13 @@ int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t
   EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention: ctx must be 16-byte aligned rows");
   EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention: B*S too large");
   if (S > 256) return attention_long_launch<kHD>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
+  return attention_short_launch<false>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream);
+}
+
+// S <= 256, head size 64: attention2_kernel.  Argument checks are the caller's.
+template <bool BIAS>
+int attention_short_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
+                           int heads, float scale, cudaStream_t stream, const RelBias& rb) {
   const int SK = (S + 15) / 16 * 16;
   const uint64_t rows = static_cast<uint64_t>(B) * S;
   const int q_tiles = (Sq + kQRows - 1) / kQRows;
@@ -1138,16 +1307,37 @@ int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t
   q.n_mt = n_mt;
   q.q_tiles = q_tiles;
   q.scale_log2e = scale_log2e;
-  const int fixed = 1024 + 2 * kQTileBytes + kSoftmaxWarps * kStgWarpBytes + (2 * kMaxKV + 12) * 8 + 16;
+  const int fixed = 1024 + 2 * kQTileBytes + kSoftmaxWarps * kStgWarpBytes + (2 * kMaxKV + 12) * 8 + 16 +
+                    (BIAS ? bias_smem_bytes(SK, rb.n) : 0);
   int n_kv = (max_smem - fixed) / (2 * SK * 128);
   if (n_kv > kMaxKV) n_kv = kMaxKV;
   if (n_kv < 2) return fail(EVT_ERR_UNSUPPORTED, "attention: sequence too long for two K/V stages");
   q.n_kv = n_kv;
   const int smem2 = fixed + n_kv * 2 * SK * 128;
-  EVT_TRY(opt_in_smem<attention2_kernel>(max_smem));
-  EVT_CUDA(launch_pdl(attention2_kernel, dim3(grid), dim3(kThreads2), smem2, stream, pdl, tmQ, tmKV, tmO, q));
+  EVT_TRY(opt_in_smem<attention2_kernel<BIAS>>(max_smem));
+  EVT_CUDA(launch_pdl(attention2_kernel<BIAS>, dim3(grid), dim3(kThreads2), smem2, stream, pdl, tmQ, tmKV, tmO, q, rb));
   EVT_LAUNCH_CHECK("attention2_kernel");
   return EVT_OK;
+}
+
+int attention_rel_bias_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, const float* table, int grid,
+                              int B, int S, int Sq, int heads, int head_size, float scale, cudaStream_t stream) {
+  EVT_CHECK_ARG(qkv && ctx && table, "attention_rel_bias: null pointer");
+  EVT_CHECK_ARG(B > 0 && S > 0 && heads > 0 && grid > 0, "attention_rel_bias: B, S, heads, grid must be positive");
+  EVT_CHECK_ARG(Sq > 0 && Sq <= S, "attention_rel_bias: query rows must be in 1..S");
+  if (head_size != kHD) return fail(EVT_ERR_UNSUPPORTED, "attention_rel_bias: only head size 64 is implemented");
+  if (S != grid * grid + 1)
+    return fail(EVT_ERR_UNSUPPORTED, "attention_rel_bias: S must be grid^2 + 1 (a cls token before grid x grid patches; no "
+                                     "distillation token)");
+  if (S > EVT_ATTN_MAX_TOKENS)
+    return fail(EVT_ERR_UNSUPPORTED, "attention_rel_bias: sequence length above " + std::to_string(EVT_ATTN_MAX_TOKENS) + " is not implemented");
+  EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(table) % 16 == 0, "attention_rel_bias: table must be 16-byte aligned");
+  EVT_CHECK_ARG(ldq >= 3ll * heads * kHD && ldc >= static_cast<int64_t>(heads) * kHD, "attention_rel_bias: leading dimension too small");
+  EVT_CHECK_ARG(ldc % 8 == 0 && reinterpret_cast<uintptr_t>(ctx) % 16 == 0, "attention_rel_bias: ctx must be 16-byte aligned rows");
+  EVT_CHECK_ARG(static_cast<int64_t>(B) * S < (1ll << 31) - 512, "attention_rel_bias: B*S too large");
+  const RelBias rb{table, grid, (2 * grid - 1) * (2 * grid - 1) + 3};  // n % 4 == 0: (2 grid - 1)^2 = 1 mod 8
+  if (S > 256) return attention_long_launch<kHD, true>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream, rb);
+  return attention_short_launch<true>(qkv, ldq, ctx, ldc, head_mask, B, S, Sq, heads, scale, stream, rb);
 }
 
 int attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask, int B, int S,
@@ -1211,4 +1401,25 @@ extern "C" int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx,
   if (rc != EVT_OK) return rc;
   return evt::attention_tf32_launch(qkv, ldq, ctx, ldc, head_mask, B, S, heads, head_size, scale,
                                     static_cast<cudaStream_t>(stream));
+}
+
+// BEiT relative position bias, see include/evt.h.
+extern "C" int evt_attention_rel_bias_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, const float* table,
+                                          int grid, int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::attention_rel_bias_launch(qkv, ldq, ctx, ldc, head_mask, table, grid, B, S, Sq, heads, head_size, scale,
+                                        static_cast<cudaStream_t>(stream));
+}
+
+// Host only: the dense bias the kernels add, from the same index arithmetic.
+extern "C" int evt_beit_score_bias(const float* table, int heads, int grid, float* out) {
+  EVT_CHECK_ARG(table != nullptr && out != nullptr, "beit_score_bias: null pointer");
+  EVT_CHECK_ARG(heads > 0 && grid > 0 && grid <= 64, "beit_score_bias: heads must be positive and grid in 1..64");
+  const int n = (2 * grid - 1) * (2 * grid - 1) + 3, S = grid * grid + 1;
+  for (int h = 0; h < heads; ++h)
+    for (int q = 0; q < S; ++q)
+      for (int k = 0; k < S; ++k)
+        out[(static_cast<size_t>(h) * S + q) * S + k] = table[static_cast<size_t>(h) * n + evt::beit_rel_index(q, k, grid)];
+  return EVT_OK;
 }

@@ -245,6 +245,79 @@ __global__ void __launch_bounds__(1024) ln2d_kernel(const float* __restrict__ x,
   }
 }
 
+// BEiT / data2vec-vision head (BeitPooler with use_mean_pooling, SITE/models/beit/modeling_beit.py:767-783):
+// y[image] = LayerNorm(mean of rows 1 .. T-1 of x[image]) in bf16 -- the mean first, then the norm (Swin's
+// ln_mean_tokens_kernel is the other order).  One CTA per image: warp w sums rows 1 + w, 1 + w + 8, .. with 4 columns per lane
+// per 128-column slab, the 8 partial rows are added in a fixed order through shared memory, and thread i normalises columns
+// [4i, 4i + 4) of the mean row.  D % 4 == 0, D <= 1024, x 16-byte aligned.
+constexpr int kPoolWarps = 8;
+__global__ void __launch_bounds__(kPoolWarps * 32) patch_mean_ln_kernel(const float* x, const float* __restrict__ gamma,
+                                                                        const float* __restrict__ beta, __nv_bfloat16* __restrict__ y,
+                                                                        int T, int D, float eps) {
+  __shared__ float4 part[kPoolWarps][256];
+  __shared__ float red[2][kPoolWarps];
+  ptx::grid_dep_launch();
+  ptx::grid_dep_wait();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const float* xi = x + static_cast<long long>(blockIdx.x) * T * D;
+  float4 acc[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 1
+  for (int t = 1 + warp; t < T; t += kPoolWarps) {
+    const float* xr = xi + static_cast<long long>(t) * D;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int c = i * 128 + lane * 4;
+      if (c < D) {
+        float4 v;
+        asm volatile("ld.global.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];"
+                     : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
+                     : "l"(xr + c));
+        acc[i].x += v.x, acc[i].y += v.y, acc[i].z += v.z, acc[i].w += v.w;
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i)
+    if (i * 128 + lane * 4 < D) part[warp][i * 32 + lane] = acc[i];
+  __syncthreads();
+  const int c = threadIdx.x * 4;
+  const bool live = c < D;
+  float4 m = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (live) {
+#pragma unroll
+    for (int w = 0; w < kPoolWarps; ++w) {
+      const float4 p = part[w][threadIdx.x];
+      m.x += p.x, m.y += p.y, m.z += p.z, m.w += p.w;
+    }
+    const float n = static_cast<float>(T - 1);
+    m = make_float4(m.x / n, m.y / n, m.z / n, m.w / n);
+  }
+  auto block_sum = [&](float v, float* r) {
+    v = ptx::warp_sum(v);
+    if (lane == 0) r[warp] = v;
+    __syncthreads();
+    float t = 0.f;
+#pragma unroll
+    for (int w = 0; w < kPoolWarps; ++w) t += r[w];
+    return t;
+  };
+  const float mean = block_sum(live ? (m.x + m.y) + (m.z + m.w) : 0.f, red[0]) / static_cast<float>(D);
+  const float a0 = m.x - mean, a1 = m.y - mean, a2 = m.z - mean, a3 = m.w - mean;
+  const float var = block_sum(live ? (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3) : 0.f, red[1]) / static_cast<float>(D);
+  const float rstd = rsqrtf(var + eps);
+  if (!live) return;
+  const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
+  const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
+  const __nv_bfloat162 lo = __floats2bfloat162_rn(a0 * rstd * g.x + b.x, a1 * rstd * g.y + b.y);
+  const __nv_bfloat162 hi = __floats2bfloat162_rn(a2 * rstd * g.z + b.z, a3 * rstd * g.w + b.w);
+  uint2 o;
+  o.x = *reinterpret_cast<const uint32_t*>(&lo);
+  o.y = *reinterpret_cast<const uint32_t*>(&hi);
+  *reinterpret_cast<uint2*>(y + static_cast<long long>(blockIdx.x) * D + c) = o;
+}
+
 template <int OUT>
 int launch_rows(const float* x, long long xs, const float* g, const float* b, void* y, long long ys, float* yc,
                 long long rows, int D, float eps, cudaStream_t st) {
@@ -308,6 +381,21 @@ int launch_rows(const float* x, long long xs, const float* g, const float* b, vo
 
 }  // namespace
 
+int layernorm_patch_mean_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
+                                cudaStream_t st) {
+  EVT_CHECK_ARG(x && gamma && beta && y, "layernorm_patch_mean: null pointer");
+  EVT_CHECK_ARG(images > 0 && images < (1ll << 31) && T >= 2, "layernorm_patch_mean: images must be positive and T >= 2");
+  EVT_CHECK_ARG(eps >= 0.f, "layernorm_patch_mean: negative eps");
+  if (D <= 0 || D % 4 != 0 || D > 1024) return fail(EVT_ERR_UNSUPPORTED, "layernorm_patch_mean: D must be a multiple of 4 in 4..1024");
+  EVT_CHECK_ARG(reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(gamma) % 16 == 0 &&
+                    reinterpret_cast<uintptr_t>(beta) % 16 == 0 && reinterpret_cast<uintptr_t>(y) % 8 == 0,
+                "layernorm_patch_mean: x, gamma, beta must be 16-byte and y 8-byte aligned");
+  EVT_CUDA(launch_pdl(patch_mean_ln_kernel, dim3(static_cast<unsigned>(images)), dim3(kPoolWarps * 32), 0, st, pdl_for_rows(images), x, gamma,
+                      beta, static_cast<__nv_bfloat16*>(y), T, D, eps));
+  EVT_LAUNCH_CHECK("patch_mean_ln");
+  return EVT_OK;
+}
+
 int layernorm_launch(const float* x, int64_t x_stride, const float* gamma, const float* beta, void* y, int y_dtype,
                      int64_t y_stride, float* y_copy, int64_t rows, int D, float eps, cudaStream_t st) {
   EVT_CHECK_ARG(x && gamma && beta && y, "layernorm: null pointer");
@@ -341,4 +429,11 @@ extern "C" int evt_layernorm2d_fwd(const float* x, const float* addend, const fl
                                                                                                  y, nh, eps);
   EVT_LAUNCH_CHECK("layernorm2d");
   return EVT_OK;
+}
+
+extern "C" int evt_layernorm_patch_mean(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D,
+                                        float eps, evt_stream stream) {
+  int rc = evt_device_check();
+  if (rc != EVT_OK) return rc;
+  return evt::layernorm_patch_mean_launch(x, gamma, beta, y, images, T, D, eps, static_cast<cudaStream_t>(stream));
 }

@@ -62,6 +62,7 @@ struct LayerW {
   uint8_t *wqkv = nullptr, *wo = nullptr, *w1 = nullptr, *w2 = nullptr;  // bf16 or f32 (tf32 mode) matrices
   float *bqkv = nullptr, *bo = nullptr, *b1 = nullptr, *b2 = nullptr;
   float *ln1_g = nullptr, *ln1_b = nullptr, *ln2_g = nullptr, *ln2_b = nullptr;
+  float* rel_tab = nullptr;  // BEiT relative position bias: [heads, (2W-1)^2 + 3] times log2(e), or null
   int a = 0, inter = 0, inter_ld = 0;
 };
 
@@ -95,6 +96,7 @@ struct evt_model {
   uint8_t* w_cls = nullptr;
   float* b_cls = nullptr;
   evt::PerformerW perf[2];   // spec.t2t: the two TokenPerformers of the tokens-to-token module
+  int rel_grid = 0;          // W of the BEiT relative position bias (layers[l].rel_tab), 0 without it
   std::vector<void*> allocs;
   // evt_model_profile_begin/end: one event before the first launch and one after every launch of a forward
   bool profiling = false;
@@ -184,6 +186,14 @@ int validate_spec(const evt_model_spec* s) {
     EVT_CHECK_ARG(s->tokens == patches + 2 && s->final_ln != 0 && s->head_hidden == 0,
                   "head_rows = 2 (two-head distilled DeiT) needs 198 tokens, the final LayerNorm and a single Linear head");
   EVT_CHECK_ARG(s->precision == EVT_PREC_BF16 || s->precision == EVT_PREC_TF32, "precision must be bf16 (0) or tf32 (1)");
+  EVT_CHECK_ARG(s->final_ln >= 0 && s->final_ln <= 2, "final_ln must be 0 (none), 1 (LayerNorm, classifier on the cls row) or 2 (LayerNorm "
+                                                      "of the mean of the patch rows)");
+  if (s->final_ln == 2) {
+    if (s->precision != EVT_PREC_BF16) return fail(EVT_ERR_UNSUPPORTED, "final_ln = 2 (mean-pooled head) is implemented in the bf16 mode only");
+    EVT_CHECK_ARG(s->tokens == patches + 1 && s->head_rows <= 1, "final_ln = 2 (mean-pooled head) needs tokens = patches + 1 and head_rows 0 or 1");
+    if (s->hidden % 4 != 0 || s->hidden > 1024)
+      return fail(EVT_ERR_UNSUPPORTED, "final_ln = 2 (mean-pooled head) is implemented for hidden sizes that are multiples of 4 up to 1024");
+  }
   EVT_CHECK_ARG(s->embed_k >= 0 && s->embed_k % 8 == 0, "embed_k must be a non-negative multiple of 8");
   EVT_CHECK_ARG(s->t2t >= 0 && s->t2t <= 3, "t2t must be 0 (patch embedding), 1 (T2T front-end, NHWC f32 pixels), 2 (T2T front-end, "
                                             "NCHW pixels) or 3 (T2T front-end with token transformers, NCHW pixels)");
@@ -405,6 +415,33 @@ extern "C" int evt_model_load_weights(evt_model* m, const evt_tensor_view* tenso
       EVT_TRY(L.vec(p + "mlp.fc2.bias", 64, true, &pw.bb2));
     }
   }
+  // BEiT relative position bias: per layer [(2W-1)^2 + 3, heads] in the HF layout, repacked to [heads, n] times log2(e) (the
+  // attention kernels' softmax runs in log2 units)
+  auto tab_name = [](int l) {
+    return "vit.encoder.layer." + std::to_string(l) + ".attention.attention.relative_position_bias.relative_position_bias_table";
+  };
+  if (L.find(tab_name(0)) != nullptr) {
+    const int W = s.image / s.patch, n = (2 * W - 1) * (2 * W - 1) + 3;
+    if (s.precision != EVT_PREC_BF16) return fail(EVT_ERR_UNSUPPORTED, "the relative position bias (BEiT) is implemented in the bf16 mode only");
+    if (s.tokens != W * W + 1)
+      return fail(EVT_ERR_UNSUPPORTED, "the relative position bias (BEiT) needs tokens = patches + 1 (no distillation token)");
+    if (s.head_size != 64) return fail(EVT_ERR_UNSUPPORTED, "the relative position bias (BEiT) is implemented for head size 64 only");
+    for (int l = 0; l < s.layers; ++l) {
+      const int h = s.heads[l];
+      std::vector<float> t;
+      EVT_TRY(L.host_copy(tab_name(l), static_cast<int64_t>(n) * h, &t));
+      std::vector<float> r(t.size());
+      for (int i = 0; i < n; ++i)
+        for (int j = 0; j < h; ++j) r[static_cast<size_t>(j) * n + i] = static_cast<float>(static_cast<double>(t[static_cast<size_t>(i) * h + j]) * 1.4426950408889634);
+      EVT_TRY(L.upload(r, &m->layers[l].rel_tab));
+    }
+    m->rel_grid = W;
+  } else {
+    for (int l = 1; l < s.layers; ++l)
+      if (L.find(tab_name(l)) != nullptr)
+        return fail(EVT_ERR_INVALID, "relative position bias tables must be given for every layer or for none (layer 0 has none, layer " +
+                                         std::to_string(l) + " has one)");
+  }
   if (s.final_ln) {
     EVT_TRY(L.vec("vit.layernorm.weight", D, false, &m->lnf_g));
     EVT_TRY(L.vec("vit.layernorm.bias", D, false, &m->lnf_b));
@@ -555,10 +592,10 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   // FC1 and FC2 run on `batch` rows: row i is image i's cls row (residual stream stride tokens * D, context and FC1
   // output packed).  Same launches, same kernels, so the cls row gets the same bits as in a full layer.  Full layer
   // instead when a caller asks for the last layer's context of every row (ctx_out), in the tf32 mode (its attention
-  // kernel has no query-row count) and for the two-head distilled DeiT (rows 0 and 1 of every image are not one strided
-  // row set).
+  // kernel has no query-row count), for the two-head distilled DeiT (rows 0 and 1 of every image are not one strided
+  // row set) and for the mean-pooled head (final_ln = 2: it reads every patch row).
   const int64_t tok_stride = static_cast<int64_t>(s.tokens) * D;
-  const bool cls_tail = !tf32 && s.head_rows <= 1 && !(o.ctx_out != nullptr && o.ctx_out[s.layers - 1] != nullptr);
+  const bool cls_tail = !tf32 && s.head_rows <= 1 && s.final_ln != 2 && !(o.ctx_out != nullptr && o.ctx_out[s.layers - 1] != nullptr);
   bool xn_ready = false;  // w.xn already holds LN1 of the current layer (written by the previous layer's FC2 epilogue)
   for (int l = 0; l < s.layers; ++l) {
     const LayerW& lw = m->layers[l];
@@ -589,6 +626,9 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
     if (tf32)
       EVT_STAGE(EVT_STAGE_ATTN, attention_tf32_launch(reinterpret_cast<const float*>(w.qkv), 3 * a, reinterpret_cast<float*>(ctx), a, hmask,
                                     batch, s.tokens, s.heads[l], s.head_size, scale, st));
+    else if (lw.rel_tab != nullptr)
+      EVT_STAGE(EVT_STAGE_ATTN, attention_rel_bias_launch(w.qkv, 3 * a, ctx, a, hmask, lw.rel_tab, m->rel_grid, batch, s.tokens,
+                                                          tail ? 1 : s.tokens, s.heads[l], s.head_size, scale, st));
     else
       EVT_STAGE(EVT_STAGE_ATTN, attention_launch(w.qkv, 3 * a, ctx, a, hmask, batch, s.tokens, tail ? 1 : s.tokens, s.heads[l], s.head_size,
                                                  scale, st));
@@ -614,7 +654,9 @@ static int forward_impl(evt_model* m, const void* pixels, const evt_forward_opts
   }
   // head: only the cls row of every image is consumed (SITE/models/vit/modeling_vit.py:641)
   const int head_rows = s.head_rows > 1 ? s.head_rows : 1;
-  if (s.final_ln) {
+  if (s.final_ln == 2) {  // BeitPooler with use_mean_pooling: LayerNorm of the mean of the patch rows
+    EVT_STAGE(EVT_STAGE_HEAD, layernorm_patch_mean_launch(w.resid, m->lnf_g, m->lnf_b, w.clsn, batch, s.tokens, D, s.eps, st));
+  } else if (s.final_ln) {
     // head_rows = 2 (DeiTForImageClassificationWithTeacher, SITE/models/deit/modeling_deit.py: logits = (cls_classifier(x[:, 0]) +
     // distillation_classifier(x[:, 1])) / 2): rows 0 and 1 of every image are normalised side by side into one 2D-wide row, and
     // ONE classifier GEMM with K = 2D over [W_cls | W_dist] / 2 produces the averaged logits.

@@ -51,9 +51,17 @@ int attention_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const
 int attention_any_length_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, int B, int S, int Sq,
                                 int heads, float scale, cudaStream_t stream);
 
+// BEiT relative position bias (attention.cu): attention_launch with table[h][rel(q, k)] added to the scaled scores; table f32
+// [heads, (2 grid - 1)^2 + 3] times log2(e), S = grid^2 + 1, head size 64, bf16 (evt_attention_rel_bias_fwd in include/evt.h)
+int attention_rel_bias_launch(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, const float* table, int grid,
+                              int B, int S, int Sq, int heads, int head_size, float scale, cudaStream_t stream);
+
 int attention_tf32_launch(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask, int B, int S,
                           int heads, int head_size, float scale, cudaStream_t stream);
 
+// BEiT mean-pooled head: y bf16 [images, D] = LayerNorm(mean of rows 1..T-1 of x f32 [images * T, D]) (evt_layernorm_patch_mean)
+int layernorm_patch_mean_launch(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D, float eps,
+                                cudaStream_t st);
 int layernorm_launch(const float* x, int64_t x_stride, const float* gamma, const float* beta, void* y, int y_dtype,
                      int64_t y_stride, float* y_copy, int64_t rows, int D, float eps, cudaStream_t st);
 

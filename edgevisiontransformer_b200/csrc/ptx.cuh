@@ -115,6 +115,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 // overlaps the predecessor's tail; NO global memory may be touched before it.  Both are no-ops for a plain launch.
 __device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+// Barrier `id` (1..15; 0 is __syncthreads) over `count` threads (a multiple of 32), whole warps arriving.
+__device__ __forceinline__ void named_bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 // ---------------------------------------------------------------- TMA
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* m) {

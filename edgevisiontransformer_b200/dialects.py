@@ -165,15 +165,22 @@ def _timm_blocks_to_canonical(sd: Dict[str, torch.Tensor], out: Dict[str, torch.
             raise ValueError(f"block {l} has LayerScale on one residual branch only")
         for g, dst in ((g1, "attention.output.dense"), (g2, "output.dense")):
             if g is not None:
-                w, b = out[q + dst + ".weight"], out[q + dst + ".bias"]
-                dt = torch.promote_types(w.dtype, torch.float32)        # f32 at least (f64 weights stay f64)
-                g = g.to(dt).reshape(-1)
-                if g.numel() != D:
-                    raise ValueError(f"block {l}: LayerScale has {g.numel()} entries, expected {D}")
-                out[q + dst + ".weight"] = w.to(dt) * g[:, None]
-                out[q + dst + ".bias"] = b.to(dt) * g
+                fold_layerscale(out, q + dst, g, D, f"block {l}")
         l += 1
     return l
+
+
+def fold_layerscale(sd: Dict[str, torch.Tensor], linear: str, gamma: torch.Tensor, D: int, where: str) -> None:
+    """In place: LayerScale ``gamma * linear(x)`` folded into the Linear ``linear`` of ``sd`` (``.weight`` [D, in], ``.bias`` [D]):
+    ``W' = diag(gamma) W``, ``b' = gamma * b``, computed in f32 at least (f64 weights stay f64).  ``where`` names the block in
+    the error for a gamma of the wrong length."""
+    w, b = sd[linear + ".weight"], sd[linear + ".bias"]
+    dt = torch.promote_types(w.dtype, torch.float32)
+    g = gamma.to(dt).reshape(-1)
+    if g.numel() != D:
+        raise ValueError(f"{where}: LayerScale has {g.numel()} entries, expected {D}")
+    sd[linear + ".weight"] = w.to(dt) * g[:, None]
+    sd[linear + ".bias"] = b.to(dt) * g
 
 
 def unwrap_checkpoint(ck: dict, use_ema: bool = True) -> Dict[str, torch.Tensor]:

@@ -224,6 +224,60 @@ def attention(qkv: torch.Tensor, B: int, S: int, heads: int, head_size: int = 64
     return ctx
 
 
+LOG2E = 1.4426950408889634
+
+
+def _beit_table(table: torch.Tensor, grid: int) -> torch.Tensor:
+    """HF relative_position_bias_table [(2 grid - 1)^2 + 3, heads] -> the library's [heads, n] f32 in log2 units."""
+    n = (2 * grid - 1) ** 2 + 3
+    if table.dim() != 2 or table.shape[0] != n:
+        raise ValueError(f"relative_position_bias_table must be [{n}, heads] for grid {grid}")
+    return (table.detach().double().t() * LOG2E).float().contiguous()
+
+
+def attention_rel_bias(qkv: torch.Tensor, table: torch.Tensor, grid: int, B: int, heads: int, scale: Optional[float] = None,
+                       head_mask: Optional[torch.Tensor] = None, q_rows: Optional[int] = None) -> torch.Tensor:
+    """BEiT attention (include/evt.h evt_attention_rel_bias_fwd): softmax(q k^T * scale + table[rel(q, k), h]) v for images of
+    grid x grid patches behind a cls token (S = grid^2 + 1), head size 64.  qkv bf16 [B*S, 3*heads*64]; table: the HF
+    relative_position_bias_table [(2 grid - 1)^2 + 3, heads] (natural-log units; repacked here); q_rows: just the first q_rows
+    queries of every image -> ctx bf16 [B*q_rows, heads*64]."""
+    _need_cuda(qkv, head_mask)
+    S = grid * grid + 1
+    if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.stride(1) != 1 or qkv.shape[0] != B * S or qkv.shape[1] < 3 * heads * 64:
+        raise ValueError("attention_rel_bias wants a bf16 [B*(grid^2+1), >= 3*heads*64] qkv matrix")
+    tab = _beit_table(table, grid).to(qkv.device)
+    Sq = S if q_rows is None else int(q_rows)
+    ctx = torch.empty((B * Sq, heads * 64), dtype=torch.bfloat16, device=qkv.device)
+    scale = float(64 ** -0.5 if scale is None else scale)
+    _lib.check(_lib.load().evt_attention_rel_bias_fwd(qkv.data_ptr(), qkv.stride(0), ctx.data_ptr(), ctx.stride(0), _ptr(head_mask),
+                                                      tab.data_ptr(), grid, B, S, Sq, heads, 64, scale, _stream()), "attention_rel_bias")
+    return ctx
+
+
+def beit_score_bias(table: torch.Tensor, grid: int) -> torch.Tensor:
+    """Dense [heads, S, S] form (S = grid^2 + 1) of what evt_attention_rel_bias_fwd adds to the scores, in natural-log units,
+    from the kernels' index arithmetic (evt_beit_score_bias).  table: HF layout [(2 grid - 1)^2 + 3, heads].  No GPU."""
+    n = (2 * grid - 1) ** 2 + 3
+    if table.dim() != 2 or table.shape[0] != n:
+        raise ValueError(f"beit_score_bias: table must be [{n}, heads]")
+    t = table.detach().float().cpu().t().contiguous()
+    S = grid * grid + 1
+    out = torch.empty((t.shape[0], S, S), dtype=torch.float32)
+    _lib.check(_lib.load().evt_beit_score_bias(t.data_ptr(), t.shape[0], grid, out.data_ptr()), "beit_score_bias")
+    return out
+
+
+def layernorm_patch_mean(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, images: int, T: int) -> torch.Tensor:
+    """BEiT's mean-pooled head input: LayerNorm of the mean of rows 1..T-1 of each image, x f32 [images*T, D] -> bf16 [images, D]."""
+    _need_cuda(x, gamma, beta)
+    if x.dtype != torch.float32 or x.dim() != 2 or not x.is_contiguous() or x.shape[0] != images * T:
+        raise ValueError("layernorm_patch_mean wants a contiguous f32 [images*T, D] matrix")
+    y = torch.empty((images, x.shape[1]), dtype=torch.bfloat16, device=x.device)
+    _lib.check(_lib.load().evt_layernorm_patch_mean(x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), images, T, x.shape[1],
+                                                    float(eps), _stream()), "layernorm_patch_mean")
+    return y
+
+
 def gather_layernorm(x: torch.Tensor, idx: torch.Tensor, gamma: Optional[torch.Tensor], beta: Optional[torch.Tensor], eps: float,
                      images: int, T_in: int, T_out: int, G: int = 1, out_dtype: Optional[torch.dtype] = torch.bfloat16,
                      copy: bool = False):

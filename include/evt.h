@@ -177,6 +177,20 @@ int evt_attention_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, cons
 int evt_attention_query_rows_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask,
                                  int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream);
 
+/* evt_attention_query_rows_fwd with BEiT's relative position bias (BeitRelativePositionBias,
+ * SITE/models/beit/modeling_beit.py:511-591) added to the scaled scores:
+ *   ctx = softmax(q k^T * scale + bias_h[rel(q, k)]) v   for an image of grid x grid patches behind one cls token
+ *   table : DEVICE f32 [heads, (2 grid - 1)^2 + 3], 16-byte aligned: head h's column of the checkpoint's
+ *           relative_position_bias_table times log2(e); rel is generate_relative_position_index (patch pairs: the Swin relative
+ *           index over the grid; cls query row: n - 3; cls key column: n - 2; cls with cls: n - 1, n = the table length)
+ * bf16, head size 64, S = grid^2 + 1 <= EVT_ATTN_MAX_TOKENS (anything else is EVT_ERR_UNSUPPORTED), Sq as in
+ * evt_attention_query_rows_fwd (rows bit-identical to the same rows of an Sq = S call). */
+int evt_attention_rel_bias_fwd(const void* qkv, int64_t ldq, void* ctx, int64_t ldc, const float* head_mask, const float* table,
+                               int grid, int B, int S, int Sq, int heads, int head_size, float scale, evt_stream stream);
+/* HOST only: out [heads, S, S] (S = grid^2 + 1) = table[h][rel(q, k)], the dense form of the bias evt_attention_rel_bias_fwd
+ * adds, from the same index arithmetic; table HOST f32 [heads, (2 grid - 1)^2 + 3]; grid 1..64. */
+int evt_beit_score_bias(const float* table, int heads, int grid, float* out);
+
 /* tf32 flavour of evt_attention_fwd: qkv and ctx are f32 (leading dims multiples of 4); S <= 256 only. */
 int evt_attention_fwd_tf32(const float* qkv, int64_t ldq, float* ctx, int64_t ldc, const float* head_mask,
                            int B, int S, int heads, int head_size, float scale, evt_stream stream);
@@ -307,6 +321,11 @@ int evt_layernorm_mean_tokens(const float* x, const float* gamma, const float* b
 /* The same with y_dtype EVT_BF16 or EVT_TF32 (f32 rounded to nearest tf32). */
 int evt_layernorm_mean_tokens_ex(const float* x, const float* gamma, const float* beta, void* y, int y_dtype, int64_t images, int T,
                                  int D, float eps, evt_stream stream);
+/* y[image, :] (bf16) = LayerNorm(mean over tokens 1..T-1 of x[image, t, :]) -- BeitPooler with use_mean_pooling
+ * (SITE/models/beit/modeling_beit.py:767-783): the mean of the patch rows first, then the norm.  x f32 [images, T, D],
+ * 16-byte aligned; T >= 2; D a multiple of 4 up to 1024. */
+int evt_layernorm_patch_mean(const float* x, const float* gamma, const float* beta, void* y, int64_t images, int T, int D,
+                             float eps, evt_stream stream);
 
 /* ---- Swin V2 block (SITE/models/swinv2/modeling_swinv2.py, microsoft/Swin-Transformer swin_transformer_v2.py).  Same window
  * order of the token rows as the V1 ops above. */
@@ -378,7 +397,9 @@ typedef struct evt_model_spec {
   float eps;                   /* LayerNorm epsilon */
   int heads[EVT_MAX_LAYERS];   /* surviving heads per layer (HF prune_heads semantics)       */
   int inter[EVT_MAX_LAYERS];   /* FFN width per layer (optimize_model semantics), any int>0  */
-  int final_ln;                /* 1: LayerNorm before the head (HF, T2T); 0: TF-dialect DeiT */
+  int final_ln;                /* 1: LayerNorm before the head (HF, T2T); 0: TF-dialect DeiT; 2: LayerNorm of the mean of
+                                  the patch rows 1..tokens-1 ("vit.layernorm.*" = BEiT's pooler.layernorm; BEiT /
+                                  data2vec-vision with use_mean_pooling); needs tokens = patches + 1 and the bf16 mode */
   int head_hidden;             /* 0: single Linear head; >0: Dense(head_hidden, gelu)->Dense */
   int t2t;                     /* T2T front-end instead of the patch embed: 1 NHWC f32 pixels (TF T2T); 2 NCHW
                                   f32 / bf16 / u8 pixels, the PyTorch T2T (stage-1 columns in (kh, kw, c) order); 3 as 2
@@ -403,7 +424,11 @@ typedef struct evt_tensor_view {
 /* Validate the spec and allocate an empty model on the current device (allocates; not async). */
 int evt_model_create(const evt_model_spec* spec, evt_model** out);
 /* Repack weights into the library's own padded bf16 / f32 buffers (allocates; synchronises `stream`).
- * The caller keeps ownership of the views.  Missing or mis-shaped tensors -> EVT_ERR_INVALID. */
+ * The caller keeps ownership of the views.  Missing or mis-shaped tensors -> EVT_ERR_INVALID.
+ * BEiT relative position bias: tensors "vit.encoder.layer.{l}.attention.attention.relative_position_bias.relative_position_bias_table"
+ * ([(2 W - 1)^2 + 3, heads[l]], W = image / patch, the HF layout), for every layer or for none, add table[rel(q, k), h] to the
+ * scaled scores of head h (evt_attention_rel_bias_fwd).  They need tokens = W^2 + 1, head size 64 and the bf16 mode
+ * (EVT_ERR_UNSUPPORTED otherwise). */
 int evt_model_load_weights(evt_model* m, const evt_tensor_view* tensors, int n, evt_stream stream);
 /* Bytes of caller-provided scratch needed for a forward at `batch`. */
 int evt_model_workspace_bytes(const evt_model* m, int batch, size_t* out);
